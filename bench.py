@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path, BASELINE configs[2] (x N = configs[3] weak)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path on the host cores
     python bench.py --config single|512|1080p|2160p|mixed    # the other BASELINE configs (see DESIGN.md section 7)
+    python bench.py --steps K --dump-outputs DIR             # also write what the last timed step computed (OutputDump)
 
 Default workload (BASELINE.json configs[2] per GPU): 64 independent synthetic 1280x720 road videos per GPU, one frame per
 stream per batch, full process() semantics (sliding-window search on the first frame, band-search tracking afterwards,
@@ -39,6 +40,7 @@ PLANE_PIXELS = 1080 * 1100
 MORPH_ALGO_BYTES_PER_FRAME = 4 * PLANE_PIXELS         # per morphology stage: two u8 planes (R, Lab-b) read + two written
 PARITY_FRAMES = 6                    # frames per stream compared with the oracle by the in-bench parity check
 PARITY_RTOL = 1e-6                   # polynomial coefficients vs np.polyfit (BASELINE.json north_star)
+DUMP_FRAME_SAMPLES = 12288           # --dump-outputs: bytes of each annotated frame kept (16 x 64 x 12288 float32 = 50 MB)
 
 
 def measured_peak_hbm():
@@ -337,6 +339,50 @@ def parity_check(ctx, trk, pool_dev, want, S):
             "morph_bands": list(trk.morph_bands())}
 
 
+class OutputDump:
+    """--dump-outputs: what a DevicePipeline caller receives from the last timed step, kept for comparing two builds.
+    Each batch of that step writes its annotated frames to a buffer of its own, and its lt_result records are copied
+    out on a side stream; before the pipeline reuses a results buffer (two batches later) the launch stream waits for
+    that copy.  The inputs depend only on the arguments (seeded synthetic streams), so runs are comparable file by file."""
+
+    def __init__(self, torch, like, batches):
+        from lane_tracker_b200.tracker import RESULT_DTYPE
+        self.torch, self.dtype = torch, RESULT_DTYPE
+        self.frames = [torch.empty_like(like) for _ in range(batches)]
+        self.results = torch.empty((batches, like.shape[0] * RESULT_DTYPE.itemsize), dtype=torch.uint8, device=like.device)
+        self.copied = [None] * batches
+        self.stream = torch.cuda.Stream(like.device)
+
+    def submit(self, pipe, frames, j):
+        """Batch j of the last step through `pipe`."""
+        torch = self.torch
+        if j >= 2:
+            torch.cuda.current_stream(frames.device).wait_event(self.copied[j - 2])
+        done = pipe.submit(frames, self.frames[j])
+        self.stream.wait_event(done)
+        with torch.cuda.stream(self.stream):
+            self.results[j].copy_(pipe.last_results_dev()[:self.results.shape[1]])
+            self.copied[j] = torch.cuda.Event()
+            self.copied[j].record(self.stream)
+
+    def write(self, path):
+        """DIR/frames_sample.npy: float32 [batch, stream, DUMP_FRAME_SAMPLES], the annotated frames' bytes at fixed
+        positions (ascending, drawn with numpy.random.default_rng(0)); DIR/result_<field>.npy: float64 [batch, stream
+        (, 3)], every lt_result field."""
+        torch = self.torch
+        self.stream.synchronize()
+        os.makedirs(path, exist_ok=True)
+        S, n = self.frames[0].shape[0], self.frames[0][0].numel()
+        pos = np.sort(np.random.default_rng(0).choice(n, DUMP_FRAME_SAMPLES, replace=False))
+        pos = torch.from_numpy(pos).to(self.results.device)
+        sample = torch.stack([f.view(S, -1)[:, pos] for f in self.frames]).cpu().numpy()
+        np.save(os.path.join(path, "frames_sample.npy"), sample.astype(np.float32))
+        res = self.results.cpu().numpy().view(self.dtype)
+        for name in self.dtype.names:
+            if not name.startswith("reserved"):
+                np.save(os.path.join(path, "result_%s.npy" % name), res[name].astype(np.float64))
+
+
 def render_pool(ctx, S, P, first_seed, scale=1.0, photos=None):
     """[P, S, H, W, 3] device pool and its pinned host twin; `photos`: frames that replace the LAST len(photos) streams."""
     torch = ctx.torch
@@ -422,19 +468,25 @@ def run_default(args, photos_in_batch=False):
     if rank == 0:
         sampler.start()
     nb = args.steps * B
+    dump = OutputDump(torch, pool_dev[0], B) if args.dump_outputs and rank == 0 else None
     trk.profile_select(["warp", "erode55", "tophat55"])
     trk.profile_begin(min(nb, 400))                            # the first 400 batches of the region
     launches0 = lib.lt_launch_count()
 
     def region():
         nonlocal k
-        for _ in range(nb):
+        for _ in range(nb - (B if dump else 0)):
             dpipe.submit(pool_dev[k % P], out_ring[k & 1]); k += 1
+        for j in range(B if dump else 0):                      # the last step, kept for --dump-outputs
+            dump.submit(dpipe, pool_dev[k % P], j); k += 1
         dpipe.join()                                            # the launch stream waits for the last back half
     ms = timed(ctx, stream, region)
     launches = lib.lt_launch_count() - launches0
     morph_ms, morph_calls = trk.profile_read()
     res = dpipe.fetch_results(S)
+    if dump:
+        dump.write(args.dump_outputs)
+        dump = None
     tracking = {"valid_fraction_last_batch": float(res["valid_lane_lines"].mean()),
                 "band_search_fraction_last_batch": float((res["search_mode"] == 1).mean()),
                 "two_attempt_fraction_last_batch": float((res["attempts"] == 2).mean())}
@@ -872,7 +924,14 @@ def main():
     ap.add_argument("--check-frames", type=int, default=64, help="--config single: frames compared free-running with the oracle")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-budget", type=float, default=20.0)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="--config 64|mixed: write the annotated frames (a fixed sample) and the result records of every "
+                         "batch of the last timed step of rank 0 to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config not in ("64", "mixed")):
+        ap.error("--dump-outputs applies to --impl ours with --config 64 or mixed")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
     if args.impl == "reference":
         return run_reference_arm(args)

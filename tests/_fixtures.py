@@ -9,8 +9,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 GOLDEN_DIR = os.path.join(HERE, "golden")
 
 
-def golden():
-    with open(os.path.join(GOLDEN_DIR, "golden.json")) as f:
+def golden(name="golden.json"):
+    with open(os.path.join(GOLDEN_DIR, name)) as f:
         return json.load(f)
 
 

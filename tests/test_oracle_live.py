@@ -1,54 +1,35 @@
-"""Oracle vs the LIVE reference (only in the build container, where /root/reference exists)."""
+"""Oracle vs the original project's outputs, recorded in tests/golden/live_reference.json by
+tests/golden/make_live_golden.py (the records compared are defined in tests/_live_records.py)."""
 import warnings
 
-import numpy as np
 import pytest
 
 import _fixtures as fx
-import _liveref
+import _live_records as records
 from lane_tracker_b200 import synth
 from oracle.tracker import OracleLaneTracker
 
-pytestmark = pytest.mark.skipif(not _liveref.available(), reason="/root/reference not present")
+LIVE = fx.golden("live_reference.json")
+CAL = synth.shipped_calibration()
+
+
+def _same_records(got, want):
+    assert len(got) == len(want)
+    for i, (g, w) in enumerate(zip(got, want)):
+        assert g == w, i
 
 
 def test_process_matches_live_reference_on_a_sequence():
     warnings.simplefilter("ignore")
-    vid = synth.RoadVideo(3)
-    ref = _liveref.make_tracker()
-    orc = OracleLaneTracker(**synth.shipped_calibration(), backend="cv2")
-    frames = [vid.frame(t) for t in range(4)] + [fx.load_frame("test4.jpg")] * 2 + [vid.frame(6)]
-    for f in frames:
-        a = _liveref.quiet(ref.process, f.copy())
-        b = orc.process(f.copy())
-        assert fx.out_digest(a) == fx.out_digest(b)
-        assert ref.last_detection == orc.last_detection and ref.valid_lane_lines == orc.valid_lane_lines
-        for nm in ("left_x", "left_y", "right_x", "right_y", "left_avg_x", "right_avg_x"):
-            assert np.array_equal(getattr(ref, nm), getattr(orc, nm)), nm
-        assert ref.average_curve_radius == orc.average_curve_radius
-        assert ref.eccentricity == orc.eccentricity
+    _same_records(records.sequence(OracleLaneTracker(**CAL, backend="cv2")), LIVE["sequence"])
 
 
 def test_sliding_window_restatement_on_adversarial_masks():
-    """The integer restatement of sliding_window_search equals the reference on masks built to hit the quirks:
+    """The integer restatement of sliding_window_search equals the original on masks built to hit the quirks:
     windows leaving the frame (NumPy slice wrap-around), one-sided masks, coupling fallback, limits 8 and 50."""
-    import _masks
-    ref = _liveref.make_tracker()
-    orc = OracleLaneTracker(**synth.shipped_calibration())
-    n_detected = 0
-    for i, m in enumerate(_masks.random_masks(36, seed=5)):
-        for nsl, partial, mu in ((8, 1.0, 0.1), (50, 1.0, 0.1), (8, 0.5, 0.35)):
-            ref.detected_pixels = orc.detected_pixels = False
-            _liveref.quiet(ref.sliding_window_search, m, 30, 40, 20, mu, nsl, 0.25, 360, 30, partial)
-            orc.sliding_window_search(m, 30, 40, 20, mu, nsl, 0.25, 360, 30, partial)
-            assert ref.detected_pixels == orc.detected_pixels, (i, nsl)
-            if ref.detected_pixels:
-                n_detected += 1
-                for nm in ("left_x", "left_y", "right_x", "right_y"):
-                    assert np.array_equal(getattr(ref, nm), getattr(orc, nm)), (i, nsl, nm)
-                assert list(ref.left_window_centroids) == list(orc.left_window_centroids), (i, nsl)
-                assert list(ref.right_window_centroids) == list(orc.right_window_centroids), (i, nsl)
-    assert n_detected > 20
+    want = LIVE["sliding_window"]
+    assert sum(w["detected"] for w in want) > 20
+    _same_records(records.sliding_window(OracleLaneTracker(**CAL)), want)
 
 
 @pytest.mark.parametrize("backend", ["cv2", "numpy"])
@@ -56,17 +37,7 @@ def test_debug_views_match_live_reference(backend):
     """visualize_search / split_view (lane_tracker.py:689-793, 1130-1209, utils.py:57-103): sliding-window frame,
     band-search frames, a frame that fails both attempts (still pixels -> SWS view of attempt 2) and a recovery."""
     warnings.simplefilter("ignore")
-    vid = synth.RoadVideo(5)
-    frames = [vid.frame(t) for t in range(3)] + [fx.load_frame("test4.jpg")] + [vid.frame(4)]
-    for mode in ("visualize_search", "split_view"):
-        ref = _liveref.make_tracker()
-        orc = OracleLaneTracker(**synth.shipped_calibration(), backend=backend)
-        for i, f in enumerate(frames):
-            a = _liveref.quiet(ref.process, f.copy(), **{mode: True})
-            b = orc.process(f.copy(), **{mode: True})
-            if mode == "visualize_search":
-                assert np.array_equal(a[0], b[0]), i
-                assert a[1].shape == b[1].shape and np.array_equal(a[1], b[1]), i
-            else:
-                assert a.shape == b.shape == (720 + 652, 1280, 3)
-                assert np.array_equal(a, b), i
+    got = records.debug_views(lambda: OracleLaneTracker(**CAL, backend=backend))
+    assert all(w["shape"] == [720 + 652, 1280, 3] for w in LIVE["debug_views"]["split_view"])
+    for mode in records.DEBUG_VIEW_MODES:
+        _same_records(got[mode], LIVE["debug_views"][mode])
