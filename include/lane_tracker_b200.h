@@ -131,6 +131,13 @@ int64_t lt_launch_count(void);
 
 /* ---- the per-frame hot path ---------------------------------------------- */
 
+/* Frame buffers.  Every full-size frame buffer the caller passes -- d_frames and d_out of lt_process,
+ * lt_process_front, lt_process_back and lt_draw_lane, d_frames of lt_remap, lt_warp_frame and lt_draw_text -- must
+ * start at a 4-byte aligned address: the kernels read and write frames as 32-bit words.  A buffer that is not is
+ * refused with an error before anything is launched.  (Frames are contiguous [n][img_h][img_w][3] and img_w is a
+ * multiple of 4, so every row and every frame of an aligned buffer is aligned too.)  The bird's-eye images
+ * (d_bv_rgb), masks, debug views and resize buffers are accessed byte by byte and need no alignment. */
+
 /* LaneTracker.process (lane_tracker.py:876-1209) for streams 0..n_streams-1.
  *   d_frames : [n_streams][img_h][img_w][3]
  *   d_out    : same shape, NULL for fits-only mode (no overlay rendered), or == d_frames to annotate in place

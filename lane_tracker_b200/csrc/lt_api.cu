@@ -395,10 +395,22 @@ static int process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, i
     return 0;
 }
 
+// Full-size frame buffers (the caller's frames and annotated output) are read and written as 32-bit words: by the
+// undistort (three words per tap pair) and by the overlay (three words per four pixels, in place when out == frames).
+// A buffer that is not 4-byte aligned is refused here, before anything is launched.
+static int check_frame_buffer(const void* p, const char* what) {
+    if ((uintptr_t)p & 3) {
+        lt_set_error("%s must be 4-byte aligned (got address %p)", what, p);
+        return -1;
+    }
+    return 0;
+}
+
 static int process_args(lt_handle* h, const uint8_t* d_frames, int n, const lt_params* params, int set, LtAttemptParams* p1) {
     int rc;
     if ((rc = check_n(h, n))) return rc;
     if (!d_frames || !params) { lt_set_error("null argument"); return -1; }
+    if ((rc = check_frame_buffer(d_frames, "d_frames"))) return rc;
     if (set != 0 && set != 1) { lt_set_error("buffer set must be 0 or 1"); return -1; }
     *p1 = attempt_from(*params);
     if ((rc = check_params(h, *p1))) return rc;
@@ -418,6 +430,7 @@ extern "C" int lt_process(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out,
                           lt_result* d_results, void* stream) {
     int rc;
     LtAttemptParams p1;
+    if ((rc = check_frame_buffer(d_out, "d_out"))) return rc;
     if ((rc = process_args(h, d_frames, n, params, 0, &p1))) return rc;
     if (!d_results) { lt_set_error("null argument"); return -1; }
     if ((rc = process_front(h, d_frames, n, p1, (cudaStream_t)stream))) return rc;
@@ -436,6 +449,7 @@ extern "C" int lt_process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d
                                int32_t set, lt_result* d_results, void* stream) {
     int rc;
     LtAttemptParams p1;
+    if ((rc = check_frame_buffer(d_out, "d_out"))) return rc;
     if ((rc = process_args(h, d_frames, n, params, set, &p1))) return rc;
     if (!d_results) { lt_set_error("null argument"); return -1; }
     return process_back(h, d_frames, d_out, n, params, p1, d_results, (cudaStream_t)stream, true);
@@ -663,6 +677,7 @@ extern "C" int lt_remap(lt_handle* h, const uint8_t* d_frames, uint8_t* d_bv_rgb
     int rc;
     if ((rc = check_n(h, n))) return rc;
     if (!d_frames) { lt_set_error("null argument"); return -1; }
+    if ((rc = check_frame_buffer(d_frames, "d_frames"))) return rc;     // (the bird's-eye output is written byte by byte)
     cudaStream_t st = (cudaStream_t)stream;
     if (h->remap_mode == 1) return lt_launch_warp_fused(h, d_frames, d_bv_rgb, n, st);
     if ((rc = lt_launch_undistort(h, d_frames, n, st))) return rc;
@@ -789,6 +804,7 @@ extern "C" int lt_draw_lane(lt_handle* h, const uint8_t* d_frames, uint8_t* d_ou
     int rc;
     if ((rc = check_n(h, n))) return rc;
     if (!d_frames || !d_out || !d_x || !d_counts) { lt_set_error("null argument"); return -1; }
+    if ((rc = check_frame_buffer(d_frames, "d_frames")) || (rc = check_frame_buffer(d_out, "d_out"))) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     // own polygon rows and draw flags: the per-stream ones cache the last valid lane of process() (the polygon a
     // failing frame re-draws, lane_tracker.py:1160-1166) and must survive a stage call
@@ -888,6 +904,7 @@ extern "C" int lt_draw_text(lt_handle* h, uint8_t* d_frames, int32_t n, const in
     int rc;
     if ((rc = check_n(h, n))) return rc;
     if (!d_frames || !h_kind || !h_counter) { lt_set_error("null argument"); return -1; }
+    if ((rc = check_frame_buffer(d_frames, "d_frames"))) return rc;
     if (!h->txt_tables) { lt_set_error("no text sprites installed (lt_set_text_sprites)"); return -1; }
     LT_CUDA(cudaSetDevice(h->cfg.device));
     if (!h->txt_state) {
@@ -927,8 +944,9 @@ extern "C" int lt_draw_text(lt_handle* h, uint8_t* d_frames, int32_t n, const in
 
 extern "C" int lt_warp_frame(lt_handle* h, const uint8_t* d_frames, int32_t n, uint8_t* d_bv_rgb, void* stream) {
     if (!h || !d_frames || !d_bv_rgb) { lt_set_error("null argument"); return -1; }
-    LT_CUDA(cudaSetDevice(h->cfg.device));
     int rc;
+    if ((rc = check_frame_buffer(d_frames, "d_frames"))) return rc;
+    LT_CUDA(cudaSetDevice(h->cfg.device));
     if ((rc = check_any_n(h, n))) return rc;
     return lt_launch_warp_frame(h, d_frames, d_bv_rgb, n, (cudaStream_t)stream);
 }

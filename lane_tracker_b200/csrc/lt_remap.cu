@@ -201,7 +201,7 @@ static_assert(UND_SPC == 4 || UND_SPC == 8 || UND_SPC == 16, "streams per CTA");
 
 __global__ void __launch_bounds__(256, LT_UND_MINB)
 k_undistort_roi(const uint8_t* __restrict__ frames, uint32_t* __restrict__ und, const int2* __restrict__ desc, LtDims d, int n,
-                int aligned, size_t group_words) {
+                size_t group_words) {
     __shared__ uint4 tile[256 * UND_CH];               // [pixel][chunk of four streams], chunk slot rotated by the pixel
     const int p0 = blockIdx.x * blockDim.x, p = p0 + threadIdx.x;
     const int roi_px = (d.roi1 - d.roi0) * d.img_w;
@@ -212,7 +212,7 @@ k_undistort_roi(const uint8_t* __restrict__ frames, uint32_t* __restrict__ und, 
         uint32_t wA, wB;
         blend_weights(f, wA, wB);
         const uint32_t m = (f >> 10) & 15u;
-        const bool fast = aligned && (f >> 14);
+        const bool fast = f >> 14;          // word loads: the API refuses frames that are not 4-byte aligned
         const size_t frame_bytes = (size_t)d.img_w * d.img_h * 3;
         const int pitch = d.img_w * 3;
         const int wi = q.x >> 2, sh = (q.x & 3) * 8, wpitch = pitch >> 2;
@@ -292,8 +292,8 @@ int lt_launch_warp_frame(lt_handle* h, const uint8_t* d_frames, uint8_t* d_bv_rg
 int lt_launch_undistort(lt_handle* h, const uint8_t* d_frames, int n, cudaStream_t st) {
     const LtDims& d = h->d;
     dim3 g(lt_div_up((d.roi1 - d.roi0) * d.img_w, 256), lt_div_up(n, UND_SPC));
-    const int aligned = ((uintptr_t)d_frames & 3) == 0 && ((d.img_w * 3) & 3) == 0;     // word loads need 4-byte aligned rows
-    k_undistort_roi<<<g, 256, 0, st>>>(d_frames, h->und_roi, h->und_desc, d, n, aligned, lt_und_group_words(d));
+    // the word loads of the fast path need 4-byte aligned rows: the frames are (lt_api.cu) and img_w % 4 == 0 (lt_create)
+    k_undistort_roi<<<g, 256, 0, st>>>(d_frames, h->und_roi, h->und_desc, d, n, lt_und_group_words(d));
     LT_LAUNCH_CHECK();
     return 0;
 }

@@ -249,9 +249,20 @@ class BatchedLaneTracker:
         if not (isinstance(frames, torch.Tensor) and frames.is_cuda and frames.dtype == torch.uint8 and
                 frames.is_contiguous() and frames.dim() == 4 and tuple(frames.shape[1:]) == (h, w, 3)):
             raise ValueError("frames must be a contiguous CUDA uint8 tensor [n, %d, %d, 3]" % (h, w))
+        if frames.data_ptr() % 4:
+            raise ValueError("frames must start at a 4-byte aligned address (the kernels access frames as 32-bit words)")
         if frames.shape[0] < 1 or frames.shape[0] > self.n_streams:
             raise ValueError("got %d frames for %d streams" % (frames.shape[0], self.n_streams))
         return int(frames.shape[0])
+
+    @staticmethod
+    def _check_out(out, frames):
+        if out is None:
+            return
+        if out.shape != frames.shape or out.dtype != torch.uint8 or not out.is_cuda or not out.is_contiguous():
+            raise ValueError("out must match frames")
+        if out.data_ptr() % 4:
+            raise ValueError("out must start at a 4-byte aligned address (the kernels access frames as 32-bit words)")
 
     def process_async(self, frames, out=None, params=None, results_dev=None, **kw):
         """Enqueue one frame per stream on the current CUDA stream; returns the number of streams.
@@ -259,9 +270,7 @@ class BatchedLaneTracker:
         frames: uint8 CUDA tensor [n, H, W, 3] (RGB).  out: same shape or None (fits-only mode).
         results_dev: optional uint8 CUDA buffer of n * RESULT_DTYPE.itemsize bytes (default: internal)."""
         n = self._check_frames(frames)
-        if out is not None and (out.shape != frames.shape or out.dtype != torch.uint8 or not out.is_cuda or
-                                not out.is_contiguous()):
-            raise ValueError("out must match frames")
+        self._check_out(out, frames)
         p = params if params is not None else make_params(**kw)
         res = self._results_dev if results_dev is None else results_dev
         if res.numel() < n * RESULT_DTYPE.itemsize or not res.is_cuda:
@@ -282,9 +291,7 @@ class BatchedLaneTracker:
         """Second half of ``process_async`` (searches, second attempt, state machine, overlay) from intermediate
         buffer set 0 or 1, on the current CUDA stream.  Advances the per-stream state."""
         n = self._check_frames(frames)
-        if out is not None and (out.shape != frames.shape or out.dtype != torch.uint8 or not out.is_cuda or
-                                not out.is_contiguous()):
-            raise ValueError("out must match frames")
+        self._check_out(out, frames)
         p = params if params is not None else make_params(**kw)
         res = self._results_dev if results_dev is None else results_dev
         if res.numel() < n * RESULT_DTYPE.itemsize or not res.is_cuda:

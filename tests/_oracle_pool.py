@@ -3,8 +3,12 @@ initialised, so it must not fork).  Test infrastructure only.
 
     python tests/_oracle_pool.py jobs.json out.json
 
-jobs.json: {"jobs": [{"kind": "synth", "seed": 3, "frames": 6} | {"kind": "image", "name": "test1.jpg", "frames": 6}, ...],
+jobs.json: {"jobs": [{"kind": "synth", "seed": 3, "frames": 6} | {"kind": "image", "name": "test1.jpg", "frames": 6}
+                     | {"kind": "plan", "plan": [<frame spec>, ...]}, ...],
             "params": {process() keyword overrides}}
+           A job may also carry "scale" (calibration and synthetic video scale, default 1.0).  A plan lists one
+           frame spec per frame (see frame_from_spec), so a stream can mix synthetic video, photographs, noise and
+           blank frames.
 out.json : per job, per frame: the fields a parity test compares (state, digests of the mask, the pixel sets and the
            output frame).
 """
@@ -18,6 +22,31 @@ ROOT = os.path.dirname(HERE)
 for p in (ROOT, HERE):
     if p not in sys.path:
         sys.path.insert(0, p)
+
+
+_VIDEOS = {}
+
+
+def frame_from_spec(spec, scale=1.0):
+    """One RGB frame from a plan entry: ["synth", seed, t] (synth.RoadVideo), ["image", name] (bundled photograph,
+    shipped scale only), ["noise", seed] (uniform random bytes), ["blank", value] (one grey level)."""
+    import numpy as np
+    import _fixtures as fx
+    from lane_tracker_b200 import synth
+    w, h = synth.shipped_calibration(scale)["img_size"]
+    kind = spec[0]
+    if kind == "synth":
+        key = (int(spec[1]), float(scale))
+        if key not in _VIDEOS:
+            _VIDEOS[key] = synth.RoadVideo(key[0], scale=scale)
+        return _VIDEOS[key].frame(int(spec[2]))
+    if kind == "image":
+        return fx.load_frame(spec[1])
+    if kind == "noise":
+        return np.random.default_rng(int(spec[1])).integers(0, 256, (h, w, 3), dtype=np.uint8)
+    if kind == "blank":
+        return np.full((h, w, 3), int(spec[1]), np.uint8)
+    raise ValueError("unknown frame spec %r" % (spec,))
 
 
 def _run(job):
@@ -36,16 +65,17 @@ def _run(job):
     except Exception:
         pass
     spec, params = job
-    trk = OracleLaneTracker(**synth.shipped_calibration(), backend=backend)
+    scale = float(spec.get("scale", 1.0))
+    trk = OracleLaneTracker(**synth.shipped_calibration(scale), backend=backend)
     if spec["kind"] == "synth":
-        vid = synth.RoadVideo(spec["seed"])
-        get = vid.frame
+        plan = [["synth", spec["seed"], t] for t in range(spec["frames"])]
+    elif spec["kind"] == "image":
+        plan = [["image", spec["name"]]] * spec["frames"]
     else:
-        img = fx.load_frame(spec["name"])
-        get = lambda t: img
+        plan = spec["plan"]
     out = []
-    for t in range(spec["frames"]):
-        frame = get(t).copy()
+    for item in plan:
+        frame = frame_from_spec(item, scale).copy()
         o = trk.process(frame, **params)
         att = trk.trace["attempts"]
         last = att[-1]
