@@ -145,7 +145,7 @@ int64_t lt_launch_count(void);
  *   params   : one lt_params for all streams (the reference's defaults-are-the-
  *              config convention, README.md:34)
  *   d_results: [n_streams] lt_result, device memory (copy back asynchronously)
- * Stream s uses and updates state slot s.  The putText overlays (lane_tracker.py:653-659, 668-672) are drawn
+ * Stream s uses and updates state slot s (lt_process_streams below serves any subset of streams).  The putText overlays (lane_tracker.py:653-659, 668-672) are drawn
  * when glyph sprites are installed (lt_set_text_sprites). */
 int lt_process(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int32_t n_streams,
                const lt_params* params, lt_result* d_results, void* stream);
@@ -163,6 +163,26 @@ int lt_process_front(lt_handle* h, const uint8_t* d_frames, int32_t n_streams, c
                      int32_t set, void* stream);
 int lt_process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int32_t n_streams,
                     const lt_params* params, int32_t set, lt_result* d_results, void* stream);
+
+/* lt_process for an arbitrary set of streams, in any order: frame i of d_frames (and d_out[i], d_results[i]) belongs
+ * to stream h_ids[i].
+ *   h_ids: HOST int32 [n], 1 <= n <= max_streams, every id in [0, max_streams), pairwise distinct (two frames of
+ *          one stream in one batch would race on its state).  The ids are copied when the call is enqueued: h_ids
+ *          may be reused as soon as the call returns.  Nothing synchronises; the call is capturable in a CUDA graph.
+ * Addressing rule: frames, out frames, result records, masks and the other intermediate buffers are indexed by batch
+ * position i; the tracking state, averaged polylines, cached lane polygon and captured pixel lists by stream id
+ * h_ids[i] (lt_get_state, lt_read_capture and lt_debug_read item 9 take a stream id; lt_debug_read items 3-8 a batch
+ * position).  Streams not listed keep their tracking state, cached lane polygon and captured pixel lists byte for
+ * byte.  With h_ids = {0, 1, ..., n-1} the results equal those of lt_process bit for bit.
+ * A null h_ids, n outside [1, max_streams], an id out of range or a repeated id is refused with an error that names
+ * the id, before anything is enqueued; every check of lt_process applies as well.
+ * lt_process_streams(...) == lt_process_front(..., 0, stream) followed by lt_process_back_streams(..., 0, ..., stream)
+ * (the front half is stateless and takes no ids).  lt_process_back_streams is ordered like lt_process_back: back(k)
+ * after front(k) and after back(k-1), front(k+2) after back(k). */
+int lt_process_streams(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids, int32_t n,
+                       const lt_params* params, lt_result* d_results, void* stream);
+int lt_process_back_streams(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids, int32_t n,
+                            const lt_params* params, int32_t set, lt_result* d_results, void* stream);
 
 /* Keep the ordered lane-pixel sets and window centroids of every lt_process call so that
  * lt_read_capture can return them (the reference exposes them as the attributes left_x/left_y/
@@ -333,8 +353,9 @@ int lt_get_state(lt_handle* h, int32_t stream_id, lt_state* h_state, int32_t* h_
 int lt_set_state(lt_handle* h, int32_t stream_id, const lt_state* h_state, const int32_t* h_left_avg_x,
                  const int32_t* h_right_avg_x);
 
-/* Debug/test access to internal buffers of the last lt_process / stage call.
- * what: 0 undistort map (int32 [img_h][img_w][2]), 1 bird's-eye map (int32 [bv_h][bv_w][2]),
+/* Debug/test access to internal buffers of the last lt_process / stage call.  stream_id is a batch position for
+ * items 3-8 (buffers of the last batch) and a stream id for item 9 (per-stream cache); the two coincide for lt_process.
+ * what:0 undistort map (int32 [img_h][img_w][2]), 1 bird's-eye map (int32 [bv_h][bv_w][2]),
  *       2 overlay map (int32 [img_h][img_w][2]), 3 R plane u8 [bv_h][bv_w], 4 LAB-b plane,
  *       5 R top-hat, 6 b top-hat, 7 mask u8 {0,255}, 8 merged (pre-open) mask,
  *       9 lane row spans int32 [bv_h][2], 10 geometry int32[9] = {undistorted ROI first,last+1, overlay rows

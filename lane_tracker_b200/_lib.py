@@ -89,6 +89,8 @@ SIGNATURES = {
     "lt_process": (C.c_int, [P, P, P, i32, C.POINTER(lt_params), P, P]),
     "lt_process_front": (C.c_int, [P, P, i32, C.POINTER(lt_params), i32, P]),
     "lt_process_back": (C.c_int, [P, P, P, i32, C.POINTER(lt_params), i32, P, P]),
+    "lt_process_streams": (C.c_int, [P, P, P, C.POINTER(i32), i32, C.POINTER(lt_params), P, P]),
+    "lt_process_back_streams": (C.c_int, [P, P, P, C.POINTER(i32), i32, C.POINTER(lt_params), i32, P, P]),
     "lt_set_capture": (C.c_int, [P, i32]),
     "lt_set_pixel_capacity": (C.c_int, [P, i32]),
     "lt_read_capture": (C.c_int, [P, i32, i32, i32, P, i32, C.POINTER(i32), P, C.POINTER(i32)]),

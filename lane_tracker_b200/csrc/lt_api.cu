@@ -139,7 +139,7 @@ extern "C" int lt_destroy(lt_handle* h) {
         for (void* p : fp) if (p) cudaFree(p);
     }
     void* ptrs[] = {h->und_map, h->bv_map, h->ov_map, h->bv_desc, h->und_desc, h->lab_yz, h->fused_desc, h->lab_gamma, h->lab_cbrt, h->pixels, h->pix_counts, h->lane_rows, h->lane_bbox, h->dl_bbox,
-                    h->avg_x, h->state, h->att, h->retry_list, h->retry_count, h->draw_flags, h->scratch_bv, h->vis_scratch,
+                    h->avg_x, h->state, h->att, h->retry_list, h->retry_count, h->draw_flags, h->stream_ids, h->scratch_bv, h->vis_scratch,
                     h->cap_pixels, h->cap_counts, h->cap_cents, h->cap_ncents, h->dl_rows, h->dl_flags, h->txt_state, h->txt_flags,
                     h->txt_tables, h->txt_char_start, h->txt_dy, h->txt_dx, h->txt_lut, h->txt_advance, h->txt_pair_overlap,
                     h->txt_bitmaps};
@@ -270,7 +270,7 @@ extern "C" int lt_create(const lt_config* cfg, lt_handle** out) {
     if (!rc) select_set(h, 0);
     A(pixels, S * 2 * (size_t)h->pix_cap); A(pix_counts, S * 2);
     A(lane_rows, S * (size_t)d.bv_h); A(lane_bbox, S); A(avg_x, S * 2 * (size_t)d.bv_h);
-    A(state, S); A(att, 2 * S); A(retry_list, S); A(retry_count, 1); A(draw_flags, 2 * S);
+    A(state, S); A(att, 2 * S); A(retry_list, S); A(retry_count, 1); A(draw_flags, 2 * S); A(stream_ids, S);
 #undef A
     if (rc) { lt_destroy(h); return rc; }
     if (cudaStreamCreateWithFlags(&h->side, cudaStreamNonBlocking) != cudaSuccess ||
@@ -340,16 +340,53 @@ static int process_front(lt_handle* h, const uint8_t* d_frames, int n, const LtA
     return lt_launch_filter(h, n, p1, nullptr, nullptr, st);
 }
 
-// searches, second attempt of the streams that failed, state machine, overlay: advances the per-stream state
+// The stream ids of a batch travel to the device as kernel arguments: a launch copies its arguments when it is
+// enqueued, so the caller's host array may be reused as soon as the call returns, nothing synchronises, and the call
+// stays capturable in a CUDA graph (a pageable cudaMemcpyAsync is neither).  One chunk holds LT_IDS_CHUNK ids (4 KB
+// of arguments); larger batches take several launches.
+#define LT_IDS_CHUNK 1000
+struct LtIdsChunk {
+    int offset, count;
+    int ids[LT_IDS_CHUNK];
+};
+
+__global__ void k_set_stream_ids(LtIdsChunk c, int* __restrict__ dst) {
+    for (int i = threadIdx.x; i < c.count; i += blockDim.x) dst[c.offset + i] = c.ids[i];
+}
+
+// Writes h_ids to the handle's one device id array on the stream of the back half that reads it.  One array per
+// handle is enough: every kernel that reads it is a back-half kernel enqueued on that same stream after this write,
+// and the back half of batch k must follow the back half of batch k-1 (lt_process_back), so a write for batch k
+// cannot overtake a read of batch k-1, and no later write can overtake a read of batch k.
+static int upload_stream_ids(lt_handle* h, const int32_t* h_ids, int n, cudaStream_t st) {
+    LtIdsChunk c;
+    for (int off = 0; off < n; off += LT_IDS_CHUNK) {
+        c.offset = off;
+        c.count = n - off < LT_IDS_CHUNK ? n - off : LT_IDS_CHUNK;
+        memcpy(c.ids, h_ids + off, (size_t)c.count * sizeof(int32_t));
+        k_set_stream_ids<<<1, 256, 0, st>>>(c, h->stream_ids);
+        LT_LAUNCH_CHECK();
+    }
+    return 0;
+}
+
+// searches, second attempt of the streams that failed, state machine, overlay: advances the per-stream state.
+// h_ids (host, validated by check_ids) maps batch position i to state slot h_ids[i]; NULL: the identity.
 static int process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, const lt_params* params,
-                        const LtAttemptParams& p1, lt_result* d_results, cudaStream_t st, bool own_begin) {
+                        const LtAttemptParams& p1, lt_result* d_results, cudaStream_t st, bool own_begin,
+                        const int32_t* h_ids = nullptr) {
     int rc;
     const LtAttemptParams p2 = second_attempt();
     const bool two = (params->n_tries >= 2) || (params->n_tries == -1);
     if (own_begin) lt_prof_mark(h, ST_BEGIN, st);       // stage times are differences of marks on ONE stream
+    const int* ids = nullptr;
+    if (h_ids) {
+        if ((rc = upload_stream_ids(h, h_ids, n, st))) return rc;
+        ids = h->stream_ids;
+    }
     LtSearchArgs sa;
     memset(&sa, 0, sizeof(sa));
-    sa.mask = h->mask; sa.mode = 0; sa.att = h->att; sa.do_fit = 1;
+    sa.mask = h->mask; sa.mode = 0; sa.att = h->att; sa.do_fit = 1; sa.ids = ids;
     const size_t S = h->S;
     if (h->capture) {
         sa.by_stream = 1; sa.pixels = h->cap_pixels; sa.pix_cap = h->pix_cap; sa.pix_counts = h->cap_counts;
@@ -371,7 +408,7 @@ static int process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, i
         if ((rc = lt_launch_search(h, n, p2, sa, h->retry_list, h->retry_count, st))) return rc;
         lt_prof_mark(h, ST_SEARCH, st);
     }
-    if ((rc = lt_launch_update_state(h, n, d_results, two ? 2 : 1, st))) return rc;
+    if ((rc = lt_launch_update_state(h, n, ids, d_results, two ? 2 : 1, st))) return rc;
     lt_prof_mark(h, ST_UPDATE, st);
     if (d_out) {
         // (copying the untouched rows on a side stream under the search kernels was measured: the copy saturates HBM
@@ -383,11 +420,11 @@ static int process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, i
         if (text_under_blend) {
             if (d_out != d_frames)
                 LT_CUDA(cudaMemcpyAsync(d_out, d_frames, (size_t)n * h->d.img_w * h->d.img_h * 3, cudaMemcpyDeviceToDevice, st));
-            if ((rc = lt_launch_text(h, d_out, n, st))) return rc;
-            if ((rc = lt_launch_overlay(h, d_out, d_out, n, h->draw_flags, st))) return rc;
+            if ((rc = lt_launch_text(h, d_out, n, ids, st))) return rc;
+            if ((rc = lt_launch_overlay(h, d_out, d_out, n, h->draw_flags, ids, st))) return rc;
         } else {
-            if ((rc = lt_launch_overlay(h, d_frames, d_out, n, h->draw_flags, st))) return rc;
-            if ((rc = lt_launch_text(h, d_out, n, st))) return rc;
+            if ((rc = lt_launch_overlay(h, d_frames, d_out, n, h->draw_flags, ids, st))) return rc;
+            if ((rc = lt_launch_text(h, d_out, n, ids, st))) return rc;
         }
         lt_prof_mark(h, ST_OVERLAY, st);
     }
@@ -453,6 +490,45 @@ extern "C" int lt_process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d
     if ((rc = process_args(h, d_frames, n, params, set, &p1))) return rc;
     if (!d_results) { lt_set_error("null argument"); return -1; }
     return process_back(h, d_frames, d_out, n, params, p1, d_results, (cudaStream_t)stream, true);
+}
+
+// Stream ids of lt_process_streams / lt_process_back_streams: 1 <= n <= S ids in [0, S), pairwise distinct (two
+// frames of one stream in a batch would race on its state).  Checked before anything is enqueued.
+static int check_ids(lt_handle* h, const int32_t* h_ids, int n) {
+    int rc;
+    if ((rc = check_n(h, n))) return rc;
+    if (!h_ids) { lt_set_error("null stream id list"); return -1; }
+    std::vector<unsigned char> seen(h->S, 0);
+    for (int i = 0; i < n; ++i) {
+        const int id = h_ids[i];
+        if (id < 0 || id >= h->S) { lt_set_error("stream id %d at batch position %d outside [0, %d)", id, i, h->S); return -1; }
+        if (seen[id]) { lt_set_error("stream id %d appears twice in the batch (position %d)", id, i); return -1; }
+        seen[id] = 1;
+    }
+    return 0;
+}
+
+extern "C" int lt_process_streams(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids, int32_t n,
+                                  const lt_params* params, lt_result* d_results, void* stream) {
+    int rc;
+    LtAttemptParams p1;
+    if ((rc = check_ids(h, h_ids, n))) return rc;
+    if ((rc = check_frame_buffer(d_out, "d_out"))) return rc;
+    if ((rc = process_args(h, d_frames, n, params, 0, &p1))) return rc;
+    if (!d_results) { lt_set_error("null argument"); return -1; }
+    if ((rc = process_front(h, d_frames, n, p1, (cudaStream_t)stream))) return rc;
+    return process_back(h, d_frames, d_out, n, params, p1, d_results, (cudaStream_t)stream, false, h_ids);
+}
+
+extern "C" int lt_process_back_streams(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids,
+                                       int32_t n, const lt_params* params, int32_t set, lt_result* d_results, void* stream) {
+    int rc;
+    LtAttemptParams p1;
+    if ((rc = check_ids(h, h_ids, n))) return rc;
+    if ((rc = check_frame_buffer(d_out, "d_out"))) return rc;
+    if ((rc = process_args(h, d_frames, n, params, set, &p1))) return rc;
+    if (!d_results) { lt_set_error("null argument"); return -1; }
+    return process_back(h, d_frames, d_out, n, params, p1, d_results, (cudaStream_t)stream, true, h_ids);
 }
 
 static const char* STAGE_NAMES[LT_NSTAGES] = {"begin", "undistort", "warp", "erode55", "erode29", "tophat55", "tophat29",
@@ -819,7 +895,7 @@ extern "C" int lt_draw_lane(lt_handle* h, const uint8_t* d_frames, uint8_t* d_ou
     view.lane_bbox = h->dl_bbox;
     view.draw_flags = h->dl_flags;
     if ((rc = lt_launch_lane_rows(&view, d_x, d_counts, n, st))) return rc;
-    return lt_launch_overlay(&view, d_frames, d_out, n, view.draw_flags, st);
+    return lt_launch_overlay(&view, d_frames, d_out, n, view.draw_flags, nullptr, st);
 }
 
 // get_curve_radius / get_eccentricity (lane_tracker.py:530-559) for caller-supplied fits and polylines.
@@ -931,7 +1007,7 @@ extern "C" int lt_draw_text(lt_handle* h, uint8_t* d_frames, int32_t n, const in
     lt_handle view = *h;
     view.state = h->txt_state;
     view.draw_flags = h->txt_flags;
-    return lt_launch_text(&view, d_frames, n, s);
+    return lt_launch_text(&view, d_frames, n, nullptr, s);
 }
 
 // ---------------------------------------------------------------------------

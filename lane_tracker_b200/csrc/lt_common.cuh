@@ -106,6 +106,7 @@ struct lt_handle {
     LtAttemptOut* att;           // [S]
     int* retry_list; int* retry_count;      // streams that need attempt 2
     int* draw_flags;             // [S]
+    int* stream_ids;             // [S] state slot of each batch position of the last call with stream ids (lt_process_streams)
     int capture;                 // lt_set_capture
     uint32_t* cap_pixels;        // [2 attempts][S][2][pix_cap]
     int* cap_counts;             // [2][S][2]
@@ -158,6 +159,9 @@ int lt_ensure_smem(const void* func, size_t bytes);
 // ---- stage launchers (defined in the .cu files) -----------------------------
 // `list`/`count` (device pointers, may be NULL) restrict a launch to the streams
 // list[0..*count): CTAs whose stream slot is >= *count exit immediately.
+// `ids` (device pointer, may be NULL = identity) maps a batch position to the state slot of its stream: frames,
+// masks, attempt outputs, draw flags and result records are indexed by batch position, the per-stream state
+// (tracking state, averaged polylines, cached lane polygon, captured pixel lists) by ids[position].
 
 int lt_launch_build_maps(lt_handle* h, cudaStream_t st);
 int lt_launch_build_desc(lt_handle* h, cudaStream_t st);
@@ -169,7 +173,7 @@ int lt_launch_undistort(lt_handle* h, const uint8_t* d_frames, int n, cudaStream
 int lt_launch_warp(lt_handle* h, uint8_t* d_bv_rgb, int n, cudaStream_t st);
 int lt_launch_planes_from_bv(lt_handle* h, const uint8_t* d_bv_rgb, int n, cudaStream_t st);
 int lt_launch_overlay(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, const int* d_draw,
-                      cudaStream_t st, bool rows_already_copied = false);
+                      const int* ids, cudaStream_t st, bool rows_already_copied = false);
 int lt_launch_nv12_to_rgb(const uint8_t* d_nv12, uint8_t* d_rgb, int n, int w, int h, cudaStream_t st);
 int lt_launch_copy_untouched_rows(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, cudaStream_t st);
 
@@ -189,18 +193,20 @@ struct LtSearchArgs {
     LtAttemptOut* att;           // [n] out
     int do_fit;                  // also fit + validity
     int by_stream;               // index pixel/centroid outputs by stream id instead of launch slot
+    const int* ids;              // [n] state slot per batch position (NULL: identity): state reads, by_stream outputs
 };
 int lt_launch_search(lt_handle* h, int n, const LtAttemptParams& p, const LtSearchArgs& a, const int* list,
                      const int* count, cudaStream_t st);
 int lt_launch_select_retry(lt_handle* h, int n, int n_tries, cudaStream_t st);
-int lt_launch_update_state(lt_handle* h, int n, lt_result* d_results, int attempts_allowed, cudaStream_t st);
+int lt_launch_update_state(lt_handle* h, int n, const int* ids, lt_result* d_results, int attempts_allowed,
+                           cudaStream_t st);
 int lt_launch_fit_pixels(lt_handle* h, const uint32_t* d_pixels, int cap, const int* d_counts, int n,
                          double* d_fits, cudaStream_t st);
 int lt_launch_validity(lt_handle* h, const double* d_fits, int n, int* d_valid, double* d_diffs, cudaStream_t st);
 int lt_launch_poly_points(lt_handle* h, const double* d_fits, int n, double partial, int* d_x, int* d_counts,
                           cudaStream_t st);
 int lt_launch_lane_rows(lt_handle* h, const int* d_x, const int* d_counts, int n, cudaStream_t st);
-int lt_launch_text(lt_handle* h, uint8_t* d_out, int n, cudaStream_t st);
+int lt_launch_text(lt_handle* h, uint8_t* d_out, int n, const int* ids, cudaStream_t st);
 // debug views (lt_vis.cu, and the two helpers that live next to the code they reuse)
 int lt_launch_warp_frame(lt_handle* h, const uint8_t* d_frames, uint8_t* d_bv_rgb, int n, cudaStream_t st);
 int lt_launch_band_rows(lt_handle* h, const int* d_x, const int* d_counts, int bandwidth, int2* rows_l, int2* rows_r,

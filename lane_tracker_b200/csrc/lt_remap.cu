@@ -673,7 +673,8 @@ __device__ __forceinline__ int lane_tap(const int2* __restrict__ rows, const LtD
 
 __global__ void __launch_bounds__(256)
 k_overlay(const uint8_t* frames, uint8_t* out, const int2* __restrict__ map,
-          const int2* __restrict__ lane_rows, const int4* __restrict__ lane_bbox, const int* __restrict__ draw, LtDims d, int row0) {
+          const int2* __restrict__ lane_rows, const int4* __restrict__ lane_bbox, const int* __restrict__ draw, LtDims d, int row0,
+          const int* __restrict__ ids) {
     // one thread = 4 pixels = 12 bytes (three aligned 32-bit words); img_w % 4 == 0 is checked at create.
     // `out` may alias `frames` (in-place annotation): every thread reads and writes only its own 12 bytes.
     int q = blockIdx.x * blockDim.x + threadIdx.x;
@@ -688,12 +689,13 @@ k_overlay(const uint8_t* frames, uint8_t* out, const int2* __restrict__ map,
         // bounding box (taps of a pixel: columns sx, sx + 1, rows sy, sy + 1) skips the span look-ups
         const int4* mp = reinterpret_cast<const int4*>(map + (size_t)y * d.img_w + q * 4);
         const int4 m01 = __ldg(mp), m23 = __ldg(mp + 1);
-        const int4 bb = __ldg(&lane_bbox[s]);
+        const int sid = ids ? __ldg(&ids[s]) : s;        // the cached polygon belongs to the stream, not the position
+        const int4 bb = __ldg(&lane_bbox[sid]);
         const int qx[4] = {m01.x, m01.z, m23.x, m23.z}, qy[4] = {m01.y, m01.w, m23.y, m23.w};
         const int sx_lo = min(min(qx[0], qx[1]), min(qx[2], qx[3])) >> 5, sx_hi = max(max(qx[0], qx[1]), max(qx[2], qx[3])) >> 5;
         const int sy_lo = min(min(qy[0], qy[1]), min(qy[2], qy[3])) >> 5, sy_hi = max(max(qy[0], qy[1]), max(qy[2], qy[3])) >> 5;
         if (sx_hi + 1 >= bb.x && sx_lo <= bb.y && sy_hi + 1 >= bb.z && sy_lo <= bb.w) {
-            const int2* rows = lane_rows + (size_t)s * d.bv_h;
+            const int2* rows = lane_rows + (size_t)sid * d.bv_h;
             uint32_t gch[4] = {(w0 >> 8) & 255, w1 & 255, (w1 >> 24) & 255, (w2 >> 16) & 255};
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
@@ -770,14 +772,14 @@ int lt_launch_copy_untouched_rows(lt_handle* h, const uint8_t* d_frames, uint8_t
 }
 
 int lt_launch_overlay(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, const int* d_draw,
-                      cudaStream_t st, bool rows_already_copied) {
+                      const int* ids, cudaStream_t st, bool rows_already_copied) {
     const LtDims& d = h->d;
     int r0, r1; bool vec_ok;
     overlay_rows(h, d_frames, d_out, r0, r1, vec_ok);
     if (!rows_already_copied) { int rc = lt_launch_copy_untouched_rows(h, d_frames, d_out, n, st); if (rc) return rc; }
     if (r1 > r0) {
         dim3 g(lt_div_up(d.img_w / 4, 256), r1 - r0, n);
-        k_overlay<<<g, 256, 0, st>>>(d_frames, d_out, h->ov_map, h->lane_rows, h->lane_bbox, d_draw, d, r0);
+        k_overlay<<<g, 256, 0, st>>>(d_frames, d_out, h->ov_map, h->lane_rows, h->lane_bbox, d_draw, d, r0, ids);
         LT_LAUNCH_CHECK();
     }
     return 0;

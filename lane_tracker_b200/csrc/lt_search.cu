@@ -299,10 +299,11 @@ k_search(LtDims d, LtAttemptParams p, LtSearchArgs a, const LtDevState* __restri
          size_t bits_stride, const int* __restrict__ list, const int* __restrict__ count, int lev_chunk) {
     int slot = blockIdx.x;
     if (count != nullptr && slot >= *count) return;
-    const int s = list ? list[slot] : slot;
+    const int s = list ? list[slot] : slot;              // batch position: mask, att, coeffs
+    const int sid = a.ids ? a.ids[s] : s;                // state slot of its stream: state, by_stream outputs
     const int W = d.bv_w, H = d.bv_h, tid = threadIdx.x;
     const uint32_t* mask = a.mask + (size_t)s * bits_stride;
-    const int oidx = a.by_stream ? s : slot;
+    const int oidx = a.by_stream ? sid : slot;
 
     extern __shared__ unsigned char smem_raw[];
     __shared__ SearchShared sh;
@@ -319,14 +320,14 @@ k_search(LtDims d, LtAttemptParams p, LtSearchArgs a, const LtDevState* __restri
     int* Sbuf = cnt + 2 * H;                            // [W + 64]
 
     int mode = a.mode;
-    if (mode == 0) mode = (state[s].s.last_detection > n_reset) ? 1 : 2;
+    if (mode == 0) mode = (state[sid].s.last_detection > n_reset) ? 1 : 2;
     if (tid == 0) {
         sh.nroi[0] = sh.nroi[1] = 0; sh.ncent[0] = sh.ncent[1] = 0; sh.nvisit[0] = sh.nvisit[1] = 0;
         if (mode == 2) {
             const double* cf = a.coeffs ? a.coeffs + (size_t)s * 6 : nullptr;
             for (int j = 0; j < 3; ++j) {
-                sh.coeffs[0][j] = cf ? cf[j] : state[s].s.last_left[j];
-                sh.coeffs[1][j] = cf ? cf[3 + j] : state[s].s.last_right[j];
+                sh.coeffs[0][j] = cf ? cf[j] : state[sid].s.last_left[j];
+                sh.coeffs[1][j] = cf ? cf[3 + j] : state[sid].s.last_right[j];
             }
         }
     }
@@ -728,20 +729,22 @@ __device__ void lane_rows_from_polylines(const int* xl, int nl, const int* xr, i
 __global__ void __launch_bounds__(SEARCH_THREADS)
 k_update_state(LtDims d, lt_config cfg, LtDevState* __restrict__ state, const LtAttemptOut* __restrict__ att1,
                const LtAttemptOut* __restrict__ att2, const int* __restrict__ retry, int* __restrict__ avg_x,
-               int2* __restrict__ lane_rows, int4* __restrict__ lane_bbox, int* __restrict__ draw, lt_result* __restrict__ results) {
-    const int s = blockIdx.x, tid = threadIdx.x, W = d.bv_w, H = d.bv_h;
+               int2* __restrict__ lane_rows, int4* __restrict__ lane_bbox, int* __restrict__ draw, lt_result* __restrict__ results,
+               const int* __restrict__ ids) {
+    // s: batch position (attempt outputs, retry and draw flags, result record); sid: state slot of its stream
+    const int s = blockIdx.x, sid = ids ? ids[s] : s, tid = threadIdx.x, W = d.bv_w, H = d.bv_h;
     extern __shared__ unsigned char smem_raw[];
     int* flags = reinterpret_cast<int*>(smem_raw);        // [H]
     int* stage = flags + H;                               // [2*H]
     __shared__ int scratch[SEARCH_THREADS + 1];
     __shared__ double avg[2][3];
     __shared__ int nkeep[2];
-    lt_state& st = state[s].s;
+    lt_state& st = state[sid].s;
     const bool second = retry && retry[s];
     const LtAttemptOut& a = second ? att2[s] : att1[s];
     const bool valid = a.detected && a.valid;
     const int nav = min(max(cfg.n_average, 1), LT_MAX_AVERAGE);
-    int* xl = avg_x + (size_t)s * 2 * H;
+    int* xl = avg_x + (size_t)sid * 2 * H;
     int* xr = xl + H;
 
     if (tid == 0) {
@@ -822,7 +825,7 @@ k_update_state(LtDims d, lt_config cfg, LtDevState* __restrict__ state, const Lt
             }
         }
         __syncthreads();
-        lane_rows_from_polylines(xl, st.n_left_avg, xr, st.n_right_avg, W, H, lane_rows + (size_t)s * H, lane_bbox + s);
+        lane_rows_from_polylines(xl, st.n_left_avg, xr, st.n_right_avg, W, H, lane_rows + (size_t)sid * H, lane_bbox + sid);
     }
     if (tid == 0) {
         int drew = valid ? 1 : ((st.has_avg && st.n_left_avg != 0 && st.last_detection <= cfg.n_fail) ? 1 : 0);
@@ -845,11 +848,12 @@ k_update_state(LtDims d, lt_config cfg, LtDevState* __restrict__ state, const Lt
     }
 }
 
-int lt_launch_update_state(lt_handle* h, int n, lt_result* d_results, int attempts_allowed, cudaStream_t st) {
+int lt_launch_update_state(lt_handle* h, int n, const int* ids, lt_result* d_results, int attempts_allowed,
+                           cudaStream_t st) {
     size_t smem = (size_t)3 * h->d.bv_h * sizeof(int);
     const int* retry = attempts_allowed >= 2 ? h->draw_flags + h->S : nullptr;
     k_update_state<<<n, SEARCH_THREADS, smem, st>>>(h->d, h->cfg, h->state, h->att, h->att + h->S, retry, h->avg_x,
-                                                    h->lane_rows, h->lane_bbox, h->draw_flags, d_results);
+                                                    h->lane_rows, h->lane_bbox, h->draw_flags, d_results, ids);
     LT_LAUNCH_CHECK();
     return 0;
 }
@@ -1044,7 +1048,7 @@ __global__ void __launch_bounds__(128)
 k_text_seq(uint8_t* out, LtDims d, const LtDevState* __restrict__ state, const int* __restrict__ draw, int print_frame_count,
            const uint8_t* __restrict__ tables, const int* __restrict__ char_start, const short* __restrict__ dy,
            const short* __restrict__ dx, const unsigned short* __restrict__ lut, const int* __restrict__ advance,
-           int nchars, int first_char);
+           int nchars, int first_char, const int* __restrict__ ids);
 
 __device__ int format_lines(TextLine* lines, const lt_state& st, int drew, int print_frame_count) {
     for (int i = 0; i < 3; ++i) { lines[i].len = 0; lines[i].x0 = 20; lines[i].y0 = 35 + 35 * i; }
@@ -1065,11 +1069,11 @@ __global__ void __launch_bounds__(128)
 k_text_seq(uint8_t* out, LtDims d, const LtDevState* __restrict__ state, const int* __restrict__ draw, int print_frame_count,
            const uint8_t* __restrict__ tables, const int* __restrict__ char_start, const short* __restrict__ dy,
            const short* __restrict__ dx, const unsigned short* __restrict__ lut, const int* __restrict__ advance,
-           int nchars, int first_char) {
-    const int s = blockIdx.x;
+           int nchars, int first_char, const int* __restrict__ ids) {
+    const int s = blockIdx.x;                       // batch position: frame, draw flag; the strings from the stream's state
     __shared__ TextLine lines[3];
     __shared__ int nlines;
-    if (threadIdx.x == 0) nlines = format_lines(lines, state[s].s, draw[s], print_frame_count);
+    if (threadIdx.x == 0) nlines = format_lines(lines, state[ids ? ids[s] : s].s, draw[s], print_frame_count);
     __syncthreads();
     uint8_t* img = out + (size_t)s * d.img_w * d.img_h * 3;
     for (int li = 0; li < nlines; ++li) {
@@ -1102,8 +1106,8 @@ k_text(uint8_t* out, LtDims d, const LtDevState* __restrict__ state, const int* 
        const uint8_t* __restrict__ tables, const int* __restrict__ char_start, const short* __restrict__ dy,
        const short* __restrict__ dx, const unsigned short* __restrict__ lut, const int* __restrict__ advance,
        const unsigned char* __restrict__ pair_overlap, const unsigned long long* __restrict__ bitmaps, int nchars,
-       int first_char) {
-    const int s = blockIdx.x, li = blockIdx.y;
+       int first_char, const int* __restrict__ ids) {
+    const int s = blockIdx.x, li = blockIdx.y;      // batch position: frame, draw flag; the strings from the stream's state
     __shared__ TextLine lines[3];
     __shared__ int nlines;
     __shared__ int cx[56], cc[56], cstart[57], cflag[56];
@@ -1111,7 +1115,7 @@ k_text(uint8_t* out, LtDims d, const LtDevState* __restrict__ state, const int* 
     const int ng = min(nchars, 128);                               // serial path of thread 0
     for (int i = threadIdx.x; i <= ng; i += blockDim.x) s_start[i] = char_start[i];
     for (int i = threadIdx.x; i < ng; i += blockDim.x) s_adv[i] = advance[i];
-    if (threadIdx.x == 0) nlines = format_lines(lines, state[s].s, draw[s], print_frame_count);
+    if (threadIdx.x == 0) nlines = format_lines(lines, state[ids ? ids[s] : s].s, draw[s], print_frame_count);
     __syncthreads();
     if (li >= nlines) return;
     if (threadIdx.x == 0) {
@@ -1153,16 +1157,16 @@ k_text(uint8_t* out, LtDims d, const LtDevState* __restrict__ state, const int* 
     }
 }
 
-int lt_launch_text(lt_handle* h, uint8_t* d_out, int n, cudaStream_t st) {
+int lt_launch_text(lt_handle* h, uint8_t* d_out, int n, const int* ids, cudaStream_t st) {
     if (!h->txt_tables || !d_out) return 0;
     if (h->txt_parallel_lines && h->txt_pair_overlap && h->txt_bitmaps)
         k_text<<<dim3(n, 3), 1024, 0, st>>>(d_out, h->d, h->state, h->draw_flags, h->cfg.print_frame_count, h->txt_tables,
                                            h->txt_char_start, h->txt_dy, h->txt_dx, h->txt_lut, h->txt_advance,
-                                           h->txt_pair_overlap, h->txt_bitmaps, h->txt_nchars, h->txt_first);
+                                           h->txt_pair_overlap, h->txt_bitmaps, h->txt_nchars, h->txt_first, ids);
     else
         k_text_seq<<<n, 128, 0, st>>>(d_out, h->d, h->state, h->draw_flags, h->cfg.print_frame_count, h->txt_tables,
                                       h->txt_char_start, h->txt_dy, h->txt_dx, h->txt_lut, h->txt_advance, h->txt_nchars,
-                                      h->txt_first);
+                                      h->txt_first, ids);
     LT_LAUNCH_CHECK();
     return 0;
 }

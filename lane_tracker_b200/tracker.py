@@ -255,6 +255,28 @@ class BatchedLaneTracker:
             raise ValueError("got %d frames for %d streams" % (frames.shape[0], self.n_streams))
         return int(frames.shape[0])
 
+    def _check_ids(self, ids, n):
+        """Stream ids of a batch of n frames -> ctypes int32 array (None: None).  Any int sequence, NumPy array or CPU
+        tensor of n distinct ids in [0, n_streams); frame i belongs to stream ids[i]."""
+        if ids is None:
+            return None
+        if isinstance(ids, torch.Tensor):
+            if ids.is_cuda:
+                raise ValueError("ids must be host data (a sequence, a NumPy array or a CPU tensor), not a CUDA tensor")
+            ids = ids.numpy()
+        a = np.asarray(ids)
+        if a.ndim != 1 or (a.size and a.dtype.kind not in "iu"):
+            raise ValueError("ids must be a 1-D sequence of integers")
+        if a.size != n:
+            raise ValueError("got %d stream ids for %d frames" % (a.size, n))
+        bad = a[(a < 0) | (a >= self.n_streams)]
+        if bad.size:
+            raise ValueError("stream id %d outside [0, %d)" % (int(bad[0]), self.n_streams))
+        u, counts = np.unique(a, return_counts=True)
+        if (counts > 1).any():
+            raise ValueError("stream id %d appears more than once in the batch" % int(u[counts > 1][0]))
+        return (C.c_int32 * n)(*[int(v) for v in a])
+
     @staticmethod
     def _check_out(out, frames):
         if out is None:
@@ -264,19 +286,27 @@ class BatchedLaneTracker:
         if out.data_ptr() % 4:
             raise ValueError("out must start at a 4-byte aligned address (the kernels access frames as 32-bit words)")
 
-    def process_async(self, frames, out=None, params=None, results_dev=None, **kw):
-        """Enqueue one frame per stream on the current CUDA stream; returns the number of streams.
+    def process_async(self, frames, out=None, params=None, results_dev=None, ids=None, **kw):
+        """Enqueue one frame per stream on the current CUDA stream; returns the number of frames.
 
         frames: uint8 CUDA tensor [n, H, W, 3] (RGB).  out: same shape or None (fits-only mode).
-        results_dev: optional uint8 CUDA buffer of n * RESULT_DTYPE.itemsize bytes (default: internal)."""
+        results_dev: optional uint8 CUDA buffer of n * RESULT_DTYPE.itemsize bytes (default: internal).
+        ids: None -- frame i belongs to stream i; else n distinct stream ids in [0, n_streams), any order (int
+        sequence, NumPy array or CPU tensor): frame i belongs to stream ids[i], and the streams not listed keep their
+        state.  out and the result records stay in batch order."""
         n = self._check_frames(frames)
         self._check_out(out, frames)
+        h_ids = self._check_ids(ids, n)
         p = params if params is not None else make_params(**kw)
         res = self._results_dev if results_dev is None else results_dev
         if res.numel() < n * RESULT_DTYPE.itemsize or not res.is_cuda:
             raise ValueError("results buffer too small")
-        check(self.lib.lt_process(self._h, _ptr(frames), _ptr(out), n, C.byref(p), _ptr(res),
-                                  _stream_ptr(self.device)))
+        if h_ids is None:
+            check(self.lib.lt_process(self._h, _ptr(frames), _ptr(out), n, C.byref(p), _ptr(res),
+                                      _stream_ptr(self.device)))
+        else:
+            check(self.lib.lt_process_streams(self._h, _ptr(frames), _ptr(out), h_ids, n, C.byref(p), _ptr(res),
+                                              _stream_ptr(self.device)))
         return n
 
     def process_front_async(self, frames, buffer_set, params=None, **kw):
@@ -287,17 +317,23 @@ class BatchedLaneTracker:
         check(self.lib.lt_process_front(self._h, _ptr(frames), n, C.byref(p), int(buffer_set), _stream_ptr(self.device)))
         return n
 
-    def process_back_async(self, frames, out, buffer_set, params=None, results_dev=None, **kw):
+    def process_back_async(self, frames, out, buffer_set, params=None, results_dev=None, ids=None, **kw):
         """Second half of ``process_async`` (searches, second attempt, state machine, overlay) from intermediate
-        buffer set 0 or 1, on the current CUDA stream.  Advances the per-stream state."""
+        buffer set 0 or 1, on the current CUDA stream.  Advances the per-stream state of the streams in ``ids``
+        (None: streams 0..n-1), as ``process_async``."""
         n = self._check_frames(frames)
         self._check_out(out, frames)
+        h_ids = self._check_ids(ids, n)
         p = params if params is not None else make_params(**kw)
         res = self._results_dev if results_dev is None else results_dev
         if res.numel() < n * RESULT_DTYPE.itemsize or not res.is_cuda:
             raise ValueError("results buffer too small")
-        check(self.lib.lt_process_back(self._h, _ptr(frames), _ptr(out), n, C.byref(p), int(buffer_set), _ptr(res),
-                                       _stream_ptr(self.device)))
+        if h_ids is None:
+            check(self.lib.lt_process_back(self._h, _ptr(frames), _ptr(out), n, C.byref(p), int(buffer_set),
+                                           _ptr(res), _stream_ptr(self.device)))
+        else:
+            check(self.lib.lt_process_back_streams(self._h, _ptr(frames), _ptr(out), h_ids, n, C.byref(p),
+                                                   int(buffer_set), _ptr(res), _stream_ptr(self.device)))
         return n
 
     def fetch_results(self, n=None):
@@ -308,8 +344,10 @@ class BatchedLaneTracker:
         torch.cuda.current_stream(self.device).synchronize()
         return self._results_host[:nbytes].numpy().view(RESULT_DTYPE).copy()
 
-    def process(self, frames, out=None, params=None, **kw):
-        n = self.process_async(frames, out, params, **kw)
+    def process(self, frames, out=None, params=None, ids=None, **kw):
+        """``process_async`` followed by ``fetch_results``: the n result records, in batch order.  With ``ids``, frame
+        i advances stream ids[i] and the other streams keep their state."""
+        n = self.process_async(frames, out, params, ids=ids, **kw)
         return self.fetch_results(n)
 
     # -- stage methods (device tensors) ---------------------------------------
@@ -625,6 +663,9 @@ class DevicePipeline:
         for frames, out in batches:            # CUDA tensors; produced on the current stream
             done = pipe.submit(frames, out)    # torch.cuda.Event: out / results of this batch are complete
         pipe.join()                            # the current stream waits for everything submitted
+
+    ``submit(frames, out, ids=...)`` advances the listed streams only (see ``BatchedLaneTracker.process_async``);
+    results stay in batch order.
     """
 
     def __init__(self, tracker, params=None):
@@ -639,8 +680,9 @@ class DevicePipeline:
         self.results_dev = [torch.zeros(tracker.n_streams * RESULT_DTYPE.itemsize, dtype=torch.uint8, device=dev)
                             for _ in range(2)]
 
-    def submit(self, frames, out=None):
+    def submit(self, frames, out=None, ids=None):
         dev = self.t.device
+        self.t._check_ids(ids, self.t._check_frames(frames))      # refuse bad ids before anything is enqueued
         k, bs = self._k, self._k & 1
         ready = torch.cuda.Event()
         ready.record(torch.cuda.current_stream(dev))            # frames (and out) belong to the caller until here
@@ -654,7 +696,7 @@ class DevicePipeline:
         with torch.cuda.stream(self.s_back):
             self.s_back.wait_event(front_done)
             self.s_back.wait_event(ready)
-            self.t.process_back_async(frames, out, bs, params=self.params, results_dev=self.results_dev[bs])
+            self.t.process_back_async(frames, out, bs, params=self.params, results_dev=self.results_dev[bs], ids=ids)
             done = torch.cuda.Event()
             done.record(self.s_back)
         self._back_done[bs] = done
@@ -701,6 +743,9 @@ class HostPipeline:
             pipe.submit(batch)
             for out, results in pipe.ready(): ...   # finished batches, oldest first
         for out, results in pipe.drain(): ...
+
+    ``submit(batch, ids=...)`` advances the listed streams only (see ``BatchedLaneTracker.process_async``); the
+    frames and records of a finished batch are in batch order.
     """
 
     def __init__(self, tracker, depth=3, overlay=True, params=None, inplace=False):
@@ -743,13 +788,14 @@ class HostPipeline:
         self.tail = 0          # oldest slot in flight
         self.inflight = 0
 
-    def submit(self, host_frames):
+    def submit(self, host_frames, ids=None):
         if self.inflight == self.depth:
             raise RuntimeError("pipeline full: collect a finished batch first")
         if not (host_frames.dtype == torch.uint8 and host_frames.is_pinned() and host_frames.is_contiguous()):
             raise ValueError("host_frames must be a contiguous pinned uint8 tensor")
         sl = self.slots[self.head]
         n = int(host_frames.shape[0])
+        self.t._check_ids(ids, n)                        # refuse bad ids before anything is enqueued
         sl["n"] = n
         with torch.cuda.stream(self.s_in):
             self.s_in.wait_event(sl["e_run"])            # the kernels that last read this input buffer are done
@@ -775,7 +821,7 @@ class HostPipeline:
             self.s_run.wait_event(e_front)
             self.s_run.wait_event(sl["e_out"])           # the previous D2H out of this output buffer is done
             d_out = sl["d_in"][:n] if self.inplace else (sl["d_out"][:n] if self.overlay else None)
-            self.t.process_back_async(sl["d_in"][:n], d_out, bs, params=self.params, results_dev=sl["d_res"])
+            self.t.process_back_async(sl["d_in"][:n], d_out, bs, params=self.params, results_dev=sl["d_res"], ids=ids)
             sl["e_run"].record(self.s_run)
         self._set_free[bs] = sl["e_run"]
         with torch.cuda.stream(self.s_out):
