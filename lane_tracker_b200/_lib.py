@@ -9,11 +9,7 @@ import ctypes as C
 import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-# LT_LIBRARY_VARIANT=<name> loads lane_tracker_b200/_variants/liblane_tracker_b200_<name>.so instead: kernel-tuning
-# builds made by tools/build_variants.py (same sources, other compile-time constants), never a different code path
-_variant = os.environ.get("LT_LIBRARY_VARIANT", "")
-LIB_PATH = (os.path.join(HERE, "_variants", "liblane_tracker_b200_%s.so" % _variant) if _variant
-            else os.path.join(HERE, "liblane_tracker_b200.so"))
+LIB_PATH = os.path.join(HERE, "liblane_tracker_b200.so")
 
 LT_MAX_AVERAGE = 8
 LT_MAX_LEVELS = 128

@@ -71,8 +71,7 @@ static int check_params(const lt_handle* h, const LtAttemptParams& a) {
         lt_set_error("Unexpected filter mode. Expected modes are 'bilateral' or 'neighborhood'.");
         return -1;
     }
-    int kmax = a.filter_type == 0 ? 255 : 255;
-    if (a.ksize_r < 1 || a.ksize_b < 1 || a.ksize_r > kmax || a.ksize_b > kmax || a.ksize_noise < 1 || a.ksize_noise > 255) {
+    if (a.ksize_r < 1 || a.ksize_b < 1 || a.ksize_r > 255 || a.ksize_b > 255 || a.ksize_noise < 1 || a.ksize_noise > 255) {
         lt_set_error("threshold kernel sizes must lie in [1, 255]");
         return -1;
     }

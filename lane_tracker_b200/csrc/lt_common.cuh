@@ -173,9 +173,8 @@ int lt_launch_undistort(lt_handle* h, const uint8_t* d_frames, int n, cudaStream
 int lt_launch_warp(lt_handle* h, uint8_t* d_bv_rgb, int n, cudaStream_t st);
 int lt_launch_planes_from_bv(lt_handle* h, const uint8_t* d_bv_rgb, int n, cudaStream_t st);
 int lt_launch_overlay(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, const int* d_draw,
-                      const int* ids, cudaStream_t st, bool rows_already_copied = false);
+                      const int* ids, cudaStream_t st);
 int lt_launch_nv12_to_rgb(const uint8_t* d_nv12, uint8_t* d_rgb, int n, int w, int h, cudaStream_t st);
-int lt_launch_copy_untouched_rows(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, cudaStream_t st);
 
 int lt_launch_filter(lt_handle* h, int n, const LtAttemptParams& p, const int* list, const int* count,
                      cudaStream_t st);

@@ -3,12 +3,9 @@
 //   or box-mean adaptive threshold on the raw planes                        > OR -> open 5x5 -> bit mask
 // The ellipse erosion / dilation / top-hat kernels live in lt_morph.cu; this file holds the thresholds, the 5x5 opening
 // of the bit mask, the layout converters and the launcher of one filter attempt.
-#include <cstdlib>
 #include <cstdio>
-#include <cuda.h>                    // CUtensorMap (types only)
 #include "lt_common.cuh"
-
-int lt_plane_tensor_map(lt_handle* h, const uint32_t* plane, int box_w, CUtensorMap* out);      // lt_morph.cu
+#include "lt_tma.cuh"
 
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::: "memory"); }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;\n" ::: "memory"); }
@@ -56,10 +53,7 @@ __device__ __forceinline__ void warp_row_prefix(const uint32_t* __restrict__ pro
 // 32-column mask words from two shift registers.  Rows sit in different banks (the row pitch is 2 * odd half-words), so
 // the walk is conflict-free.
 constexpr int CROSSH_ROWS = 32;
-#ifndef LT_CROSSH_WARPS
-#define LT_CROSSH_WARPS 8
-#endif
-constexpr int CROSSH_WARPS = LT_CROSSH_WARPS;
+constexpr int CROSSH_WARPS = 8;
 static_assert(CROSSH_ROWS <= LT_HALO_Y && CROSSH_ROWS % CROSSH_WARPS == 0, "a tile may run into the pad rows below the plane");
 
 __device__ __forceinline__ uint32_t unpack_pair(uint32_t v16) {            // (hi<<8 | lo) -> hi<<16 | lo
@@ -190,7 +184,7 @@ k_cross_h_wide(const uint32_t* __restrict__ plane_all, uint32_t* __restrict__ bi
 
 // Vertical half: one thread per packed column walks a band of rows with running sums U, D (packed u16x2).  The rows a
 // step needs (y + k + 1 to add, y + 1 as the next centre, y - k to drop) come from a per-warp ring of plane rows in
-// shared memory that is filled CV_PF chunks of CV_CHUNK rows ahead of the walk -- by TMA for row-padded planes
+// shared memory that is filled CV_PF chunks of CV_CHUNK rows ahead of the walk -- by TMA for packed, row-padded planes
 // (k_cross_v_tma, the hot path), by 4-byte cp.async otherwise (k_cross_v).
 // PACKED: k*255 + C*k + 1 < 2^15, the compare is done on both lanes at once with a guard bit.
 // ROWPAD: k + 2 * CV_CHUNK <= LT_HALO_Y, every row the walk touches or prefetches exists in the padded plane (pad rows are zero, which
@@ -199,10 +193,7 @@ k_cross_h_wide(const uint32_t* __restrict__ plane_all, uint32_t* __restrict__ bi
 // two 32x32 bit matrices column-major, transposes them with five shuffle stages each, and lane r flushes the two
 // mask words of row r with one RED.OR each -- no per-row ballot.
 constexpr int CV_CHUNK = 8;
-#ifndef LT_CV_BAND
-#define LT_CV_BAND 288
-#endif
-constexpr int CV_BAND = LT_CV_BAND;  // rows per CTA (multiple of 32)
+constexpr int CV_BAND = 288;         // rows per CTA (multiple of 32)
 constexpr int CV_BAND_FEW = 96;      // ... when fewer than 16 streams are processed (latency, not throughput)
 static_assert(CV_BAND % 32 == 0 && CV_BAND % CV_CHUNK == 0 && 32 % CV_CHUNK == 0, "band geometry");
 
@@ -224,10 +215,7 @@ __device__ __forceinline__ uint32_t warp_transpose32(uint32_t w, int lane) {
 // conflict-free, and a thread only ever reads what it fetched itself, so no barrier is needed).  Rows enter the ring
 // by 4-byte cp.async CV_PF chunks ahead of the walk: every plane row is fetched from L2/HBM once per band (instead of
 // three times, as p[y+k+1], p[y+1] and p[y-k]) and 8 * (CV_PF + 1) rows per warp are in flight without holding registers.
-#ifndef LT_CV_PF
-#define LT_CV_PF 3
-#endif
-constexpr int CV_PF = LT_CV_PF;      // prefetch distance in chunks
+constexpr int CV_PF = 3;             // prefetch distance in chunks
 
 __device__ __forceinline__ void cp_async4_zfill(void* smem_dst, const void* gsrc, bool valid) {
     unsigned sa = (unsigned)__cvta_generic_to_shared(smem_dst);
@@ -362,24 +350,6 @@ k_cross_v(const uint32_t* __restrict__ plane0, const uint32_t* __restrict__ plan
 // One lane requests a whole chunk -- a box of 32 columns x 8 rows of the plane's tensor map lands as eight consecutive
 // ring slots -- and the warp waits on the chunk's mbarrier: the eight cp.async per chunk, their address arithmetic and
 // the group bookkeeping leave the instruction stream (the walk is issue-bound).
-__device__ __forceinline__ void v_mbar_init(uint64_t* bar, int count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"((unsigned)__cvta_generic_to_shared(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void v_mbar_expect_tx(uint64_t* bar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"((unsigned)__cvta_generic_to_shared(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void v_mbar_wait(uint64_t* bar, unsigned parity) {
-    asm volatile(
-        "{\n.reg .pred p;\nWAIT_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@!p bra WAIT_%=;\n}\n" ::"r"((unsigned)__cvta_generic_to_shared(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void v_tma_load_2d(void* smem_dst, const CUtensorMap* map, int x, int y, uint64_t* bar) {
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-                 ::"r"((unsigned)__cvta_generic_to_shared(smem_dst)), "l"(map), "r"(x), "r"(y),
-                   "r"((unsigned)__cvta_generic_to_shared(bar)) : "memory");
-}
-
 constexpr int CV_NST = CV_PF + 1;    // chunk mbarriers (chunks in flight)
 static_assert(CV_CHUNK == 8, "lt_plane_tensor_map builds boxes of 8 rows");
 
@@ -412,11 +382,11 @@ k_cross_v_tma(const __grid_constant__ CUtensorMap tmap0, const __grid_constant__
     const int nbox = (2 * k + 1 + CV_CHUNK - 1) / CV_CHUNK;                            // fill boxes: they end at row yb0 + k
     const int r_last = yb1 + k + CV_CHUNK;                                             // rows >= r_last are never read
     if (lane == 0) {
-        for (int i = 0; i <= CV_NST; ++i) v_mbar_init(&bar[i], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        v_mbar_expect_tx(&bar[CV_NST], BOX * nbox);
+        for (int i = 0; i <= CV_NST; ++i) mbar_init(&bar[i], 1);
+        mbar_init_fence();
+        mbar_expect_tx(&bar[CV_NST], BOX * nbox);
         for (int j = 0; j < nbox; ++j)
-            v_tma_load_2d(ring + (R - CV_CHUNK * (nbox - j)) * 32, tm, tx, ty0 + yb0 + k + 1 - CV_CHUNK * (nbox - j), &bar[CV_NST]);
+            tma_load_2d(ring + (R - CV_CHUNK * (nbox - j)) * 32, tm, tx, ty0 + yb0 + k + 1 - CV_CHUNK * (nbox - j), &bar[CV_NST]);
     }
     __syncwarp();
     // chunk c adds rows yb0 + k + 1 + 8c .. + 7 to slots (8c) mod R (and their mirror when that is slot 0)
@@ -425,11 +395,11 @@ k_cross_v_tma(const __grid_constant__ CUtensorMap tmap0, const __grid_constant__
         if (r0 >= r_last) return;
         const int slot_row = (CV_CHUNK * c) % R;
         if (lane == 0) {
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            fence_proxy_async();
             uint64_t* b = &bar[c % CV_NST];
-            v_mbar_expect_tx(b, slot_row == 0 ? 2 * BOX : BOX);
-            v_tma_load_2d(ring + slot_row * 32, tm, tx, ty0 + r0, b);
-            if (slot_row == 0) v_tma_load_2d(ring + R * 32, tm, tx, ty0 + r0, b);
+            mbar_expect_tx(b, slot_row == 0 ? 2 * BOX : BOX);
+            tma_load_2d(ring + slot_row * 32, tm, tx, ty0 + r0, b);
+            if (slot_row == 0) tma_load_2d(ring + R * 32, tm, tx, ty0 + r0, b);
         }
     };
 #pragma unroll
@@ -444,12 +414,12 @@ k_cross_v_tma(const __grid_constant__ CUtensorMap tmap0, const __grid_constant__
         __syncwarp();                                  // every lane has finished reading the slots the next copy overwrites
         fetch_chunk(c + CV_PF);
         if (yc == yb0) {
-            v_mbar_wait(&bar[CV_NST], 0u);
+            mbar_wait(&bar[CV_NST], 0u);
             const uint32_t* f = rl + (R - 2 * k - 1) * 32;
             for (int i = 0; i < k; ++i) { U += f[i * 32]; D += f[(k + 1 + i) * 32]; }
             p = f[k * 32];
         }
-        v_mbar_wait(&bar[c % CV_NST], (unsigned)(c / CV_NST) & 1u);
+        mbar_wait(&bar[c % CV_NST], (unsigned)(c / CV_NST) & 1u);
         const uint32_t* const pn = rl + r_new * 32;
         const uint32_t* const pcur = rl + r_cur * 32;
         const uint32_t* const pold = rl + r_old * 32;
@@ -833,12 +803,7 @@ static int launch_cross_v(lt_handle* h, const uint32_t* plane, uint32_t* bits, i
     const int band = n >= 16 ? CV_BAND : CV_BAND_FEW;               // few streams: shorter sequential walks, more warps
     dim3 gv(d.p2 / 32, lt_div_up(d.bv_h, band), plane1 ? 2 * n : n);
     const int kmax = (plane1 && k1 > k) ? k1 : k;
-    const int ring_rows = crossv_ring_rows(kmax);
-    const size_t ring_bytes = (size_t)(ring_rows + CV_CHUNK) * 32 * sizeof(uint32_t);      // + the mirror slots
-#define LT_CROSS_V(PK, RP) do { int rc_ = lt_ensure_smem((const void*)k_cross_v<PK, RP>, ring_bytes); if (rc_) return rc_; \
-        k_cross_v<PK, RP><<<gv, 32, ring_bytes, st>>>(plane, plane1, bits, d, k, C, k1, C1, n, ppitch, pstride, h->stream_mask, list, count, ring_rows, band); } while (0)
-    static const bool v_tma = [] { const char* e = getenv("LT_CROSSV_TMA"); return !(e && e[0] == '0'); }();      // default on
-    if (packed && rowpad && v_tma) {
+    if (packed && rowpad) {
         CUtensorMap tm0, tm1;
         int rc_ = lt_plane_tensor_map(h, plane, 32, &tm0);
         if (!rc_) { if (plane1) rc_ = lt_plane_tensor_map(h, plane1, 32, &tm1); else tm1 = tm0; }
@@ -847,8 +812,16 @@ static int launch_cross_v(lt_handle* h, const uint32_t* plane, uint32_t* bits, i
         const size_t bytes = (size_t)(rr + CV_CHUNK) * 32 * sizeof(uint32_t) + (CV_NST + 1) * sizeof(uint64_t);
         if ((rc_ = lt_ensure_smem((const void*)k_cross_v_tma, bytes))) return rc_;
         k_cross_v_tma<<<gv, 32, bytes, st>>>(tm0, tm1, bits, d, k, C, k1, C1, n, h->stream_mask, list, count, rr, band);
-    } else if (packed && rowpad) LT_CROSS_V(true, true);
-    else if (packed) LT_CROSS_V(true, false);
+        LT_LAUNCH_CHECK();
+        return 0;
+    }
+    // the cp.async ring serves what TMA cannot: unpacked lanes, a plane whose pad rows are not zero (the raw plane of
+    // mask_noise) and k > 40
+    const int ring_rows = crossv_ring_rows(kmax);
+    const size_t ring_bytes = (size_t)(ring_rows + CV_CHUNK) * 32 * sizeof(uint32_t);      // + the mirror slots
+#define LT_CROSS_V(PK, RP) do { int rc_ = lt_ensure_smem((const void*)k_cross_v<PK, RP>, ring_bytes); if (rc_) return rc_; \
+        k_cross_v<PK, RP><<<gv, 32, ring_bytes, st>>>(plane, plane1, bits, d, k, C, k1, C1, n, ppitch, pstride, h->stream_mask, list, count, ring_rows, band); } while (0)
+    if (packed) LT_CROSS_V(true, false);
     else if (rowpad) LT_CROSS_V(false, true);
     else LT_CROSS_V(false, false);
 #undef LT_CROSS_V
@@ -899,7 +872,7 @@ int lt_launch_filter(lt_handle* h, int n, const LtAttemptParams& p, const int* l
         lt_prof_mark(h, ST_ERODE55, st);            // both erosions (55x55 on Lab-b, 29x29 on R), two concurrent kernels
         if ((rc = lt_launch_morph_pair(h, true, n, list, count, st))) return rc;
         lt_prof_mark(h, ST_TOPHAT55, st);           // both dilations + top-hat epilogues
-        if (list == nullptr && h->side) {
+        if (list == nullptr) {
             // The four threshold halves (R/Lab-b x horizontal/vertical) only OR bits into the merged mask and each
             // of them fills about half of the issue slots: the horizontal pair runs on a side stream, the vertical
             // pair on the caller's stream.  (Stage "cross_b" then reports both planes.)

@@ -11,12 +11,13 @@
 // busy.  Hence the WARP-SPECIALISED layout of this file:
 //
 //   * CTA = 6 consumer warps (192 packed columns, one per thread) + 2 producer warps, one tile x one row band.
-//   * Producers stage 8 source rows at a time (16-byte cp.async from the padded planes), build the byte-packed window
-//     tables of the 4 row pairs (T1 = the rows themselves, T4 -> T8, T16, T32) into one of TWO table buffers and
-//     signal "full"; consumers walk a buffer and signal "empty".  Named barriers (bar.sync / bar.arrive) only: a
-//     consumer never waits at a CTA-wide barrier and never executes a table build, a producer never walks.
+//   * Producers stage 8 source rows at a time (one TMA bulk-tensor copy per block from the padded plane's tensor map),
+//     build the byte-packed window tables of the 4 row pairs (T1 = the rows themselves, T4 -> T8, T16, T32) into one
+//     of TWO table buffers and signal "full"; consumers walk a buffer and signal "empty".  Named barriers (bar.sync /
+//     bar.arrive) only: a consumer never waits at a CTA-wide barrier and never executes a table build, a producer
+//     never walks.
 //   * The 55x55 (Lab-b) and the 29x29 (R) structuring elements are separate kernels with their own register budgets
-//     (3 resp. 4 CTAs per SM) launched on two streams, so the lighter one fills the SM slots the heavy one leaves.
+//     (2 resp. 3 CTAs per SM) launched on two streams, so the lighter one fills the SM slots the heavy one leaves.
 //   * A consumer derives the distinct Hop_w lazily in width order and feeds stages j and K-2-j (the ellipse is
 //     symmetric: they need the same two widths) right away, ping-ponging between two register copies of the pipeline,
 //     so only ~4 window values are live next to the K accumulators: no spills (round 1: 92 bytes of spill stores).
@@ -33,28 +34,15 @@
 #include <map>
 #include <mutex>
 #include <tuple>
-#include <cstring>
-#include <cuda.h>                    // CUtensorMap (types only: the encoder is fetched with cudaGetDriverEntryPoint)
 #include "lt_common.cuh"
 #include "lt_ellipse.cuh"
+#include "lt_tma.cuh"
 
 namespace {
 
 constexpr int TW = 192;             // packed columns per CTA = consumer threads
-#ifndef LT_MORPH_NPW
-#define LT_MORPH_NPW 2
-#endif
-constexpr int NPW = LT_MORPH_NPW;   // producer warps
-#ifndef LT_MORPH_UNROLL4
-#define LT_MORPH_UNROLL4 4
-#endif
-#ifndef LT_MORPH_UNROLL8
-#define LT_MORPH_UNROLL8 4
-#endif
-#ifndef LT_MORPH_T32_FROM_T16
-#define LT_MORPH_T32_FROM_T16 0
-#endif
-constexpr int UNROLL4 = LT_MORPH_UNROLL4, UNROLL8 = LT_MORPH_UNROLL8;   // unroll factors of the producers' task loops
+constexpr int NPW = 2;              // producer warps
+constexpr int UNROLL4 = 4, UNROLL8 = 4;   // unroll factors of the producers' task loops
 constexpr int NPROD = 32 * NPW;
 constexpr int NTHREADS = TW + NPROD;
 constexpr int RB = 8, RP = RB / 2;  // source rows / row pairs per table build
@@ -64,33 +52,6 @@ constexpr int BAR_FULL = 1, BAR_EMPTY = 3, BAR_PROD = 5;
 
 __device__ __forceinline__ void bar_sync(int id, int count) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(count) : "memory"); }
 __device__ __forceinline__ void bar_arrive(int id, int count) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(count) : "memory"); }
-
-__device__ __forceinline__ void cp_async16(void* smem_dst, const void* gsrc) {
-    unsigned sa = (unsigned)__cvta_generic_to_shared(smem_dst);
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(sa), "l"(gsrc) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::: "memory"); }
-__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;\n" ::: "memory"); }
-
-// ---- TMA (cp.async.bulk.tensor) + mbarrier: the alternative row-block staging of the producers (LT_MORPH_TMA=1)
-__device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"((unsigned)__cvta_generic_to_shared(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"((unsigned)__cvta_generic_to_shared(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, unsigned parity) {
-    asm volatile(
-        "{\n.reg .pred p;\nWAIT_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@!p bra WAIT_%=;\n}\n" ::"r"((unsigned)__cvta_generic_to_shared(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* map, int x, int y, uint64_t* bar) {
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-                 ::"r"((unsigned)__cvta_generic_to_shared(smem_dst)), "l"(map), "r"(x), "r"(y),
-                   "r"((unsigned)__cvta_generic_to_shared(bar)) : "memory");
-}
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
 template <bool IS_MAX> __device__ __forceinline__ uint32_t op2(uint32_t a, uint32_t b) { return IS_MAX ? __vmaxu2(a, b) : __vminu2(a, b); }
 template <bool IS_MAX> __device__ __forceinline__ uint32_t op3(uint32_t a, uint32_t b, uint32_t c) {
@@ -110,8 +71,8 @@ template <int K> struct Geo {
     static constexpr int TEP = TE + 4;                 // raw row pitch: slack read by the last T4 chunk
     static constexpr int PRIV = RP * TEA + 2 * RB * TEP;   // producer-private words: T4[RP][TEA], RAW[2][RB][TEP]
     static constexpr int OGW = 2 * RB * TW;            // words of the two original-row buffers of the top-hat epilogue
-    static constexpr size_t smem(bool tophat) { return (size_t)(2 * TBUF + PRIV + (tophat ? OGW : 0)) * sizeof(uint32_t) + 32; }   // + four mbarriers (TMA staging)
-    static_assert((2 * TBUF + RP * TEA) % 32 == 0 && (RB * TEP) % 32 == 0 && TE <= 256, "the raw row buffers must be 128-byte aligned for the TMA variant");
+    static constexpr size_t smem(bool tophat) { return (size_t)(2 * TBUF + PRIV + (tophat ? OGW : 0)) * sizeof(uint32_t) + 32; }   // + four mbarriers
+    static_assert((2 * TBUF + RP * TEA) % 32 == 0 && (RB * TEP) % 32 == 0 && TE <= 256, "the raw row buffers must be 128-byte aligned for the TMA copies");
     static_assert((2 * TBUF + PRIV) % 32 == 0 && (RB * TW) % 32 == 0, "so must the original-row buffers");
     static_assert(HA >= R && HA <= LT_HALO_X && R + RB <= LT_HALO_Y && TE % 4 == 0, "staging must be 16-byte granular and inside the plane padding");
 };
@@ -154,14 +115,16 @@ __device__ __forceinline__ void pair_step(const uint32_t (&S)[K], uint32_t (&D)[
 }
 
 struct MorphArgs {
-    const uint32_t* src; uint32_t* dst; const uint32_t* orig;     // padded planes (pitch d.pp), stream 0
-    int bands, band_rows, tiles, n, sms;
+    uint32_t* dst;                                                // padded plane (pitch d.pp), stream 0; the sources come as tensor maps
+    int bands, band_rows, tiles, n;
     size_t stride;                                                // words per stream
     const int* list; const int* count;
 };
 
-template <int K, bool IS_MAX, bool TOPHAT, int MINB, bool TMA>
-__global__ void __launch_bounds__(NTHREADS, MINB)
+// Resident CTAs per SM each kernel is compiled for (register budget): two for 55x55, three for 29x29; three / four were
+// measured slower (spills, DESIGN.md section 4).
+template <int K, bool IS_MAX, bool TOPHAT>
+__global__ void __launch_bounds__(NTHREADS, K == 55 ? 2 : 3)
 k_morph(MorphArgs a, LtDims d, const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap omap) {
     using G = Geo<K>;
     using E = Ellipse<K>;
@@ -174,7 +137,6 @@ k_morph(MorphArgs a, LtDims d, const __grid_constant__ CUtensorMap tmap, const _
     const int tile = item % a.tiles, band = item / a.tiles;
     if (a.count != nullptr && slot >= *a.count) return;
     const int s = a.list ? a.list[slot] : slot;
-    const uint32_t* src = a.src + (size_t)s * a.stride;
     uint32_t* dst = a.dst + (size_t)s * a.stride;
     const int pitch = d.pp;
 
@@ -183,7 +145,7 @@ k_morph(MorphArgs a, LtDims d, const __grid_constant__ CUtensorMap tmap, const _
     uint32_t* const T4 = smem + 2 * G::TBUF;            // [RP][TEA]            producer private
     uint32_t* const RAW = T4 + RP * TEA;                // [2 buffers][RB][TEP] producer private
     uint32_t* const OG = RAW + 2 * RB * G::TEP;         // [2 buffers][RB][TW]  original rows of the top-hat epilogue
-    uint64_t* const mbar = reinterpret_cast<uint64_t*>(smem + 2 * G::TBUF + G::PRIV + (TOPHAT ? G::OGW : 0));   // [4], TMA variant: raw rows, original rows
+    uint64_t* const mbar = reinterpret_cast<uint64_t*>(smem + 2 * G::TBUF + G::PRIV + (TOPHAT ? G::OGW : 0));   // [4]: raw rows, original rows
 
     const int x0 = tile * TW;
     const int yb0 = band * a.band_rows;
@@ -194,65 +156,33 @@ k_morph(MorphArgs a, LtDims d, const __grid_constant__ CUtensorMap tmap, const _
     const int r_end = yb1 + R;                          // exclusive
     const int nblk = (r_end - r_begin + RB - 1) / RB;
 
-    // Roles.  Warp w issues on SM sub-partition w % 4; the producers are warps {6, 7} in one CTA and {4, 5} in the CTA it
-    // most likely shares the SM with (launch order alternates over the SMs), so that every sub-partition carries three
-    // consumer warps and one producer warp instead of four consumers here and two producers there.
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int pfirst = ((blockIdx.x / a.sms) & 1) ? 4 : 6;
-    const bool producer = warp >= pfirst && warp < pfirst + NPW;
-    const int tid = ((warp >= pfirst + NPW ? warp - NPW : warp) << 5) | lane;   // consumer: column within the tile
+    // Roles: warps 0-5 (threads 0 .. TW - 1) are the consumers, thread = packed column within the tile; warps 6-7 are
+    // the producers.
+    const int tid = threadIdx.x;
 
-    if (producer) {
+    if (tid >= TW) {
         // ================================================================= producers
-        constexpr int TEP = G::TEP;
-        const int pt = ((warp - pfirst) << 5) | lane;
-        // staging: 16-byte cp.async chunks; TPR producer threads per row, each takes every TPR-th chunk of its row
-        constexpr int TPR = NPROD / RB;
-        const int srow = pt / TPR, sc0 = pt % TPR;
-        const uint32_t* sp = src + (ptrdiff_t)(r_begin + srow) * pitch + (x0 - HA) + 4 * sc0;   // this thread's row of the next block
-        uint32_t* const sdst = RAW + srow * TEP + 4 * sc0;
-        auto stage = [&](int buf) {
-            uint32_t* t = sdst + buf * RB * TEP;
-#pragma unroll
-            for (int c = 0; c < G::CH; c += TPR)
-                if (c + sc0 < G::CH) cp_async16(t + 4 * c, sp + 4 * c);
-            sp += (ptrdiff_t)RB * pitch;
-            cp_async_commit();
-        };
-        // original rows of the block's OUTPUT rows (source rows - R), columns of the tile itself
-        const uint32_t* op = TOPHAT ? a.orig + (size_t)s * a.stride + (ptrdiff_t)(r_begin - R + srow) * pitch + x0 + 4 * sc0 : nullptr;
-        uint32_t* const odst = OG + srow * TW + 4 * sc0;
-        int oy = r_begin - R + srow;                     // image row of this thread's original row of the next block
-        auto stage_orig = [&](int buf) {
-            if ((unsigned)oy < (unsigned)d.bv_h) {       // warm-up / overrun rows are never emitted (and may lie outside the plane)
-                uint32_t* t = odst + buf * RB * TW;
-#pragma unroll
-                for (int c = 0; c < TW / 4; c += TPR)
-                    if (c + sc0 < TW / 4) cp_async16(t + 4 * c, op + 4 * c);
-            }
-            op += (ptrdiff_t)RB * pitch;
-            oy += RB;
-            cp_async_commit();
-        };
-        // TMA variant: ONE producer thread requests the whole 8-row block (box TE x RB of the plane's tensor map, rows
-        // dense in shared memory) and every producer waits on the buffer's mbarrier instead of its own cp.async groups
-        constexpr int RPITCH = TMA ? G::TE : TEP;        // row pitch of a raw buffer
-        constexpr unsigned BLOCK_BYTES = RB * G::TE * sizeof(uint32_t);
+        const int pt = tid - TW;
+        // ONE producer thread requests the whole 8-row block (box TE x RB of the plane's tensor map, rows dense in shared
+        // memory, TE apart) and every producer waits on the buffer's mbarrier
+        constexpr int TE = G::TE;
+        constexpr unsigned BLOCK_BYTES = RB * TE * sizeof(uint32_t);
         const int tx = LT_HALO_X + x0 - HA;              // box origin in the padded plane: column ...
         int ty = s * (d.bv_h + 2 * LT_HALO_Y) + LT_HALO_Y + r_begin;     // ... and row (advances RB per block)
-        auto stage_tma = [&](int buf) {
+        auto stage = [&](int buf) {
             if (pt == 0) {
                 fence_proxy_async();                     // the generic-proxy reads of this buffer are ordered before the bulk copy
                 mbar_expect_tx(&mbar[buf], BLOCK_BYTES);
-                tma_load_2d(RAW + buf * RB * TEP, &tmap, tx, ty, &mbar[buf]);
+                tma_load_2d(RAW + buf * RB * G::TEP, &tmap, tx, ty, &mbar[buf]);
             }
             ty += RB;
         };
-        // ... and the original rows of the top-hat epilogue (box TW x RB of the original plane's map; rows outside the
-        // plane are pad rows of the layout and are never emitted)
+        // ... and the original rows of the block's OUTPUT rows (source rows - R) for the top-hat epilogue (box TW x RB of
+        // the original plane's map, columns of the tile itself; rows outside the plane are pad rows of the layout and
+        // are never emitted)
         const int ox = LT_HALO_X + x0;
         int oyt = s * (d.bv_h + 2 * LT_HALO_Y) + LT_HALO_Y + r_begin - R;
-        auto stage_orig_tma = [&](int buf) {
+        auto stage_orig = [&](int buf) {
             if (pt == 0) {
                 fence_proxy_async();
                 mbar_expect_tx(&mbar[2 + buf], (unsigned)(RB * TW * sizeof(uint32_t)));
@@ -260,25 +190,21 @@ k_morph(MorphArgs a, LtDims d, const __grid_constant__ CUtensorMap tmap, const _
             }
             oyt += RB;
         };
-        if (TMA) {
-            if (pt == 0) {
-                mbar_init(&mbar[0], 1); mbar_init(&mbar[1], 1); mbar_init(&mbar[2], 1); mbar_init(&mbar[3], 1);
-                asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-            }
-            bar_sync(BAR_PROD, NPROD);
-            stage_tma(0);
-        } else {
-            stage(0);
+        if (pt == 0) {
+            mbar_init(&mbar[0], 1); mbar_init(&mbar[1], 1); mbar_init(&mbar[2], 1); mbar_init(&mbar[3], 1);
+            mbar_init_fence();
         }
+        bar_sync(BAR_PROD, NPROD);
+        stage(0);
         for (int blk = 0; blk < nblk; ++blk) {
             const int b = blk & 1;
-            if (TMA) mbar_wait(&mbar[b], (unsigned)(blk >> 1) & 1u); else cp_async_wait_all();
+            mbar_wait(&mbar[b], (unsigned)(blk >> 1) & 1u);
             bar_sync(BAR_PROD, NPROD);                   // rows of this block landed; everybody is done with T4 and RAW[b ^ 1]
-            if (blk + 1 < nblk) { if (TMA) stage_tma(b ^ 1); else stage(b ^ 1); }     // next block's rows: in flight during the whole build
+            if (blk + 1 < nblk) stage(b ^ 1);            // next block's rows: in flight during the whole build
             if (blk >= 2) bar_sync(BAR_EMPTY + b, NTHREADS);     // the consumers have left table buffer b (and OG[b])
-            if (TOPHAT) { if (TMA) stage_orig_tma(b); else stage_orig(b); }      // lands during the build (waited for before "full" is signalled)
+            if (TOPHAT) stage_orig(b);                   // lands during the build (waited for before "full" is signalled)
             uint32_t* const Tb = TB + b * G::TBUF;
-            const uint32_t* const Rw = RAW + b * RB * TEP;     // (rows RPITCH apart)
+            const uint32_t* const Rw = RAW + b * RB * G::TEP;
             // ---- T1 (the rows themselves) and T4, four consecutive columns per task
             constexpr int NTASK = RP * G::CH, NIT = (NTASK + NPROD - 1) / NPROD;
 #pragma unroll UNROLL4
@@ -286,8 +212,8 @@ k_morph(MorphArgs a, LtDims d, const __grid_constant__ CUtensorMap tmap, const _
                 const int q = pt + it * NPROD;
                 if (q >= NTASK) break;
                 const int pr = q / G::CH, c = (q - pr * G::CH) * 4;
-                const uint4* ra = reinterpret_cast<const uint4*>(Rw + (2 * pr) * RPITCH + c);
-                const uint4* rb = reinterpret_cast<const uint4*>(Rw + (2 * pr + 1) * RPITCH + c);
+                const uint4* ra = reinterpret_cast<const uint4*>(Rw + (2 * pr) * TE + c);
+                const uint4* rb = reinterpret_cast<const uint4*>(Rw + (2 * pr + 1) * TE + c);
                 const uint4 a0 = ra[0], a1 = ra[1], b0 = rb[0], b1 = rb[1];
                 // raw lanes are plain values (or the 16-bit pad): their low bytes are the table bytes
                 uint4 t1;
@@ -310,19 +236,17 @@ k_morph(MorphArgs a, LtDims d, const __grid_constant__ CUtensorMap tmap, const _
                 *reinterpret_cast<uint4*>(T4 + pr * TEA + c) = t4;
             }
             bar_sync(BAR_PROD, NPROD);
-            // ---- T8, T16 from T4 (entry i = op over T4[i + 4k]); T32 either straight from T4 as well (one phase, 8 vector
-            // loads and 13 min/max-pipe operations per entry) or from T16 in a third phase (T32[i] = op(T16[i], T16[i + 16]):
-            // one more producer barrier, 9 operations per entry)
-            constexpr bool T32_DIRECT = G::HAS32 && !LT_MORPH_T32_FROM_T16;
+            // ---- T8, T16 and (HAS32) T32 from T4: entry i = op over T4[i + 4k]; T32 takes 8 vector loads and 13 min/max-pipe
+            // operations per entry
 #pragma unroll UNROLL8
             for (int it = 0; it < NIT; ++it) {
                 const int q = pt + it * NPROD;
                 if (q >= NTASK) break;
                 const int pr = q / G::CH, c = (q - pr * G::CH) * 4;
                 const uint4* t = reinterpret_cast<const uint4*>(T4 + pr * TEA + c);
-                uint4 v[T32_DIRECT ? 8 : 4];
+                uint4 v[G::HAS32 ? 8 : 4];
 #pragma unroll
-                for (int k = 0; k < (T32_DIRECT ? 8 : 4); ++k) v[k] = t[k];
+                for (int k = 0; k < (G::HAS32 ? 8 : 4); ++k) v[k] = t[k];
                 uint32_t o8[4], o16[4], o32[4];
 #pragma unroll
                 for (int e = 0; e < 4; ++e) {
@@ -331,7 +255,7 @@ k_morph(MorphArgs a, LtDims d, const __grid_constant__ CUtensorMap tmap, const _
                     const uint32_t a16 = op3<IS_MAX>(a8, w(2) << 8, w(3) << 8), b16 = op3<IS_MAX>(b8, w(2), w(3));
                     o8[e] = __byte_perm(a8, b8, 0x7351);          // value bytes back to {a.lo, b.lo, a.hi, b.hi}
                     o16[e] = __byte_perm(a16, b16, 0x7351);
-                    if (T32_DIRECT) {
+                    if (G::HAS32) {
                         const uint32_t a32 = op3<IS_MAX>(a16, op2<IS_MAX>(w(4) << 8, w(5) << 8), op2<IS_MAX>(w(6) << 8, w(7) << 8));
                         const uint32_t b32 = op3<IS_MAX>(b16, op2<IS_MAX>(w(4), w(5)), op2<IS_MAX>(w(6), w(7)));
                         o32[e] = __byte_perm(a32, b32, 0x7351);
@@ -340,25 +264,9 @@ k_morph(MorphArgs a, LtDims d, const __grid_constant__ CUtensorMap tmap, const _
                 uint32_t* o = Tb + RP * TEA + pr * TEA + c;
                 *reinterpret_cast<uint4*>(o) = make_uint4(o8[0], o8[1], o8[2], o8[3]);
                 *reinterpret_cast<uint4*>(o + RP * TEA) = make_uint4(o16[0], o16[1], o16[2], o16[3]);
-                if (T32_DIRECT) *reinterpret_cast<uint4*>(o + 2 * RP * TEA) = make_uint4(o32[0], o32[1], o32[2], o32[3]);
+                if (G::HAS32) *reinterpret_cast<uint4*>(o + 2 * RP * TEA) = make_uint4(o32[0], o32[1], o32[2], o32[3]);
             }
-            if (G::HAS32 && !T32_DIRECT) {
-                bar_sync(BAR_PROD, NPROD);
-                // entries whose window runs past the tabulated columns read slack / the next pair's row: never used by the walk
-#pragma unroll UNROLL8
-                for (int it = 0; it < NIT; ++it) {
-                    const int q = pt + it * NPROD;
-                    if (q >= NTASK) break;
-                    const int pr = q / G::CH, c = (q - pr * G::CH) * 4;
-                    const uint32_t* t16 = Tb + 2 * RP * TEA + pr * TEA + c;
-                    const uint4 u = *reinterpret_cast<const uint4*>(t16), v = *reinterpret_cast<const uint4*>(t16 + 16);
-                    auto m = [](uint32_t x, uint32_t y) {
-                        return __byte_perm(op2<IS_MAX>(x << 8, y << 8), op2<IS_MAX>(x, y), 0x7351);
-                    };
-                    *reinterpret_cast<uint4*>(Tb + 3 * RP * TEA + pr * TEA + c) = make_uint4(m(u.x, v.x), m(u.y, v.y), m(u.z, v.z), m(u.w, v.w));
-                }
-            }
-            if (TOPHAT) { if (TMA) mbar_wait(&mbar[2 + b], (unsigned)(blk >> 1) & 1u); else cp_async_wait_all(); }   // OG[b] has landed
+            if (TOPHAT) mbar_wait(&mbar[2 + b], (unsigned)(blk >> 1) & 1u);     // OG[b] has landed
             bar_arrive(BAR_FULL + b, NTHREADS);
         }
         return;
@@ -419,9 +327,30 @@ k_morph(MorphArgs a, LtDims d, const __grid_constant__ CUtensorMap tmap, const _
     }
 }
 
-// Tensor map of one padded plane allocation for the TMA variant: 2-D uint32 [rows][pp], box = TE x RB.  Cached per
-// (device, allocation, geometry); the encoder comes from the driver through cudaGetDriverEntryPoint (no -lcuda).
-static int plane_tensor_map(lt_handle* h, const uint32_t* plane, int box_w, CUtensorMap* out) {
+template <int K, bool IS_MAX, bool TOPHAT>
+int launch_one(lt_handle* h, const uint32_t* src, uint32_t* dst, const uint32_t* orig, int bands, int n, const int* list,
+               const int* count, cudaStream_t st) {
+    const LtDims& d = h->d;
+    MorphArgs a;
+    a.dst = dst;
+    a.band_rows = (lt_div_up(d.bv_h, bands) + 1) & ~1;          // even: output rows come out in aligned pairs
+    a.bands = lt_div_up(d.bv_h, a.band_rows);
+    a.tiles = lt_div_up(d.p2, TW);
+    a.n = n; a.stride = h->stream_pad; a.list = list; a.count = count;
+    CUtensorMap tm, om = {};                                     // om: original rows, top-hat only
+    int rc;
+    if ((rc = lt_plane_tensor_map(h, src, Geo<K>::TE, &tm))) return rc;
+    if (TOPHAT && (rc = lt_plane_tensor_map(h, orig, TW, &om))) return rc;
+    if ((rc = lt_ensure_smem((const void*)k_morph<K, IS_MAX, TOPHAT>, Geo<K>::smem(TOPHAT)))) return rc;
+    k_morph<K, IS_MAX, TOPHAT><<<n * a.tiles * a.bands, NTHREADS, Geo<K>::smem(TOPHAT), st>>>(a, d, tm, om);
+    LT_LAUNCH_CHECK();
+    return 0;
+}
+
+}  // namespace
+
+// The encoder comes from the driver through cudaGetDriverEntryPoint (no -lcuda).
+int lt_plane_tensor_map(lt_handle* h, const uint32_t* plane, int box_w, CUtensorMap* out) {
     typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -457,53 +386,6 @@ static int plane_tensor_map(lt_handle* h, const uint32_t* plane, int box_w, CUte
     return 0;
 }
 
-template <int K, bool IS_MAX, bool TOPHAT, int MINB>
-int launch_occ(lt_handle* h, const uint32_t* src, uint32_t* dst, const uint32_t* orig, int bands, int n, const int* list,
-               const int* count, cudaStream_t st) {
-    const LtDims& d = h->d;
-    MorphArgs a;
-    a.src = src; a.dst = dst; a.orig = orig;
-    a.band_rows = (lt_div_up(d.bv_h, bands) + 1) & ~1;          // even: output rows come out in aligned pairs
-    a.bands = lt_div_up(d.bv_h, a.band_rows);
-    a.tiles = lt_div_up(d.p2, TW);
-    a.n = n; a.stride = h->stream_pad; a.list = list; a.count = count;
-    a.sms = h->sm_count > 0 ? h->sm_count : 148;
-    static const bool parity = [] { const char* e = getenv("LT_MORPH_PARITY"); return e && e[0] == '1'; }();
-    if (!parity) a.sms = 1 << 30;
-    // The producers stage their row blocks with cp.async.bulk.tensor + mbarrier (one request per block by one thread);
-    // LT_MORPH_TMA=0 selects the 16-byte cp.async staging it replaced (measured 3 % slower: the producers are the
-    // critical path and every instruction they do not issue counts)
-    static const bool tma = [] { const char* e = getenv("LT_MORPH_TMA"); return !(e && e[0] == '0'); }();      // default on
-    CUtensorMap tm;
-    memset(&tm, 0, sizeof(tm));
-    int rc;
-    CUtensorMap om = tm;
-    if (tma) {
-        if ((rc = plane_tensor_map(h, src, Geo<K>::TE, &tm))) return rc;
-        if (TOPHAT && (rc = plane_tensor_map(h, orig, TW, &om))) return rc;
-        if ((rc = lt_ensure_smem((const void*)k_morph<K, IS_MAX, TOPHAT, MINB, true>, Geo<K>::smem(TOPHAT)))) return rc;
-        k_morph<K, IS_MAX, TOPHAT, MINB, true><<<n * a.tiles * a.bands, NTHREADS, Geo<K>::smem(TOPHAT), st>>>(a, d, tm, om);
-    } else {
-        if ((rc = lt_ensure_smem((const void*)k_morph<K, IS_MAX, TOPHAT, MINB, false>, Geo<K>::smem(TOPHAT)))) return rc;
-        k_morph<K, IS_MAX, TOPHAT, MINB, false><<<n * a.tiles * a.bands, NTHREADS, Geo<K>::smem(TOPHAT), st>>>(a, d, tm, om);
-    }
-    LT_LAUNCH_CHECK();
-    return 0;
-}
-
-// resident CTAs per SM each kernel is compiled for (register budget): two for 55x55 (106 registers), three for 29x29
-// (76 registers); three / four were measured slower (spills, DESIGN.md section 4)
-template <int K, bool IS_MAX, bool TOPHAT>
-int launch_one(lt_handle* h, const uint32_t* src, uint32_t* dst, const uint32_t* orig, int bands, int n, const int* list,
-               const int* count, cudaStream_t st) {
-    return launch_occ<K, IS_MAX, TOPHAT, K == 55 ? 2 : 3>(h, src, dst, orig, bands, n, list, count, st);
-}
-
-}  // namespace
-
-// (also used by the vertical threshold, lt_filter.cu: box = box_w columns x 8 rows of a padded plane)
-int lt_plane_tensor_map(lt_handle* h, const uint32_t* plane, int box_w, CUtensorMap* out) { return plane_tensor_map(h, plane, box_w, out); }
-
 // Band counts of the two jobs: simulate list scheduling of both grids (55x55 CTAs first, they are the long ones) on
 // the CTA slots of the device.  Per-row costs: measured relative walk costs of the two structuring elements.
 static void choose_bands(lt_handle* h, int n, int tiles, int H, int* b55, int* b29) {
@@ -516,8 +398,8 @@ static void choose_bands(lt_handle* h, int n, int tiles, int H, int* b55, int* b
         else c55 = c29 = 1;
     }
     if (!fixed) {
-        // an SM holds 3 CTAs of the 55x55 kernel or 4 of the 29x29 kernel (registers); model it as 12 "quarter slots"
-        // where a 55x55 CTA takes 4 and a 29x29 CTA 3, scheduled greedily in launch order
+        // a cost model, not the hardware's CTA counts: every CTA takes one of 3.5 slots per SM for (band rows + warm-up
+        // rows) x the relative walk cost of its structuring element, scheduled greedily in launch order
         double best = 1e300;
         std::vector<double> freeat;
         for (int a = 1; a <= 16; ++a)
@@ -525,7 +407,6 @@ static void choose_bands(lt_handle* h, int n, int tiles, int H, int* b55, int* b
                 const int ra = (lt_div_up(H, a) + 1) & ~1, rb = (lt_div_up(H, b) + 1) & ~1;
                 const int na = n * tiles * lt_div_up(H, ra), nb = n * tiles * lt_div_up(H, rb);
                 const double ta = (ra + 56) * 1.0, tb = (rb + 30) * 0.55;
-                // greedy: 3.5 concurrent CTAs per SM on average
                 const int slots = (7 * sms) / 2;
                 freeat.assign(slots, 0.0);
                 std::make_heap(freeat.begin(), freeat.end(), std::greater<double>());
@@ -551,11 +432,9 @@ int lt_launch_morph_pair(lt_handle* h, bool tophat, int n, const int* list, cons
     const LtDims& d = h->d;
     int b55, b29, rc;
     choose_bands(h, n, lt_div_up(d.p2, TW), d.bv_h, &b55, &b29);
-    cudaStream_t s2 = h->side ? h->side : st;
-    if (s2 != st) {
-        LT_CUDA(cudaEventRecord(h->ev_fork, st));
-        LT_CUDA(cudaStreamWaitEvent(s2, h->ev_fork, 0));
-    }
+    cudaStream_t s2 = h->side;
+    LT_CUDA(cudaEventRecord(h->ev_fork, st));
+    LT_CUDA(cudaStreamWaitEvent(s2, h->ev_fork, 0));
     if (!tophat) {
         if ((rc = launch_one<55, false, false>(h, h->planeB, h->tmpB, nullptr, b55, n, list, count, st))) return rc;
         if ((rc = launch_one<29, false, false>(h, h->planeR, h->tmpR, nullptr, b29, n, list, count, s2))) return rc;
@@ -563,9 +442,7 @@ int lt_launch_morph_pair(lt_handle* h, bool tophat, int n, const int* list, cons
         if ((rc = launch_one<55, true, true>(h, h->tmpB, h->topB, h->planeB, b55, n, list, count, st))) return rc;
         if ((rc = launch_one<29, true, true>(h, h->tmpR, h->topR, h->planeR, b29, n, list, count, s2))) return rc;
     }
-    if (s2 != st) {
-        LT_CUDA(cudaEventRecord(h->ev_join, s2));
-        LT_CUDA(cudaStreamWaitEvent(st, h->ev_join, 0));
-    }
+    LT_CUDA(cudaEventRecord(h->ev_join, s2));
+    LT_CUDA(cudaStreamWaitEvent(st, h->ev_join, 0));
     return 0;
 }

@@ -189,17 +189,12 @@ constexpr int NSW = LT_UND_GROUP;      // streams per group
 // a warp read 32 neighbouring pixels of one frame: whole sectors).  The stream-minor output goes through shared memory
 // so that a warp stores whole 32-byte sectors.  Fast path: the six bytes of a tap pair come from three aligned 32-bit
 // words and two funnel shifts.
-#ifndef LT_UND_SPC
-#define LT_UND_SPC 8
-#endif
-constexpr int UND_SPC = LT_UND_SPC;    // streams per CTA: 4, 8 or 16 (a CTA covers UND_SPC / 4 of the four 16-byte chunks of a pixel)
+constexpr int UND_SPC = 8;             // streams per CTA: 4, 8 or 16 (a CTA covers UND_SPC / 4 of the four 16-byte chunks of a pixel)
 constexpr int UND_CH = UND_SPC / 4;
-#ifndef LT_UND_MINB
-#define LT_UND_MINB 6
-#endif
+constexpr int UND_MINB = 6;            // resident CTAs per SM the undistort is compiled for
 static_assert(UND_SPC == 4 || UND_SPC == 8 || UND_SPC == 16, "streams per CTA");
 
-__global__ void __launch_bounds__(256, LT_UND_MINB)
+__global__ void __launch_bounds__(256, UND_MINB)
 k_undistort_roi(const uint8_t* __restrict__ frames, uint32_t* __restrict__ und, const int2* __restrict__ desc, LtDims d, int n,
                 size_t group_words) {
     __shared__ uint4 tile[256 * UND_CH];               // [pixel][chunk of four streams], chunk slot rotated by the pixel
@@ -435,16 +430,11 @@ __device__ __forceinline__ void blend_weights(uint32_t f, uint32_t& wA, uint32_t
 __device__ __forceinline__ uint32_t u4_at(const uint4& v, int k) { return k == 0 ? v.x : (k == 1 ? v.y : (k == 2 ? v.z : v.w)); }
 
 constexpr int WARP_ITEMS = 64;        // packed columns per pass of a CTA (x 4 stream chunks = 256 threads)
-#ifndef LT_WARP_NB
-#define LT_WARP_NB 8
-#endif
-constexpr int WARP_NB = LT_WARP_NB;   // passes per CTA (the Lab tables are loaded once per CTA)
+constexpr int WARP_NB = 8;            // passes per CTA (the Lab tables are loaded once per CTA)
+constexpr int WARP_MINB = 4;          // resident CTAs per SM the warp is compiled for
 
-#ifndef LT_WARP_MINB
-#define LT_WARP_MINB 4
-#endif
 template <bool RGB_OUT>
-__global__ void __launch_bounds__(256, LT_WARP_MINB)
+__global__ void __launch_bounds__(256, WARP_MINB)
 k_warp_planes(const uint32_t* __restrict__ und_all, const int2* __restrict__ desc, uint32_t* __restrict__ planeR,
               uint32_t* __restrict__ planeB, uint8_t* __restrict__ bv_rgb, const uint2* __restrict__ yz,
               const unsigned short* __restrict__ cb, LtDims d, unsigned stream_pad, int n, size_t group_words) {
@@ -755,7 +745,7 @@ static void overlay_rows(const lt_handle* h, const uint8_t* d_frames, const uint
     if (d_out != d_frames && !vec_ok) { r0 = 0; r1 = d.img_h; }   // generic path: k_overlay copies every row itself
 }
 
-int lt_launch_copy_untouched_rows(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, cudaStream_t st) {
+static int copy_untouched_rows(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, cudaStream_t st) {
     const LtDims& d = h->d;
     const size_t row_bytes = (size_t)d.img_w * 3, frame_bytes = row_bytes * d.img_h;
     int r0, r1; bool vec_ok;
@@ -772,11 +762,11 @@ int lt_launch_copy_untouched_rows(lt_handle* h, const uint8_t* d_frames, uint8_t
 }
 
 int lt_launch_overlay(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, const int* d_draw,
-                      const int* ids, cudaStream_t st, bool rows_already_copied) {
+                      const int* ids, cudaStream_t st) {
     const LtDims& d = h->d;
     int r0, r1; bool vec_ok;
     overlay_rows(h, d_frames, d_out, r0, r1, vec_ok);
-    if (!rows_already_copied) { int rc = lt_launch_copy_untouched_rows(h, d_frames, d_out, n, st); if (rc) return rc; }
+    { int rc = copy_untouched_rows(h, d_frames, d_out, n, st); if (rc) return rc; }
     if (r1 > r0) {
         dim3 g(lt_div_up(d.img_w / 4, 256), r1 - r0, n);
         k_overlay<<<g, 256, 0, st>>>(d_frames, d_out, h->ov_map, h->lane_rows, h->lane_bbox, d_draw, d, r0, ids);

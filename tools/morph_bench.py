@@ -1,5 +1,5 @@
 #!/usr/bin/env python3
-"""Stage times of the filter front half at S=64 for a list of (implementation, band split) settings.
+"""Stage times of the filter front half at S=64 for a list of morphology band splits.
 The morphology kernels do not branch on pixel values, so random frames are as good as rendered ones."""
 import json
 import os
@@ -34,23 +34,16 @@ def one():
     e1.record()
     torch.cuda.synchronize()
     st, calls = trk.profile_read()
-    print(json.dumps({"bands": os.environ.get("LT_MORPH_BANDS", "auto"), "variant": os.environ.get("LT_LIBRARY_VARIANT", "-"),
-                      "chosen": trk.morph_bands(), "ms_per_step": e0.elapsed_time(e1) / n,
+    print(json.dumps({"bands": os.environ.get("LT_MORPH_BANDS", "auto"), "chosen": trk.morph_bands(), "ms_per_step": e0.elapsed_time(e1) / n,
                       "stages": {k: round(v / calls, 4) for k, v in st.items() if v > 0}}), flush=True)
 
 
 def main():
     if len(sys.argv) > 1 and sys.argv[1] == "--one":
         return one()
-    settings = sys.argv[1:] or ["new:auto", "new:2,5", "new:2,4", "new:3,5", "new:3,6", "new:2,6", "new:4,8"]
-    for s in settings:
-        impl, bands = s.split(":")[:2]
+    for bands in sys.argv[1:] or ["auto", "2,5", "2,4", "3,5", "3,6", "2,6", "4,8"]:
         env = dict(os.environ)
         env.pop("LT_MORPH_BANDS", None)
-        env.pop("LT_MORPH_PARITY", None)
-        env.pop("LT_LIBRARY_VARIANT", None)
-        if len(s.split(":")) > 3 and s.split(":")[3]:
-            env["LT_LIBRARY_VARIANT"] = s.split(":")[3]
         if bands != "auto":
             env["LT_MORPH_BANDS"] = bands
         subprocess.run([sys.executable, os.path.abspath(__file__), "--one"], env=env, check=False)
