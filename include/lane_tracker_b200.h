@@ -13,7 +13,8 @@
  *   - int return: 0 = ok, <0 = error (see lt_last_error); no exceptions;
  *   - one handle per GPU; a handle is not thread-safe (the reference object is
  *     not re-entrant either: it carries tracking state);
- *   - images are uint8, RGB, row-major HWC, tightly packed.
+ *   - images are uint8, RGB, row-major HWC, tightly packed; the input frames of the
+ *     hot path may be NV12 instead (lt_set_frame_format).
  *   - a handle serves `max_streams` independent video streams; per-stream
  *     tracking state (lane_tracker.py:139-176) lives in device memory.
  */
@@ -139,9 +140,9 @@ int64_t lt_launch_count(void);
  * (d_bv_rgb), masks, debug views and resize buffers are accessed byte by byte and need no alignment. */
 
 /* LaneTracker.process (lane_tracker.py:876-1209) for streams 0..n_streams-1.
- *   d_frames : [n_streams][img_h][img_w][3]
- *   d_out    : same shape, NULL for fits-only mode (no overlay rendered), or == d_frames to annotate in place
- *              (only the rows the lane overlay can reach are rewritten)
+ *   d_frames : [n_streams][img_h][img_w][3], or NV12 [n_streams][img_h * 3 / 2][img_w] (lt_set_frame_format)
+ *   d_out    : [n_streams][img_h][img_w][3], NULL for fits-only mode (no overlay rendered), or, for RGB frames,
+ *              == d_frames to annotate in place (only the rows the lane overlay can reach are rewritten)
  *   params   : one lt_params for all streams (the reference's defaults-are-the-
  *              config convention, README.md:34)
  *   d_results: [n_streams] lt_result, device memory (copy back asynchronously)
@@ -214,9 +215,28 @@ int lt_set_text_sprites(lt_handle* h, const uint8_t* h_tables, int32_t n_tables,
  * mask IoU >= 0.6 per frame and >= 0.8 on average (measured: tests/test_gpu_parity.py::test_fused_remap_variant). */
 int lt_set_remap_mode(lt_handle* h, int32_t mode);
 
+/* Layout of the input frames d_frames.  LT_FRAME_RGB (default): [n][img_h][img_w][3].  LT_FRAME_NV12: what video
+ * decoders deliver, [n][img_h * 3 / 2][img_w] uint8 per frame (the luma plane, then img_h / 2 rows of interleaved U, V
+ * pairs), converted as cv2.cvtColor(COLOR_YUV2RGB_NV12) (ITU-R BT.601 limited range, chroma not interpolated) inside
+ * the kernels that read the frames, with no RGB copy of the frame in between.  The results are bit for bit those of
+ * the RGB path fed lt_nv12_to_rgb of the same frames.
+ *   - The format applies to d_frames of lt_process, lt_process_front, lt_process_back, lt_process_streams,
+ *     lt_process_back_streams and lt_remap, and to lt_memcpy_rows.  lt_draw_lane, lt_warp_frame and lt_draw_text
+ *     always take RGB frames.  d_out stays RGB [n][img_h][img_w][3]: every row of it is written (the annotation cannot
+ *     happen in place), and a d_out whose bytes overlap the NV12 input is refused.
+ *   - NV12 buffers must be 4-byte aligned, like RGB frames.
+ *   - The format is read when a call is enqueued, so it may change between calls with work in flight.
+ *   - Refused with an error: an unknown format, NV12 on a handle with odd img_h, and NV12 together with remap mode 1
+ *     (the fused variant samples raw RGB), whichever of lt_set_frame_format / lt_set_remap_mode comes second. */
+#define LT_FRAME_RGB 0
+#define LT_FRAME_NV12 1
+int lt_set_frame_format(lt_handle* h, int32_t format);
+
 /* Copy frame rows [row0, row1) of n_frames frames between a host (pinned) and a device batch of full frames
  * (one cudaMemcpy2DAsync: pitch = frame size).  to_device: 1 host->device, 0 device->host.  Used to move only
- * the rows the tracker reads / the overlay can change (lt_debug_read geometry) across PCIe. */
+ * the rows the tracker reads / the overlay can change (lt_debug_read geometry) across PCIe.  Under LT_FRAME_NV12
+ * the frames are NV12 and the copy moves luma rows [row0, row1) plus the chroma rows that cover them
+ * ([row0 / 2, (row1 + 1) / 2) of the chroma plane): two cudaMemcpy2DAsync. */
 int lt_memcpy_rows(lt_handle* h, void* dst, const void* src, int32_t n_frames, int32_t row0, int32_t row1,
                    int32_t to_device, void* stream);
 

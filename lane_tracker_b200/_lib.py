@@ -92,6 +92,7 @@ SIGNATURES = {
     "lt_read_capture": (C.c_int, [P, i32, i32, i32, P, i32, C.POINTER(i32), P, C.POINTER(i32)]),
     "lt_set_text_sprites": (C.c_int, [P, P, i32, P, i32, P, P, P, i32, P, i32]),
     "lt_set_remap_mode": (C.c_int, [P, i32]),
+    "lt_set_frame_format": (C.c_int, [P, i32]),
     "lt_memcpy_rows": (C.c_int, [P, P, P, i32, i32, i32, i32, P]),
     "lt_profile_begin": (C.c_int, [P, i32]),
     "lt_profile_read": (C.c_int, [P, C.POINTER(f64), C.POINTER(i32)]),

@@ -416,13 +416,21 @@ static int process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, i
         // geometry the text rows and the rows the lane overlay can reach are disjoint and the order is immaterial;
         // when they overlap (other calibrations) the text goes first and the blend runs in place over it.
         const bool text_under_blend = h->txt_nchars > 0 && h->txt_row0 < h->d.ov1 && h->d.ov0 < h->txt_row1;
+        // NV12 input: the frame is converted where it is read; with text under the blend, the whole frame is converted
+        // into d_out first and the text and the blend then run on d_out as for RGB.
+        const bool nv12 = h->frame_format == LT_FRAME_NV12;
         if (text_under_blend) {
-            if (d_out != d_frames)
+            if (nv12) {
+                if ((rc = lt_launch_nv12_to_rgb(d_frames, d_out, n, h->d.img_w, h->d.img_h, 0, h->d.img_h, st))) return rc;
+            } else if (d_out != d_frames) {
                 LT_CUDA(cudaMemcpyAsync(d_out, d_frames, (size_t)n * h->d.img_w * h->d.img_h * 3, cudaMemcpyDeviceToDevice, st));
+            }
             if ((rc = lt_launch_text(h, d_out, n, ids, st))) return rc;
             if ((rc = lt_launch_overlay(h, d_out, d_out, n, h->draw_flags, ids, st))) return rc;
         } else {
-            if ((rc = lt_launch_overlay(h, d_frames, d_out, n, h->draw_flags, ids, st))) return rc;
+            if (nv12) rc = lt_launch_overlay_nv12(h, d_frames, d_out, n, h->draw_flags, ids, st);
+            else rc = lt_launch_overlay(h, d_frames, d_out, n, h->draw_flags, ids, st);
+            if (rc) return rc;
             if ((rc = lt_launch_text(h, d_out, n, ids, st))) return rc;
         }
         lt_prof_mark(h, ST_OVERLAY, st);
@@ -438,6 +446,23 @@ static int check_frame_buffer(const void* p, const char* what) {
     if ((uintptr_t)p & 3) {
         lt_set_error("%s must be 4-byte aligned (got address %p)", what, p);
         return -1;
+    }
+    return 0;
+}
+
+// d_out of the process calls: 4-byte aligned; under LT_FRAME_NV12 it is a separate RGB buffer, so its bytes may not
+// overlap the NV12 input (the annotation cannot happen in place).
+static int check_out(const lt_handle* h, const uint8_t* d_frames, const uint8_t* d_out, int n) {
+    int rc;
+    if ((rc = check_frame_buffer(d_out, "d_out"))) return rc;
+    if (h && d_out && d_frames && n > 0 && h->frame_format == LT_FRAME_NV12) {
+        const size_t fb = (size_t)h->d.img_w * h->d.img_h;
+        const uintptr_t o0 = (uintptr_t)d_out, o1 = o0 + (size_t)n * fb * 3;
+        const uintptr_t f0 = (uintptr_t)d_frames, f1 = f0 + (size_t)n * (fb + fb / 2);
+        if (o0 < f1 && f0 < o1) {
+            lt_set_error("d_out overlaps the NV12 input frames: NV12 frames are annotated into a separate RGB buffer");
+            return -1;
+        }
     }
     return 0;
 }
@@ -466,7 +491,7 @@ extern "C" int lt_process(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out,
                           lt_result* d_results, void* stream) {
     int rc;
     LtAttemptParams p1;
-    if ((rc = check_frame_buffer(d_out, "d_out"))) return rc;
+    if ((rc = check_out(h, d_frames, d_out, n))) return rc;
     if ((rc = process_args(h, d_frames, n, params, 0, &p1))) return rc;
     if (!d_results) { lt_set_error("null argument"); return -1; }
     if ((rc = process_front(h, d_frames, n, p1, (cudaStream_t)stream))) return rc;
@@ -485,7 +510,7 @@ extern "C" int lt_process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d
                                int32_t set, lt_result* d_results, void* stream) {
     int rc;
     LtAttemptParams p1;
-    if ((rc = check_frame_buffer(d_out, "d_out"))) return rc;
+    if ((rc = check_out(h, d_frames, d_out, n))) return rc;
     if ((rc = process_args(h, d_frames, n, params, set, &p1))) return rc;
     if (!d_results) { lt_set_error("null argument"); return -1; }
     return process_back(h, d_frames, d_out, n, params, p1, d_results, (cudaStream_t)stream, true);
@@ -512,7 +537,7 @@ extern "C" int lt_process_streams(lt_handle* h, const uint8_t* d_frames, uint8_t
     int rc;
     LtAttemptParams p1;
     if ((rc = check_ids(h, h_ids, n))) return rc;
-    if ((rc = check_frame_buffer(d_out, "d_out"))) return rc;
+    if ((rc = check_out(h, d_frames, d_out, n))) return rc;
     if ((rc = process_args(h, d_frames, n, params, 0, &p1))) return rc;
     if (!d_results) { lt_set_error("null argument"); return -1; }
     if ((rc = process_front(h, d_frames, n, p1, (cudaStream_t)stream))) return rc;
@@ -524,7 +549,7 @@ extern "C" int lt_process_back_streams(lt_handle* h, const uint8_t* d_frames, ui
     int rc;
     LtAttemptParams p1;
     if ((rc = check_ids(h, h_ids, n))) return rc;
-    if ((rc = check_frame_buffer(d_out, "d_out"))) return rc;
+    if ((rc = check_out(h, d_frames, d_out, n))) return rc;
     if ((rc = process_args(h, d_frames, n, params, set, &p1))) return rc;
     if (!d_results) { lt_set_error("null argument"); return -1; }
     return process_back(h, d_frames, d_out, n, params, p1, d_results, (cudaStream_t)stream, true, h_ids);
@@ -667,6 +692,10 @@ extern "C" int lt_set_text_sprites(lt_handle* h, const uint8_t* tables, int32_t 
 
 extern "C" int lt_set_remap_mode(lt_handle* h, int32_t mode) {
     if (!h || (mode != 0 && mode != 1)) { lt_set_error("remap mode must be 0 (exact) or 1 (fused single resample)"); return -1; }
+    if (mode == 1 && h->frame_format == LT_FRAME_NV12) {
+        lt_set_error("remap mode 1 (fused single resample) samples RGB frames: not available with NV12 frames");
+        return -1;
+    }
     LT_CUDA(cudaSetDevice(h->cfg.device));
     if (mode == 1 && !h->fused_desc) {
         int rc = dev_alloc(&h->fused_desc, (size_t)h->d.bv_w * h->d.bv_h);
@@ -678,14 +707,42 @@ extern "C" int lt_set_remap_mode(lt_handle* h, int32_t mode) {
     return 0;
 }
 
+extern "C" int lt_set_frame_format(lt_handle* h, int32_t format) {
+    if (!h) { lt_set_error("null handle"); return -1; }
+    if (format != LT_FRAME_RGB && format != LT_FRAME_NV12) {
+        lt_set_error("frame format must be %d (RGB) or %d (NV12), got %d", LT_FRAME_RGB, LT_FRAME_NV12, format);
+        return -1;
+    }
+    if (format == LT_FRAME_NV12 && (h->d.img_h & 1)) {
+        lt_set_error("NV12 frames need an even image height (got %d)", h->d.img_h);
+        return -1;
+    }
+    if (format == LT_FRAME_NV12 && h->remap_mode == 1) {
+        lt_set_error("NV12 frames are not available with remap mode 1 (fused single resample), which samples RGB frames");
+        return -1;
+    }
+    h->frame_format = format;
+    return 0;
+}
+
 extern "C" int lt_memcpy_rows(lt_handle* h, void* dst, const void* src, int32_t n, int32_t row0, int32_t row1,
                               int32_t to_device, void* stream) {
     if (!h || !dst || !src || n < 1 || row0 < 0 || row1 > h->d.img_h || row0 >= row1) { lt_set_error("bad argument"); return -1; }
+    const cudaMemcpyKind kind = to_device ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToHost;
+    if (h->frame_format == LT_FRAME_NV12) {     // luma rows [row0, row1), then the chroma rows that cover them
+        const size_t W = (size_t)h->d.img_w, H = (size_t)h->d.img_h, frame_bytes = W * (H + H / 2);
+        const size_t c0 = H + (size_t)row0 / 2, c1 = H + (size_t)(row1 + 1) / 2;
+        LT_CUDA(cudaMemcpy2DAsync((char*)dst + row0 * W, frame_bytes, (const char*)src + row0 * W, frame_bytes,
+                                  (size_t)(row1 - row0) * W, (size_t)n, kind, (cudaStream_t)stream));
+        LT_CUDA(cudaMemcpy2DAsync((char*)dst + c0 * W, frame_bytes, (const char*)src + c0 * W, frame_bytes, (c1 - c0) * W,
+                                  (size_t)n, kind, (cudaStream_t)stream));
+        return 0;
+    }
     const size_t row_bytes = (size_t)h->d.img_w * 3, frame_bytes = row_bytes * h->d.img_h;
     const char* s = (const char*)src + (size_t)row0 * row_bytes;
     char* d = (char*)dst + (size_t)row0 * row_bytes;
-    LT_CUDA(cudaMemcpy2DAsync(d, frame_bytes, s, frame_bytes, (size_t)(row1 - row0) * row_bytes, (size_t)n,
-                              to_device ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToHost, (cudaStream_t)stream));
+    LT_CUDA(cudaMemcpy2DAsync(d, frame_bytes, s, frame_bytes, (size_t)(row1 - row0) * row_bytes, (size_t)n, kind,
+                              (cudaStream_t)stream));
     return 0;
 }
 
@@ -765,7 +822,7 @@ extern "C" int lt_nv12_to_rgb(const uint8_t* d_nv12, uint8_t* d_rgb, int32_t n, 
         lt_set_error("lt_nv12_to_rgb: width must be a multiple of 4, height even, buffers 4-byte aligned");
         return -1;
     }
-    return lt_launch_nv12_to_rgb(d_nv12, d_rgb, n, width, height, (cudaStream_t)stream);
+    return lt_launch_nv12_to_rgb(d_nv12, d_rgb, n, width, height, 0, height, (cudaStream_t)stream);
 }
 
 extern "C" int lt_filter_lane_points(lt_handle* h, const uint8_t* d_bv_rgb, uint8_t* d_mask, int32_t n,

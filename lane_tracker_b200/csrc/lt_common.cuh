@@ -83,6 +83,7 @@ struct lt_handle {
     int2* bv_desc;               // [bv_h][bv_w] tap descriptors derived from bv_map and the ROI
     int2* fused_desc;            // [bv_h][bv_w] single-resample variant (lazily built by lt_set_remap_mode)
     int remap_mode;              // 0 exact two-stage (default), 1 fused single resample
+    int frame_format;            // LT_FRAME_RGB (default) or LT_FRAME_NV12: layout of d_frames, read when a call is enqueued
     unsigned short* lab_gamma;   // [256]
     unsigned short* lab_cbrt;    // [3072]
     uint2* lab_yz;               // [3][256] Lab partial sums per channel value (lt_remap.cu)
@@ -169,12 +170,16 @@ int lt_launch_build_lab_yz(lt_handle* h, cudaStream_t st);
 int lt_launch_build_und_desc(lt_handle* h, cudaStream_t st);
 int lt_launch_build_fused_desc(lt_handle* h, cudaStream_t st);
 int lt_launch_warp_fused(lt_handle* h, const uint8_t* d_frames, uint8_t* d_bv_rgb, int n, cudaStream_t st);
-int lt_launch_undistort(lt_handle* h, const uint8_t* d_frames, int n, cudaStream_t st);
+int lt_launch_undistort(lt_handle* h, const uint8_t* d_frames, int n, cudaStream_t st);   // RGB or NV12 (h->frame_format)
 int lt_launch_warp(lt_handle* h, uint8_t* d_bv_rgb, int n, cudaStream_t st);
 int lt_launch_planes_from_bv(lt_handle* h, const uint8_t* d_bv_rgb, int n, cudaStream_t st);
 int lt_launch_overlay(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, const int* d_draw,
                       const int* ids, cudaStream_t st);
-int lt_launch_nv12_to_rgb(const uint8_t* d_nv12, uint8_t* d_rgb, int n, int w, int h, cudaStream_t st);
+// NV12 frames -> overlay-annotated RGB frames (every row of d_out written; d_out cannot alias d_frames)
+int lt_launch_overlay_nv12(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, const int* d_draw,
+                           const int* ids, cudaStream_t st);
+// rows [r0, r1) of NV12 frames -> RGB (nothing outside those rows is written)
+int lt_launch_nv12_to_rgb(const uint8_t* d_nv12, uint8_t* d_rgb, int n, int w, int h, int r0, int r1, cudaStream_t st);
 
 int lt_launch_filter(lt_handle* h, int n, const LtAttemptParams& p, const int* list, const int* count,
                      cudaStream_t st);

@@ -123,6 +123,23 @@ __device__ __forceinline__ Tap4 make_taps(int2 q) {
 }
 
 // ---------------------------------------------------------------------------
+// NV12 sampling: cv::cvtColor(COLOR_YUV2RGB_NV12) restated (SURVEY section 8 (f) #2: the reference gets RGB frames from
+// moviepy / ffmpeg, process_video.py:42-44; a hardware decoder delivers NV12).  ITU-R BT.601 limited range in Q20 fixed
+// point, one chroma sample per 2x2 block, no interpolation (oracle.cvops.yuv2rgb_nv12, pinned against cv2 in
+// tests/test_oracle_cvops.py).  Frame layout [img_h * 3 / 2][img_w]: luma plane, then rows of interleaved U, V pairs;
+// pixel (y, x) takes luma byte y * W + x and the pair at (H + (y >> 1)) * W + (x & ~1).
+// ---------------------------------------------------------------------------
+
+__device__ __forceinline__ uint32_t sat_q20(int v) { return (uint32_t)min(255, max(0, v >> 20)); }
+
+// one luma byte and one chroma pair (U in bits 0-7, V in bits 8-15; higher bits ignored) -> R | G << 8 | B << 16
+__device__ __forceinline__ uint32_t yuv_to_rgb(uint32_t luma, uint32_t uv) {
+    const int u = (int)(uv & 255u) - 128, v = (int)((uv >> 8) & 255u) - 128;
+    const int y = max(0, (int)luma - 16) * 1220542 + (1 << 19);
+    return sat_q20(y + 1673527 * v) | (sat_q20(y - 852492 * v - 409993 * u) << 8) | (sat_q20(y + 2116026 * u) << 16);
+}
+
+// ---------------------------------------------------------------------------
 // undistort: frame rows -> undistorted ROI rows [roi0, roi1), RGBX
 // ---------------------------------------------------------------------------
 
@@ -194,6 +211,27 @@ constexpr int UND_CH = UND_SPC / 4;
 constexpr int UND_MINB = 6;            // resident CTAs per SM the undistort is compiled for
 static_assert(UND_SPC == 4 || UND_SPC == 8 || UND_SPC == 16, "streams per CTA");
 
+// rotate the chunk slot with the pixel index: the 16-byte accesses of a quarter warp land in distinct banks
+__device__ __forceinline__ int und_slot(int px, int c) { return px * UND_CH + ((c + (px * UND_CH >> 3)) & (UND_CH - 1)); }
+
+// Second half of k_undistort_roi_nv12, as in k_undistort_roi (which keeps its own copy so that its code stays as
+// measured): the blended pixels of the CTA (tile, [pixel][chunk of four streams]) go to the
+// stream-minor und layout.  The UND_CH chunks of this CTA inside the pixel's 64 bytes: streams s0 .. s0 + UND_SPC - 1
+// of group s0 / NSW.
+__device__ __forceinline__ void und_store_tile(const uint4* tile, uint32_t* __restrict__ und, int p0, int roi_px, int s0,
+                                               const LtDims& d, size_t group_words) {
+    uint32_t* const base = und + (size_t)(s0 / NSW) * group_words + (s0 % NSW);
+#pragma unroll
+    for (int r = 0; r < UND_CH; ++r) {
+        const int e = r * 256 + threadIdx.x;           // (pixel, chunk) in output order
+        const int px = e / UND_CH, c = e % UND_CH, pp = p0 + px;
+        if (pp >= roi_px) break;
+        const int i = pp / d.img_w, j = pp - i * d.img_w;
+        uint4* out = reinterpret_cast<uint4*>(base + ((size_t)(i + 1) * (d.img_w + 1) + (j + 1)) * NSW);
+        out[c] = tile[und_slot(px, c)];
+    }
+}
+
 __global__ void __launch_bounds__(256, UND_MINB)
 k_undistort_roi(const uint8_t* __restrict__ frames, uint32_t* __restrict__ und, const int2* __restrict__ desc, LtDims d, int n,
                 size_t group_words) {
@@ -264,6 +302,78 @@ k_undistort_roi(const uint8_t* __restrict__ frames, uint32_t* __restrict__ und, 
     }
 }
 
+// k_undistort_roi of NV12 frames: same descriptor, blend and store; only the tap fetch differs.  The descriptor's byte
+// offset 3 (sy W + sx) gives the tap (sy, sx) back (sx = -1 when the left tap column lies outside the frame).  A tap
+// outside the frame is RGB 0 (BORDER_CONSTANT applies to the RGB image), not the conversion of YUV (0, 0, 0).
+// With all four taps inside, each needed byte or U,V pair comes from an aligned word of its own row (img_w % 4 == 0):
+// two luma words and two chroma words per tap row, all requested before the first conversion.  The 32 words of four
+// streams in flight need 64 registers: 4 resident CTAs per SM (at the 6 of k_undistort_roi they spill).
+constexpr int UND_NV12_MINB = 4;
+__global__ void __launch_bounds__(256, UND_NV12_MINB)
+k_undistort_roi_nv12(const uint8_t* __restrict__ frames, uint32_t* __restrict__ und, const int2* __restrict__ desc, LtDims d,
+                     int n, size_t group_words) {
+    __shared__ uint4 tile[256 * UND_CH];
+    const int p0 = blockIdx.x * blockDim.x, p = p0 + threadIdx.x;
+    const int roi_px = (d.roi1 - d.roi0) * d.img_w;
+    const int s0 = blockIdx.y * UND_SPC, ns = min(UND_SPC, n - s0);
+    if (p < roi_px) {
+        const int2 q = __ldg(&desc[p]);
+        const uint32_t f = (uint32_t)q.y;
+        uint32_t wA, wB;
+        blend_weights(f, wA, wB);
+        const uint32_t m = (f >> 10) & 15u;
+        const int W = d.img_w, H = d.img_h;
+        const size_t frame_bytes = (size_t)W * (H + H / 2);
+        const int lo = (m & 5u) ? 0 : 1;                 // left tap column outside the frame: sx = -1
+        const int t = q.x / 3 + lo + W;                  // (sy + 1) W + sx + lo >= 0
+        const int sy = t / W - 1, sx = t - (sy + 1) * W - lo;
+        const int ly = sy * W, cy0 = (H + (sy >> 1)) * W, cy1 = (H + ((sy + 1) >> 1)) * W;     // luma row, chroma rows
+        const int xa = sx, xb = sx + 1, ca = sx & ~1, cb = (sx + 1) & ~1;
+#pragma unroll
+        for (int c = 0; c < UND_CH; ++c) {
+            uint32_t o[4] = {0u, 0u, 0u, 0u};
+            if (4 * c < ns) {
+                if (m == 15u) {
+                    const int sa = 8 * (xa & 3), sb = 8 * (xb & 3), ua = 8 * (ca & 2), ub = 8 * (cb & 2);
+                    uint32_t y[4][4], uv[4][4];          // [stream][tap], taps 00 01 10 11
+#pragma unroll
+                    for (int k = 0; k < 4; ++k) {
+                        if (4 * c + k >= ns) break;
+                        const uint32_t* w = reinterpret_cast<const uint32_t*>(frames + (size_t)(s0 + 4 * c + k) * frame_bytes);
+                        y[k][0] = __ldg(w + ((ly + xa) >> 2));     y[k][1] = __ldg(w + ((ly + xb) >> 2));
+                        y[k][2] = __ldg(w + ((ly + W + xa) >> 2)); y[k][3] = __ldg(w + ((ly + W + xb) >> 2));
+                        uv[k][0] = __ldg(w + ((cy0 + ca) >> 2));   uv[k][1] = __ldg(w + ((cy0 + cb) >> 2));
+                        uv[k][2] = __ldg(w + ((cy1 + ca) >> 2));   uv[k][3] = __ldg(w + ((cy1 + cb) >> 2));
+                    }
+#pragma unroll
+                    for (int k = 0; k < 4; ++k) {
+                        if (4 * c + k >= ns) break;
+                        o[k] = blend_taps(yuv_to_rgb((y[k][0] >> sa) & 255u, uv[k][0] >> ua),
+                                          yuv_to_rgb((y[k][1] >> sb) & 255u, uv[k][1] >> ub),
+                                          yuv_to_rgb((y[k][2] >> sa) & 255u, uv[k][2] >> ua),
+                                          yuv_to_rgb((y[k][3] >> sb) & 255u, uv[k][3] >> ub), wA, wB);
+                    }
+                } else if (m) {
+#pragma unroll 1
+                    for (int k = 0; k < 4; ++k) {
+                        if (4 * c + k >= ns) break;
+                        const uint8_t* img = frames + (size_t)(s0 + 4 * c + k) * frame_bytes;
+                        auto tap = [&](uint32_t bit, int lrow, int crow, int x, int cx) -> uint32_t {     // BORDER_CONSTANT 0
+                            if (!(m & bit)) return 0u;
+                            return yuv_to_rgb(__ldg(img + lrow + x), __ldg(reinterpret_cast<const unsigned short*>(img + crow + cx)));
+                        };
+                        o[k] = blend_taps(tap(1u, ly, cy0, xa, ca), tap(2u, ly, cy0, xb, cb), tap(4u, ly + W, cy1, xa, ca),
+                                          tap(8u, ly + W, cy1, xb, cb), wA, wB);
+                    }
+                }
+            }
+            tile[und_slot(threadIdx.x, c)] = make_uint4(o[0], o[1], o[2], o[3]);
+        }
+    }
+    __syncthreads();
+    und_store_tile(tile, und, p0, roi_px, s0, d, group_words);
+}
+
 // cv2.warpPerspective(img, M, warped_size) of the RAW frame (lane_tracker.py:1035, the split view's middle panel)
 __global__ void __launch_bounds__(256)
 k_warp_frame(const uint8_t* __restrict__ frames, uint8_t* __restrict__ bv_rgb, const int2* __restrict__ map, LtDims d) {
@@ -288,7 +398,10 @@ int lt_launch_undistort(lt_handle* h, const uint8_t* d_frames, int n, cudaStream
     const LtDims& d = h->d;
     dim3 g(lt_div_up((d.roi1 - d.roi0) * d.img_w, 256), lt_div_up(n, UND_SPC));
     // the word loads of the fast path need 4-byte aligned rows: the frames are (lt_api.cu) and img_w % 4 == 0 (lt_create)
-    k_undistort_roi<<<g, 256, 0, st>>>(d_frames, h->und_roi, h->und_desc, d, n, lt_und_group_words(d));
+    if (h->frame_format == LT_FRAME_NV12)
+        k_undistort_roi_nv12<<<g, 256, 0, st>>>(d_frames, h->und_roi, h->und_desc, d, n, lt_und_group_words(d));
+    else
+        k_undistort_roi<<<g, 256, 0, st>>>(d_frames, h->und_roi, h->und_desc, d, n, lt_und_group_words(d));
     LT_LAUNCH_CHECK();
     return 0;
 }
@@ -661,6 +774,50 @@ __device__ __forceinline__ int lane_tap(const int2* __restrict__ rows, const LtD
     return (x >= r.x && x <= r.y) ? 255 : 0;
 }
 
+// Lane overlay of four pixels of frame row y, columns 4q .. 4q + 3, held as three RGB words (12 bytes): only G changes.
+// The same steps as k_overlay, which keeps its own copy so that its code stays as measured.
+__device__ __forceinline__ void overlay_words(uint32_t& w0, uint32_t& w1, uint32_t& w2, const int2* __restrict__ map,
+                                              const int2* __restrict__ lane_rows, const int4* __restrict__ lane_bbox,
+                                              const int* __restrict__ draw, const LtDims& d, int y, int q, int s,
+                                              const int* __restrict__ ids) {
+    if (draw[s] && y >= d.ov0 && y < d.ov1) {
+        // Q5 canvas coordinates of the four pixels; most of them cannot reach the polygon: one test against its
+        // bounding box (taps of a pixel: columns sx, sx + 1, rows sy, sy + 1) skips the span look-ups
+        const int4* mp = reinterpret_cast<const int4*>(map + (size_t)y * d.img_w + q * 4);
+        const int4 m01 = __ldg(mp), m23 = __ldg(mp + 1);
+        const int sid = ids ? __ldg(&ids[s]) : s;        // the cached polygon belongs to the stream, not the position
+        const int4 bb = __ldg(&lane_bbox[sid]);
+        const int qx[4] = {m01.x, m01.z, m23.x, m23.z}, qy[4] = {m01.y, m01.w, m23.y, m23.w};
+        const int sx_lo = min(min(qx[0], qx[1]), min(qx[2], qx[3])) >> 5, sx_hi = max(max(qx[0], qx[1]), max(qx[2], qx[3])) >> 5;
+        const int sy_lo = min(min(qy[0], qy[1]), min(qy[2], qy[3])) >> 5, sy_hi = max(max(qy[0], qy[1]), max(qy[2], qy[3])) >> 5;
+        if (sx_hi + 1 >= bb.x && sx_lo <= bb.y && sy_hi + 1 >= bb.z && sy_lo <= bb.w) {
+            const int2* rows = lane_rows + (size_t)sid * d.bv_h;
+            uint32_t gch[4] = {(w0 >> 8) & 255, w1 & 255, (w1 >> 24) & 255, (w2 >> 16) & 255};
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                Tap4 t = make_taps(make_int2(qx[k], qy[k]));
+                // the two taps of a canvas row share its [lo, hi] span: two span loads instead of four
+                const int2 none = make_int2(1, 0);
+                const int2 s0 = ((unsigned)t.sy < (unsigned)d.bv_h) ? __ldg(&rows[t.sy]) : none;
+                const int2 s1 = ((unsigned)(t.sy + 1) < (unsigned)d.bv_h) ? __ldg(&rows[t.sy + 1]) : none;
+                const int xa = t.sx, xb = t.sx + 1;
+                const bool ina = (unsigned)xa < (unsigned)d.bv_w, inb = (unsigned)xb < (unsigned)d.bv_w;
+                int v = ((ina && xa >= s0.x && xa <= s0.y) ? t.w00 : 0) + ((inb && xb >= s0.x && xb <= s0.y) ? t.w01 : 0) +
+                        ((ina && xa >= s1.x && xa <= s1.y) ? t.w10 : 0) + ((inb && xb >= s1.x && xb <= s1.y) ? t.w11 : 0);
+                v = (v * 255 + 512) >> 10;
+                if (v) {
+                    // cv2.addWeighted(img,1,lane,0.3,0): float32 a + b*0.3f, round half to even, saturate
+                    float f = __fadd_rn((float)gch[k], __fmul_rn((float)v, 0.3f));
+                    gch[k] = (uint32_t)min(255, __float2int_rn(f));
+                }
+            }
+            w0 = (w0 & 0xFFFF00FFu) | (gch[0] << 8);
+            w1 = (w1 & 0x00FFFF00u) | gch[1] | (gch[2] << 24);
+            w2 = (w2 & 0xFF00FFFFu) | (gch[3] << 16);
+        }
+    }
+}
+
 __global__ void __launch_bounds__(256)
 k_overlay(const uint8_t* frames, uint8_t* out, const int2* __restrict__ map,
           const int2* __restrict__ lane_rows, const int4* __restrict__ lane_bbox, const int* __restrict__ draw, LtDims d, int row0,
@@ -711,6 +868,28 @@ k_overlay(const uint8_t* frames, uint8_t* out, const int2* __restrict__ map,
         }
     }
     uint32_t* dst = reinterpret_cast<uint32_t*>(out + base);
+    dst[0] = w0; dst[1] = w1; dst[2] = w2;
+}
+
+
+// k_overlay of NV12 frames: one thread converts 4 pixels (one luma word, one chroma word = two U,V pairs) to the three
+// RGB words k_overlay reads, blends them the same way and writes them to the RGB output (which cannot alias the input).
+__global__ void __launch_bounds__(256)
+k_overlay_nv12(const uint8_t* __restrict__ frames, uint8_t* __restrict__ out, const int2* __restrict__ map,
+               const int2* __restrict__ lane_rows, const int4* __restrict__ lane_bbox, const int* __restrict__ draw, LtDims d,
+               int row0, const int* __restrict__ ids) {
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    const int y = row0 + blockIdx.y, s = blockIdx.z;
+    if (q >= (d.img_w >> 2)) return;
+    const uint8_t* f = frames + (size_t)s * d.img_w * (d.img_h + d.img_h / 2);
+    const uint32_t luma = __ldg(reinterpret_cast<const uint32_t*>(f + (size_t)y * d.img_w) + q);
+    const uint32_t uv = __ldg(reinterpret_cast<const uint32_t*>(f + (size_t)(d.img_h + (y >> 1)) * d.img_w) + q);
+    uint32_t px[4];
+#pragma unroll
+    for (int i = 0; i < 4; ++i) px[i] = yuv_to_rgb((luma >> (8 * i)) & 255u, uv >> (16 * (i >> 1)));
+    uint32_t w0 = px[0] | (px[1] << 24), w1 = (px[1] >> 8) | (px[2] << 16), w2 = (px[2] >> 16) | (px[3] << 8);
+    overlay_words(w0, w1, w2, map, lane_rows, lane_bbox, draw, d, y, q, s, ids);
+    uint32_t* dst = reinterpret_cast<uint32_t*>(out + (((size_t)s * d.img_h + y) * d.img_w + (size_t)q * 4) * 3);
     dst[0] = w0; dst[1] = w1; dst[2] = w2;
 }
 
@@ -776,52 +955,56 @@ int lt_launch_overlay(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int
 }
 
 // ---------------------------------------------------------------------------
-// Decoder output -> RGB frames (SURVEY section 8 (f) #2: the reference gets RGB frames from moviepy / ffmpeg,
-// process_video.py:42-44; a hardware decoder delivers NV12).  cv::cvtColor(COLOR_YUV2RGB_NV12) restated: ITU-R BT.601
-// limited range in Q20 fixed point, one chroma sample per 2x2 block, no interpolation (oracle.cvops.yuv2rgb_nv12,
-// pinned against cv2 in tests/test_oracle_cvops.py).  HBM-bound: 1.5 bytes in, 3 bytes out per pixel.
-// One thread = 4 x 2 pixels: two aligned luma words, one chroma word (two U,V pairs), six RGB words out.
+// Decoder output -> RGB frames (lt_nv12_to_rgb), and the rows of an NV12 frame that the lane overlay cannot reach.
+// HBM-bound: 1.5 bytes in, 3 bytes out per pixel.  One thread = 4 x 2 pixels: two aligned luma words, one chroma word
+// (two U,V pairs), six RGB words out.  Only rows [r0, r1) are written: a row range may start or end in the middle of
+// a chroma row pair, and the rows outside it belong to another kernel.
 // ---------------------------------------------------------------------------
 
-__device__ __forceinline__ uint32_t sat_q20(int v) { return (uint32_t)min(255, max(0, v >> 20)); }
-
 __global__ void __launch_bounds__(256)
-k_nv12_to_rgb(const uint8_t* __restrict__ nv12, uint8_t* __restrict__ rgb, int w, int h) {
+k_nv12_to_rgb(const uint8_t* __restrict__ nv12, uint8_t* __restrict__ rgb, int w, int h, int r0, int r1) {
     const int qx = blockIdx.x * blockDim.x + threadIdx.x;            // group of four columns
-    const int yp = blockIdx.y, s = blockIdx.z;                         // row pair
+    const int yp = (r0 >> 1) + blockIdx.y, s = blockIdx.z;             // row pair
     if (qx * 4 >= w) return;
     const uint8_t* f = nv12 + (size_t)s * w * (h + h / 2);
     const uint32_t y0 = __ldg(reinterpret_cast<const uint32_t*>(f + (size_t)(2 * yp) * w) + qx);
     const uint32_t y1 = __ldg(reinterpret_cast<const uint32_t*>(f + (size_t)(2 * yp + 1) * w) + qx);
     const uint32_t uv = __ldg(reinterpret_cast<const uint32_t*>(f + (size_t)(h + yp) * w) + qx);   // U0 V0 U1 V1
-    int ruv[2], guv[2], buv[2];
-#pragma unroll
-    for (int c = 0; c < 2; ++c) {
-        const int u = (int)((uv >> (16 * c)) & 255u) - 128, v = (int)((uv >> (16 * c + 8)) & 255u) - 128;
-        ruv[c] = (1 << 19) + 1673527 * v;
-        guv[c] = (1 << 19) - 852492 * v - 409993 * u;
-        buv[c] = (1 << 19) + 2116026 * u;
-    }
 #pragma unroll
     for (int r = 0; r < 2; ++r) {
+        const int row = 2 * yp + r;
+        if (row < r0 || row >= r1) continue;
         const uint32_t yy = r ? y1 : y0;
         uint32_t px[4];                                                // R | G << 8 | B << 16
 #pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            const int y = max(0, (int)((yy >> (8 * i)) & 255u) - 16) * 1220542;
-            const int c = i >> 1;
-            px[i] = sat_q20(y + ruv[c]) | (sat_q20(y + guv[c]) << 8) | (sat_q20(y + buv[c]) << 16);
-        }
-        uint32_t* o = reinterpret_cast<uint32_t*>(rgb + (((size_t)s * h + 2 * yp + r) * w + (size_t)qx * 4) * 3);
+        for (int i = 0; i < 4; ++i) px[i] = yuv_to_rgb((yy >> (8 * i)) & 255u, uv >> (16 * (i >> 1)));
+        uint32_t* o = reinterpret_cast<uint32_t*>(rgb + (((size_t)s * h + row) * w + (size_t)qx * 4) * 3);
         o[0] = px[0] | (px[1] << 24);
         o[1] = (px[1] >> 8) | (px[2] << 16);
         o[2] = (px[2] >> 16) | (px[3] << 8);
     }
 }
 
-int lt_launch_nv12_to_rgb(const uint8_t* d_nv12, uint8_t* d_rgb, int n, int w, int h, cudaStream_t st) {
-    dim3 g(lt_div_up(w / 4, 256), h / 2, n);
-    k_nv12_to_rgb<<<g, 256, 0, st>>>(d_nv12, d_rgb, w, h);
+int lt_launch_nv12_to_rgb(const uint8_t* d_nv12, uint8_t* d_rgb, int n, int w, int h, int r0, int r1, cudaStream_t st) {
+    if (r1 <= r0) return 0;
+    dim3 g(lt_div_up(w / 4, 256), (r1 + 1) / 2 - r0 / 2, n);
+    k_nv12_to_rgb<<<g, 256, 0, st>>>(d_nv12, d_rgb, w, h, r0, r1);
     LT_LAUNCH_CHECK();
+    return 0;
+}
+
+// The annotated RGB frames of NV12 input: k_overlay_nv12 on the rows the overlay can reach, the converter on the others.
+int lt_launch_overlay_nv12(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, const int* d_draw,
+                           const int* ids, cudaStream_t st) {
+    const LtDims& d = h->d;
+    int r0 = d.ov0, r1 = d.ov1, rc;
+    if (r0 >= r1) { r0 = 0; r1 = 0; }
+    if ((rc = lt_launch_nv12_to_rgb(d_frames, d_out, n, d.img_w, d.img_h, 0, r0, st))) return rc;
+    if ((rc = lt_launch_nv12_to_rgb(d_frames, d_out, n, d.img_w, d.img_h, r1 > r0 ? r1 : 0, d.img_h, st))) return rc;
+    if (r1 > r0) {
+        dim3 g(lt_div_up(d.img_w / 4, 256), r1 - r0, n);
+        k_overlay_nv12<<<g, 256, 0, st>>>(d_frames, d_out, h->ov_map, h->lane_rows, h->lane_bbox, d_draw, d, r0, ids);
+        LT_LAUNCH_CHECK();
+    }
     return 0;
 }

@@ -146,3 +146,24 @@ def _render_one(job):
     seed, n_frames, scale = job
     v = RoadVideo(seed, scale)
     return np.stack([v.frame(t) for t in range(n_frames)])
+
+
+def rgb_to_nv12(frames):
+    """RGB frames uint8 [..., H, W, 3] -> NV12 uint8 [..., H * 3 / 2, W] (H and W even): ITU-R BT.601 limited range,
+    each chroma sample the mean of its 2x2 block, rounded to nearest -- what a camera or a decoder delivers for road
+    video.  (The inverse, cv2.cvtColor(COLOR_YUV2RGB_NV12), is lossy: converting back does not give the input.)"""
+    rgb = np.asarray(frames)
+    if rgb.dtype != np.uint8 or rgb.ndim < 3 or rgb.shape[-1] != 3 or rgb.shape[-3] % 2 or rgb.shape[-2] % 2:
+        raise ValueError("rgb_to_nv12: expected uint8 [..., H, W, 3] with even H and W")
+    h, w = rgb.shape[-3], rgb.shape[-2]
+    lead = rgb.shape[:-3]
+    f = rgb.astype(np.float64)
+    r, g, b = f[..., 0], f[..., 1], f[..., 2]
+    y = 16 + (65.481 * r + 128.553 * g + 24.966 * b) / 255
+    cb = 128 + (-37.797 * r - 74.203 * g + 112.0 * b) / 255
+    cr = 128 + (112.0 * r - 93.786 * g - 18.214 * b) / 255
+    sub = lambda c: c.reshape(lead + (h // 2, 2, w // 2, 2)).mean(axis=(-3, -1))
+    out = np.empty(lead + (h * 3 // 2, w), dtype=np.uint8)
+    out[..., :h, :] = np.clip(np.rint(y), 0, 255)
+    out[..., h:, :] = np.clip(np.rint(np.stack([sub(cb), sub(cr)], axis=-1)), 0, 255).reshape(lead + (h // 2, w))
+    return out

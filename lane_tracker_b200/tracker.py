@@ -21,6 +21,10 @@ RESULT_DTYPE = np.dtype(lt_result)
 
 _FILTER_TYPES = {"bilateral": 0, "neighborhood": 1}
 
+# layouts of the input frames of the hot path (lt_set_frame_format)
+FRAME_RGB, FRAME_NV12 = 0, 1
+_FRAME_FORMATS = {"rgb": FRAME_RGB, "nv12": FRAME_NV12}
+
 # keyword defaults of the reference methods (SURVEY.md B.2)
 PROCESS_DEFAULTS = dict(
     ksize_r=15, C_r=8, ksize_b=35, C_b=5, filter_type="bilateral", mask_noise=False, noise_thresh=140,
@@ -123,6 +127,7 @@ class BatchedLaneTracker:
         with torch.cuda.device(self.device):
             check(self.lib.lt_create(C.byref(cfg), C.byref(h)))
         self._h = h
+        self._format_set = FRAME_RGB           # what the handle was last set to (lt_set_frame_format)
         S = self.n_streams
         self._results_dev = torch.zeros(S * RESULT_DTYPE.itemsize, dtype=torch.uint8, device=self.device)
         self._results_host = torch.zeros(S * RESULT_DTYPE.itemsize, dtype=torch.uint8).pin_memory()
@@ -196,8 +201,10 @@ class BatchedLaneTracker:
 
     def copy_rows(self, dst, src, row0, row1, to_device):
         """Copy frame rows [row0, row1) of a batch of full frames between pinned host and device tensors on the
-        current stream (strided 2-D copy, no staging)."""
+        current stream (strided 2-D copy, no staging).  NV12 batches ([n, H * 3 / 2, W]) move luma rows [row0, row1)
+        and the chroma rows that cover them."""
         n = int(src.shape[0])
+        self._use_format(FRAME_NV12 if src.dim() == 3 else FRAME_RGB)
         check(self.lib.lt_memcpy_rows(self._h, _ptr(dst), _ptr(src), n, int(row0), int(row1), int(bool(to_device)),
                                       _stream_ptr(self.device)))
 
@@ -244,6 +251,37 @@ class BatchedLaneTracker:
         return {self.lib.lt_stage_name(i).decode(): float(ms[i]) for i in range(1, _lib.LT_NSTAGES)}, calls.value
 
     # -- hot path -----------------------------------------------------------
+    def _frame_format(self, frames):
+        """-> (n, format) of an input batch: uint8 [n, H, W, 3] is RGB, uint8 [n, H * 3 / 2, W] is NV12."""
+        w, h = self.img_size
+        if not (isinstance(frames, torch.Tensor) and frames.dtype == torch.uint8):
+            raise ValueError("frames must be a uint8 tensor")
+        if frames.dim() == 4 and tuple(frames.shape[1:]) == (h, w, 3):
+            fmt = FRAME_RGB
+        elif frames.dim() == 3 and tuple(frames.shape[1:]) == (h * 3 // 2, w) and h % 2 == 0:
+            fmt = FRAME_NV12
+        else:
+            raise ValueError("frames must be RGB [n, %d, %d, 3] or NV12 [n, %d, %d], got %s"
+                             % (h, w, h * 3 // 2, w, list(frames.shape)))
+        if not (frames.is_cuda and frames.is_contiguous()):
+            raise ValueError("frames must be a contiguous CUDA tensor")
+        if frames.data_ptr() % 4:
+            raise ValueError("frames must start at a 4-byte aligned address (the kernels access frames as 32-bit words)")
+        if frames.shape[0] < 1 or frames.shape[0] > self.n_streams:
+            raise ValueError("got %d frames for %d streams" % (frames.shape[0], self.n_streams))
+        return int(frames.shape[0]), fmt
+
+    def _use_format(self, fmt):
+        if fmt != self._format_set:
+            check(self.lib.lt_set_frame_format(self._h, int(fmt)))
+            self._format_set = fmt
+
+    def _input(self, frames):
+        """Check an input batch of RGB or NV12 frames and set the handle's frame format to it; -> n."""
+        n, fmt = self._frame_format(frames)
+        self._use_format(fmt)
+        return n
+
     def _check_frames(self, frames):
         w, h = self.img_size
         if not (isinstance(frames, torch.Tensor) and frames.is_cuda and frames.dtype == torch.uint8 and
@@ -277,24 +315,28 @@ class BatchedLaneTracker:
             raise ValueError("stream id %d appears more than once in the batch" % int(u[counts > 1][0]))
         return (C.c_int32 * n)(*[int(v) for v in a])
 
-    @staticmethod
-    def _check_out(out, frames):
+    def _check_out(self, out, frames):
+        """out: RGB [n, H, W, 3] for RGB and NV12 frames alike."""
         if out is None:
             return
-        if out.shape != frames.shape or out.dtype != torch.uint8 or not out.is_cuda or not out.is_contiguous():
-            raise ValueError("out must match frames")
+        w, h = self.img_size
+        if (tuple(out.shape) != (int(frames.shape[0]), h, w, 3) or out.dtype != torch.uint8 or not out.is_cuda or
+                not out.is_contiguous()):
+            raise ValueError("out must be a contiguous CUDA uint8 tensor [n, %d, %d, 3] for n frames" % (h, w))
         if out.data_ptr() % 4:
             raise ValueError("out must start at a 4-byte aligned address (the kernels access frames as 32-bit words)")
 
     def process_async(self, frames, out=None, params=None, results_dev=None, ids=None, **kw):
         """Enqueue one frame per stream on the current CUDA stream; returns the number of frames.
 
-        frames: uint8 CUDA tensor [n, H, W, 3] (RGB).  out: same shape or None (fits-only mode).
+        frames: uint8 CUDA tensor [n, H, W, 3] (RGB) or [n, H * 3 / 2, W] (NV12: the luma plane, then interleaved
+        U, V rows, as video decoders deliver it; same results as RGB frames converted by ``nv12_to_rgb``).
+        out: RGB [n, H, W, 3] or None (fits-only mode); for NV12 frames it is a separate buffer.
         results_dev: optional uint8 CUDA buffer of n * RESULT_DTYPE.itemsize bytes (default: internal).
         ids: None -- frame i belongs to stream i; else n distinct stream ids in [0, n_streams), any order (int
         sequence, NumPy array or CPU tensor): frame i belongs to stream ids[i], and the streams not listed keep their
         state.  out and the result records stay in batch order."""
-        n = self._check_frames(frames)
+        n = self._input(frames)
         self._check_out(out, frames)
         h_ids = self._check_ids(ids, n)
         p = params if params is not None else make_params(**kw)
@@ -311,8 +353,8 @@ class BatchedLaneTracker:
 
     def process_front_async(self, frames, buffer_set, params=None, **kw):
         """First half of ``process_async`` (undistort, warp, first-attempt filter) into intermediate buffer set
-        0 or 1, on the current CUDA stream.  Stateless.  See ``DevicePipeline``."""
-        n = self._check_frames(frames)
+        0 or 1, on the current CUDA stream.  Stateless.  See ``DevicePipeline``.  RGB or NV12 frames."""
+        n = self._input(frames)
         p = params if params is not None else make_params(**kw)
         check(self.lib.lt_process_front(self._h, _ptr(frames), n, C.byref(p), int(buffer_set), _stream_ptr(self.device)))
         return n
@@ -320,8 +362,8 @@ class BatchedLaneTracker:
     def process_back_async(self, frames, out, buffer_set, params=None, results_dev=None, ids=None, **kw):
         """Second half of ``process_async`` (searches, second attempt, state machine, overlay) from intermediate
         buffer set 0 or 1, on the current CUDA stream.  Advances the per-stream state of the streams in ``ids``
-        (None: streams 0..n-1), as ``process_async``."""
-        n = self._check_frames(frames)
+        (None: streams 0..n-1), as ``process_async``.  RGB or NV12 frames, as given to the front half."""
+        n = self._input(frames)
         self._check_out(out, frames)
         h_ids = self._check_ids(ids, n)
         p = params if params is not None else make_params(**kw)
@@ -352,7 +394,8 @@ class BatchedLaneTracker:
 
     # -- stage methods (device tensors) ---------------------------------------
     def remap(self, frames, want_bv=True):
-        n = self._check_frames(frames)
+        """Undistort + warp of RGB or NV12 frames -> bird's-eye RGB [n, bv_h, bv_w, 3] (None without want_bv)."""
+        n = self._input(frames)
         bw, bh = self.warped_size
         bv = torch.empty((n, bh, bw, 3), dtype=torch.uint8, device=self.device) if want_bv else None
         check(self.lib.lt_remap(self._h, _ptr(frames), _ptr(bv), n, _stream_ptr(self.device)))
@@ -616,14 +659,18 @@ class GraphedProcess:
         g.frames.copy_(batch, non_blocking=True); g.replay(); results = g.fetch_results()
     """
 
-    def __init__(self, tracker, n=None, overlay=True, params=None):
+    def __init__(self, tracker, n=None, overlay=True, params=None, frame_format="rgb"):
+        """frame_format 'nv12': ``self.frames`` is NV12 [n, H * 3 / 2, W]; ``self.out`` stays RGB."""
+        if frame_format not in _FRAME_FORMATS:
+            raise ValueError("frame_format must be 'rgb' or 'nv12'")
         self.t = tracker
         n = tracker.n_streams if n is None else int(n)
         dev = tracker.device
         w, h = tracker.img_size
         self.n = n
-        self.frames = torch.zeros((n, h, w, 3), dtype=torch.uint8, device=dev)
-        self.out = torch.empty_like(self.frames) if overlay else None
+        shape = (n, h * 3 // 2, w) if frame_format == "nv12" else (n, h, w, 3)
+        self.frames = torch.zeros(shape, dtype=torch.uint8, device=dev)
+        self.out = torch.empty((n, h, w, 3), dtype=torch.uint8, device=dev) if overlay else None
         self.results_dev = torch.zeros(n * RESULT_DTYPE.itemsize, dtype=torch.uint8, device=dev)
         self.params = params if params is not None else make_params()
         # first-use initialisation (module load, shared-memory attributes) cannot happen inside a capture: run the
@@ -665,7 +712,7 @@ class DevicePipeline:
         pipe.join()                            # the current stream waits for everything submitted
 
     ``submit(frames, out, ids=...)`` advances the listed streams only (see ``BatchedLaneTracker.process_async``);
-    results stay in batch order.
+    results stay in batch order.  ``frames`` may be RGB or NV12 (``out`` is RGB either way), batch by batch.
     """
 
     def __init__(self, tracker, params=None):
@@ -682,7 +729,7 @@ class DevicePipeline:
 
     def submit(self, frames, out=None, ids=None):
         dev = self.t.device
-        self.t._check_ids(ids, self.t._check_frames(frames))      # refuse bad ids before anything is enqueued
+        self.t._check_ids(ids, self.t._frame_format(frames)[0])   # refuse bad frames / ids before anything is enqueued
         k, bs = self._k, self._k & 1
         ready = torch.cuda.Event()
         ready.record(torch.cuda.current_stream(dev))            # frames (and out) belong to the caller until here
@@ -748,22 +795,34 @@ class HostPipeline:
     frames and records of a finished batch are in batch order.
     """
 
-    def __init__(self, tracker, depth=3, overlay=True, params=None, inplace=False):
+    def __init__(self, tracker, depth=3, overlay=True, params=None, inplace=False, frame_format="rgb"):
         """inplace=True: annotate the caller's pinned frames in place.  Only the frame rows the tracker reads
         (geometry['source_rows'] + overlay rows) go host->device and only the rows the overlay can change
         (geometry['overlay_rows']) come back, written into the submitted tensor; every other row of the frame is
         already identical to the annotated frame, so the host ends up with the same image as overlay mode while
-        about a third of the bytes cross PCIe."""
+        about a third of the bytes cross PCIe.
+
+        frame_format='nv12': submitted batches are pinned NV12 [n, H * 3 / 2, W], as video decoders deliver them.
+        With overlay=True whole NV12 frames go host->device and whole annotated RGB frames come back; with
+        overlay=False only the rows the tracker reads (geometry['source_rows']) and the chroma rows that cover them
+        go host->device.  inplace is RGB only (an RGB annotation cannot be written into NV12 frames)."""
+        if frame_format not in _FRAME_FORMATS:
+            raise ValueError("frame_format must be 'rgb' or 'nv12'")
         self.t = tracker
         self.depth = int(depth)
         self.overlay = overlay
         self.inplace = bool(inplace)
+        self.nv12 = frame_format == "nv12"
         if self.inplace and not overlay:
             raise ValueError('inplace needs overlay=True')
+        if self.inplace and self.nv12:
+            raise ValueError("inplace annotation needs RGB frames: NV12 frames are annotated into separate RGB frames")
         g = tracker.geometry
         h_img = tracker.img_size[1]     # +-2 rows of slack: the fused remap variant samples the raw frame directly
         self.rows_in = (max(0, min(g['source_rows'][0], g['overlay_rows'][0]) - 2),
                         min(h_img, max(g['source_rows'][1], g['overlay_rows'][1]) + 2))
+        if self.nv12:       # the fused variant refuses NV12: the undistort reads exactly the source rows
+            self.rows_in = tuple(g['source_rows'])
         self.rows_out = g['overlay_rows']
         self.rows_text = tracker.text_rows if tracker.text_enabled else (0, 0)   # putText rows: read and rewritten
         self.params = params if params is not None else make_params()
@@ -778,7 +837,7 @@ class HostPipeline:
         self.slots = []
         for _ in range(self.depth):
             self.slots.append(dict(
-                d_in=torch.empty((S, h, w, 3), dtype=torch.uint8, device=dev),
+                d_in=torch.empty((S, h * 3 // 2, w) if self.nv12 else (S, h, w, 3), dtype=torch.uint8, device=dev),
                 d_out=torch.empty((S, h, w, 3), dtype=torch.uint8, device=dev) if (overlay and not inplace) else None,
                 d_res=torch.zeros(S * RESULT_DTYPE.itemsize, dtype=torch.uint8, device=dev),
                 h_out=torch.empty((S, h, w, 3), dtype=torch.uint8).pin_memory() if (overlay and not inplace) else None,
@@ -795,6 +854,10 @@ class HostPipeline:
             raise ValueError("host_frames must be a contiguous pinned uint8 tensor")
         sl = self.slots[self.head]
         n = int(host_frames.shape[0])
+        if host_frames.shape[1:] != sl["d_in"].shape[1:] or not 1 <= n <= self.t.n_streams:
+            raise ValueError("host_frames must be %s [n, %s] with 1 <= n <= %d, got %s"
+                             % ("NV12" if self.nv12 else "RGB", ", ".join(map(str, sl["d_in"].shape[1:])),
+                                self.t.n_streams, list(host_frames.shape)))
         self.t._check_ids(ids, n)                        # refuse bad ids before anything is enqueued
         sl["n"] = n
         with torch.cuda.stream(self.s_in):
@@ -805,6 +868,8 @@ class HostPipeline:
                 for ta, tb in _rows_minus(self.rows_text, (a, b)):      # text rows outside the rows already sent
                     self.t.copy_rows(sl["d_in"], host_frames, ta, tb, True)
                 sl["frames"] = host_frames
+            elif self.nv12 and not self.overlay:
+                self.t.copy_rows(sl["d_in"], host_frames, self.rows_in[0], self.rows_in[1], True)
             else:
                 sl["d_in"][:n].copy_(host_frames, non_blocking=True)
             sl["e_in"].record(self.s_in)
