@@ -137,8 +137,8 @@ extern "C" int lt_destroy(lt_handle* h) {
                       f.merged, f.mask};
         for (void* p : fp) if (p) cudaFree(p);
     }
-    void* ptrs[] = {h->und_map, h->bv_map, h->ov_map, h->bv_desc, h->und_desc, h->lab_yz, h->fused_desc, h->lab_gamma, h->lab_cbrt, h->pixels, h->pix_counts, h->lane_rows, h->lane_bbox, h->dl_bbox,
-                    h->avg_x, h->state, h->att, h->retry_list, h->retry_count, h->draw_flags, h->stream_ids, h->scratch_bv, h->vis_scratch,
+    void* ptrs[] = {h->und_map, h->bv_map, h->ov_map, h->bv_desc, h->und_desc, h->lab_yz, h->fused_desc, h->lab_gamma, h->lab_cbrt, h->lane_rows, h->lane_bbox, h->dl_bbox,
+                    h->avg_x, h->state, h->att, h->retry_list, h->retry_count, h->draw_flags, h->stream_ids, h->vis_scratch,
                     h->cap_pixels, h->cap_counts, h->cap_cents, h->cap_ncents, h->dl_rows, h->dl_flags, h->txt_state, h->txt_flags,
                     h->txt_tables, h->txt_char_start, h->txt_dy, h->txt_dx, h->txt_lut, h->txt_advance, h->txt_pair_overlap,
                     h->txt_bitmaps};
@@ -177,12 +177,10 @@ static void select_set(lt_handle* h, int k) {
     const LtFrontSet& f = h->fs[k];
     const size_t origin = (size_t)LT_HALO_Y * h->d.pp + LT_HALO_X;
     h->und_roi = f.und_roi;
-    for (int i = 0; i < 6; ++i) h->pad_alloc[i] = f.pad_alloc[i];
     h->planeR = f.pad_alloc[0] + origin; h->planeB = f.pad_alloc[1] + origin;
     h->tmpR = f.pad_alloc[2] + origin;   h->tmpB = f.pad_alloc[3] + origin;
     h->topR = f.pad_alloc[4] + origin;   h->topB = f.pad_alloc[5] + origin;
     h->merged = f.merged; h->mask = f.mask;
-    h->cur_set = k;
 }
 
 extern "C" int lt_create(const lt_config* cfg, lt_handle** out) {
@@ -267,7 +265,6 @@ extern "C" int lt_create(const lt_config* cfg, lt_handle** out) {
     if (!rc) rc = lt_launch_build_lab_yz(h, st);
     if (!rc) rc = alloc_front_set(h, 0);
     if (!rc) select_set(h, 0);
-    A(pixels, S * 2 * (size_t)h->pix_cap); A(pix_counts, S * 2);
     A(lane_rows, S * (size_t)d.bv_h); A(lane_bbox, S); A(avg_x, S * 2 * (size_t)d.bv_h);
     A(state, S); A(att, 2 * S); A(retry_list, S); A(retry_count, 1); A(draw_flags, 2 * S); A(stream_ids, S);
 #undef A
@@ -373,7 +370,7 @@ static int upload_stream_ids(lt_handle* h, const int32_t* h_ids, int n, cudaStre
 // h_ids (host, validated by check_ids) maps batch position i to state slot h_ids[i]; NULL: the identity.
 static int process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, const lt_params* params,
                         const LtAttemptParams& p1, lt_result* d_results, cudaStream_t st, bool own_begin,
-                        const int32_t* h_ids = nullptr) {
+                        const int32_t* h_ids) {
     int rc;
     const LtAttemptParams p2 = second_attempt();
     const bool two = (params->n_tries >= 2) || (params->n_tries == -1);
@@ -487,35 +484,6 @@ static int process_args(lt_handle* h, const uint8_t* d_frames, int n, const lt_p
     return 0;
 }
 
-extern "C" int lt_process(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int32_t n, const lt_params* params,
-                          lt_result* d_results, void* stream) {
-    int rc;
-    LtAttemptParams p1;
-    if ((rc = check_out(h, d_frames, d_out, n))) return rc;
-    if ((rc = process_args(h, d_frames, n, params, 0, &p1))) return rc;
-    if (!d_results) { lt_set_error("null argument"); return -1; }
-    if ((rc = process_front(h, d_frames, n, p1, (cudaStream_t)stream))) return rc;
-    return process_back(h, d_frames, d_out, n, params, p1, d_results, (cudaStream_t)stream, false);
-}
-
-extern "C" int lt_process_front(lt_handle* h, const uint8_t* d_frames, int32_t n, const lt_params* params, int32_t set,
-                                void* stream) {
-    int rc;
-    LtAttemptParams p1;
-    if ((rc = process_args(h, d_frames, n, params, set, &p1))) return rc;
-    return process_front(h, d_frames, n, p1, (cudaStream_t)stream);
-}
-
-extern "C" int lt_process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int32_t n, const lt_params* params,
-                               int32_t set, lt_result* d_results, void* stream) {
-    int rc;
-    LtAttemptParams p1;
-    if ((rc = check_out(h, d_frames, d_out, n))) return rc;
-    if ((rc = process_args(h, d_frames, n, params, set, &p1))) return rc;
-    if (!d_results) { lt_set_error("null argument"); return -1; }
-    return process_back(h, d_frames, d_out, n, params, p1, d_results, (cudaStream_t)stream, true);
-}
-
 // Stream ids of lt_process_streams / lt_process_back_streams: 1 <= n <= S ids in [0, S), pairwise distinct (two
 // frames of one stream in a batch would race on its state).  Checked before anything is enqueued.
 static int check_ids(lt_handle* h, const int32_t* h_ids, int n) {
@@ -532,27 +500,47 @@ static int check_ids(lt_handle* h, const int32_t* h_ids, int n) {
     return 0;
 }
 
-extern "C" int lt_process_streams(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids, int32_t n,
-                                  const lt_params* params, lt_result* d_results, void* stream) {
+// What one process entry point does: the front half, the back half or both, with or without a stream id list.
+enum { PROC_FRONT = 1, PROC_BACK = 2, PROC_IDS = 4 };
+
+// The checks of the process entry points, in this order and all before anything is enqueued, then the halves.
+static int process_call(lt_handle* h, int what, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids, int n,
+                        const lt_params* params, int set, lt_result* d_results, void* stream) {
     int rc;
     LtAttemptParams p1;
-    if ((rc = check_ids(h, h_ids, n))) return rc;
-    if ((rc = check_out(h, d_frames, d_out, n))) return rc;
-    if ((rc = process_args(h, d_frames, n, params, 0, &p1))) return rc;
-    if (!d_results) { lt_set_error("null argument"); return -1; }
-    if ((rc = process_front(h, d_frames, n, p1, (cudaStream_t)stream))) return rc;
-    return process_back(h, d_frames, d_out, n, params, p1, d_results, (cudaStream_t)stream, false, h_ids);
+    const bool front = what & PROC_FRONT, back = what & PROC_BACK;
+    const cudaStream_t st = (cudaStream_t)stream;
+    if ((what & PROC_IDS) && (rc = check_ids(h, h_ids, n))) return rc;
+    if (back && (rc = check_out(h, d_frames, d_out, n))) return rc;
+    if ((rc = process_args(h, d_frames, n, params, set, &p1))) return rc;
+    if (back && !d_results) { lt_set_error("null argument"); return -1; }
+    if (front && (rc = process_front(h, d_frames, n, p1, st))) return rc;
+    return back ? process_back(h, d_frames, d_out, n, params, p1, d_results, st, !front, h_ids) : 0;
+}
+
+extern "C" int lt_process(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int32_t n, const lt_params* params,
+                          lt_result* d_results, void* stream) {
+    return process_call(h, PROC_FRONT | PROC_BACK, d_frames, d_out, nullptr, n, params, 0, d_results, stream);
+}
+
+extern "C" int lt_process_front(lt_handle* h, const uint8_t* d_frames, int32_t n, const lt_params* params, int32_t set,
+                                void* stream) {
+    return process_call(h, PROC_FRONT, d_frames, nullptr, nullptr, n, params, set, nullptr, stream);
+}
+
+extern "C" int lt_process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int32_t n, const lt_params* params,
+                               int32_t set, lt_result* d_results, void* stream) {
+    return process_call(h, PROC_BACK, d_frames, d_out, nullptr, n, params, set, d_results, stream);
+}
+
+extern "C" int lt_process_streams(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids, int32_t n,
+                                  const lt_params* params, lt_result* d_results, void* stream) {
+    return process_call(h, PROC_FRONT | PROC_BACK | PROC_IDS, d_frames, d_out, h_ids, n, params, 0, d_results, stream);
 }
 
 extern "C" int lt_process_back_streams(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids,
                                        int32_t n, const lt_params* params, int32_t set, lt_result* d_results, void* stream) {
-    int rc;
-    LtAttemptParams p1;
-    if ((rc = check_ids(h, h_ids, n))) return rc;
-    if ((rc = check_out(h, d_frames, d_out, n))) return rc;
-    if ((rc = process_args(h, d_frames, n, params, set, &p1))) return rc;
-    if (!d_results) { lt_set_error("null argument"); return -1; }
-    return process_back(h, d_frames, d_out, n, params, p1, d_results, (cudaStream_t)stream, true, h_ids);
+    return process_call(h, PROC_BACK | PROC_IDS, d_frames, d_out, h_ids, n, params, set, d_results, stream);
 }
 
 static const char* STAGE_NAMES[LT_NSTAGES] = {"begin", "undistort", "warp", "erode55", "erode29", "tophat55", "tophat29",

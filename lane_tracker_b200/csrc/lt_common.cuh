@@ -22,7 +22,7 @@ struct LtDims {
     int p2;        // pair-plane width in entries (multiple of 32)
     int mwords;    // mask words per row = 2*p2/32
     int roi0, roi1;   // undistorted rows materialised: [roi0, roi1)
-    int ov0, ov1;     // frame rows whose overlay taps can hit the bird's-eye view: [ov0, ov1)
+    int ov0, ov1;     // frame rows whose overlay taps can hit the bird's-eye view: [ov0, ov1), [0, 0) if none
     int pp;           // row pitch of the PADDED pair planes (morphology inputs) = p2 + 2*LT_HALO_X
 };
 
@@ -93,13 +93,9 @@ struct lt_handle {
     uint32_t* planeR; uint32_t* planeB;     // padded [S][bv_h + 2*LT_HALO_Y][pp]; lanes beyond the image / halo: 0xFFFF
     uint32_t* tmpR;   uint32_t* tmpB;       // padded eroded planes; lanes beyond the image / halo: 0
     uint32_t* topR;   uint32_t* topB;       // padded top-hat planes / box row sums; halo and pad rows: 0
-    uint32_t* pad_alloc[6];                 // the allocations behind the six padded planes
     LtFrontSet fs[2];                       // [0] always allocated, [1] on first use; the fields above mirror the selected one
-    int cur_set;
     uint32_t* merged; uint32_t* mask;       // [S][bv_h][mwords]
-    uint32_t* pixels;            // [S][2][pix_cap]
-    int pix_cap;
-    int* pix_counts;             // [S][2]
+    int pix_cap;                 // entries per stream and side of the captured pixel lists
     int2* lane_rows;             // [S][bv_h]
     int4* lane_bbox;             // [S] bounding box of the polygon rows: (min lo, max hi, first row, last row); empty: (W, -1, H, -1)
     int* avg_x;                  // [S][2][bv_h]   averaged polylines (state)
@@ -123,7 +119,6 @@ struct lt_handle {
     unsigned char* txt_pair_overlap;   // [nchars][nchars]: glyph b drawn right after glyph a shares pixels with it
     cudaEvent_t* prof_ev; int* prof_stage; int prof_cap, prof_n, prof_active, prof_calls, prof_max_calls;
     uint32_t prof_mask;          // 0: every stage boundary is marked; else only the boundaries whose bit is set
-    uint8_t* scratch_bv;         // lazily allocated [S][bv_h][bv_w][3] for stage calls
     unsigned char* vis_scratch;  // lazily allocated work area of lt_visualize_search
     cudaStream_t side;           // carries the horizontal threshold halves next to the vertical ones (lt_launch_filter)
     cudaEvent_t ev_fork, ev_join;

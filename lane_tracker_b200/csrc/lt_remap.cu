@@ -139,6 +139,17 @@ __device__ __forceinline__ uint32_t yuv_to_rgb(uint32_t luma, uint32_t uv) {
     return sat_q20(y + 1673527 * v) | (sat_q20(y - 852492 * v - 409993 * u) << 8) | (sat_q20(y + 2116026 * u) << 16);
 }
 
+// four pixels of one row: one aligned luma word and the chroma word under it (two U,V pairs) -> the three words of
+// their 12 RGB bytes
+__device__ __forceinline__ void nv12_to_rgb_words(uint32_t luma, uint32_t uv, uint32_t& w0, uint32_t& w1, uint32_t& w2) {
+    uint32_t px[4];                                                    // R | G << 8 | B << 16
+#pragma unroll
+    for (int i = 0; i < 4; ++i) px[i] = yuv_to_rgb((luma >> (8 * i)) & 255u, uv >> (16 * (i >> 1)));
+    w0 = px[0] | (px[1] << 24);
+    w1 = (px[1] >> 8) | (px[2] << 16);
+    w2 = (px[2] >> 16) | (px[3] << 8);
+}
+
 // ---------------------------------------------------------------------------
 // undistort: frame rows -> undistorted ROI rows [roi0, roi1), RGBX
 // ---------------------------------------------------------------------------
@@ -214,8 +225,7 @@ static_assert(UND_SPC == 4 || UND_SPC == 8 || UND_SPC == 16, "streams per CTA");
 // rotate the chunk slot with the pixel index: the 16-byte accesses of a quarter warp land in distinct banks
 __device__ __forceinline__ int und_slot(int px, int c) { return px * UND_CH + ((c + (px * UND_CH >> 3)) & (UND_CH - 1)); }
 
-// Second half of k_undistort_roi_nv12, as in k_undistort_roi (which keeps its own copy so that its code stays as
-// measured): the blended pixels of the CTA (tile, [pixel][chunk of four streams]) go to the
+// Second half of the undistort kernels: the blended pixels of the CTA (tile, [pixel][chunk of four streams]) go to the
 // stream-minor und layout.  The UND_CH chunks of this CTA inside the pixel's 64 bytes: streams s0 .. s0 + UND_SPC - 1
 // of group s0 / NSW.
 __device__ __forceinline__ void und_store_tile(const uint4* tile, uint32_t* __restrict__ und, int p0, int roi_px, int s0,
@@ -284,22 +294,11 @@ k_undistort_roi(const uint8_t* __restrict__ frames, uint32_t* __restrict__ und, 
                     }
                 }
             }
-            // rotate the chunk slot with the pixel index: the 16-byte accesses of a quarter warp land in distinct banks
-            tile[threadIdx.x * UND_CH + ((c + (threadIdx.x * UND_CH >> 3)) & (UND_CH - 1))] = make_uint4(o[0], o[1], o[2], o[3]);
+            tile[und_slot(threadIdx.x, c)] = make_uint4(o[0], o[1], o[2], o[3]);
         }
     }
     __syncthreads();
-    // the UND_CH chunks of this CTA inside the pixel's 64 bytes: streams s0 .. s0 + UND_SPC - 1 of group s0 / NSW
-    uint32_t* const base = und + (size_t)(s0 / NSW) * group_words + (s0 % NSW);
-#pragma unroll
-    for (int r = 0; r < UND_CH; ++r) {
-        const int e = r * 256 + threadIdx.x;           // (pixel, chunk) in output order
-        const int px = e / UND_CH, c = e % UND_CH, pp = p0 + px;
-        if (pp >= roi_px) break;
-        const int i = pp / d.img_w, j = pp - i * d.img_w;
-        uint4* out = reinterpret_cast<uint4*>(base + ((size_t)(i + 1) * (d.img_w + 1) + (j + 1)) * NSW);
-        out[c] = tile[px * UND_CH + ((c + (px * UND_CH >> 3)) & (UND_CH - 1))];
-    }
+    und_store_tile(tile, und, p0, roi_px, s0, d, group_words);
 }
 
 // k_undistort_roi of NV12 frames: same descriptor, blend and store; only the tap fetch differs.  The descriptor's byte
@@ -775,7 +774,6 @@ __device__ __forceinline__ int lane_tap(const int2* __restrict__ rows, const LtD
 }
 
 // Lane overlay of four pixels of frame row y, columns 4q .. 4q + 3, held as three RGB words (12 bytes): only G changes.
-// The same steps as k_overlay, which keeps its own copy so that its code stays as measured.
 __device__ __forceinline__ void overlay_words(uint32_t& w0, uint32_t& w1, uint32_t& w2, const int2* __restrict__ map,
                                               const int2* __restrict__ lane_rows, const int4* __restrict__ lane_bbox,
                                               const int* __restrict__ draw, const LtDims& d, int y, int q, int s,
@@ -831,46 +829,10 @@ k_overlay(const uint8_t* frames, uint8_t* out, const int2* __restrict__ map,
     size_t base = (((size_t)s * d.img_h + y) * d.img_w + (size_t)q * 4) * 3;
     const uint32_t* src = reinterpret_cast<const uint32_t*>(frames + base);
     uint32_t w0 = src[0], w1 = src[1], w2 = src[2];
-    if (draw[s] && y >= d.ov0 && y < d.ov1) {
-        // Q5 canvas coordinates of the four pixels; most of them cannot reach the polygon: one test against its
-        // bounding box (taps of a pixel: columns sx, sx + 1, rows sy, sy + 1) skips the span look-ups
-        const int4* mp = reinterpret_cast<const int4*>(map + (size_t)y * d.img_w + q * 4);
-        const int4 m01 = __ldg(mp), m23 = __ldg(mp + 1);
-        const int sid = ids ? __ldg(&ids[s]) : s;        // the cached polygon belongs to the stream, not the position
-        const int4 bb = __ldg(&lane_bbox[sid]);
-        const int qx[4] = {m01.x, m01.z, m23.x, m23.z}, qy[4] = {m01.y, m01.w, m23.y, m23.w};
-        const int sx_lo = min(min(qx[0], qx[1]), min(qx[2], qx[3])) >> 5, sx_hi = max(max(qx[0], qx[1]), max(qx[2], qx[3])) >> 5;
-        const int sy_lo = min(min(qy[0], qy[1]), min(qy[2], qy[3])) >> 5, sy_hi = max(max(qy[0], qy[1]), max(qy[2], qy[3])) >> 5;
-        if (sx_hi + 1 >= bb.x && sx_lo <= bb.y && sy_hi + 1 >= bb.z && sy_lo <= bb.w) {
-            const int2* rows = lane_rows + (size_t)sid * d.bv_h;
-            uint32_t gch[4] = {(w0 >> 8) & 255, w1 & 255, (w1 >> 24) & 255, (w2 >> 16) & 255};
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                Tap4 t = make_taps(make_int2(qx[k], qy[k]));
-                // the two taps of a canvas row share its [lo, hi] span: two span loads instead of four
-                const int2 none = make_int2(1, 0);
-                const int2 s0 = ((unsigned)t.sy < (unsigned)d.bv_h) ? __ldg(&rows[t.sy]) : none;
-                const int2 s1 = ((unsigned)(t.sy + 1) < (unsigned)d.bv_h) ? __ldg(&rows[t.sy + 1]) : none;
-                const int xa = t.sx, xb = t.sx + 1;
-                const bool ina = (unsigned)xa < (unsigned)d.bv_w, inb = (unsigned)xb < (unsigned)d.bv_w;
-                int v = ((ina && xa >= s0.x && xa <= s0.y) ? t.w00 : 0) + ((inb && xb >= s0.x && xb <= s0.y) ? t.w01 : 0) +
-                        ((ina && xa >= s1.x && xa <= s1.y) ? t.w10 : 0) + ((inb && xb >= s1.x && xb <= s1.y) ? t.w11 : 0);
-                v = (v * 255 + 512) >> 10;
-                if (v) {
-                    // cv2.addWeighted(img,1,lane,0.3,0): float32 a + b*0.3f, round half to even, saturate
-                    float f = __fadd_rn((float)gch[k], __fmul_rn((float)v, 0.3f));
-                    gch[k] = (uint32_t)min(255, __float2int_rn(f));
-                }
-            }
-            w0 = (w0 & 0xFFFF00FFu) | (gch[0] << 8);
-            w1 = (w1 & 0x00FFFF00u) | gch[1] | (gch[2] << 24);
-            w2 = (w2 & 0xFF00FFFFu) | (gch[3] << 16);
-        }
-    }
+    overlay_words(w0, w1, w2, map, lane_rows, lane_bbox, draw, d, y, q, s, ids);
     uint32_t* dst = reinterpret_cast<uint32_t*>(out + base);
     dst[0] = w0; dst[1] = w1; dst[2] = w2;
 }
-
 
 // k_overlay of NV12 frames: one thread converts 4 pixels (one luma word, one chroma word = two U,V pairs) to the three
 // RGB words k_overlay reads, blends them the same way and writes them to the RGB output (which cannot alias the input).
@@ -884,10 +846,8 @@ k_overlay_nv12(const uint8_t* __restrict__ frames, uint8_t* __restrict__ out, co
     const uint8_t* f = frames + (size_t)s * d.img_w * (d.img_h + d.img_h / 2);
     const uint32_t luma = __ldg(reinterpret_cast<const uint32_t*>(f + (size_t)y * d.img_w) + q);
     const uint32_t uv = __ldg(reinterpret_cast<const uint32_t*>(f + (size_t)(d.img_h + (y >> 1)) * d.img_w) + q);
-    uint32_t px[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) px[i] = yuv_to_rgb((luma >> (8 * i)) & 255u, uv >> (16 * (i >> 1)));
-    uint32_t w0 = px[0] | (px[1] << 24), w1 = (px[1] >> 8) | (px[2] << 16), w2 = (px[2] >> 16) | (px[3] << 8);
+    uint32_t w0, w1, w2;
+    nv12_to_rgb_words(luma, uv, w0, w1, w2);
     overlay_words(w0, w1, w2, map, lane_rows, lane_bbox, draw, d, y, q, s, ids);
     uint32_t* dst = reinterpret_cast<uint32_t*>(out + (((size_t)s * d.img_h + y) * d.img_w + (size_t)q * 4) * 3);
     dst[0] = w0; dst[1] = w1; dst[2] = w2;
@@ -914,38 +874,25 @@ k_copy_rows(const uint4* __restrict__ src, uint4* __restrict__ dst, size_t frame
         if (i0 + (size_t)u * blockDim.x < total) fd[idx[u]] = v[u];
 }
 
-// The rows of the output frame that the lane overlay cannot reach are a plain copy of the input.
-static void overlay_rows(const lt_handle* h, const uint8_t* d_frames, const uint8_t* d_out, int& r0, int& r1, bool& vec_ok) {
-    const LtDims& d = h->d;
-    const size_t row_bytes = (size_t)d.img_w * 3;
-    r0 = d.ov0; r1 = d.ov1;
-    if (r0 >= r1) { r0 = 0; r1 = 0; }
-    vec_ok = (row_bytes % 16 == 0) && (((uintptr_t)d_frames | (uintptr_t)d_out) % 16 == 0);
-    if (d_out != d_frames && !vec_ok) { r0 = 0; r1 = d.img_h; }   // generic path: k_overlay copies every row itself
-}
-
-static int copy_untouched_rows(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, cudaStream_t st) {
-    const LtDims& d = h->d;
-    const size_t row_bytes = (size_t)d.img_w * 3, frame_bytes = row_bytes * d.img_h;
-    int r0, r1; bool vec_ok;
-    overlay_rows(h, d_frames, d_out, r0, r1, vec_ok);
-    if (d_out != d_frames && vec_ok && (r0 > 0 || r1 < d.img_h)) {
-        const size_t a_vec = (size_t)r0 * row_bytes / 16, b_off = (size_t)r1 * row_bytes / 16;
-        const size_t b_vec = (size_t)(d.img_h - r1) * row_bytes / 16;
-        dim3 g((unsigned)((a_vec + b_vec + 1023) / 1024), n);
-        k_copy_rows<<<g, 256, 0, st>>>(reinterpret_cast<const uint4*>(d_frames), reinterpret_cast<uint4*>(d_out),
-                                        frame_bytes / 16, a_vec, b_off, b_vec);
-        LT_LAUNCH_CHECK();
-    }
-    return 0;
-}
-
+// k_overlay runs on the rows [ov0, ov1) that the lane overlay can reach; out of place, the other rows of the output
+// frame are a plain copy of the input.
 int lt_launch_overlay(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, const int* d_draw,
                       const int* ids, cudaStream_t st) {
     const LtDims& d = h->d;
-    int r0, r1; bool vec_ok;
-    overlay_rows(h, d_frames, d_out, r0, r1, vec_ok);
-    { int rc = copy_untouched_rows(h, d_frames, d_out, n, st); if (rc) return rc; }
+    const size_t row_bytes = (size_t)d.img_w * 3, frame_bytes = row_bytes * d.img_h;
+    int r0 = d.ov0, r1 = d.ov1;
+    if (d_out != d_frames) {
+        if (row_bytes % 16 || ((uintptr_t)d_frames | (uintptr_t)d_out) % 16) {
+            r0 = 0; r1 = d.img_h;                       // generic path: k_overlay copies every row itself
+        } else if (r0 > 0 || r1 < d.img_h) {
+            const size_t a_vec = (size_t)r0 * row_bytes / 16, b_off = (size_t)r1 * row_bytes / 16;
+            const size_t b_vec = (size_t)(d.img_h - r1) * row_bytes / 16;
+            dim3 g((unsigned)((a_vec + b_vec + 1023) / 1024), n);
+            k_copy_rows<<<g, 256, 0, st>>>(reinterpret_cast<const uint4*>(d_frames), reinterpret_cast<uint4*>(d_out),
+                                            frame_bytes / 16, a_vec, b_off, b_vec);
+            LT_LAUNCH_CHECK();
+        }
+    }
     if (r1 > r0) {
         dim3 g(lt_div_up(d.img_w / 4, 256), r1 - r0, n);
         k_overlay<<<g, 256, 0, st>>>(d_frames, d_out, h->ov_map, h->lane_rows, h->lane_bbox, d_draw, d, r0, ids);
@@ -974,14 +921,8 @@ k_nv12_to_rgb(const uint8_t* __restrict__ nv12, uint8_t* __restrict__ rgb, int w
     for (int r = 0; r < 2; ++r) {
         const int row = 2 * yp + r;
         if (row < r0 || row >= r1) continue;
-        const uint32_t yy = r ? y1 : y0;
-        uint32_t px[4];                                                // R | G << 8 | B << 16
-#pragma unroll
-        for (int i = 0; i < 4; ++i) px[i] = yuv_to_rgb((yy >> (8 * i)) & 255u, uv >> (16 * (i >> 1)));
         uint32_t* o = reinterpret_cast<uint32_t*>(rgb + (((size_t)s * h + row) * w + (size_t)qx * 4) * 3);
-        o[0] = px[0] | (px[1] << 24);
-        o[1] = (px[1] >> 8) | (px[2] << 16);
-        o[2] = (px[2] >> 16) | (px[3] << 8);
+        nv12_to_rgb_words(r ? y1 : y0, uv, o[0], o[1], o[2]);
     }
 }
 
@@ -997,13 +938,12 @@ int lt_launch_nv12_to_rgb(const uint8_t* d_nv12, uint8_t* d_rgb, int n, int w, i
 int lt_launch_overlay_nv12(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, const int* d_draw,
                            const int* ids, cudaStream_t st) {
     const LtDims& d = h->d;
-    int r0 = d.ov0, r1 = d.ov1, rc;
-    if (r0 >= r1) { r0 = 0; r1 = 0; }
-    if ((rc = lt_launch_nv12_to_rgb(d_frames, d_out, n, d.img_w, d.img_h, 0, r0, st))) return rc;
-    if ((rc = lt_launch_nv12_to_rgb(d_frames, d_out, n, d.img_w, d.img_h, r1 > r0 ? r1 : 0, d.img_h, st))) return rc;
-    if (r1 > r0) {
-        dim3 g(lt_div_up(d.img_w / 4, 256), r1 - r0, n);
-        k_overlay_nv12<<<g, 256, 0, st>>>(d_frames, d_out, h->ov_map, h->lane_rows, h->lane_bbox, d_draw, d, r0, ids);
+    int rc;
+    if ((rc = lt_launch_nv12_to_rgb(d_frames, d_out, n, d.img_w, d.img_h, 0, d.ov0, st))) return rc;
+    if ((rc = lt_launch_nv12_to_rgb(d_frames, d_out, n, d.img_w, d.img_h, d.ov1, d.img_h, st))) return rc;
+    if (d.ov1 > d.ov0) {
+        dim3 g(lt_div_up(d.img_w / 4, 256), d.ov1 - d.ov0, n);
+        k_overlay_nv12<<<g, 256, 0, st>>>(d_frames, d_out, h->ov_map, h->lane_rows, h->lane_bbox, d_draw, d, d.ov0, ids);
         LT_LAUNCH_CHECK();
     }
     return 0;

@@ -283,15 +283,12 @@ class BatchedLaneTracker:
         return n
 
     def _check_frames(self, frames):
-        w, h = self.img_size
-        if not (isinstance(frames, torch.Tensor) and frames.is_cuda and frames.dtype == torch.uint8 and
-                frames.is_contiguous() and frames.dim() == 4 and tuple(frames.shape[1:]) == (h, w, 3)):
-            raise ValueError("frames must be a contiguous CUDA uint8 tensor [n, %d, %d, 3]" % (h, w))
-        if frames.data_ptr() % 4:
-            raise ValueError("frames must start at a 4-byte aligned address (the kernels access frames as 32-bit words)")
-        if frames.shape[0] < 1 or frames.shape[0] > self.n_streams:
-            raise ValueError("got %d frames for %d streams" % (frames.shape[0], self.n_streams))
-        return int(frames.shape[0])
+        """Check an input batch of RGB frames (the stage calls take no NV12); -> n."""
+        n, fmt = self._frame_format(frames)
+        if fmt != FRAME_RGB:
+            w, h = self.img_size
+            raise ValueError("frames must be RGB [n, %d, %d, 3] here, got NV12 frames" % (h, w))
+        return n
 
     def _check_ids(self, ids, n):
         """Stream ids of a batch of n frames -> ctypes int32 array (None: None).  Any int sequence, NumPy array or CPU
@@ -336,20 +333,7 @@ class BatchedLaneTracker:
         ids: None -- frame i belongs to stream i; else n distinct stream ids in [0, n_streams), any order (int
         sequence, NumPy array or CPU tensor): frame i belongs to stream ids[i], and the streams not listed keep their
         state.  out and the result records stay in batch order."""
-        n = self._input(frames)
-        self._check_out(out, frames)
-        h_ids = self._check_ids(ids, n)
-        p = params if params is not None else make_params(**kw)
-        res = self._results_dev if results_dev is None else results_dev
-        if res.numel() < n * RESULT_DTYPE.itemsize or not res.is_cuda:
-            raise ValueError("results buffer too small")
-        if h_ids is None:
-            check(self.lib.lt_process(self._h, _ptr(frames), _ptr(out), n, C.byref(p), _ptr(res),
-                                      _stream_ptr(self.device)))
-        else:
-            check(self.lib.lt_process_streams(self._h, _ptr(frames), _ptr(out), h_ids, n, C.byref(p), _ptr(res),
-                                              _stream_ptr(self.device)))
-        return n
+        return self._process_call(frames, out, None, params, results_dev, ids, kw)
 
     def process_front_async(self, frames, buffer_set, params=None, **kw):
         """First half of ``process_async`` (undistort, warp, first-attempt filter) into intermediate buffer set
@@ -363,6 +347,10 @@ class BatchedLaneTracker:
         """Second half of ``process_async`` (searches, second attempt, state machine, overlay) from intermediate
         buffer set 0 or 1, on the current CUDA stream.  Advances the per-stream state of the streams in ``ids``
         (None: streams 0..n-1), as ``process_async``.  RGB or NV12 frames, as given to the front half."""
+        return self._process_call(frames, out, buffer_set, params, results_dev, ids, kw)
+
+    def _process_call(self, frames, out, buffer_set, params, results_dev, ids, kw):
+        """Checks and C call of ``process_async`` (buffer_set None: both halves) or ``process_back_async``; -> n."""
         n = self._input(frames)
         self._check_out(out, frames)
         h_ids = self._check_ids(ids, n)
@@ -370,19 +358,22 @@ class BatchedLaneTracker:
         res = self._results_dev if results_dev is None else results_dev
         if res.numel() < n * RESULT_DTYPE.itemsize or not res.is_cuda:
             raise ValueError("results buffer too small")
-        if h_ids is None:
-            check(self.lib.lt_process_back(self._h, _ptr(frames), _ptr(out), n, C.byref(p), int(buffer_set),
-                                           _ptr(res), _stream_ptr(self.device)))
+        if buffer_set is None:
+            plain, streams, set_arg = self.lib.lt_process, self.lib.lt_process_streams, ()
         else:
-            check(self.lib.lt_process_back_streams(self._h, _ptr(frames), _ptr(out), h_ids, n, C.byref(p),
-                                                   int(buffer_set), _ptr(res), _stream_ptr(self.device)))
+            plain, streams, set_arg = self.lib.lt_process_back, self.lib.lt_process_back_streams, (int(buffer_set),)
+        fn, ids_arg = (plain, ()) if h_ids is None else (streams, (h_ids,))
+        check(fn(self._h, _ptr(frames), _ptr(out), *ids_arg, n, C.byref(p), *set_arg, _ptr(res),
+                 _stream_ptr(self.device)))
         return n
 
-    def fetch_results(self, n=None):
-        """Copy the last results to pinned host memory and return them as a structured array."""
+    def fetch_results(self, n=None, results_dev=None):
+        """Copy the first n result records of ``results_dev`` (default: the internal buffer ``process_async`` fills
+        when given none) to pinned host memory and return them as a structured array (synchronises)."""
         n = self.n_streams if n is None else n
+        res = self._results_dev if results_dev is None else results_dev
         nbytes = n * RESULT_DTYPE.itemsize
-        self._results_host[:nbytes].copy_(self._results_dev[:nbytes], non_blocking=True)
+        self._results_host[:nbytes].copy_(res[:nbytes], non_blocking=True)
         torch.cuda.current_stream(self.device).synchronize()
         return self._results_host[:nbytes].numpy().view(RESULT_DTYPE).copy()
 
@@ -693,10 +684,7 @@ class GraphedProcess:
         self.graph.replay()
 
     def fetch_results(self):
-        nbytes = self.n * RESULT_DTYPE.itemsize
-        self.t._results_host[:nbytes].copy_(self.results_dev[:nbytes], non_blocking=True)
-        torch.cuda.current_stream(self.t.device).synchronize()
-        return self.t._results_host[:nbytes].numpy().view(RESULT_DTYPE).copy()
+        return self.t.fetch_results(self.n, self.results_dev)
 
 
 class DevicePipeline:
@@ -761,12 +749,8 @@ class DevicePipeline:
 
     def fetch_results(self, n=None):
         """Results of the most recently submitted batch as a structured array (synchronises)."""
-        n = self.t.n_streams if n is None else n
         self.join()
-        nbytes = n * RESULT_DTYPE.itemsize
-        self.t._results_host[:nbytes].copy_(self.last_results_dev()[:nbytes], non_blocking=True)
-        torch.cuda.current_stream(self.t.device).synchronize()
-        return self.t._results_host[:nbytes].numpy().view(RESULT_DTYPE).copy()
+        return self.t.fetch_results(n, self.last_results_dev())
 
 
 def _rows_minus(rows, covered):
