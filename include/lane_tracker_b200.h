@@ -29,6 +29,7 @@ extern "C" {
 
 #define LT_ABI_VERSION 4
 #define LT_MAX_AVERAGE 8          /* capacity of the n_average rings */
+#define LT_MAX_PROFILES 16        /* parameter profiles per handle (lt_set_profile) */
 
 typedef struct lt_handle lt_handle;
 
@@ -185,6 +186,37 @@ int lt_process_streams(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, co
 int lt_process_back_streams(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids, int32_t n,
                             const lt_params* params, int32_t set, lt_result* d_results, void* stream);
 
+/* Parameter profiles: one batch whose frames use different lt_params and check_validity windows (cameras on different
+ * roads or mounted differently; tracker_settings.md of the reference documents one set per demo video).
+ * lt_set_profile stores profile `profile` (0 <= profile < LT_MAX_PROFILES) on the handle: `params`, checked like the
+ * lt_params of lt_process (same messages), and the windows `validity` (NULL: the shipped ones).  Synchronous; a profile
+ * never set is "unset".  It may be called with work in flight: a batch uses the profile table as it stood when its
+ * front half was enqueued (the front half copies the profiles into its intermediate buffer set, the back half reads
+ * that copy only). */
+int lt_set_profile(lt_handle* h, int32_t profile, const lt_params* params, const lt_validity* validity);
+
+/* lt_process_streams / lt_process_front / lt_process_back_streams with a profile per batch position:
+ *   h_profiles: HOST int32 [n], position i uses profile h_profiles[i] (its filter, searches, validity windows and
+ *               n_tries; the second attempt keeps the reference's hard-coded parameters and uses the profile's
+ *               windows).  Profiles belong to batch positions, like frames: a caller that keeps a profile per camera
+ *               passes profile_of[ids], and a stream may change profile from one frame to the next.  Copied when the
+ *               call is enqueued (kernel arguments): nothing synchronises and the calls are capturable in a CUDA graph.
+ *   h_ids     : as lt_process_streams; NULL means the identity 0..n-1.
+ * The front half filters each group of positions that share a filter configuration (filter_type, ksize_r, C_r,
+ * ksize_b, C_b, mask_noise, and noise_thresh, ksize_noise, C_noise under mask_noise) with one launch sequence; with a
+ * single group the launches are those of lt_process.  Refused before anything is enqueued, naming the position: a NULL
+ * h_profiles, an index outside [0, LT_MAX_PROFILES), an unset profile; every check of lt_process_streams applies as
+ * well (the pixel-capacity check of capture mode takes the widest bandwidth of the profiles used).
+ * lt_process_back_profiles refuses a buffer set whose last front half was not lt_process_front_profiles, or had
+ * another n or other profile indices (naming the first position that differs).  Ordering as lt_process_back.
+ * lt_process_profiles(...) == lt_process_front_profiles(..., 0, stream) + lt_process_back_profiles(..., 0, ..., stream). */
+int lt_process_profiles(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids,
+                        const int32_t* h_profiles, int32_t n, lt_result* d_results, void* stream);
+int lt_process_front_profiles(lt_handle* h, const uint8_t* d_frames, const int32_t* h_profiles, int32_t n, int32_t set,
+                              void* stream);
+int lt_process_back_profiles(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids,
+                             const int32_t* h_profiles, int32_t n, int32_t set, lt_result* d_results, void* stream);
+
 /* Keep the ordered lane-pixel sets and window centroids of every lt_process call so that
  * lt_read_capture can return them (the reference exposes them as the attributes left_x/left_y/
  * right_x/right_y/left_window_centroids, lane_tracker.py:159-166).  Off by default: the
@@ -244,7 +276,8 @@ int lt_memcpy_rows(lt_handle* h, void* dst, const void* src, int32_t n_frames, i
  * lt_profile_begin arms CUDA-event recording at every stage boundary of the next `max_calls`
  * lt_process calls (events are recorded on the caller's stream, no synchronisation);
  * lt_profile_read synchronises, sums the per-stage durations [ms] over the recorded calls,
- * and disarms.  Stage ids: lt_stage_name(0..LT_NSTAGES-1). */
+ * and disarms.  Stage ids: lt_stage_name(0..LT_NSTAGES-1).  A call with parameter profiles marks the threshold stages
+ * once per filter group; their times add up. */
 #define LT_NSTAGES 16
 int lt_profile_begin(lt_handle* h, int32_t max_calls);
 int lt_profile_read(lt_handle* h, double* h_stage_ms, int32_t* h_calls);

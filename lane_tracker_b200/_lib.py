@@ -12,6 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "liblane_tracker_b200.so")
 
 LT_MAX_AVERAGE = 8
+LT_MAX_PROFILES = 16
 LT_MAX_LEVELS = 128
 LT_ABI_VERSION = 4
 LT_NSTAGES = 16
@@ -87,6 +88,10 @@ SIGNATURES = {
     "lt_process_back": (C.c_int, [P, P, P, i32, C.POINTER(lt_params), i32, P, P]),
     "lt_process_streams": (C.c_int, [P, P, P, C.POINTER(i32), i32, C.POINTER(lt_params), P, P]),
     "lt_process_back_streams": (C.c_int, [P, P, P, C.POINTER(i32), i32, C.POINTER(lt_params), i32, P, P]),
+    "lt_set_profile": (C.c_int, [P, i32, C.POINTER(lt_params), C.POINTER(lt_validity)]),
+    "lt_process_profiles": (C.c_int, [P, P, P, C.POINTER(i32), C.POINTER(i32), i32, P, P]),
+    "lt_process_front_profiles": (C.c_int, [P, P, C.POINTER(i32), i32, i32, P]),
+    "lt_process_back_profiles": (C.c_int, [P, P, P, C.POINTER(i32), C.POINTER(i32), i32, i32, P, P]),
     "lt_set_capture": (C.c_int, [P, i32]),
     "lt_set_pixel_capacity": (C.c_int, [P, i32]),
     "lt_read_capture": (C.c_int, [P, i32, i32, i32, P, i32, C.POINTER(i32), P, C.POINTER(i32)]),

@@ -123,6 +123,27 @@ extern "C" int lt_get_validity(lt_handle* h, lt_validity* v) {
     return 0;
 }
 
+static int check_params(const lt_handle* h, const LtAttemptParams& a);
+
+extern "C" int lt_set_profile(lt_handle* h, int32_t profile, const lt_params* params, const lt_validity* validity) {
+    if (!h) { lt_set_error("null handle"); return -1; }
+    if (profile < 0 || profile >= LT_MAX_PROFILES) {
+        lt_set_error("profile %d outside [0, %d)", profile, LT_MAX_PROFILES);
+        return -1;
+    }
+    if (!params) { lt_set_error("null params"); return -1; }
+    LtProfile q;
+    memset(&q, 0, sizeof(q));
+    q.p = attempt_from(*params);
+    int rc;
+    if ((rc = check_params(h, q.p))) return rc;
+    q.val = validity ? *validity : SHIPPED_VALIDITY;
+    q.n_tries = params->n_tries;
+    h->profiles[profile] = q;
+    h->profiles_set |= 1u << profile;
+    return 0;
+}
+
 static void init_state(lt_handle* h, lt_state* s) {
     memset(s, 0, sizeof(*s));
     s->last_detection = h->cfg.n_reset + 1;     // lane_tracker.py:140
@@ -134,8 +155,9 @@ extern "C" int lt_destroy(lt_handle* h) {
     for (int k = 0; k < 2; ++k) {
         const LtFrontSet& f = h->fs[k];
         void* fp[] = {f.und_roi, f.pad_alloc[0], f.pad_alloc[1], f.pad_alloc[2], f.pad_alloc[3], f.pad_alloc[4], f.pad_alloc[5],
-                      f.merged, f.mask};
+                      f.merged, f.mask, f.group_pos, f.pos_profile, f.profiles};
         for (void* p : fp) if (p) cudaFree(p);
+        delete[] f.h_pos_profile;
     }
     void* ptrs[] = {h->und_map, h->bv_map, h->ov_map, h->bv_desc, h->und_desc, h->lab_yz, h->fused_desc, h->lab_gamma, h->lab_cbrt, h->lane_rows, h->lane_bbox, h->dl_bbox,
                     h->avg_x, h->state, h->att, h->retry_list, h->retry_count, h->draw_flags, h->stream_ids, h->vis_scratch,
@@ -169,6 +191,10 @@ static int alloc_front_set(lt_handle* h, int k) {
     }
     if (!rc) rc = dev_alloc(&f.merged, S * h->stream_mask);
     if (!rc) rc = dev_alloc(&f.mask, S * h->stream_mask);
+    if (!rc) rc = dev_alloc(&f.group_pos, S);
+    if (!rc) rc = dev_alloc(&f.pos_profile, S);
+    if (!rc) rc = dev_alloc(&f.profiles, LT_MAX_PROFILES);
+    if (!rc) f.h_pos_profile = new int[S];
     return rc;
 }
 
@@ -320,8 +346,9 @@ static int check_n(lt_handle* h, int n) {
 // process()
 // ---------------------------------------------------------------------------
 
-// find_lane_points (lane_tracker.py:795-874) of the first attempt up to the binary mask, all streams: stateless
-static int process_front(lt_handle* h, const uint8_t* d_frames, int n, const LtAttemptParams& p1, cudaStream_t st) {
+// find_lane_points (lane_tracker.py:795-874) of the first attempt up to the binary mask, all streams: stateless.
+// The filter groups g[0..ng) cover the batch (one group {p1, NULL, n} without profiles).
+static int process_front(lt_handle* h, const uint8_t* d_frames, int n, const LtFilterGroup* g, int ng, cudaStream_t st) {
     int rc;
     if (h->prof_active && h->prof_calls >= h->prof_max_calls) h->prof_active = 0;
     lt_prof_mark(h, ST_BEGIN, st);
@@ -333,7 +360,7 @@ static int process_front(lt_handle* h, const uint8_t* d_frames, int n, const LtA
         if ((rc = lt_launch_warp(h, nullptr, n, st))) return rc;
     }
     lt_prof_mark(h, ST_WARP, st);
-    return lt_launch_filter(h, n, p1, nullptr, nullptr, st);
+    return lt_launch_filter_groups(h, n, g, ng, nullptr, st);
 }
 
 // The stream ids of a batch travel to the device as kernel arguments: a launch copies its arguments when it is
@@ -350,30 +377,100 @@ __global__ void k_set_stream_ids(LtIdsChunk c, int* __restrict__ dst) {
     for (int i = threadIdx.x; i < c.count; i += blockDim.x) dst[c.offset + i] = c.ids[i];
 }
 
-// Writes h_ids to the handle's one device id array on the stream of the back half that reads it.  One array per
-// handle is enough: every kernel that reads it is a back-half kernel enqueued on that same stream after this write,
-// and the back half of batch k must follow the back half of batch k-1 (lt_process_back), so a write for batch k
-// cannot overtake a read of batch k-1, and no later write can overtake a read of batch k.
-static int upload_stream_ids(lt_handle* h, const int32_t* h_ids, int n, cudaStream_t st) {
+// Writes the host ints h_src[0..n) to the device array dst on stream st, as kernel arguments.
+static int upload_ints(const int32_t* h_src, int n, int* dst, cudaStream_t st) {
     LtIdsChunk c;
     for (int off = 0; off < n; off += LT_IDS_CHUNK) {
         c.offset = off;
         c.count = n - off < LT_IDS_CHUNK ? n - off : LT_IDS_CHUNK;
-        memcpy(c.ids, h_ids + off, (size_t)c.count * sizeof(int32_t));
-        k_set_stream_ids<<<1, 256, 0, st>>>(c, h->stream_ids);
+        memcpy(c.ids, h_src + off, (size_t)c.count * sizeof(int32_t));
+        k_set_stream_ids<<<1, 256, 0, st>>>(c, dst);
         LT_LAUNCH_CHECK();
     }
     return 0;
 }
 
+// Writes h_ids to the handle's one device id array on the stream of the back half that reads it.  One array per
+// handle is enough: every kernel that reads it is a back-half kernel enqueued on that same stream after this write,
+// and the back half of batch k must follow the back half of batch k-1 (lt_process_back), so a write for batch k
+// cannot overtake a read of batch k-1, and no later write can overtake a read of batch k.
+static int upload_stream_ids(lt_handle* h, const int32_t* h_ids, int n, cudaStream_t st) {
+    return upload_ints(h_ids, n, h->stream_ids, st);
+}
+
+struct LtProfileTable {
+    LtProfile e[LT_MAX_PROFILES];
+};
+
+__global__ void k_set_profiles(LtProfileTable t, LtProfile* __restrict__ dst) {
+    if (threadIdx.x < LT_MAX_PROFILES) dst[threadIdx.x] = t.e[threadIdx.x];
+}
+
+static bool same_filter(const LtAttemptParams& a, const LtAttemptParams& b) {
+    if (a.filter_type != b.filter_type || a.ksize_r != b.ksize_r || a.C_r != b.C_r || a.ksize_b != b.ksize_b ||
+        a.C_b != b.C_b || a.mask_noise != b.mask_noise)
+        return false;
+    return !a.mask_noise || (a.noise_thresh == b.noise_thresh && a.ksize_noise == b.ksize_noise && a.C_noise == b.C_noise);
+}
+
+// Front half with profiles: snapshot the profile table and the batch's profile indices into buffer set `set` (on the
+// front stream: the back half of this batch runs after it, the front half of batch k+2 after that back half), group
+// the positions by filter configuration, and run the front half over the groups.
+static int process_front_profiles(lt_handle* h, const uint8_t* d_frames, const int32_t* h_prof, int n, int set,
+                                  cudaStream_t st) {
+    LtFrontSet& f = h->fs[set];
+    LtProfileTable t;
+    memcpy(t.e, h->profiles, sizeof(t.e));
+    int rc;
+    if ((rc = upload_ints(h_prof, n, f.pos_profile, st))) return rc;
+    k_set_profiles<<<1, 32, 0, st>>>(t, f.profiles);
+    LT_LAUNCH_CHECK();
+    memcpy(f.snap, h->profiles, sizeof(f.snap));
+    memcpy(f.h_pos_profile, h_prof, (size_t)n * sizeof(int32_t));
+    f.snap_n = n;
+    // one representative profile per filter configuration, bilateral configurations first
+    int rep[LT_MAX_PROFILES], nrep = 0, group_of[LT_MAX_PROFILES];
+    for (int pass = 0; pass < 2; ++pass)
+        for (int k = 0; k < LT_MAX_PROFILES; ++k) {
+            if (!((h->profiles_set >> k) & 1u) || (h->profiles[k].p.filter_type == 0) != (pass == 0)) continue;
+            bool used = false;
+            for (int i = 0; i < n && !used; ++i) used = h_prof[i] == k;
+            if (!used) continue;
+            int r = 0;
+            while (r < nrep && !same_filter(h->profiles[rep[r]].p, h->profiles[k].p)) ++r;
+            if (r == nrep) rep[nrep++] = k;
+            group_of[k] = r;
+        }
+    LtFilterGroup g[LT_MAX_PROFILES];
+    if (nrep == 1) {
+        g[0] = {h->profiles[rep[0]].p, nullptr, n};
+    } else {
+        std::vector<int> pos;
+        pos.reserve(n);
+        for (int r = 0; r < nrep; ++r) {
+            const size_t first = pos.size();
+            for (int i = 0; i < n; ++i) if (group_of[h_prof[i]] == r) pos.push_back(i);
+            g[r] = {h->profiles[rep[r]].p, f.group_pos + first, (int)(pos.size() - first)};
+        }
+        if ((rc = upload_ints(pos.data(), n, f.group_pos, st))) return rc;
+    }
+    return process_front(h, d_frames, n, g, nrep, st);
+}
+
+static bool allows_retry(int n_tries) { return n_tries >= 2 || n_tries == -1; }
+
 // searches, second attempt of the streams that failed, state machine, overlay: advances the per-stream state.
 // h_ids (host, validated by check_ids) maps batch position i to state slot h_ids[i]; NULL: the identity.
-static int process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, const lt_params* params,
+// fs: the buffer set whose profile snapshot the batch uses (NULL: p1 and the handle's windows for every position);
+// n_tries: of the batch (with profiles: 2 when some position may take a second attempt, else 1).
+static int process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, int n_tries,
                         const LtAttemptParams& p1, lt_result* d_results, cudaStream_t st, bool own_begin,
-                        const int32_t* h_ids) {
+                        const int32_t* h_ids, const LtFrontSet* fs) {
     int rc;
     const LtAttemptParams p2 = second_attempt();
-    const bool two = (params->n_tries >= 2) || (params->n_tries == -1);
+    const LtProfile* prof = fs ? fs->profiles : nullptr;
+    const int* pos_prof = fs ? fs->pos_profile : nullptr;
+    const bool two = allows_retry(n_tries);
     if (own_begin) lt_prof_mark(h, ST_BEGIN, st);       // stage times are differences of marks on ONE stream
     const int* ids = nullptr;
     if (h_ids) {
@@ -388,12 +485,12 @@ static int process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, i
         sa.by_stream = 1; sa.pixels = h->cap_pixels; sa.pix_cap = h->pix_cap; sa.pix_counts = h->cap_counts;
         sa.centroids = h->cap_cents; sa.ncentroids = h->cap_ncents;
     }
-    if ((rc = lt_launch_search(h, n, p1, sa, nullptr, nullptr, st))) return rc;
+    if ((rc = lt_launch_search(h, n, p1, sa, nullptr, nullptr, st, prof, pos_prof, 1))) return rc;
     lt_prof_mark(h, ST_SEARCH, st);
     if (two) {
         // second attempt only for the streams whose first attempt failed (lane_tracker.py:1071-1128).
         // The reference re-runs undistort + warp here; their outputs are unchanged, so the planes are reused.
-        if ((rc = lt_launch_select_retry(h, n, params->n_tries, st))) return rc;
+        if ((rc = lt_launch_select_retry(h, n, n_tries, st, prof, pos_prof))) return rc;
         lt_prof_mark(h, ST_RETRY_SELECT, st);
         if ((rc = lt_launch_filter(h, n, p2, h->retry_list, h->retry_count, st))) return rc;
         sa.att = h->att + h->S;
@@ -401,7 +498,7 @@ static int process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, i
             sa.pixels = h->cap_pixels + S * 2 * (size_t)h->pix_cap; sa.pix_counts = h->cap_counts + S * 2;
             sa.centroids = h->cap_cents + S * 2 * LT_MAX_LEVELS; sa.ncentroids = h->cap_ncents + S * 2;
         }
-        if ((rc = lt_launch_search(h, n, p2, sa, h->retry_list, h->retry_count, st))) return rc;
+        if ((rc = lt_launch_search(h, n, p2, sa, h->retry_list, h->retry_count, st, prof, pos_prof, 0))) return rc;
         lt_prof_mark(h, ST_SEARCH, st);
     }
     if ((rc = lt_launch_update_state(h, n, ids, d_results, two ? 2 : 1, st))) return rc;
@@ -464,19 +561,25 @@ static int check_out(const lt_handle* h, const uint8_t* d_frames, const uint8_t*
     return 0;
 }
 
-static int process_args(lt_handle* h, const uint8_t* d_frames, int n, const lt_params* params, int set, LtAttemptParams* p1) {
+// The checks every process call makes on its batch size, frames and buffer set (has_params: params or the profile
+// list is not NULL).
+static int process_args(lt_handle* h, const uint8_t* d_frames, int n, bool has_params, int set) {
     int rc;
     if ((rc = check_n(h, n))) return rc;
-    if (!d_frames || !params) { lt_set_error("null argument"); return -1; }
+    if (!d_frames || !has_params) { lt_set_error("null argument"); return -1; }
     if ((rc = check_frame_buffer(d_frames, "d_frames"))) return rc;
     if (set != 0 && set != 1) { lt_set_error("buffer set must be 0 or 1"); return -1; }
-    *p1 = attempt_from(*params);
-    if ((rc = check_params(h, *p1))) return rc;
+    return 0;
+}
+
+// bandwidth: the widest band-search bandwidth the batch uses.  Then selects buffer set `set`.
+static int process_set(lt_handle* h, int set, int bandwidth) {
+    int rc;
     // captured pixel lists: a band-search row holds up to 2*bandwidth - 1 pixels (attempt 2 uses bandwidth 30)
-    const int bw = p1->bandwidth > 30 ? p1->bandwidth : 30;
+    const int bw = bandwidth > 30 ? bandwidth : 30;
     if (h->capture && (long long)(2 * bw - 1) * h->d.bv_h > (long long)h->pix_cap) {
         lt_set_error("bandwidth %d can overflow the captured pixel lists (capacity %d): raise it with lt_set_pixel_capacity",
-                     p1->bandwidth, h->pix_cap);
+                     bandwidth, h->pix_cap);
         return -1;
     }
     if ((rc = alloc_front_set(h, set))) return rc;
@@ -500,47 +603,133 @@ static int check_ids(lt_handle* h, const int32_t* h_ids, int n) {
     return 0;
 }
 
-// What one process entry point does: the front half, the back half or both, with or without a stream id list.
-enum { PROC_FRONT = 1, PROC_BACK = 2, PROC_IDS = 4 };
+// Profile indices of lt_process_*_profiles: every entry names a profile that is set.  Returns the widest bandwidth
+// and the batch's n_tries (2 when a profile used allows a second attempt, else 1).
+static int check_profiles(lt_handle* h, const int32_t* h_prof, int n, int* bandwidth, int* n_tries) {
+    if (!h_prof) { lt_set_error("null profile list"); return -1; }
+    *bandwidth = 0;
+    *n_tries = 1;
+    for (int i = 0; i < n; ++i) {
+        const int k = h_prof[i];
+        if (k < 0 || k >= LT_MAX_PROFILES) {
+            lt_set_error("profile %d at batch position %d outside [0, %d)", k, i, LT_MAX_PROFILES);
+            return -1;
+        }
+        if (!((h->profiles_set >> k) & 1u)) { lt_set_error("profile %d at batch position %d is unset", k, i); return -1; }
+        const LtProfile& q = h->profiles[k];
+        if (q.p.bandwidth > *bandwidth) *bandwidth = q.p.bandwidth;
+        if (allows_retry(q.n_tries)) *n_tries = 2;
+    }
+    return 0;
+}
+
+// What one process entry point does: the front half, the back half or both, with or without a stream id list, with
+// one lt_params or with a parameter profile per batch position.
+enum { PROC_FRONT = 1, PROC_BACK = 2, PROC_IDS = 4, PROC_PROFILES = 8 };
 
 // The checks of the process entry points, in this order and all before anything is enqueued, then the halves.
 static int process_call(lt_handle* h, int what, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids, int n,
-                        const lt_params* params, int set, lt_result* d_results, void* stream) {
+                        const lt_params* params, const int32_t* h_prof, int set, lt_result* d_results, void* stream) {
     int rc;
     LtAttemptParams p1;
-    const bool front = what & PROC_FRONT, back = what & PROC_BACK;
+    const bool front = what & PROC_FRONT, back = what & PROC_BACK, profiles = what & PROC_PROFILES;
     const cudaStream_t st = (cudaStream_t)stream;
     if ((what & PROC_IDS) && (rc = check_ids(h, h_ids, n))) return rc;
     if (back && (rc = check_out(h, d_frames, d_out, n))) return rc;
-    if ((rc = process_args(h, d_frames, n, params, set, &p1))) return rc;
+    if ((rc = process_args(h, d_frames, n, profiles || params, set))) return rc;
+    int bandwidth, n_tries;
+    if (profiles) {
+        if ((rc = check_profiles(h, h_prof, n, &bandwidth, &n_tries))) return rc;
+        if (back && !front) {    // the front half of this set must have taken these profiles
+            const LtFrontSet& f = h->fs[set];
+            if (f.snap_n == 0) {
+                lt_set_error("buffer set %d was last filled by a front half without profiles", set);
+                return -1;
+            }
+            if (f.snap_n != n) {
+                lt_set_error("buffer set %d holds a front half of %d frames, not %d", set, f.snap_n, n);
+                return -1;
+            }
+            for (int i = 0; i < n; ++i)
+                if (f.h_pos_profile[i] != h_prof[i]) {
+                    lt_set_error("profile %d at batch position %d differs from the front half's profile %d", h_prof[i], i,
+                                 f.h_pos_profile[i]);
+                    return -1;
+                }
+            // the back half uses the snapshot of the front half: its bandwidths and n_tries
+            bandwidth = 0; n_tries = 1;
+            for (int i = 0; i < n; ++i) {
+                const LtProfile& q = f.snap[h_prof[i]];
+                if (q.p.bandwidth > bandwidth) bandwidth = q.p.bandwidth;
+                if (allows_retry(q.n_tries)) n_tries = 2;
+            }
+        }
+        // the launchers' own checks see a valid parameter set; every kernel reads its position's profile instead
+        p1 = ((back && !front) ? h->fs[set].snap : h->profiles)[h_prof[0]].p;
+    } else {
+        p1 = attempt_from(*params);
+        if ((rc = check_params(h, p1))) return rc;
+        bandwidth = p1.bandwidth;
+        n_tries = params->n_tries;
+    }
+    if ((rc = process_set(h, set, bandwidth))) return rc;
     if (back && !d_results) { lt_set_error("null argument"); return -1; }
-    if (front && (rc = process_front(h, d_frames, n, p1, st))) return rc;
-    return back ? process_back(h, d_frames, d_out, n, params, p1, d_results, st, !front, h_ids) : 0;
+    if (front) {
+        if (profiles) {
+            rc = process_front_profiles(h, d_frames, h_prof, n, set, st);
+        } else {
+            h->fs[set].snap_n = 0;
+            const LtFilterGroup g = {p1, nullptr, n};
+            rc = process_front(h, d_frames, n, &g, 1, st);
+        }
+        if (rc) return rc;
+    }
+    return back ? process_back(h, d_frames, d_out, n, n_tries, p1, d_results, st, !front, h_ids, profiles ? &h->fs[set] : nullptr)
+                : 0;
 }
 
 extern "C" int lt_process(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int32_t n, const lt_params* params,
                           lt_result* d_results, void* stream) {
-    return process_call(h, PROC_FRONT | PROC_BACK, d_frames, d_out, nullptr, n, params, 0, d_results, stream);
+    return process_call(h, PROC_FRONT | PROC_BACK, d_frames, d_out, nullptr, n, params, nullptr, 0, d_results, stream);
 }
 
 extern "C" int lt_process_front(lt_handle* h, const uint8_t* d_frames, int32_t n, const lt_params* params, int32_t set,
                                 void* stream) {
-    return process_call(h, PROC_FRONT, d_frames, nullptr, nullptr, n, params, set, nullptr, stream);
+    return process_call(h, PROC_FRONT, d_frames, nullptr, nullptr, n, params, nullptr, set, nullptr, stream);
 }
 
 extern "C" int lt_process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int32_t n, const lt_params* params,
                                int32_t set, lt_result* d_results, void* stream) {
-    return process_call(h, PROC_BACK, d_frames, d_out, nullptr, n, params, set, d_results, stream);
+    return process_call(h, PROC_BACK, d_frames, d_out, nullptr, n, params, nullptr, set, d_results, stream);
 }
 
 extern "C" int lt_process_streams(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids, int32_t n,
                                   const lt_params* params, lt_result* d_results, void* stream) {
-    return process_call(h, PROC_FRONT | PROC_BACK | PROC_IDS, d_frames, d_out, h_ids, n, params, 0, d_results, stream);
+    return process_call(h, PROC_FRONT | PROC_BACK | PROC_IDS, d_frames, d_out, h_ids, n, params, nullptr, 0, d_results, stream);
 }
 
 extern "C" int lt_process_back_streams(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids,
                                        int32_t n, const lt_params* params, int32_t set, lt_result* d_results, void* stream) {
-    return process_call(h, PROC_BACK | PROC_IDS, d_frames, d_out, h_ids, n, params, set, d_results, stream);
+    return process_call(h, PROC_BACK | PROC_IDS, d_frames, d_out, h_ids, n, params, nullptr, set, d_results, stream);
+}
+
+extern "C" int lt_process_profiles(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids,
+                                   const int32_t* h_profiles, int32_t n, lt_result* d_results, void* stream) {
+    return process_call(h, PROC_FRONT | PROC_BACK | PROC_PROFILES | (h_ids ? PROC_IDS : 0), d_frames, d_out, h_ids, n,
+                        nullptr, h_profiles, 0, d_results, stream);
+}
+
+extern "C" int lt_process_front_profiles(lt_handle* h, const uint8_t* d_frames, const int32_t* h_profiles, int32_t n,
+                                         int32_t set, void* stream) {
+    return process_call(h, PROC_FRONT | PROC_PROFILES, d_frames, nullptr, nullptr, n, nullptr, h_profiles, set, nullptr,
+                        stream);
+}
+
+extern "C" int lt_process_back_profiles(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids,
+                                        const int32_t* h_profiles, int32_t n, int32_t set, lt_result* d_results,
+                                        void* stream) {
+    return process_call(h, PROC_BACK | PROC_PROFILES | (h_ids ? PROC_IDS : 0), d_frames, d_out, h_ids, n, nullptr,
+                        h_profiles, set, d_results, stream);
 }
 
 static const char* STAGE_NAMES[LT_NSTAGES] = {"begin", "undistort", "warp", "erode55", "erode29", "tophat55", "tophat29",
@@ -559,7 +748,8 @@ void lt_prof_mark(lt_handle* h, int stage, cudaStream_t st) {
 extern "C" int lt_profile_begin(lt_handle* h, int32_t max_calls) {
     if (!h || max_calls < 1 || max_calls > 4096) { lt_set_error("bad argument"); return -1; }
     LT_CUDA(cudaSetDevice(h->cfg.device));
-    int need = max_calls * 32;
+    // a call marks at most about 20 boundaries, plus the threshold and noise stages once per filter group
+    int need = max_calls * (32 + 2 * LT_MAX_PROFILES);
     if (need > h->prof_cap) {
         cudaEvent_t* ev = new cudaEvent_t[need];
         for (int i = 0; i < need; ++i) LT_CUDA(cudaEventCreate(&ev[i]));

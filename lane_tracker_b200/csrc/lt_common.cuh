@@ -50,6 +50,13 @@ struct LtAttemptParams {   // parameters of one attempt, device-visible
     double mu, start_slice, partial;
 };
 
+// One parameter profile (lt_set_profile) as the kernels read it.
+struct LtProfile {
+    LtAttemptParams p;
+    lt_validity val;
+    int n_tries;
+};
+
 // Scratch result of one search+fit+validity pass for one stream.
 struct LtAttemptOut {
     int detected, valid, mode, rank_def;
@@ -62,10 +69,19 @@ struct LtAttemptOut {
 // The buffers the stateless front half of a frame (undistort, warp, filter) produces and the stateful back half
 // (search, second attempt, state update, overlay) consumes.  A handle owns two sets so that the front half of batch
 // k+1 can run on one CUDA stream while the back half of batch k runs on another (lt_process_front / lt_process_back).
+// A front half with profiles (lt_process_front_profiles) also leaves the batch's profile snapshot in its set: the
+// back half reads the snapshot, never the live table, so lt_set_profile may run with work in flight.
 struct LtFrontSet {
     uint32_t* und_roi;
     uint32_t* pad_alloc[6];
     uint32_t* merged; uint32_t* mask;
+    int* group_pos;              // [S] batch positions ordered by filter group (bilateral groups first)
+    int* pos_profile;            // [S] profile index of each batch position
+    LtProfile* profiles;         // [LT_MAX_PROFILES] copy of the profile table
+    // host copy of the snapshot: lt_process_back_profiles checks its arguments against it
+    int* h_pos_profile;          // [S]
+    int snap_n;                  // batch size of the last front half with profiles; 0: the last front half took lt_params
+    LtProfile snap[LT_MAX_PROFILES];
 };
 
 struct lt_handle {
@@ -73,6 +89,8 @@ struct lt_handle {
     LtDims d;
     int S;                       // max streams
     lt_validity val;             // check_validity windows
+    LtProfile profiles[LT_MAX_PROFILES];   // lt_set_profile
+    unsigned profiles_set;       // bit k: profile k was set
     int bands_key[3], bands_val[2];   // cached band split of the paired morphology launch (n, height, slots)
     int sm_count;
     int src0, src1;              // frame rows the undistort of the ROI reads: [src0, src1)
@@ -176,8 +194,19 @@ int lt_launch_overlay_nv12(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out
 // rows [r0, r1) of NV12 frames -> RGB (nothing outside those rows is written)
 int lt_launch_nv12_to_rgb(const uint8_t* d_nv12, uint8_t* d_rgb, int n, int w, int h, int r0, int r1, cudaStream_t st);
 
+// The filter of one attempt over the whole batch, or over list[0..*count) when count != NULL (the retry list).
 int lt_launch_filter(lt_handle* h, int n, const LtAttemptParams& p, const int* list, const int* count,
                      cudaStream_t st);
+// One filter group of a batch: the positions list[0..n) (list == NULL: positions 0..n-1) filtered with p.
+struct LtFilterGroup {
+    LtAttemptParams p;
+    const int* list;
+    int n;
+};
+// The filter of a batch of n positions split into disjoint groups g[0..ng) that cover it.  The bilateral groups come
+// first and their lists are consecutive in one device array, so that g[0].list covers all their positions (the
+// morphology runs once over them).  count != NULL (device count of a retry list) only with ng == 1.
+int lt_launch_filter_groups(lt_handle* h, int n, const LtFilterGroup* g, int ng, const int* count, cudaStream_t st);
 int lt_launch_morph_pair(lt_handle* h, bool tophat, int n, const int* list, const int* count, cudaStream_t st);
 int lt_launch_mask_to_u8(lt_handle* h, const uint32_t* bits, uint8_t* d_mask, int n, cudaStream_t st);
 int lt_launch_u8_to_mask(lt_handle* h, const uint8_t* d_mask, uint32_t* bits, int n, cudaStream_t st);
@@ -194,9 +223,13 @@ struct LtSearchArgs {
     int by_stream;               // index pixel/centroid outputs by stream id instead of launch slot
     const int* ids;              // [n] state slot per batch position (NULL: identity): state reads, by_stream outputs
 };
+// prof / pos_prof (device, may be NULL): position s takes its validity windows -- and, with prof_params, its attempt
+// parameters instead of p -- from prof[pos_prof[s]]; its n_tries in lt_launch_select_retry.
 int lt_launch_search(lt_handle* h, int n, const LtAttemptParams& p, const LtSearchArgs& a, const int* list,
-                     const int* count, cudaStream_t st);
-int lt_launch_select_retry(lt_handle* h, int n, int n_tries, cudaStream_t st);
+                     const int* count, cudaStream_t st, const LtProfile* prof = nullptr, const int* pos_prof = nullptr,
+                     int prof_params = 0);
+int lt_launch_select_retry(lt_handle* h, int n, int n_tries, cudaStream_t st, const LtProfile* prof = nullptr,
+                           const int* pos_prof = nullptr);
 int lt_launch_update_state(lt_handle* h, int n, const int* ids, lt_result* d_results, int attempts_allowed,
                            cudaStream_t st);
 int lt_launch_fit_pixels(lt_handle* h, const uint32_t* d_pixels, int cap, const int* d_counts, int n,

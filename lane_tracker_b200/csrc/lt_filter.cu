@@ -851,7 +851,7 @@ static int launch_box_pair(lt_handle* h, int block_r, int c_r, int block_b, int 
     const int pitch_r = box_pitch(half_r), pitch_b = box_pitch(half_b);
     size_t smem = (size_t)CROSSH_ROWS * (pitch_r > pitch_b ? pitch_r : pitch_b) * sizeof(unsigned short);
     { int rc = lt_ensure_smem((const void*)k_box_h, smem); if (rc) return rc; }
-    const int zs = list ? (n < 8 ? n : 8) : n;      // retry-list launches: few slots, each CTA loops over the list
+    const int zs = count ? (n < 8 ? n : 8) : n;     // retry-list launches: few slots, each CTA loops over the list
     dim3 gh(lt_div_up(d.bv_h, CROSSH_ROWS), zs, 2);
     k_box_h<<<gh, CROSSH_WARPS * 32, smem, st>>>(h->planeR, h->planeB, h->topR, h->topB, d, half_r, half_b, pitch_r, pitch_b, d.pp,
                                                  h->stream_pad, h->stream_pad, list, count, n);
@@ -865,44 +865,65 @@ static int launch_box_pair(lt_handle* h, int block_r, int c_r, int block_b, int 
 
 int lt_launch_filter(lt_handle* h, int n, const LtAttemptParams& p, const int* list, const int* count,
                      cudaStream_t st) {
+    const LtFilterGroup g = {p, list, n};
+    return lt_launch_filter_groups(h, n, &g, 1, count, st);
+}
+
+int lt_launch_filter_groups(lt_handle* h, int n, const LtFilterGroup* g, int ng, const int* count, cudaStream_t st) {
     const LtDims& d = h->d;
     int rc;
-    if (p.filter_type == 0) {
-        if ((rc = lt_launch_morph_pair(h, false, n, list, count, st))) return rc;
+    // the morphology has no parameters: one pair of launches over the positions of every bilateral group
+    int n_morph = 0;
+    for (int i = 0; i < ng && g[i].p.filter_type == 0; ++i) n_morph += g[i].n;
+    if (n_morph > 0) {
+        const int* ml = (n_morph == n && count == nullptr) ? nullptr : g[0].list;
+        if ((rc = lt_launch_morph_pair(h, false, n_morph, ml, count, st))) return rc;
         lt_prof_mark(h, ST_ERODE55, st);            // both erosions (55x55 on Lab-b, 29x29 on R), two concurrent kernels
-        if ((rc = lt_launch_morph_pair(h, true, n, list, count, st))) return rc;
+        if ((rc = lt_launch_morph_pair(h, true, n_morph, ml, count, st))) return rc;
         lt_prof_mark(h, ST_TOPHAT55, st);           // both dilations + top-hat epilogues
-        if (list == nullptr) {
-            // The four threshold halves (R/Lab-b x horizontal/vertical) only OR bits into the merged mask and each
-            // of them fills about half of the issue slots: the horizontal pair runs on a side stream, the vertical
-            // pair on the caller's stream.  (Stage "cross_b" then reports both planes.)
-            LT_CUDA(cudaMemsetAsync(h->merged, 0, (size_t)n * h->stream_mask * sizeof(uint32_t), st));
-            LT_CUDA(cudaEventRecord(h->ev_fork, st));
-            LT_CUDA(cudaStreamWaitEvent(h->side, h->ev_fork, 0));
-            if ((rc = launch_cross_h(h, h->topR, h->merged, p.ksize_r, p.C_r, 1, n, list, count, h->side, h->topB, p.ksize_b, p.C_b))) return rc;
-            LT_CUDA(cudaEventRecord(h->ev_join, h->side));
-            if ((rc = launch_cross_v(h, h->topR, h->merged, p.ksize_r, p.C_r, n, list, count, st, true, h->topB, p.ksize_b, p.C_b))) return rc;
-            LT_CUDA(cudaStreamWaitEvent(st, h->ev_join, 0));
-            lt_prof_mark(h, ST_CROSS_B, st);
+    }
+    bool zeroed = false;
+    for (int i = 0; i < ng; ++i) {
+        const LtAttemptParams& p = g[i].p;
+        const int* list = g[i].list;
+        const int gn = g[i].n;
+        if (p.filter_type == 0) {
+            if (count == nullptr) {
+                // The four threshold halves (R/Lab-b x horizontal/vertical) only OR bits into the merged mask and each
+                // of them fills about half of the issue slots: the horizontal pair runs on a side stream, the vertical
+                // pair on the caller's stream.  (Stage "cross_b" then reports both planes.)  The merged masks of the
+                // whole batch are cleared once: the box threshold of a neighbourhood group rewrites every word.
+                if (!zeroed) LT_CUDA(cudaMemsetAsync(h->merged, 0, (size_t)n * h->stream_mask * sizeof(uint32_t), st));
+                zeroed = true;
+                LT_CUDA(cudaEventRecord(h->ev_fork, st));
+                LT_CUDA(cudaStreamWaitEvent(h->side, h->ev_fork, 0));
+                if ((rc = launch_cross_h(h, h->topR, h->merged, p.ksize_r, p.C_r, 1, gn, list, nullptr, h->side, h->topB, p.ksize_b, p.C_b))) return rc;
+                LT_CUDA(cudaEventRecord(h->ev_join, h->side));
+                if ((rc = launch_cross_v(h, h->topR, h->merged, p.ksize_r, p.C_r, gn, list, nullptr, st, true, h->topB, p.ksize_b, p.C_b))) return rc;
+                LT_CUDA(cudaStreamWaitEvent(st, h->ev_join, 0));
+                lt_prof_mark(h, ST_CROSS_B, st);
+            } else {
+                if ((rc = launch_cross(h, h->topR, h->merged, p.ksize_r, p.C_r, 0, gn, list, count, st, true))) return rc;
+                lt_prof_mark(h, ST_CROSS_R, st);
+                if ((rc = launch_cross(h, h->topB, h->merged, p.ksize_b, p.C_b, 1, gn, list, count, st, true))) return rc;
+                lt_prof_mark(h, ST_CROSS_B, st);
+            }
         } else {
-            if ((rc = launch_cross(h, h->topR, h->merged, p.ksize_r, p.C_r, 0, n, list, count, st, true))) return rc;
-            lt_prof_mark(h, ST_CROSS_R, st);
-            if ((rc = launch_cross(h, h->topB, h->merged, p.ksize_b, p.C_b, 1, n, list, count, st, true))) return rc;
-            lt_prof_mark(h, ST_CROSS_B, st);
+            if ((rc = launch_box_pair(h, p.ksize_r, p.C_r, p.ksize_b, p.C_b, gn, list, count, st))) return rc;
+            lt_prof_mark(h, ST_BOX, st);
         }
-    } else {
-        if ((rc = launch_box_pair(h, p.ksize_r, p.C_r, p.ksize_b, p.C_b, n, list, count, st))) return rc;
-        lt_prof_mark(h, ST_BOX, st);
+        if (p.mask_noise) {
+            // h->mask of the group's own positions holds the noise bits until k_open5 overwrites it
+            if ((rc = launch_cross(h, h->planeB, h->mask, p.ksize_noise, p.C_noise, 0, gn, list, count, st, false))) return rc;
+            dim3 gz(d.p2 / 32, d.bv_h, gn);
+            k_noise_combine<<<gz, 32, 0, st>>>(h->planeB, h->mask, h->merged, d, p.noise_thresh, d.pp, h->stream_pad,
+                                               h->stream_mask, list, count);
+            LT_LAUNCH_CHECK();
+            lt_prof_mark(h, ST_NOISE, st);
+        }
     }
-    if (p.mask_noise) {
-        if ((rc = launch_cross(h, h->planeB, h->mask, p.ksize_noise, p.C_noise, 0, n, list, count, st, false))) return rc;
-        dim3 g(d.p2 / 32, d.bv_h, n);
-        k_noise_combine<<<g, 32, 0, st>>>(h->planeB, h->mask, h->merged, d, p.noise_thresh, d.pp, h->stream_pad,
-                                          h->stream_mask, list, count);
-        LT_LAUNCH_CHECK();
-        lt_prof_mark(h, ST_NOISE, st);
-    }
-    const int zs = list ? (n < 8 ? n : 8) : n;
+    const int* list = ng == 1 ? g[0].list : nullptr;
+    const int zs = count ? (n < 8 ? n : 8) : n;
     const int band = zs >= 16 ? OPEN_BAND : OPEN_BAND_FEW;
     dim3 go(lt_div_up(lt_div_up(d.mwords, OPEN_CORE), 2), lt_div_up(d.bv_h, band), zs);
     k_open5<<<go, 64, 0, st>>>(h->merged, h->mask, d, h->stream_mask, list, count, n, band);

@@ -294,12 +294,21 @@ __device__ int poly_points(const double* cf, double partial, int W, int H, int* 
 // search + fit + validity for one attempt
 // ---------------------------------------------------------------------------
 
+// PROF: position s takes its validity windows, and with prof_params its attempt parameters, from prof[pos_prof[s]]
+// (the parameter profiles of the batch) instead of V and p.
+template <bool PROF>
 __global__ void __launch_bounds__(SEARCH_THREADS)
 k_search(LtDims d, LtAttemptParams p, LtSearchArgs a, const LtDevState* __restrict__ state, int n_reset, lt_validity V,
-         size_t bits_stride, const int* __restrict__ list, const int* __restrict__ count, int lev_chunk) {
+         size_t bits_stride, const int* __restrict__ list, const int* __restrict__ count, int lev_chunk,
+         const LtProfile* __restrict__ prof, const int* __restrict__ pos_prof, int prof_params) {
     int slot = blockIdx.x;
     if (count != nullptr && slot >= *count) return;
     const int s = list ? list[slot] : slot;              // batch position: mask, att, coeffs
+    if (PROF) {
+        const LtProfile& q = prof[pos_prof[s]];
+        V = q.val;
+        if (prof_params) p = q.p;
+    }
     const int sid = a.ids ? a.ids[s] : s;                // state slot of its stream: state, by_stream outputs
     const int W = d.bv_w, H = d.bv_h, tid = threadIdx.x;
     const uint32_t* mask = a.mask + (size_t)s * bits_stride;
@@ -586,15 +595,22 @@ k_search(LtDims d, LtAttemptParams p, LtSearchArgs a, const LtDevState* __restri
 static size_t search_smem(const LtDims& d) { return (size_t)(10 * d.bv_h + d.bv_w + 64 + 2 * d.bv_h) * sizeof(int); }
 
 int lt_launch_search(lt_handle* h, int n, const LtAttemptParams& p, const LtSearchArgs& a, const int* list,
-                     const int* count, cudaStream_t st) {
+                     const int* count, cudaStream_t st, const LtProfile* prof, const int* pos_prof, int prof_params) {
     if (p.window_width < 1 || p.window_height < 1) { lt_set_error("window size must be positive"); return -1; }
     // + prefix-sum rows of the sliding-window levels: as many levels per chunk as fit next to the per-row tables
     const size_t base = search_smem(h->d), per_level = (size_t)(h->d.bv_w + 1) * sizeof(int), budget = 200 * 1024;
     int lev_chunk = base + per_level < budget ? (int)((budget - base) / per_level) : 1;
     lev_chunk = lev_chunk < 1 ? 1 : (lev_chunk > LT_MAX_LEVELS ? LT_MAX_LEVELS : lev_chunk);
     const size_t smem = base + (size_t)lev_chunk * per_level;
-    { int rc = lt_ensure_smem((const void*)k_search, smem); if (rc) return rc; }
-    k_search<<<n, SEARCH_THREADS, smem, st>>>(h->d, p, a, h->state, h->cfg.n_reset, h->val, h->stream_mask, list, count, lev_chunk);
+    if (prof) {
+        { int rc = lt_ensure_smem((const void*)k_search<true>, smem); if (rc) return rc; }
+        k_search<true><<<n, SEARCH_THREADS, smem, st>>>(h->d, p, a, h->state, h->cfg.n_reset, h->val, h->stream_mask, list, count,
+                                                        lev_chunk, prof, pos_prof, prof_params);
+    } else {
+        { int rc = lt_ensure_smem((const void*)k_search<false>, smem); if (rc) return rc; }
+        k_search<false><<<n, SEARCH_THREADS, smem, st>>>(h->d, p, a, h->state, h->cfg.n_reset, h->val, h->stream_mask, list, count,
+                                                         lev_chunk, nullptr, nullptr, 0);
+    }
     LT_LAUNCH_CHECK();
     return 0;
 }
@@ -603,12 +619,15 @@ int lt_launch_search(lt_handle* h, int n, const LtAttemptParams& p, const LtSear
 // attempt-2 selection (lane_tracker.py:1071)
 // ---------------------------------------------------------------------------
 
+// PROF: n_tries of position s is prof[pos_prof[s]].n_tries
+template <bool PROF>
 __global__ void k_select_retry(const LtAttemptOut* __restrict__ att, int n, int n_tries, int* list, int* count,
-                               int* flags) {
+                               int* flags, const LtProfile* __restrict__ prof, const int* __restrict__ pos_prof) {
     // single CTA, ordered compaction so that the retry list is deterministic
     if (threadIdx.x == 0) {
         int c = 0;
         for (int s = 0; s < n; ++s) {
+            if (PROF) n_tries = prof[pos_prof[s]].n_tries;
             bool retry = ((!att[s].detected) | (!att[s].valid)) & ((n_tries >= 2) | (n_tries == -1));
             flags[s] = retry;
             if (retry) list[c++] = s;
@@ -617,8 +636,13 @@ __global__ void k_select_retry(const LtAttemptOut* __restrict__ att, int n, int 
     }
 }
 
-int lt_launch_select_retry(lt_handle* h, int n, int n_tries, cudaStream_t st) {
-    k_select_retry<<<1, 32, 0, st>>>(h->att, n, n_tries, h->retry_list, h->retry_count, h->draw_flags + h->S);
+int lt_launch_select_retry(lt_handle* h, int n, int n_tries, cudaStream_t st, const LtProfile* prof, const int* pos_prof) {
+    if (prof)
+        k_select_retry<true><<<1, 32, 0, st>>>(h->att, n, n_tries, h->retry_list, h->retry_count, h->draw_flags + h->S, prof,
+                                               pos_prof);
+    else
+        k_select_retry<false><<<1, 32, 0, st>>>(h->att, n, n_tries, h->retry_list, h->retry_count, h->draw_flags + h->S,
+                                                nullptr, nullptr);
     LT_LAUNCH_CHECK();
     return 0;
 }

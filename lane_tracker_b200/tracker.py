@@ -175,6 +175,27 @@ class BatchedLaneTracker:
             setattr(v, k, float(val))
         check(self.lib.lt_set_validity(self._h, C.byref(v)))
 
+    def set_profile(self, k, params=None, validity=None, **kw):
+        """Store parameter profile k (0 <= k < LT_MAX_PROFILES) for the ``profiles=`` argument of the process calls:
+        ``params`` (default: ``make_params(**kw)``) and the check_validity windows ``validity``, a dict with the keys of
+        ``set_validity`` (missing keys and None: the shipped windows).  A batch uses the profiles as they stood when its
+        front half was enqueued, so this may be called with work in flight.
+
+            bt.set_profile(1, validity=presets.DEMO_1["validity"], **presets.DEMO_1["process"])
+        """
+        p = params if params is not None else make_params(**kw)
+        if params is not None and kw:
+            raise ValueError("pass either params or keyword options, not both")
+        v = None
+        if validity is not None:
+            from .presets import SHIPPED_VALIDITY
+            v = _lib.lt_validity(**{key: float(val) for key, val in SHIPPED_VALIDITY.items()})
+            for key, val in validity.items():
+                if not hasattr(v, key):
+                    raise TypeError("unknown validity option %r" % key)
+                setattr(v, key, float(val))
+        check(self.lib.lt_set_profile(self._h, int(k), C.byref(p), C.byref(v) if v is not None else None))
+
     def set_text(self, enable=True):
         """Install (or remove) the glyph sprites of the reference's putText overlays (lane_tracker.py:653-659, 668-672)."""
         from .text import TextSprites
@@ -312,6 +333,31 @@ class BatchedLaneTracker:
             raise ValueError("stream id %d appears more than once in the batch" % int(u[counts > 1][0]))
         return (C.c_int32 * n)(*[int(v) for v in a])
 
+    def _check_profiles(self, profiles, n):
+        """Profile indices of a batch of n frames -> ctypes int32 array (None: None).  Any int sequence, NumPy array or
+        CPU tensor of n indices in [0, LT_MAX_PROFILES); frame i uses profile profiles[i] (see ``set_profile``)."""
+        if profiles is None:
+            return None
+        if isinstance(profiles, torch.Tensor):
+            if profiles.is_cuda:
+                raise ValueError("profiles must be host data (a sequence, a NumPy array or a CPU tensor), not a CUDA tensor")
+            profiles = profiles.numpy()
+        a = np.asarray(profiles)
+        if a.ndim != 1 or (a.size and a.dtype.kind not in "iu"):
+            raise ValueError("profiles must be a 1-D sequence of integers")
+        if a.size != n:
+            raise ValueError("got %d profile indices for %d frames" % (a.size, n))
+        bad = np.flatnonzero((a < 0) | (a >= _lib.LT_MAX_PROFILES))
+        if bad.size:
+            raise ValueError("profile %d at batch position %d outside [0, %d)"
+                             % (int(a[bad[0]]), int(bad[0]), _lib.LT_MAX_PROFILES))
+        return (C.c_int32 * n)(*[int(v) for v in a])
+
+    @staticmethod
+    def _no_params_with_profiles(profiles, params, kw):
+        if profiles is not None and (params is not None or kw):
+            raise ValueError("profiles= selects the parameters of every frame: pass it without params or keyword options")
+
     def _check_out(self, out, frames):
         """out: RGB [n, H, W, 3] for RGB and NV12 frames alike."""
         if out is None:
@@ -323,7 +369,7 @@ class BatchedLaneTracker:
         if out.data_ptr() % 4:
             raise ValueError("out must start at a 4-byte aligned address (the kernels access frames as 32-bit words)")
 
-    def process_async(self, frames, out=None, params=None, results_dev=None, ids=None, **kw):
+    def process_async(self, frames, out=None, params=None, results_dev=None, ids=None, profiles=None, **kw):
         """Enqueue one frame per stream on the current CUDA stream; returns the number of frames.
 
         frames: uint8 CUDA tensor [n, H, W, 3] (RGB) or [n, H * 3 / 2, W] (NV12: the luma plane, then interleaved
@@ -332,32 +378,53 @@ class BatchedLaneTracker:
         results_dev: optional uint8 CUDA buffer of n * RESULT_DTYPE.itemsize bytes (default: internal).
         ids: None -- frame i belongs to stream i; else n distinct stream ids in [0, n_streams), any order (int
         sequence, NumPy array or CPU tensor): frame i belongs to stream ids[i], and the streams not listed keep their
-        state.  out and the result records stay in batch order."""
-        return self._process_call(frames, out, None, params, results_dev, ids, kw)
+        state.  out and the result records stay in batch order.
+        profiles: None -- every frame uses ``params`` (or ``make_params(**kw)``); else n profile indices (any int
+        sequence, NumPy array or CPU tensor; see ``set_profile``): frame i uses profile profiles[i], and ``params`` /
+        keyword options may not be given."""
+        return self._process_call(frames, out, None, params, results_dev, ids, kw, profiles)
 
-    def process_front_async(self, frames, buffer_set, params=None, **kw):
+    def process_front_async(self, frames, buffer_set, params=None, profiles=None, **kw):
         """First half of ``process_async`` (undistort, warp, first-attempt filter) into intermediate buffer set
-        0 or 1, on the current CUDA stream.  Stateless.  See ``DevicePipeline``.  RGB or NV12 frames."""
+        0 or 1, on the current CUDA stream.  Stateless.  See ``DevicePipeline``.  RGB or NV12 frames.  With
+        ``profiles``, the back half of this buffer set must be given the same profile indices."""
         n = self._input(frames)
+        self._no_params_with_profiles(profiles, params, kw)
+        h_prof = self._check_profiles(profiles, n)
+        if h_prof is not None:
+            check(self.lib.lt_process_front_profiles(self._h, _ptr(frames), h_prof, n, int(buffer_set),
+                                                     _stream_ptr(self.device)))
+            return n
         p = params if params is not None else make_params(**kw)
         check(self.lib.lt_process_front(self._h, _ptr(frames), n, C.byref(p), int(buffer_set), _stream_ptr(self.device)))
         return n
 
-    def process_back_async(self, frames, out, buffer_set, params=None, results_dev=None, ids=None, **kw):
+    def process_back_async(self, frames, out, buffer_set, params=None, results_dev=None, ids=None, profiles=None, **kw):
         """Second half of ``process_async`` (searches, second attempt, state machine, overlay) from intermediate
         buffer set 0 or 1, on the current CUDA stream.  Advances the per-stream state of the streams in ``ids``
-        (None: streams 0..n-1), as ``process_async``.  RGB or NV12 frames, as given to the front half."""
-        return self._process_call(frames, out, buffer_set, params, results_dev, ids, kw)
+        (None: streams 0..n-1), as ``process_async``.  RGB or NV12 frames, as given to the front half.  ``profiles``:
+        those the front half of this buffer set was given."""
+        return self._process_call(frames, out, buffer_set, params, results_dev, ids, kw, profiles)
 
-    def _process_call(self, frames, out, buffer_set, params, results_dev, ids, kw):
+    def _process_call(self, frames, out, buffer_set, params, results_dev, ids, kw, profiles=None):
         """Checks and C call of ``process_async`` (buffer_set None: both halves) or ``process_back_async``; -> n."""
         n = self._input(frames)
         self._check_out(out, frames)
         h_ids = self._check_ids(ids, n)
-        p = params if params is not None else make_params(**kw)
+        self._no_params_with_profiles(profiles, params, kw)
+        h_prof = self._check_profiles(profiles, n)
         res = self._results_dev if results_dev is None else results_dev
         if res.numel() < n * RESULT_DTYPE.itemsize or not res.is_cuda:
             raise ValueError("results buffer too small")
+        if h_prof is not None:
+            if buffer_set is None:
+                check(self.lib.lt_process_profiles(self._h, _ptr(frames), _ptr(out), h_ids, h_prof, n, _ptr(res),
+                                                   _stream_ptr(self.device)))
+            else:
+                check(self.lib.lt_process_back_profiles(self._h, _ptr(frames), _ptr(out), h_ids, h_prof, n,
+                                                        int(buffer_set), _ptr(res), _stream_ptr(self.device)))
+            return n
+        p = params if params is not None else make_params(**kw)
         if buffer_set is None:
             plain, streams, set_arg = self.lib.lt_process, self.lib.lt_process_streams, ()
         else:
@@ -377,10 +444,11 @@ class BatchedLaneTracker:
         torch.cuda.current_stream(self.device).synchronize()
         return self._results_host[:nbytes].numpy().view(RESULT_DTYPE).copy()
 
-    def process(self, frames, out=None, params=None, ids=None, **kw):
+    def process(self, frames, out=None, params=None, ids=None, profiles=None, **kw):
         """``process_async`` followed by ``fetch_results``: the n result records, in batch order.  With ``ids``, frame
-        i advances stream ids[i] and the other streams keep their state."""
-        n = self.process_async(frames, out, params, ids=ids, **kw)
+        i advances stream ids[i] and the other streams keep their state; with ``profiles``, frame i uses parameter
+        profile profiles[i] (``set_profile``)."""
+        n = self.process_async(frames, out, params, ids=ids, profiles=profiles, **kw)
         return self.fetch_results(n)
 
     # -- stage methods (device tensors) ---------------------------------------
@@ -648,12 +716,17 @@ class GraphedProcess:
 
         g = GraphedProcess(tracker, n_streams)          # static device buffers g.frames / g.out
         g.frames.copy_(batch, non_blocking=True); g.replay(); results = g.fetch_results()
+
+    With ``profiles`` (n profile indices, see ``BatchedLaneTracker.set_profile``) frame i uses profile profiles[i].
+    The graph holds the profile indices and the profile table as they stood at capture time: a later ``set_profile``
+    does not reach it (capture a new ``GraphedProcess`` instead).
     """
 
-    def __init__(self, tracker, n=None, overlay=True, params=None, frame_format="rgb"):
+    def __init__(self, tracker, n=None, overlay=True, params=None, frame_format="rgb", profiles=None):
         """frame_format 'nv12': ``self.frames`` is NV12 [n, H * 3 / 2, W]; ``self.out`` stays RGB."""
         if frame_format not in _FRAME_FORMATS:
             raise ValueError("frame_format must be 'rgb' or 'nv12'")
+        BatchedLaneTracker._no_params_with_profiles(profiles, params, {})
         self.t = tracker
         n = tracker.n_streams if n is None else int(n)
         dev = tracker.device
@@ -663,20 +736,24 @@ class GraphedProcess:
         self.frames = torch.zeros(shape, dtype=torch.uint8, device=dev)
         self.out = torch.empty((n, h, w, 3), dtype=torch.uint8, device=dev) if overlay else None
         self.results_dev = torch.zeros(n * RESULT_DTYPE.itemsize, dtype=torch.uint8, device=dev)
-        self.params = params if params is not None else make_params()
+        self.params = params if params is not None or profiles is not None else make_params()
+        self.profiles = None if profiles is None else np.array(profiles, dtype=np.int64)
+        tracker._check_profiles(self.profiles, n)
         # first-use initialisation (module load, shared-memory attributes) cannot happen inside a capture: run the
         # chain once for real on a side stream, with the tracking state saved and restored around it
         saved = [tracker.get_state(s) for s in range(n)]
         side = torch.cuda.Stream(dev)
         side.wait_stream(torch.cuda.current_stream(dev))
         with torch.cuda.stream(side):
-            tracker.process_async(self.frames, self.out, params=self.params, results_dev=self.results_dev)
+            tracker.process_async(self.frames, self.out, params=self.params, results_dev=self.results_dev,
+                                  profiles=self.profiles)
         side.synchronize()
         for s, (st, lx, rx) in enumerate(saved):
             tracker.set_state(s, st, lx, rx)
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph, stream=side):
-            tracker.process_async(self.frames, self.out, params=self.params, results_dev=self.results_dev)
+            tracker.process_async(self.frames, self.out, params=self.params, results_dev=self.results_dev,
+                                  profiles=self.profiles)
         torch.cuda.current_stream(dev).wait_stream(side)
 
     def replay(self):
@@ -701,6 +778,8 @@ class DevicePipeline:
 
     ``submit(frames, out, ids=...)`` advances the listed streams only (see ``BatchedLaneTracker.process_async``);
     results stay in batch order.  ``frames`` may be RGB or NV12 (``out`` is RGB either way), batch by batch.
+    ``submit(..., profiles=...)`` gives frame i parameter profile profiles[i] (``BatchedLaneTracker.set_profile``)
+    instead of the pipeline's ``params``.
     """
 
     def __init__(self, tracker, params=None):
@@ -715,9 +794,12 @@ class DevicePipeline:
         self.results_dev = [torch.zeros(tracker.n_streams * RESULT_DTYPE.itemsize, dtype=torch.uint8, device=dev)
                             for _ in range(2)]
 
-    def submit(self, frames, out=None, ids=None):
+    def submit(self, frames, out=None, ids=None, profiles=None):
         dev = self.t.device
-        self.t._check_ids(ids, self.t._frame_format(frames)[0])   # refuse bad frames / ids before anything is enqueued
+        n = self.t._frame_format(frames)[0]
+        self.t._check_ids(ids, n)                      # refuse bad frames / ids / profiles before anything is enqueued
+        self.t._check_profiles(profiles, n)
+        params = self.params if profiles is None else None
         k, bs = self._k, self._k & 1
         ready = torch.cuda.Event()
         ready.record(torch.cuda.current_stream(dev))            # frames (and out) belong to the caller until here
@@ -725,13 +807,14 @@ class DevicePipeline:
             self.s_front.wait_event(ready)
             if self._back_done[bs] is not None:
                 self.s_front.wait_event(self._back_done[bs])    # set `bs` is free again
-            self.t.process_front_async(frames, bs, params=self.params)
+            self.t.process_front_async(frames, bs, params=params, profiles=profiles)
             front_done = torch.cuda.Event()
             front_done.record(self.s_front)
         with torch.cuda.stream(self.s_back):
             self.s_back.wait_event(front_done)
             self.s_back.wait_event(ready)
-            self.t.process_back_async(frames, out, bs, params=self.params, results_dev=self.results_dev[bs], ids=ids)
+            self.t.process_back_async(frames, out, bs, params=params, results_dev=self.results_dev[bs], ids=ids,
+                                      profiles=profiles)
             done = torch.cuda.Event()
             done.record(self.s_back)
         self._back_done[bs] = done
@@ -776,7 +859,8 @@ class HostPipeline:
         for out, results in pipe.drain(): ...
 
     ``submit(batch, ids=...)`` advances the listed streams only (see ``BatchedLaneTracker.process_async``); the
-    frames and records of a finished batch are in batch order.
+    frames and records of a finished batch are in batch order.  ``submit(batch, profiles=...)`` gives frame i
+    parameter profile profiles[i] (``BatchedLaneTracker.set_profile``) instead of the pipeline's ``params``.
     """
 
     def __init__(self, tracker, depth=3, overlay=True, params=None, inplace=False, frame_format="rgb"):
@@ -831,7 +915,7 @@ class HostPipeline:
         self.tail = 0          # oldest slot in flight
         self.inflight = 0
 
-    def submit(self, host_frames, ids=None):
+    def submit(self, host_frames, ids=None, profiles=None):
         if self.inflight == self.depth:
             raise RuntimeError("pipeline full: collect a finished batch first")
         if not (host_frames.dtype == torch.uint8 and host_frames.is_pinned() and host_frames.is_contiguous()):
@@ -842,7 +926,9 @@ class HostPipeline:
             raise ValueError("host_frames must be %s [n, %s] with 1 <= n <= %d, got %s"
                              % ("NV12" if self.nv12 else "RGB", ", ".join(map(str, sl["d_in"].shape[1:])),
                                 self.t.n_streams, list(host_frames.shape)))
-        self.t._check_ids(ids, n)                        # refuse bad ids before anything is enqueued
+        self.t._check_ids(ids, n)                        # refuse bad ids / profiles before anything is enqueued
+        self.t._check_profiles(profiles, n)
+        params = self.params if profiles is None else None
         sl["n"] = n
         with torch.cuda.stream(self.s_in):
             self.s_in.wait_event(sl["e_run"])            # the kernels that last read this input buffer are done
@@ -863,14 +949,15 @@ class HostPipeline:
             self.s_front.wait_event(sl["e_in"])
             if self._set_free[bs] is not None:
                 self.s_front.wait_event(self._set_free[bs])
-            self.t.process_front_async(sl["d_in"][:n], bs, params=self.params)
+            self.t.process_front_async(sl["d_in"][:n], bs, params=params, profiles=profiles)
             e_front = torch.cuda.Event()
             e_front.record(self.s_front)
         with torch.cuda.stream(self.s_run):
             self.s_run.wait_event(e_front)
             self.s_run.wait_event(sl["e_out"])           # the previous D2H out of this output buffer is done
             d_out = sl["d_in"][:n] if self.inplace else (sl["d_out"][:n] if self.overlay else None)
-            self.t.process_back_async(sl["d_in"][:n], d_out, bs, params=self.params, results_dev=sl["d_res"], ids=ids)
+            self.t.process_back_async(sl["d_in"][:n], d_out, bs, params=params, results_dev=sl["d_res"], ids=ids,
+                                      profiles=profiles)
             sl["e_run"].record(self.s_run)
         self._set_free[bs] = sl["e_run"]
         with torch.cuda.stream(self.s_out):
