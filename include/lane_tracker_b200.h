@@ -217,6 +217,51 @@ int lt_process_front_profiles(lt_handle* h, const uint8_t* d_frames, const int32
 int lt_process_back_profiles(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids,
                              const int32_t* h_profiles, int32_t n, int32_t set, lt_result* d_results, void* stream);
 
+/* Cameras: one batch whose frames come from differently calibrated cameras (another mounting: its own warp M / Minv;
+ * another lens: its own cam_matrix / dist_coeffs; and the metres per pixel of its bird's-eye view).  Image size,
+ * bird's-eye size, n_fail / n_reset / n_average and print_frame_count stay those of the handle.
+ * A handle holds up to LT_MAX_CAMERAS cameras.  Camera 0 is the calibration given to lt_create and cannot be changed;
+ * lt_set_camera sets camera `camera` (1 <= camera < LT_MAX_CAMERAS) to `cam`, the same fields lt_config carries (taken
+ * as given, like lt_create takes them).  It builds the camera's remap tables on the device and is synchronous (it
+ * synchronises the device and may reallocate the intermediate buffer the camera calls undistort into).  A camera
+ * cannot be unset.  Refused: camera 0, an index out of range, a NULL cam, and a call while a buffer set holds the front
+ * half of a camera call whose back half has not been enqueued yet (the back half would draw with tables its front half
+ * did not see). */
+#define LT_MAX_CAMERAS 64
+typedef struct lt_camera {
+    double cam_matrix[9];         /* row-major 3x3 */
+    double dist_coeffs[5];        /* k1 k2 p1 p2 k3 */
+    double M[9];                  /* warp_matrices[0] */
+    double Minv[9];               /* warp_matrices[1] */
+    double mppv, mpph;            /* mpp_conversion */
+} lt_camera;
+int lt_set_camera(lt_handle* h, int32_t camera, const lt_camera* cam);
+
+/* lt_process_streams / lt_process_profiles and their halves with a camera per batch position:
+ *   h_cameras : HOST int32 [n], position i was filmed by camera h_cameras[i] (its undistort, warp, overlay and the
+ *               metres per pixel of its curve radii and eccentricity).  Cameras belong to batch positions, like
+ *               profiles: a caller that keeps one camera per stream passes camera_of[ids].  A stream may change camera
+ *               between frames; its tracking state carries over (reset a re-mounted camera's stream with lt_reset).
+ *               Copied when the call is enqueued: nothing synchronises and the calls are capturable in a CUDA graph.
+ *   params / h_profiles: exactly one is non-NULL (lt_process_streams or lt_process_profiles semantics).
+ *   h_ids     : as lt_process_streams; NULL means the identity 0..n-1.
+ * A batch whose positions all use camera 0 runs exactly the launches of the call without cameras.  Otherwise the front
+ * half undistorts into a buffer of its own whose slots are grouped by camera; everything after the warp is indexed by
+ * batch position as before.  Every check of lt_process_streams / lt_process_profiles applies, in the same order; then,
+ * before anything is enqueued and naming the position: a NULL h_cameras, an index outside [0, LT_MAX_CAMERAS), a
+ * camera never set, and remap mode 1 (the fused variant has camera 0's calibration baked in).
+ * lt_process_back_cameras refuses a buffer set whose last front half was not lt_process_front_cameras, or had another
+ * n or other camera indices.  Ordering as lt_process_back.
+ * lt_process_cameras(...) == lt_process_front_cameras(..., 0, stream) + lt_process_back_cameras(..., 0, ..., stream). */
+int lt_process_cameras(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids,
+                       const int32_t* h_cameras, int32_t n, const lt_params* params, const int32_t* h_profiles,
+                       lt_result* d_results, void* stream);
+int lt_process_front_cameras(lt_handle* h, const uint8_t* d_frames, const int32_t* h_cameras, int32_t n,
+                             const lt_params* params, const int32_t* h_profiles, int32_t set, void* stream);
+int lt_process_back_cameras(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids,
+                            const int32_t* h_cameras, int32_t n, const lt_params* params, const int32_t* h_profiles,
+                            int32_t set, lt_result* d_results, void* stream);
+
 /* Keep the ordered lane-pixel sets and window centroids of every lt_process call so that
  * lt_read_capture can return them (the reference exposes them as the attributes left_x/left_y/
  * right_x/right_y/left_window_centroids, lane_tracker.py:159-166).  Off by default: the
@@ -415,7 +460,9 @@ int lt_set_state(lt_handle* h, int32_t stream_id, const lt_state* h_state, const
  *       first,last+1, pair-plane width, mask words per row, pixel-list capacity of lt_read_capture, frame rows the
  *       tracker reads first,last+1}, 11 int32[3] = {row bands of the 55x55 and of the 29x29 morphology jobs in the
  *       last filter launch, SM count of the device}, 12 lane row spans of the last lt_draw_lane call (int32 [bv_h][2];
- *       9 is the per-stream cache that lt_process re-draws on failing frames).
+ *       9 is the per-stream cache that lt_process re-draws on failing frames), 13 int32[6] = {undistorted ROI
+ *       first,last+1, overlay rows first,last+1, frame rows the tracker reads first,last+1} of camera stream_id
+ *       (lt_set_camera; stream_id in [0, LT_MAX_CAMERAS)).  Items 0-2 and 10 describe camera 0.
  * Copies to HOST memory; synchronous. Returns bytes written or <0. */
 int64_t lt_debug_read(lt_handle* h, int32_t what, int32_t stream_id, void* h_dst, int64_t capacity);
 

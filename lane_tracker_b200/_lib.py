@@ -13,6 +13,7 @@ LIB_PATH = os.path.join(HERE, "liblane_tracker_b200.so")
 
 LT_MAX_AVERAGE = 8
 LT_MAX_PROFILES = 16
+LT_MAX_CAMERAS = 64
 LT_MAX_LEVELS = 128
 LT_ABI_VERSION = 4
 LT_NSTAGES = 16
@@ -26,6 +27,11 @@ class lt_config(C.Structure):
                 ("mppv", f64), ("mpph", f64),
                 ("n_fail", i32), ("n_reset", i32), ("n_average", i32), ("print_frame_count", i32),
                 ("max_streams", i32), ("device", i32)]
+
+
+class lt_camera(C.Structure):
+    _fields_ = [("cam_matrix", f64 * 9), ("dist_coeffs", f64 * 5), ("M", f64 * 9), ("Minv", f64 * 9),
+                ("mppv", f64), ("mpph", f64)]
 
 
 class lt_params(C.Structure):
@@ -92,6 +98,12 @@ SIGNATURES = {
     "lt_process_profiles": (C.c_int, [P, P, P, C.POINTER(i32), C.POINTER(i32), i32, P, P]),
     "lt_process_front_profiles": (C.c_int, [P, P, C.POINTER(i32), i32, i32, P]),
     "lt_process_back_profiles": (C.c_int, [P, P, P, C.POINTER(i32), C.POINTER(i32), i32, i32, P, P]),
+    "lt_set_camera": (C.c_int, [P, i32, C.POINTER(lt_camera)]),
+    "lt_process_cameras": (C.c_int, [P, P, P, C.POINTER(i32), C.POINTER(i32), i32, C.POINTER(lt_params), C.POINTER(i32),
+                                     P, P]),
+    "lt_process_front_cameras": (C.c_int, [P, P, C.POINTER(i32), i32, C.POINTER(lt_params), C.POINTER(i32), i32, P]),
+    "lt_process_back_cameras": (C.c_int, [P, P, P, C.POINTER(i32), C.POINTER(i32), i32, C.POINTER(lt_params),
+                                          C.POINTER(i32), i32, P, P]),
     "lt_set_capture": (C.c_int, [P, i32]),
     "lt_set_pixel_capacity": (C.c_int, [P, i32]),
     "lt_read_capture": (C.c_int, [P, i32, i32, i32, P, i32, C.POINTER(i32), P, C.POINTER(i32)]),

@@ -155,9 +155,16 @@ extern "C" int lt_destroy(lt_handle* h) {
     for (int k = 0; k < 2; ++k) {
         const LtFrontSet& f = h->fs[k];
         void* fp[] = {f.und_roi, f.pad_alloc[0], f.pad_alloc[1], f.pad_alloc[2], f.pad_alloc[3], f.pad_alloc[4], f.pad_alloc[5],
-                      f.merged, f.mask, f.group_pos, f.pos_profile, f.profiles};
+                      f.merged, f.mask, f.group_pos, f.pos_profile, f.profiles, f.und_cam, f.slot_pos, f.chunk_cam,
+                      f.pos_cam, f.cams};
         for (void* p : fp) if (p) cudaFree(p);
         delete[] f.h_pos_profile;
+        delete[] f.h_pos_cam;
+    }
+    for (int k = 1; k < LT_MAX_CAMERAS; ++k) {     // camera 0's tables are the handle's own, freed below
+        const LtCamera& c = h->cams[k];
+        void* cp[] = {c.und_map, c.bv_map, c.ov_map, c.und_desc, c.bv_desc};
+        for (void* p : cp) if (p) cudaFree(p);
     }
     void* ptrs[] = {h->und_map, h->bv_map, h->ov_map, h->bv_desc, h->und_desc, h->lab_yz, h->fused_desc, h->lab_gamma, h->lab_cbrt, h->lane_rows, h->lane_bbox, h->dl_bbox,
                     h->avg_x, h->state, h->att, h->retry_list, h->retry_count, h->draw_flags, h->stream_ids, h->vis_scratch,
@@ -172,6 +179,17 @@ extern "C" int lt_destroy(lt_handle* h) {
     if (h->ev_join) cudaEventDestroy(h->ev_join);
     delete h;
     return 0;
+}
+
+// (re)allocate the camera undistort buffer of a front set at the handle's stride and capacity, zeroed: its row 0 and
+// column 0 are the zero border of the und layout and are never written
+static int alloc_und_cam(lt_handle* h, LtFrontSet& f) {
+    if (f.und_cam) cudaFree(f.und_cam);
+    f.und_cam = nullptr;
+    const size_t words = (size_t)(h->und_cam_slots / LT_UND_GROUP) * lt_und_cam_group_words(h);
+    int rc = dev_alloc(&f.und_cam, words);
+    if (!rc) LT_CUDA(cudaMemset(f.und_cam, 0, words * sizeof(uint32_t)));
+    return rc;
 }
 
 // allocate one set of front-half buffers (LtFrontSet) and give its padded planes their pad values
@@ -195,6 +213,13 @@ static int alloc_front_set(lt_handle* h, int k) {
     if (!rc) rc = dev_alloc(&f.pos_profile, S);
     if (!rc) rc = dev_alloc(&f.profiles, LT_MAX_PROFILES);
     if (!rc) f.h_pos_profile = new int[S];
+    // camera batches: at most S + 3 S slots (a run of one camera pads to a multiple of four)
+    if (!rc) rc = dev_alloc(&f.slot_pos, 4 * S);
+    if (!rc) rc = dev_alloc(&f.chunk_cam, S);
+    if (!rc) rc = dev_alloc(&f.pos_cam, S);
+    if (!rc) rc = dev_alloc(&f.cams, LT_MAX_CAMERAS);
+    if (!rc) f.h_pos_cam = new int[S];
+    if (!rc && h->und_cam_slots) rc = alloc_und_cam(h, f);
     return rc;
 }
 
@@ -207,6 +232,69 @@ static void select_set(lt_handle* h, int k) {
     h->tmpR = f.pad_alloc[2] + origin;   h->tmpB = f.pad_alloc[3] + origin;
     h->topR = f.pad_alloc[4] + origin;   h->topB = f.pad_alloc[5] + origin;
     h->merged = f.merged; h->mask = f.mask;
+}
+
+// The rows of a calibration, from its maps: rows of the undistorted frame that the bird's-eye view can touch (the ROI),
+// frame rows the undistort of the ROI reads (for partial host->device transfers), frame rows the overlay can touch.
+static int camera_rows(const lt_handle* h, LtCamera& c) {
+    const LtDims& d = h->d;
+    const size_t npx = (size_t)d.img_w * d.img_h, nbv = (size_t)d.bv_w * d.bv_h;
+    std::vector<int2> m(nbv);
+    cudaError_t e = cudaMemcpy(m.data(), c.bv_map, nbv * sizeof(int2), cudaMemcpyDeviceToHost);
+    if (e != cudaSuccess) { lt_set_error("map build failed: %s", cudaGetErrorString(e)); return -2; }
+    int r0 = d.img_h, r1 = 0;
+    for (size_t i = 0; i < nbv; ++i) {
+        int sx = m[i].x >> 5, sy = m[i].y >> 5;
+        if (sx + 1 < 0 || sx >= d.img_w) continue;
+        for (int yy = sy; yy <= sy + 1; ++yy)
+            if (yy >= 0 && yy < d.img_h) { r0 = yy < r0 ? yy : r0; r1 = yy + 1 > r1 ? yy + 1 : r1; }
+    }
+    if (r0 >= r1) { r0 = 0; r1 = 1; }
+    c.roi0 = r0; c.roi1 = r1;
+    {   // frame rows read by the undistort of the ROI rows (for partial host->device transfers)
+        std::vector<int2> u((size_t)(r1 - r0) * d.img_w);
+        cudaMemcpy(u.data(), c.und_map + (size_t)r0 * d.img_w, u.size() * sizeof(int2), cudaMemcpyDeviceToHost);
+        int s0 = d.img_h, s1 = 0;
+        for (size_t i = 0; i < u.size(); ++i) {
+            int sy = u[i].y >> 5;
+            for (int yy = sy; yy <= sy + 1; ++yy)
+                if (yy >= 0 && yy < d.img_h) { s0 = yy < s0 ? yy : s0; s1 = yy + 1 > s1 ? yy + 1 : s1; }
+        }
+        if (s0 >= s1) { s0 = 0; s1 = d.img_h; }
+        c.src0 = s0; c.src1 = s1;
+    }
+    std::vector<int2> o(npx);
+    cudaMemcpy(o.data(), c.ov_map, npx * sizeof(int2), cudaMemcpyDeviceToHost);
+    int o0 = d.img_h, o1 = 0;
+    for (int y = 0; y < d.img_h; ++y)
+        for (int x = 0; x < d.img_w; ++x) {
+            int2 q = o[(size_t)y * d.img_w + x];
+            int sx = q.x >> 5, sy = q.y >> 5;
+            if (sx + 1 >= 0 && sx < d.bv_w && sy + 1 >= 0 && sy < d.bv_h) { o0 = y < o0 ? y : o0; o1 = y + 1 > o1 ? y + 1 : o1; }
+        }
+    if (o0 >= o1) { o0 = 0; o1 = 0; }
+    c.ov0 = o0; c.ov1 = o1;
+    return 0;
+}
+
+// The tables of calibration c.cal on the device (synchronous): maps, rows, then the tap descriptors of its ROI.
+// On failure, what was allocated is left in c for the caller to free.
+static int build_camera(lt_handle* h, LtCamera& c) {
+    const size_t npx = (size_t)h->d.img_w * h->d.img_h, nbv = (size_t)h->d.bv_w * h->d.bv_h;
+    int rc = 0;
+    if (!rc) rc = dev_alloc(&c.und_map, npx);
+    if (!rc) rc = dev_alloc(&c.bv_map, nbv);
+    if (!rc) rc = dev_alloc(&c.ov_map, npx);
+    if (!rc) rc = lt_launch_build_maps(c.cal, h->d, c.und_map, c.bv_map, c.ov_map, 0);
+    if (!rc) rc = camera_rows(h, c);
+    if (rc) return rc;
+    LtDims d = h->d;
+    d.roi0 = c.roi0; d.roi1 = c.roi1; d.ov0 = c.ov0; d.ov1 = c.ov1;
+    if (!rc) rc = dev_alloc(&c.bv_desc, nbv);
+    if (!rc) rc = lt_launch_build_desc(c.bv_map, c.bv_desc, d, 0);
+    if (!rc) rc = dev_alloc(&c.und_desc, (size_t)(d.roi1 - d.roi0) * d.img_w);
+    if (!rc) rc = lt_launch_build_und_desc(c.und_map, c.und_desc, d, 0);
+    return rc;
 }
 
 extern "C" int lt_create(const lt_config* cfg, lt_handle** out) {
@@ -239,54 +327,22 @@ extern "C" int lt_create(const lt_config* cfg, lt_handle** out) {
     const size_t S = h->S, npx = (size_t)d.img_w * d.img_h, nbv = (size_t)d.bv_w * d.bv_h;
     int rc = 0;
 #define A(ptr, n) if (!rc) rc = dev_alloc(&h->ptr, (n))
-    A(und_map, npx); A(bv_map, nbv); A(ov_map, npx); A(lab_gamma, 256); A(lab_cbrt, 3072);
+    A(lab_gamma, 256); A(lab_cbrt, 3072);
     if (rc) { lt_destroy(h); return rc; }
+    LtCamera& c0 = h->cams[0];
+    memcpy(c0.cal.cam_matrix, cfg->cam_matrix, sizeof(c0.cal.cam_matrix));
+    memcpy(c0.cal.dist_coeffs, cfg->dist_coeffs, sizeof(c0.cal.dist_coeffs));
+    memcpy(c0.cal.M, cfg->M, sizeof(c0.cal.M));
+    memcpy(c0.cal.Minv, cfg->Minv, sizeof(c0.cal.Minv));
+    c0.cal.mppv = cfg->mppv; c0.cal.mpph = cfg->mpph;
+    rc = build_camera(h, c0);
+    h->und_map = c0.und_map; h->bv_map = c0.bv_map; h->ov_map = c0.ov_map; h->und_desc = c0.und_desc; h->bv_desc = c0.bv_desc;
+    if (rc) { lt_destroy(h); return rc; }
+    d.roi0 = c0.roi0; d.roi1 = c0.roi1; d.ov0 = c0.ov0; d.ov1 = c0.ov1;
+    h->src0 = c0.src0; h->src1 = c0.src1;
     cudaStream_t st = 0;
-    if ((rc = lt_launch_build_maps(h, st))) { lt_destroy(h); return rc; }
     cudaMemcpy(h->lab_gamma, LT_LAB_GAMMA, sizeof(LT_LAB_GAMMA), cudaMemcpyHostToDevice);
     cudaMemcpy(h->lab_cbrt, LT_LAB_CBRT, sizeof(LT_LAB_CBRT), cudaMemcpyHostToDevice);
-    // rows of the undistorted frame that the bird's-eye view can touch / frame rows the overlay can touch
-    {
-        std::vector<int2> m(nbv);
-        cudaError_t e = cudaMemcpy(m.data(), h->bv_map, nbv * sizeof(int2), cudaMemcpyDeviceToHost);
-        if (e != cudaSuccess) { lt_set_error("map build failed: %s", cudaGetErrorString(e)); lt_destroy(h); return -2; }
-        int r0 = d.img_h, r1 = 0;
-        for (size_t i = 0; i < nbv; ++i) {
-            int sx = m[i].x >> 5, sy = m[i].y >> 5;
-            if (sx + 1 < 0 || sx >= d.img_w) continue;
-            for (int yy = sy; yy <= sy + 1; ++yy)
-                if (yy >= 0 && yy < d.img_h) { r0 = yy < r0 ? yy : r0; r1 = yy + 1 > r1 ? yy + 1 : r1; }
-        }
-        if (r0 >= r1) { r0 = 0; r1 = 1; }
-        d.roi0 = r0; d.roi1 = r1;
-        {   // frame rows read by the undistort of the ROI rows (for partial host->device transfers)
-            std::vector<int2> u((size_t)(r1 - r0) * d.img_w);
-            cudaMemcpy(u.data(), h->und_map + (size_t)r0 * d.img_w, u.size() * sizeof(int2), cudaMemcpyDeviceToHost);
-            int s0 = d.img_h, s1 = 0;
-            for (size_t i = 0; i < u.size(); ++i) {
-                int sy = u[i].y >> 5;
-                for (int yy = sy; yy <= sy + 1; ++yy)
-                    if (yy >= 0 && yy < d.img_h) { s0 = yy < s0 ? yy : s0; s1 = yy + 1 > s1 ? yy + 1 : s1; }
-            }
-            if (s0 >= s1) { s0 = 0; s1 = d.img_h; }
-            h->src0 = s0; h->src1 = s1;
-        }
-        std::vector<int2> o(npx);
-        cudaMemcpy(o.data(), h->ov_map, npx * sizeof(int2), cudaMemcpyDeviceToHost);
-        int o0 = d.img_h, o1 = 0;
-        for (int y = 0; y < d.img_h; ++y)
-            for (int x = 0; x < d.img_w; ++x) {
-                int2 q = o[(size_t)y * d.img_w + x];
-                int sx = q.x >> 5, sy = q.y >> 5;
-                if (sx + 1 >= 0 && sx < d.bv_w && sy + 1 >= 0 && sy < d.bv_h) { o0 = y < o0 ? y : o0; o1 = y + 1 > o1 ? y + 1 : o1; }
-            }
-        if (o0 >= o1) { o0 = 0; o1 = 0; }
-        d.ov0 = o0; d.ov1 = o1;
-    }
-    A(bv_desc, nbv);
-    if (!rc) rc = lt_launch_build_desc(h, st);
-    A(und_desc, (size_t)(d.roi1 - d.roi0) * d.img_w);
-    if (!rc) rc = lt_launch_build_und_desc(h, st);
     A(lab_yz, 768);
     if (!rc) rc = lt_launch_build_lab_yz(h, st);
     if (!rc) rc = alloc_front_set(h, 0);
@@ -330,6 +386,49 @@ extern "C" int lt_reset(lt_handle* h, const int32_t* ids, int32_t n) {
     return 0;
 }
 
+extern "C" int lt_set_camera(lt_handle* h, int32_t camera, const lt_camera* cam) {
+    if (!h) { lt_set_error("null handle"); return -1; }
+    if (camera == 0) { lt_set_error("camera 0 is the calibration given to lt_create and cannot be changed"); return -1; }
+    if (camera < 1 || camera >= LT_MAX_CAMERAS) { lt_set_error("camera %d outside [1, %d)", camera, LT_MAX_CAMERAS); return -1; }
+    if (!cam) { lt_set_error("null camera"); return -1; }
+    for (int k = 0; k < 2; ++k)
+        if (h->fs[k].cam_pending) {
+            lt_set_error("buffer set %d holds the front half of a camera batch whose back half has not been enqueued: "
+                         "enqueue it before lt_set_camera", k);
+            return -1;
+        }
+    LT_CUDA(cudaSetDevice(h->cfg.device));
+    LT_CUDA(cudaDeviceSynchronize());        // no work in flight reads the tables replaced below
+    LtCamera c;
+    memset(&c, 0, sizeof(c));
+    c.cal = *cam;
+    int rc = build_camera(h, c);
+    if (!rc && cudaDeviceSynchronize() != cudaSuccess) {
+        lt_set_error("camera tables: %s", cudaGetErrorString(cudaGetLastError()));
+        rc = -2;
+    }
+    LtCamera& old = rc ? c : h->cams[camera];      // on failure the camera keeps its previous tables
+    void* cp[] = {old.und_map, old.bv_map, old.ov_map, old.und_desc, old.bv_desc};
+    for (void* p : cp) if (p) cudaFree(p);
+    if (rc) return rc;
+    h->cams[camera] = c;
+    // the camera undistort buffer: the stride of the tallest ROI, S + 3 min(S, cameras) slots in groups of 16
+    int rows = 0, ncams = 0;
+    for (int k = 0; k < LT_MAX_CAMERAS; ++k)
+        if (h->cams[k].und_map) {
+            ++ncams;
+            rows = h->cams[k].roi1 - h->cams[k].roi0 > rows ? h->cams[k].roi1 - h->cams[k].roi0 : rows;
+        }
+    const int slots = (h->S + 3 * (h->S < ncams ? h->S : ncams) + LT_UND_GROUP - 1) / LT_UND_GROUP * LT_UND_GROUP;
+    if (rows > h->und_cam_rows || slots > h->und_cam_slots) {
+        h->und_cam_rows = rows > h->und_cam_rows ? rows : h->und_cam_rows;
+        h->und_cam_slots = slots > h->und_cam_slots ? slots : h->und_cam_slots;
+        for (int k = 0; k < 2; ++k)
+            if (h->fs[k].mask && (rc = alloc_und_cam(h, h->fs[k]))) return rc;
+    }
+    return 0;
+}
+
 static int check_any_n(lt_handle* h, int n) {   // stage calls that touch no per-stream buffer of the handle
     if (!h) { lt_set_error("null handle"); return -1; }
     if (n < 1) { lt_set_error("n_streams must be positive"); return -1; }
@@ -346,13 +445,25 @@ static int check_n(lt_handle* h, int n) {
 // process()
 // ---------------------------------------------------------------------------
 
+// The undistort and warp of a camera batch: nslots slots of f.und_cam, max_rows the tallest ROI of its cameras.
+struct LtCamBatch {
+    const LtFrontSet* f;
+    int nslots, max_rows;
+};
+
 // find_lane_points (lane_tracker.py:795-874) of the first attempt up to the binary mask, all streams: stateless.
-// The filter groups g[0..ng) cover the batch (one group {p1, NULL, n} without profiles).
-static int process_front(lt_handle* h, const uint8_t* d_frames, int n, const LtFilterGroup* g, int ng, cudaStream_t st) {
+// The filter groups g[0..ng) cover the batch (one group {p1, NULL, n} without profiles).  cb: a camera batch (NULL:
+// every position uses camera 0).
+static int process_front(lt_handle* h, const uint8_t* d_frames, int n, const LtFilterGroup* g, int ng, cudaStream_t st,
+                         const LtCamBatch* cb) {
     int rc;
     if (h->prof_active && h->prof_calls >= h->prof_max_calls) h->prof_active = 0;
     lt_prof_mark(h, ST_BEGIN, st);
-    if (h->remap_mode == 1) {
+    if (cb) {
+        if ((rc = lt_launch_undistort_cams(h, *cb->f, d_frames, cb->nslots, cb->max_rows, st))) return rc;
+        lt_prof_mark(h, ST_UNDISTORT, st);
+        if ((rc = lt_launch_warp_cams(h, *cb->f, cb->nslots, st))) return rc;
+    } else if (h->remap_mode == 1) {
         if ((rc = lt_launch_warp_fused(h, d_frames, nullptr, n, st))) return rc;
     } else {
         if ((rc = lt_launch_undistort(h, d_frames, n, st))) return rc;
@@ -417,7 +528,7 @@ static bool same_filter(const LtAttemptParams& a, const LtAttemptParams& b) {
 // front stream: the back half of this batch runs after it, the front half of batch k+2 after that back half), group
 // the positions by filter configuration, and run the front half over the groups.
 static int process_front_profiles(lt_handle* h, const uint8_t* d_frames, const int32_t* h_prof, int n, int set,
-                                  cudaStream_t st) {
+                                  cudaStream_t st, const LtCamBatch* cb) {
     LtFrontSet& f = h->fs[set];
     LtProfileTable t;
     memcpy(t.e, h->profiles, sizeof(t.e));
@@ -454,7 +565,56 @@ static int process_front_profiles(lt_handle* h, const uint8_t* d_frames, const i
         }
         if ((rc = upload_ints(pos.data(), n, f.group_pos, st))) return rc;
     }
-    return process_front(h, d_frames, n, g, nrep, st);
+    return process_front(h, d_frames, n, g, nrep, st, cb);
+}
+
+struct LtCamTable {
+    LtCamDev e[LT_MAX_CAMERAS];
+};
+
+__global__ void k_set_cameras(LtCamTable t, LtCamDev* __restrict__ dst) {
+    if (threadIdx.x < LT_MAX_CAMERAS) dst[threadIdx.x] = t.e[threadIdx.x];
+}
+
+// Front half with cameras, first step: record the batch's cameras in buffer set `set`.  A batch on camera 0 alone
+// leaves it at that (it runs the launches without cameras).  Otherwise the slots of und_cam are laid out -- positions
+// stably sorted by camera, each camera's run padded to whole chunks of four slots -- and the slot positions, chunk
+// cameras, position cameras and the camera snapshot are uploaded on the front stream (kernel arguments, as the
+// profiles: the back half of this batch runs after them, the front half of batch k+2 after that back half).
+static int prepare_cameras(lt_handle* h, const int32_t* h_cams, int n, int set, cudaStream_t st, LtCamBatch* cb) {
+    LtFrontSet& f = h->fs[set];
+    memcpy(f.h_pos_cam, h_cams, (size_t)n * sizeof(int32_t));
+    f.cam_n = n;
+    int count[LT_MAX_CAMERAS] = {0};
+    for (int i = 0; i < n; ++i) count[h_cams[i]]++;
+    f.cam_plain = count[0] == n;
+    if (f.cam_plain) return 0;
+    int next[LT_MAX_CAMERAS], nslots = 0, max_rows = 0, ov0 = h->d.img_h, ov1 = 0;
+    LtCamTable t;
+    memset(&t, 0, sizeof(t));
+    for (int k = 0; k < LT_MAX_CAMERAS; ++k) {
+        const LtCamera& c = h->cams[k];
+        if (c.und_map) t.e[k] = {c.und_desc, c.bv_desc, c.ov_map, (c.roi1 - c.roi0) * h->d.img_w, c.ov0, c.ov1, c.cal.mppv, c.cal.mpph};
+        next[k] = nslots;
+        if (!count[k]) continue;
+        nslots += (count[k] + 3) & ~3;
+        max_rows = c.roi1 - c.roi0 > max_rows ? c.roi1 - c.roi0 : max_rows;
+        if (c.ov1 > c.ov0) { ov0 = c.ov0 < ov0 ? c.ov0 : ov0; ov1 = c.ov1 > ov1 ? c.ov1 : ov1; }
+    }
+    std::vector<int> slot_pos(nslots, -1), chunk_cam(nslots / 4);
+    for (int k = 0; k < LT_MAX_CAMERAS; ++k)
+        for (int s = next[k]; s < next[k] + ((count[k] + 3) & ~3); s += 4) chunk_cam[s / 4] = k;
+    for (int i = 0; i < n; ++i) slot_pos[next[h_cams[i]]++] = i;
+    int rc;
+    if ((rc = upload_ints(slot_pos.data(), nslots, f.slot_pos, st))) return rc;
+    if ((rc = upload_ints(chunk_cam.data(), nslots / 4, f.chunk_cam, st))) return rc;
+    if ((rc = upload_ints(h_cams, n, f.pos_cam, st))) return rc;
+    k_set_cameras<<<1, LT_MAX_CAMERAS, 0, st>>>(t, f.cams);
+    LT_LAUNCH_CHECK();
+    f.cam_ov0 = ov1 > ov0 ? ov0 : 0;
+    f.cam_ov1 = ov1 > ov0 ? ov1 : 0;
+    *cb = {&f, nslots, max_rows};
+    return 0;
 }
 
 static bool allows_retry(int n_tries) { return n_tries >= 2 || n_tries == -1; }
@@ -463,9 +623,10 @@ static bool allows_retry(int n_tries) { return n_tries >= 2 || n_tries == -1; }
 // h_ids (host, validated by check_ids) maps batch position i to state slot h_ids[i]; NULL: the identity.
 // fs: the buffer set whose profile snapshot the batch uses (NULL: p1 and the handle's windows for every position);
 // n_tries: of the batch (with profiles: 2 when some position may take a second attempt, else 1).
+// cf: the buffer set of a camera batch that is not on camera 0 alone (NULL otherwise).
 static int process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, int n_tries,
                         const LtAttemptParams& p1, lt_result* d_results, cudaStream_t st, bool own_begin,
-                        const int32_t* h_ids, const LtFrontSet* fs) {
+                        const int32_t* h_ids, const LtFrontSet* fs, const LtFrontSet* cf) {
     int rc;
     const LtAttemptParams p2 = second_attempt();
     const LtProfile* prof = fs ? fs->profiles : nullptr;
@@ -501,7 +662,7 @@ static int process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, i
         if ((rc = lt_launch_search(h, n, p2, sa, h->retry_list, h->retry_count, st, prof, pos_prof, 0))) return rc;
         lt_prof_mark(h, ST_SEARCH, st);
     }
-    if ((rc = lt_launch_update_state(h, n, ids, d_results, two ? 2 : 1, st))) return rc;
+    if ((rc = lt_launch_update_state(h, n, ids, d_results, two ? 2 : 1, st, cf))) return rc;
     lt_prof_mark(h, ST_UPDATE, st);
     if (d_out) {
         // (copying the untouched rows on a side stream under the search kernels was measured: the copy saturates HBM
@@ -509,7 +670,10 @@ static int process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, i
         // draw_lane writes its text into the frame BEFORE the blend (lane_tracker.py:653-662).  With the shipped
         // geometry the text rows and the rows the lane overlay can reach are disjoint and the order is immaterial;
         // when they overlap (other calibrations) the text goes first and the blend runs in place over it.
-        const bool text_under_blend = h->txt_nchars > 0 && h->txt_row0 < h->d.ov1 && h->d.ov0 < h->txt_row1;
+        // (a camera batch: the union of its cameras' overlay rows; for a camera whose rows miss the text rows, the
+        // order of text and blend does not matter)
+        const int ov0 = cf ? cf->cam_ov0 : h->d.ov0, ov1 = cf ? cf->cam_ov1 : h->d.ov1;
+        const bool text_under_blend = h->txt_nchars > 0 && h->txt_row0 < ov1 && ov0 < h->txt_row1;
         // NV12 input: the frame is converted where it is read; with text under the blend, the whole frame is converted
         // into d_out first and the text and the blend then run on d_out as for RGB.
         const bool nv12 = h->frame_format == LT_FRAME_NV12;
@@ -520,10 +684,10 @@ static int process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, i
                 LT_CUDA(cudaMemcpyAsync(d_out, d_frames, (size_t)n * h->d.img_w * h->d.img_h * 3, cudaMemcpyDeviceToDevice, st));
             }
             if ((rc = lt_launch_text(h, d_out, n, ids, st))) return rc;
-            if ((rc = lt_launch_overlay(h, d_out, d_out, n, h->draw_flags, ids, st))) return rc;
+            if ((rc = lt_launch_overlay(h, d_out, d_out, n, h->draw_flags, ids, st, cf))) return rc;
         } else {
-            if (nv12) rc = lt_launch_overlay_nv12(h, d_frames, d_out, n, h->draw_flags, ids, st);
-            else rc = lt_launch_overlay(h, d_frames, d_out, n, h->draw_flags, ids, st);
+            if (nv12) rc = lt_launch_overlay_nv12(h, d_frames, d_out, n, h->draw_flags, ids, st, cf);
+            else rc = lt_launch_overlay(h, d_frames, d_out, n, h->draw_flags, ids, st, cf);
             if (rc) return rc;
             if ((rc = lt_launch_text(h, d_out, n, ids, st))) return rc;
         }
@@ -623,13 +787,34 @@ static int check_profiles(lt_handle* h, const int32_t* h_prof, int n, int* bandw
     return 0;
 }
 
+// Camera indices of lt_process_*_cameras: every entry names a camera that is set; remap mode 1 (whose fused table
+// holds camera 0's calibration) takes camera 0 only.
+static int check_cameras(lt_handle* h, const int32_t* h_cams, int n) {
+    if (!h_cams) { lt_set_error("null camera list"); return -1; }
+    for (int i = 0; i < n; ++i) {
+        const int k = h_cams[i];
+        if (k < 0 || k >= LT_MAX_CAMERAS) {
+            lt_set_error("camera %d at batch position %d outside [0, %d)", k, i, LT_MAX_CAMERAS);
+            return -1;
+        }
+        if (!h->cams[k].und_map) { lt_set_error("camera %d at batch position %d is unset", k, i); return -1; }
+        if (k && h->remap_mode == 1) {
+            lt_set_error("camera %d at batch position %d: remap mode 1 (fused single resample) has camera 0's calibration "
+                         "built in; camera calls need remap mode 0", k, i);
+            return -1;
+        }
+    }
+    return 0;
+}
+
 // What one process entry point does: the front half, the back half or both, with or without a stream id list, with
-// one lt_params or with a parameter profile per batch position.
-enum { PROC_FRONT = 1, PROC_BACK = 2, PROC_IDS = 4, PROC_PROFILES = 8 };
+// one lt_params or with a parameter profile per batch position, and with or without a camera per batch position.
+enum { PROC_FRONT = 1, PROC_BACK = 2, PROC_IDS = 4, PROC_PROFILES = 8, PROC_CAMERAS = 16 };
 
 // The checks of the process entry points, in this order and all before anything is enqueued, then the halves.
 static int process_call(lt_handle* h, int what, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids, int n,
-                        const lt_params* params, const int32_t* h_prof, int set, lt_result* d_results, void* stream) {
+                        const lt_params* params, const int32_t* h_prof, int set, lt_result* d_results, void* stream,
+                        const int32_t* h_cams = nullptr) {
     int rc;
     LtAttemptParams p1;
     const bool front = what & PROC_FRONT, back = what & PROC_BACK, profiles = what & PROC_PROFILES;
@@ -672,20 +857,50 @@ static int process_call(lt_handle* h, int what, const uint8_t* d_frames, uint8_t
         bandwidth = p1.bandwidth;
         n_tries = params->n_tries;
     }
+    const bool cameras = what & PROC_CAMERAS;
+    if (cameras) {
+        if (profiles && params) { lt_set_error("params and h_profiles are exclusive: pass one of them"); return -1; }
+        if ((rc = check_cameras(h, h_cams, n))) return rc;
+        if (back && !front) {    // the front half of this set must have taken these cameras
+            const LtFrontSet& f = h->fs[set];
+            if (f.cam_n == 0) {
+                lt_set_error("buffer set %d was last filled by a front half without cameras", set);
+                return -1;
+            }
+            if (f.cam_n != n) {
+                lt_set_error("buffer set %d holds a camera front half of %d frames, not %d", set, f.cam_n, n);
+                return -1;
+            }
+            for (int i = 0; i < n; ++i)
+                if (f.h_pos_cam[i] != h_cams[i]) {
+                    lt_set_error("camera %d at batch position %d differs from the front half's camera %d", h_cams[i], i,
+                                 f.h_pos_cam[i]);
+                    return -1;
+                }
+        }
+    }
     if ((rc = process_set(h, set, bandwidth))) return rc;
     if (back && !d_results) { lt_set_error("null argument"); return -1; }
+    LtFrontSet& fset = h->fs[set];
     if (front) {
+        LtCamBatch cb = {nullptr, 0, 0};
+        fset.cam_n = 0;
+        if (cameras && (rc = prepare_cameras(h, h_cams, n, set, st, &cb))) return rc;
+        const LtCamBatch* cbp = cb.f ? &cb : nullptr;
         if (profiles) {
-            rc = process_front_profiles(h, d_frames, h_prof, n, set, st);
+            rc = process_front_profiles(h, d_frames, h_prof, n, set, st, cbp);
         } else {
-            h->fs[set].snap_n = 0;
+            fset.snap_n = 0;
             const LtFilterGroup g = {p1, nullptr, n};
-            rc = process_front(h, d_frames, n, &g, 1, st);
+            rc = process_front(h, d_frames, n, &g, 1, st, cbp);
         }
         if (rc) return rc;
+        fset.cam_pending = cameras && !back;
     }
-    return back ? process_back(h, d_frames, d_out, n, n_tries, p1, d_results, st, !front, h_ids, profiles ? &h->fs[set] : nullptr)
-                : 0;
+    if (!back) return 0;
+    fset.cam_pending = 0;
+    const LtFrontSet* cf = (cameras && !fset.cam_plain) ? &fset : nullptr;
+    return process_back(h, d_frames, d_out, n, n_tries, p1, d_results, st, !front, h_ids, profiles ? &fset : nullptr, cf);
 }
 
 extern "C" int lt_process(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int32_t n, const lt_params* params,
@@ -730,6 +945,26 @@ extern "C" int lt_process_back_profiles(lt_handle* h, const uint8_t* d_frames, u
                                         void* stream) {
     return process_call(h, PROC_BACK | PROC_PROFILES | (h_ids ? PROC_IDS : 0), d_frames, d_out, h_ids, n, nullptr,
                         h_profiles, set, d_results, stream);
+}
+
+extern "C" int lt_process_cameras(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids,
+                                  const int32_t* h_cameras, int32_t n, const lt_params* params, const int32_t* h_profiles,
+                                  lt_result* d_results, void* stream) {
+    return process_call(h, PROC_FRONT | PROC_BACK | PROC_CAMERAS | (h_profiles ? PROC_PROFILES : 0) | (h_ids ? PROC_IDS : 0),
+                        d_frames, d_out, h_ids, n, params, h_profiles, 0, d_results, stream, h_cameras);
+}
+
+extern "C" int lt_process_front_cameras(lt_handle* h, const uint8_t* d_frames, const int32_t* h_cameras, int32_t n,
+                                        const lt_params* params, const int32_t* h_profiles, int32_t set, void* stream) {
+    return process_call(h, PROC_FRONT | PROC_CAMERAS | (h_profiles ? PROC_PROFILES : 0), d_frames, nullptr, nullptr, n,
+                        params, h_profiles, set, nullptr, stream, h_cameras);
+}
+
+extern "C" int lt_process_back_cameras(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids,
+                                       const int32_t* h_cameras, int32_t n, const lt_params* params,
+                                       const int32_t* h_profiles, int32_t set, lt_result* d_results, void* stream) {
+    return process_call(h, PROC_BACK | PROC_CAMERAS | (h_profiles ? PROC_PROFILES : 0) | (h_ids ? PROC_IDS : 0), d_frames,
+                        d_out, h_ids, n, params, h_profiles, set, d_results, stream, h_cameras);
 }
 
 static const char* STAGE_NAMES[LT_NSTAGES] = {"begin", "undistort", "warp", "erode55", "erode29", "tophat55", "tophat29",
@@ -1362,6 +1597,15 @@ extern "C" int lt_set_state(lt_handle* h, int32_t id, const lt_state* hs, const 
 }
 
 extern "C" int64_t lt_debug_read(lt_handle* h, int32_t what, int32_t id, void* dst, int64_t cap) {
+    if (h && what == 13) {     // rows of camera `id` (host data, no synchronisation)
+        if (!dst || id < 0 || id >= LT_MAX_CAMERAS) { lt_set_error("bad argument"); return -1; }
+        const LtCamera& c = h->cams[id];
+        if (!c.und_map) { lt_set_error("camera %d is unset", id); return -1; }
+        int v[6] = {c.roi0, c.roi1, c.ov0, c.ov1, c.src0, c.src1};
+        if (cap < (int64_t)sizeof(v)) { lt_set_error("buffer too small"); return -1; }
+        memcpy(dst, v, sizeof(v));
+        return sizeof(v);
+    }
     if (!h || !dst || id < 0 || id >= h->S) { lt_set_error("bad argument"); return -1; }
     if (cudaSetDevice(h->cfg.device) != cudaSuccess || cudaDeviceSynchronize() != cudaSuccess) {
         lt_set_error("device error: %s", cudaGetErrorString(cudaGetLastError()));

@@ -57,6 +57,23 @@ struct LtProfile {
     int n_tries;
 };
 
+// One camera of a handle (lt_set_camera; camera 0 is the calibration of lt_create and uses the handle's tables).
+struct LtCamera {
+    lt_camera cal;
+    int2* und_map; int2* bv_map; int2* ov_map;    // [img_h][img_w], [bv_h][bv_w], [img_h][img_w]
+    int2* und_desc;              // [roi rows][img_w] tap descriptors of the undistort
+    int2* bv_desc;               // [bv_h][bv_w] tap descriptors of the warp (rows of this camera's ROI)
+    int roi0, roi1, ov0, ov1, src0, src1;         // as LtDims / lt_handle::src0, src1
+};
+
+// What the camera kernels read of one camera (a snapshot per front set, lt_process_front_cameras).
+struct LtCamDev {
+    const int2* und_desc; const int2* bv_desc; const int2* ov_map;
+    int roi_px;                  // undistorted ROI pixels: (roi1 - roi0) * img_w
+    int ov0, ov1;                // frame rows the overlay can reach
+    double mppv, mpph;
+};
+
 // Scratch result of one search+fit+validity pass for one stream.
 struct LtAttemptOut {
     int detected, valid, mode, rank_def;
@@ -82,6 +99,19 @@ struct LtFrontSet {
     int* h_pos_profile;          // [S]
     int snap_n;                  // batch size of the last front half with profiles; 0: the last front half took lt_params
     LtProfile snap[LT_MAX_PROFILES];
+    // Camera calls (lt_process_front_cameras): the undistorted ROI of such a batch goes to und_cam, whose slots are
+    // grouped by camera (runs of whole 16-byte chunks of four slots).  und_cam is separate from und_roi: the plain path
+    // relies on und_roi's zero rows below camera 0's ROI, which a taller camera would overwrite.
+    uint32_t* und_cam;           // [und_cam_slots / 16][lt_und_group_words of und_cam_rows rows]
+    int* slot_pos;               // [und_cam_slots] batch position of each slot, -1: pad
+    int* chunk_cam;              // [und_cam_slots / 4] camera of each chunk of four slots
+    int* pos_cam;                // [S] camera of each batch position
+    LtCamDev* cams;              // [LT_MAX_CAMERAS] snapshot of the camera tables
+    int* h_pos_cam;              // [S] host copy: lt_process_back_cameras checks its arguments against it
+    int cam_n;                   // batch size of the last front half with cameras; 0: the last front half took none
+    int cam_plain;               // that front half used camera 0 only (it ran the launches without cameras)
+    int cam_pending;             // a camera front half was enqueued alone and its back half not yet (lt_set_camera waits)
+    int cam_ov0, cam_ov1;        // union of the overlay rows of its cameras
 };
 
 struct lt_handle {
@@ -94,6 +124,8 @@ struct lt_handle {
     int bands_key[3], bands_val[2];   // cached band split of the paired morphology launch (n, height, slots)
     int sm_count;
     int src0, src1;              // frame rows the undistort of the ROI reads: [src0, src1)
+    LtCamera cams[LT_MAX_CAMERAS];   // [0] mirrors the tables above; [k] set by lt_set_camera (und_map != NULL)
+    int und_cam_rows, und_cam_slots; // stride (tallest ROI of the cameras set) and slot capacity of LtFrontSet::und_cam
     // shared tables
     int2* und_map;               // [img_h][img_w]
     int2* bv_map;                // [bv_h][bv_w]
@@ -144,6 +176,13 @@ struct lt_handle {
     size_t stream_mask;          // words per stream in a bit mask
 };
 
+// words per group of 16 slots of LtFrontSet::und_cam: the und layout at the stride of the tallest ROI of the cameras set
+static inline size_t lt_und_cam_group_words(const lt_handle* h) {
+    LtDims e = h->d;
+    e.roi0 = 0; e.roi1 = h->und_cam_rows;
+    return lt_und_group_words(e);
+}
+
 extern "C" int64_t lt_launch_count(void);
 void lt_count_launch(int n = 1);
 void lt_set_error(const char* fmt, ...);
@@ -177,20 +216,28 @@ int lt_ensure_smem(const void* func, size_t bytes);
 // masks, attempt outputs, draw flags and result records are indexed by batch position, the per-stream state
 // (tracking state, averaged polylines, cached lane polygon, captured pixel lists) by ids[position].
 
-int lt_launch_build_maps(lt_handle* h, cudaStream_t st);
-int lt_launch_build_desc(lt_handle* h, cudaStream_t st);
+// remap tables of one calibration; d: the handle's sizes and the calibration's ROI (roi0, roi1) for the descriptors
+int lt_launch_build_maps(const lt_camera& c, const LtDims& d, int2* und_map, int2* bv_map, int2* ov_map, cudaStream_t st);
+int lt_launch_build_desc(const int2* bv_map, int2* bv_desc, const LtDims& d, cudaStream_t st);
 int lt_launch_build_lab_yz(lt_handle* h, cudaStream_t st);
-int lt_launch_build_und_desc(lt_handle* h, cudaStream_t st);
+int lt_launch_build_und_desc(const int2* und_map, int2* und_desc, const LtDims& d, cudaStream_t st);
 int lt_launch_build_fused_desc(lt_handle* h, cudaStream_t st);
 int lt_launch_warp_fused(lt_handle* h, const uint8_t* d_frames, uint8_t* d_bv_rgb, int n, cudaStream_t st);
 int lt_launch_undistort(lt_handle* h, const uint8_t* d_frames, int n, cudaStream_t st);   // RGB or NV12 (h->frame_format)
 int lt_launch_warp(lt_handle* h, uint8_t* d_bv_rgb, int n, cudaStream_t st);
+// The front half of a camera batch in buffer set f: nslots slots of f->und_cam (slot_pos / chunk_cam / cams uploaded),
+// max_rows: the tallest ROI of the cameras in the batch.
+int lt_launch_undistort_cams(lt_handle* h, const LtFrontSet& f, const uint8_t* d_frames, int nslots, int max_rows,
+                             cudaStream_t st);
+int lt_launch_warp_cams(lt_handle* h, const LtFrontSet& f, int nslots, cudaStream_t st);
 int lt_launch_planes_from_bv(lt_handle* h, const uint8_t* d_bv_rgb, int n, cudaStream_t st);
+// cf (may be NULL): the buffer set of a camera batch; position s then takes its overlay map and rows from
+// cf->cams[cf->pos_cam[s]], and the launch covers the union cf->cam_ov0 .. cam_ov1 of their rows
 int lt_launch_overlay(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, const int* d_draw,
-                      const int* ids, cudaStream_t st);
+                      const int* ids, cudaStream_t st, const LtFrontSet* cf = nullptr);
 // NV12 frames -> overlay-annotated RGB frames (every row of d_out written; d_out cannot alias d_frames)
 int lt_launch_overlay_nv12(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, const int* d_draw,
-                           const int* ids, cudaStream_t st);
+                           const int* ids, cudaStream_t st, const LtFrontSet* cf = nullptr);
 // rows [r0, r1) of NV12 frames -> RGB (nothing outside those rows is written)
 int lt_launch_nv12_to_rgb(const uint8_t* d_nv12, uint8_t* d_rgb, int n, int w, int h, int r0, int r1, cudaStream_t st);
 
@@ -230,8 +277,9 @@ int lt_launch_search(lt_handle* h, int n, const LtAttemptParams& p, const LtSear
                      int prof_params = 0);
 int lt_launch_select_retry(lt_handle* h, int n, int n_tries, cudaStream_t st, const LtProfile* prof = nullptr,
                            const int* pos_prof = nullptr);
+// cf (may be NULL): the buffer set of a camera batch; position s then takes mppv / mpph from cf->cams[cf->pos_cam[s]]
 int lt_launch_update_state(lt_handle* h, int n, const int* ids, lt_result* d_results, int attempts_allowed,
-                           cudaStream_t st);
+                           cudaStream_t st, const LtFrontSet* cf = nullptr);
 int lt_launch_fit_pixels(lt_handle* h, const uint32_t* d_pixels, int cap, const int* d_counts, int n,
                          double* d_fits, cudaStream_t st);
 int lt_launch_validity(lt_handle* h, const double* d_fits, int n, int* d_valid, double* d_diffs, cudaStream_t st);

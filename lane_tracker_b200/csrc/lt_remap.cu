@@ -81,22 +81,21 @@ static void invert3x3(const double* a, double* o) {
     o[8] = (a[0] * a[4] - a[1] * a[3]) * d;
 }
 
-int lt_launch_build_maps(lt_handle* h, cudaStream_t st) {
-    const lt_config& c = h->cfg;
+int lt_launch_build_maps(const lt_camera& c, const LtDims& d, int2* und_map, int2* bv_map, int2* ov_map, cudaStream_t st) {
     UndistortCoef uc;
     invert3x3(c.cam_matrix, uc.iR);
     uc.k1 = c.dist_coeffs[0]; uc.k2 = c.dist_coeffs[1]; uc.p1 = c.dist_coeffs[2];
     uc.p2 = c.dist_coeffs[3]; uc.k3 = c.dist_coeffs[4];
     uc.fx = c.cam_matrix[0]; uc.fy = c.cam_matrix[4]; uc.cx = c.cam_matrix[2]; uc.cy = c.cam_matrix[5];
-    dim3 b(256), g1(lt_div_up(c.img_w, 256), c.img_h), g2(lt_div_up(c.bv_w, 256), c.bv_h);
-    k_build_undistort_map<<<g1, b, 0, st>>>(h->und_map, c.img_w, c.img_h, uc);
+    dim3 b(256), g1(lt_div_up(d.img_w, 256), d.img_h), g2(lt_div_up(d.bv_w, 256), d.bv_h);
+    k_build_undistort_map<<<g1, b, 0, st>>>(und_map, d.img_w, d.img_h, uc);
     LT_LAUNCH_CHECK();
     Mat9 mi;
     invert3x3(c.M, mi.m);
-    k_build_perspective_map<<<g2, b, 0, st>>>(h->bv_map, c.bv_w, c.bv_h, mi);
+    k_build_perspective_map<<<g2, b, 0, st>>>(bv_map, d.bv_w, d.bv_h, mi);
     LT_LAUNCH_CHECK();
     invert3x3(c.Minv, mi.m);
-    k_build_perspective_map<<<g1, b, 0, st>>>(h->ov_map, c.img_w, c.img_h, mi);
+    k_build_perspective_map<<<g1, b, 0, st>>>(ov_map, d.img_w, d.img_h, mi);
     LT_LAUNCH_CHECK();
     return 0;
 }
@@ -196,10 +195,9 @@ __global__ void k_build_und_desc(const int2* __restrict__ map, int2* __restrict_
     desc[(size_t)(i - d.roi0) * d.img_w + j] = make_int2((int)off, (int)f);
 }
 
-int lt_launch_build_und_desc(lt_handle* h, cudaStream_t st) {
-    const LtDims& d = h->d;
+int lt_launch_build_und_desc(const int2* und_map, int2* und_desc, const LtDims& d, cudaStream_t st) {
     dim3 g(lt_div_up(d.img_w, 256), d.roi1 - d.roi0);
-    k_build_und_desc<<<g, 256, 0, st>>>(h->und_map, h->und_desc, d);
+    k_build_und_desc<<<g, 256, 0, st>>>(und_map, und_desc, d);
     LT_LAUNCH_CHECK();
     return 0;
 }
@@ -242,13 +240,139 @@ __device__ __forceinline__ void und_store_tile(const uint4* tile, uint32_t* __re
     }
 }
 
+// Slots of a camera batch (lt_process_front_cameras): the und buffer (LtFrontSet::und_cam) holds the batch positions
+// grouped by camera, each camera's run starting at a multiple of four slots, so that every chunk of four slots (one
+// 16-byte vector of a pixel) belongs to one camera.  slot_pos: batch position of each slot (-1: pad, only at the end of
+// a run); chunk_cam: camera of each chunk; cams: the snapshot of the camera tables.  Unused by the forms without cameras.
+struct LtCamSlots {
+    const int* slot_pos;
+    const int* chunk_cam;
+    const LtCamDev* cams;
+};
+
+// The four slots of chunk c of a CTA whose first slot is s0, in a camera batch: the batch positions of their frames and
+// the number of slots of the CTA up to the last real one of the chunk (pads are skipped like slots beyond the batch).
+__device__ __forceinline__ int cam_chunk_slots(const LtCamSlots& cs, int s0, int c, int ns, int4& pos) {
+    pos = __ldg(reinterpret_cast<const int4*>(cs.slot_pos + s0 + 4 * c));
+    const int real = (pos.x >= 0) + (pos.y >= 0) + (pos.z >= 0) + (pos.w >= 0);
+    return min(ns, 4 * c + real);
+}
+
+__device__ __forceinline__ int i4_at(const int4& v, int k) { return k == 0 ? v.x : (k == 1 ? v.y : (k == 2 ? v.z : v.w)); }
+
+// One ROI pixel's tap descriptor q, decoded once for every chunk of streams.
+struct UndTap {
+    int2 q;
+    uint32_t wA, wB, m;
+    bool fast;
+    int pitch, wi, sh, wpitch;
+};
+
+__device__ __forceinline__ UndTap und_tap(int2 q, const LtDims& d) {
+    UndTap t;
+    t.q = q;
+    const uint32_t f = (uint32_t)q.y;
+    blend_weights(f, t.wA, t.wB);
+    t.m = (f >> 10) & 15u;
+    t.fast = f >> 14;                   // word loads: the API refuses frames that are not 4-byte aligned
+    t.pitch = d.img_w * 3;
+    t.wi = q.x >> 2; t.sh = (q.x & 3) * 8; t.wpitch = t.pitch >> 2;
+    return t;
+}
+
+// The blended RGBX words of the four streams of chunk c at one ROI pixel (RGB frames): stream k reads the frame at
+// frame(k); streams 4c + k >= ns give 0.
+template <typename Frame>
+__device__ __forceinline__ uint4 und_chunk_rgb(const UndTap& t, int c, int ns, Frame frame) {
+    const int2 q = t.q;
+    const uint32_t wA = t.wA, wB = t.wB, m = t.m;
+    const bool fast = t.fast;
+    const int pitch = t.pitch, wi = t.wi, sh = t.sh, wpitch = t.wpitch;
+    uint32_t o[4] = {0u, 0u, 0u, 0u};
+    if (4 * c < ns) {
+        if (fast) {
+            // all 24 words of the four streams are requested before the first blend needs one
+            uint32_t a[4][3], b[4][3];
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                if (4 * c + k >= ns) break;
+                const uint32_t* w = reinterpret_cast<const uint32_t*>(frame(k)) + wi;
+                a[k][0] = __ldg(w); a[k][1] = __ldg(w + 1); a[k][2] = __ldg(w + 2);
+                b[k][0] = __ldg(w + wpitch); b[k][1] = __ldg(w + wpitch + 1); b[k][2] = __ldg(w + wpitch + 2);
+            }
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                if (4 * c + k >= ns) break;
+                const uint32_t qa0 = __funnelshift_r(a[k][0], a[k][1], sh), qa1 = __funnelshift_r(a[k][1], a[k][2], sh);     // bytes o..o+3, o+4..o+7
+                const uint32_t qb0 = __funnelshift_r(b[k][0], b[k][1], sh), qb1 = __funnelshift_r(b[k][1], b[k][2], sh);
+                o[k] = blend_taps(qa0, __funnelshift_r(qa0, qa1, 24), qb0, __funnelshift_r(qb0, qb1, 24), wA, wB);
+            }
+        } else if (m) {
+#pragma unroll 1
+            for (int k = 0; k < 4; ++k) {
+                if (4 * c + k >= ns) break;
+                const uint8_t* img = frame(k);
+                auto tap = [&](uint32_t bit, int off) -> uint32_t {     // BORDER_CONSTANT 0
+                    if (!(m & bit)) return 0u;
+                    const uint8_t* tp = img + q.x + off;
+                    return (uint32_t)__ldg(tp) | ((uint32_t)__ldg(tp + 1) << 8) | ((uint32_t)__ldg(tp + 2) << 16);
+                };
+                o[k] = blend_taps(tap(1u, 0), tap(2u, 3), tap(4u, pitch), tap(8u, pitch + 3), wA, wB);
+            }
+        }
+    }
+    return make_uint4(o[0], o[1], o[2], o[3]);
+}
+
+// The camera form of both undistort kernels: chunk c of the CTA takes the descriptors and ROI of its own camera.  Its
+// pixels below that ROI, down to two rows past it, are written as zeros: the warp reads them (the no-tap index and the
+// bottom taps of the last ROI row) and a slot may have held a taller camera's ROI in an earlier batch.  -> the number of
+// pixels the store of this thread's chunk (threadIdx.x % UND_CH) covers.
+template <typename Chunk>
+__device__ __forceinline__ int und_cams_tile(uint4* tile, int p, int s0, int ns, const LtCamSlots& cs, const LtDims& d,
+                                             Chunk chunk) {
+    int lim_mine = 0;
+#pragma unroll
+    for (int c = 0; c < UND_CH; ++c) {
+        int lim = 0;
+        uint4 o = make_uint4(0u, 0u, 0u, 0u);
+        if (4 * c < ns) {
+            const LtCamDev* cd = cs.cams + __ldg(&cs.chunk_cam[s0 / 4 + c]);
+            const int roi_px = cd->roi_px;
+            lim = roi_px + 2 * d.img_w;
+            if (p < roi_px) {
+                int4 pos;
+                const int nsc = cam_chunk_slots(cs, s0, c, ns, pos);
+                o = chunk(__ldg(&cd->und_desc[p]), c, nsc, pos);
+            }
+        }
+        if (c == (int)(threadIdx.x % UND_CH)) lim_mine = lim;
+        if (p < lim) tile[und_slot(threadIdx.x, c)] = o;
+    }
+    return lim_mine;
+}
+
+// CAMS: a camera batch (n slots of LtFrontSet::und_cam, tables per chunk from `cs`; `desc` unused).
+template <bool CAMS>
 __global__ void __launch_bounds__(256, UND_MINB)
 k_undistort_roi(const uint8_t* __restrict__ frames, uint32_t* __restrict__ und, const int2* __restrict__ desc, LtDims d, int n,
-                size_t group_words) {
+                size_t group_words, LtCamSlots cs) {
     __shared__ uint4 tile[256 * UND_CH];               // [pixel][chunk of four streams], chunk slot rotated by the pixel
     const int p0 = blockIdx.x * blockDim.x, p = p0 + threadIdx.x;
+    if (CAMS) {
+        const int s0 = blockIdx.y * UND_SPC, ns = min(UND_SPC, n - s0);
+        const size_t frame_bytes = (size_t)d.img_w * d.img_h * 3;
+        const int lim = und_cams_tile(tile, p, s0, ns, cs, d, [&](int2 q, int c, int nsc, const int4& pos) {
+            return und_chunk_rgb(und_tap(q, d), c, nsc, [&](int k) { return frames + (size_t)i4_at(pos, k) * frame_bytes; });
+        });
+        __syncthreads();
+        und_store_tile(tile, und, p0, lim, s0, d, group_words);
+        return;
+    }
     const int roi_px = (d.roi1 - d.roi0) * d.img_w;
     const int s0 = blockIdx.y * UND_SPC, ns = min(UND_SPC, n - s0);
+    // (the form without cameras keeps its own copy of the tap fetch of und_chunk_rgb: through the helper, ptxas lays
+    // out its branches differently, and this form is meant to stay the code it was before cameras)
     if (p < roi_px) {
         const int2 q = __ldg(&desc[p]);
         const uint32_t f = (uint32_t)q.y;
@@ -308,13 +432,78 @@ k_undistort_roi(const uint8_t* __restrict__ frames, uint32_t* __restrict__ und, 
 // two luma words and two chroma words per tap row, all requested before the first conversion.  The 32 words of four
 // streams in flight need 64 registers: 4 resident CTAs per SM (at the 6 of k_undistort_roi they spill).
 constexpr int UND_NV12_MINB = 4;
-__global__ void __launch_bounds__(256, UND_NV12_MINB)
+
+template <typename Frame>
+__device__ __forceinline__ uint4 und_chunk_nv12(int2 q, uint32_t wA, uint32_t wB, int c, int ns, Frame frame, const LtDims& d) {
+    const uint32_t f = (uint32_t)q.y;
+    const uint32_t m = (f >> 10) & 15u;
+    const int W = d.img_w, H = d.img_h;
+    const int lo = (m & 5u) ? 0 : 1;                 // left tap column outside the frame: sx = -1
+    const int t = q.x / 3 + lo + W;                  // (sy + 1) W + sx + lo >= 0
+    const int sy = t / W - 1, sx = t - (sy + 1) * W - lo;
+    const int ly = sy * W, cy0 = (H + (sy >> 1)) * W, cy1 = (H + ((sy + 1) >> 1)) * W;     // luma row, chroma rows
+    const int xa = sx, xb = sx + 1, ca = sx & ~1, cb = (sx + 1) & ~1;
+    uint32_t o[4] = {0u, 0u, 0u, 0u};
+    if (4 * c < ns) {
+        if (m == 15u) {
+            const int sa = 8 * (xa & 3), sb = 8 * (xb & 3), ua = 8 * (ca & 2), ub = 8 * (cb & 2);
+            uint32_t y[4][4], uv[4][4];          // [stream][tap], taps 00 01 10 11
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                if (4 * c + k >= ns) break;
+                const uint32_t* w = reinterpret_cast<const uint32_t*>(frame(k));
+                y[k][0] = __ldg(w + ((ly + xa) >> 2));     y[k][1] = __ldg(w + ((ly + xb) >> 2));
+                y[k][2] = __ldg(w + ((ly + W + xa) >> 2)); y[k][3] = __ldg(w + ((ly + W + xb) >> 2));
+                uv[k][0] = __ldg(w + ((cy0 + ca) >> 2));   uv[k][1] = __ldg(w + ((cy0 + cb) >> 2));
+                uv[k][2] = __ldg(w + ((cy1 + ca) >> 2));   uv[k][3] = __ldg(w + ((cy1 + cb) >> 2));
+            }
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                if (4 * c + k >= ns) break;
+                o[k] = blend_taps(yuv_to_rgb((y[k][0] >> sa) & 255u, uv[k][0] >> ua),
+                                  yuv_to_rgb((y[k][1] >> sb) & 255u, uv[k][1] >> ub),
+                                  yuv_to_rgb((y[k][2] >> sa) & 255u, uv[k][2] >> ua),
+                                  yuv_to_rgb((y[k][3] >> sb) & 255u, uv[k][3] >> ub), wA, wB);
+            }
+        } else if (m) {
+#pragma unroll 1
+            for (int k = 0; k < 4; ++k) {
+                if (4 * c + k >= ns) break;
+                const uint8_t* img = frame(k);
+                auto tap = [&](uint32_t bit, int lrow, int crow, int x, int cx) -> uint32_t {     // BORDER_CONSTANT 0
+                    if (!(m & bit)) return 0u;
+                    return yuv_to_rgb(__ldg(img + lrow + x), __ldg(reinterpret_cast<const unsigned short*>(img + crow + cx)));
+                };
+                o[k] = blend_taps(tap(1u, ly, cy0, xa, ca), tap(2u, ly, cy0, xb, cb), tap(4u, ly + W, cy1, xa, ca),
+                                  tap(8u, ly + W, cy1, xb, cb), wA, wB);
+            }
+        }
+    }
+    return make_uint4(o[0], o[1], o[2], o[3]);
+}
+
+// (the camera form: 3 CTAs per SM; with the chunk's camera and slot positions live as well, 64 registers spill)
+template <bool CAMS>
+__global__ void __launch_bounds__(256, CAMS ? UND_NV12_MINB - 1 : UND_NV12_MINB)
 k_undistort_roi_nv12(const uint8_t* __restrict__ frames, uint32_t* __restrict__ und, const int2* __restrict__ desc, LtDims d,
-                     int n, size_t group_words) {
+                     int n, size_t group_words, LtCamSlots cs) {
     __shared__ uint4 tile[256 * UND_CH];
     const int p0 = blockIdx.x * blockDim.x, p = p0 + threadIdx.x;
+    if (CAMS) {
+        const int s0 = blockIdx.y * UND_SPC, ns = min(UND_SPC, n - s0);
+        const size_t frame_bytes = (size_t)d.img_w * (d.img_h + d.img_h / 2);
+        const int lim = und_cams_tile(tile, p, s0, ns, cs, d, [&](int2 q, int c, int nsc, const int4& pos) {
+            uint32_t wA, wB;
+            blend_weights((uint32_t)q.y, wA, wB);
+            return und_chunk_nv12(q, wA, wB, c, nsc, [&](int k) { return frames + (size_t)i4_at(pos, k) * frame_bytes; }, d);
+        });
+        __syncthreads();
+        und_store_tile(tile, und, p0, lim, s0, d, group_words);
+        return;
+    }
     const int roi_px = (d.roi1 - d.roi0) * d.img_w;
     const int s0 = blockIdx.y * UND_SPC, ns = min(UND_SPC, n - s0);
+    // (the form without cameras keeps its own copy of the tap fetch of und_chunk_nv12, as k_undistort_roi does)
     if (p < roi_px) {
         const int2 q = __ldg(&desc[p]);
         const uint32_t f = (uint32_t)q.y;
@@ -396,11 +585,26 @@ int lt_launch_warp_frame(lt_handle* h, const uint8_t* d_frames, uint8_t* d_bv_rg
 int lt_launch_undistort(lt_handle* h, const uint8_t* d_frames, int n, cudaStream_t st) {
     const LtDims& d = h->d;
     dim3 g(lt_div_up((d.roi1 - d.roi0) * d.img_w, 256), lt_div_up(n, UND_SPC));
+    const LtCamSlots none = {nullptr, nullptr, nullptr};
     // the word loads of the fast path need 4-byte aligned rows: the frames are (lt_api.cu) and img_w % 4 == 0 (lt_create)
     if (h->frame_format == LT_FRAME_NV12)
-        k_undistort_roi_nv12<<<g, 256, 0, st>>>(d_frames, h->und_roi, h->und_desc, d, n, lt_und_group_words(d));
+        k_undistort_roi_nv12<false><<<g, 256, 0, st>>>(d_frames, h->und_roi, h->und_desc, d, n, lt_und_group_words(d), none);
     else
-        k_undistort_roi<<<g, 256, 0, st>>>(d_frames, h->und_roi, h->und_desc, d, n, lt_und_group_words(d));
+        k_undistort_roi<false><<<g, 256, 0, st>>>(d_frames, h->und_roi, h->und_desc, d, n, lt_und_group_words(d), none);
+    LT_LAUNCH_CHECK();
+    return 0;
+}
+
+// The camera batch: the grid covers the tallest ROI of its cameras plus the two zero rows below it.
+int lt_launch_undistort_cams(lt_handle* h, const LtFrontSet& f, const uint8_t* d_frames, int nslots, int max_rows,
+                             cudaStream_t st) {
+    const LtDims& d = h->d;
+    dim3 g(lt_div_up((max_rows + 2) * d.img_w, 256), lt_div_up(nslots, UND_SPC));
+    const LtCamSlots cs = {f.slot_pos, f.chunk_cam, f.cams};
+    if (h->frame_format == LT_FRAME_NV12)
+        k_undistort_roi_nv12<true><<<g, 256, 0, st>>>(d_frames, f.und_cam, nullptr, d, nslots, lt_und_cam_group_words(h), cs);
+    else
+        k_undistort_roi<true><<<g, 256, 0, st>>>(d_frames, f.und_cam, nullptr, d, nslots, lt_und_cam_group_words(h), cs);
     LT_LAUNCH_CHECK();
     return 0;
 }
@@ -437,10 +641,9 @@ __global__ void k_build_bv_desc(const int2* __restrict__ map, int2* __restrict__
     desc[(size_t)y * d.bv_w + x] = make_int2(idx, (int)((uint32_t)(q.x & 31) | ((uint32_t)(q.y & 31) << 5)));
 }
 
-int lt_launch_build_desc(lt_handle* h, cudaStream_t st) {
-    const LtDims& d = h->d;
+int lt_launch_build_desc(const int2* bv_map, int2* bv_desc, const LtDims& d, cudaStream_t st) {
     dim3 g(lt_div_up(d.bv_w, 256), d.bv_h);
-    k_build_bv_desc<<<g, 256, 0, st>>>(h->bv_map, h->bv_desc, d);
+    k_build_bv_desc<<<g, 256, 0, st>>>(bv_map, bv_desc, d);
     LT_LAUNCH_CHECK();
     return 0;
 }
@@ -545,11 +748,16 @@ constexpr int WARP_ITEMS = 64;        // packed columns per pass of a CTA (x 4 s
 constexpr int WARP_NB = 8;            // passes per CTA (the Lab tables are loaded once per CTA)
 constexpr int WARP_MINB = 4;          // resident CTAs per SM the warp is compiled for
 
-template <bool RGB_OUT>
-__global__ void __launch_bounds__(256, WARP_MINB)
+// CAMS: a camera batch, n slots of LtFrontSet::und_cam: the chunk of a thread takes the descriptors of its camera and
+// stream k of the chunk writes the planes of batch position slot_pos[s0 + k] (`desc` unused).  Where two cameras meet
+// inside a group of 16 slots, the four threads of a column gather from different pixels.  The camera form runs at 3 CTAs
+// per SM: with its camera's descriptor pointer and the slot positions, 64 registers spill.
+template <bool RGB_OUT, bool CAMS>
+__global__ void __launch_bounds__(256, CAMS ? WARP_MINB - 1 : WARP_MINB)
 k_warp_planes(const uint32_t* __restrict__ und_all, const int2* __restrict__ desc, uint32_t* __restrict__ planeR,
               uint32_t* __restrict__ planeB, uint8_t* __restrict__ bv_rgb, const uint2* __restrict__ yz,
-              const unsigned short* __restrict__ cb, LtDims d, unsigned stream_pad, int n, size_t group_words) {
+              const unsigned short* __restrict__ cb, LtDims d, unsigned stream_pad, int n, size_t group_words,
+              LtCamSlots cs) {
     __shared__ LabSmem L;
     lab_smem_load(L, yz, cb);
     __syncthreads();
@@ -559,6 +767,7 @@ k_warp_planes(const uint32_t* __restrict__ und_all, const int2* __restrict__ des
     const int c = threadIdx.x & 3, il = threadIdx.x >> 2;
     const int s0 = blockIdx.y * NSW + 4 * c, ns = min(4, n - s0);
     if (ns <= 0) return;
+    if (CAMS) desc = cs.cams[__ldg(&cs.chunk_cam[s0 / 4])].bv_desc;
     const int up4 = (d.img_w + 1) * (NSW / 4);                      // one und row in 16-byte units
     const uint4* und = reinterpret_cast<const uint4*>(und_all + (size_t)blockIdx.y * group_words) + c;
     const int total = d.bv_h * d.p2;
@@ -595,6 +804,12 @@ k_warp_planes(const uint32_t* __restrict__ und_all, const int2* __restrict__ des
 #pragma unroll
         for (int k = 0; k < 4; ++k, pr += stream_pad, pb += stream_pad) {
             if (k >= ns) break;
+            const int pk = CAMS ? __ldg(&cs.slot_pos[s0 + k]) : 0;
+            if (CAMS) {
+                if (pk < 0) break;                                      // pads end a camera's run
+                pr = planeR + (size_t)(unsigned)pk * stream_pad + o;
+                pb = planeB + (size_t)(unsigned)pk * stream_pad + o;
+            }
             uint32_t R0, G0, B0, R1, G1, B1;
             blend_taps3(u4_at(a00, k), u4_at(a01, k), u4_at(a10, k), u4_at(a11, k), wA0, wB0, R0, G0, B0);
             blend_taps3(u4_at(b00, k), u4_at(b01, k), u4_at(b10, k), u4_at(b11, k), wA1, wB1, R1, G1, B1);
@@ -606,7 +821,7 @@ k_warp_planes(const uint32_t* __restrict__ und_all, const int2* __restrict__ des
             if (halo_l) { pr[-d.p2] = (r2 << 16) | 0xFFFFu; pb[-d.p2] = (b2 << 16) | 0xFFFFu; }      // seam-stitched halo columns
             if (halo_r) { pr[d.p2] = (r2 >> 16) | 0xFFFF0000u; pb[d.p2] = (b2 >> 16) | 0xFFFF0000u; }
             if (RGB_OUT) {
-                uint8_t* p = bv_rgb + (((size_t)(s0 + k) * d.bv_h + y) * d.bv_w + x) * 3;
+                uint8_t* p = bv_rgb + (((size_t)(CAMS ? pk : s0 + k) * d.bv_h + y) * d.bv_w + x) * 3;
                 p[0] = R0; p[1] = G0; p[2] = B0;
                 if (hi_real) { p += (size_t)d.p2 * 3; p[0] = R1; p[1] = G1; p[2] = B1; }
             }
@@ -623,12 +838,23 @@ int lt_launch_build_lab_yz(lt_handle* h, cudaStream_t st) {
 int lt_launch_warp(lt_handle* h, uint8_t* d_bv_rgb, int n, cudaStream_t st) {
     const LtDims& d = h->d;
     dim3 g(lt_div_up(d.bv_h * d.p2, WARP_ITEMS * WARP_NB), lt_div_up(n, NSW));
+    const LtCamSlots none = {nullptr, nullptr, nullptr};
     if (d_bv_rgb)
-        k_warp_planes<true><<<g, 256, 0, st>>>(h->und_roi, h->bv_desc, h->planeR, h->planeB, d_bv_rgb, h->lab_yz, h->lab_cbrt, d,
-                                               (unsigned)h->stream_pad, n, lt_und_group_words(d));
+        k_warp_planes<true, false><<<g, 256, 0, st>>>(h->und_roi, h->bv_desc, h->planeR, h->planeB, d_bv_rgb, h->lab_yz,
+                                                      h->lab_cbrt, d, (unsigned)h->stream_pad, n, lt_und_group_words(d), none);
     else
-        k_warp_planes<false><<<g, 256, 0, st>>>(h->und_roi, h->bv_desc, h->planeR, h->planeB, nullptr, h->lab_yz, h->lab_cbrt, d,
-                                                (unsigned)h->stream_pad, n, lt_und_group_words(d));
+        k_warp_planes<false, false><<<g, 256, 0, st>>>(h->und_roi, h->bv_desc, h->planeR, h->planeB, nullptr, h->lab_yz,
+                                                       h->lab_cbrt, d, (unsigned)h->stream_pad, n, lt_und_group_words(d), none);
+    LT_LAUNCH_CHECK();
+    return 0;
+}
+
+int lt_launch_warp_cams(lt_handle* h, const LtFrontSet& f, int nslots, cudaStream_t st) {
+    const LtDims& d = h->d;
+    dim3 g(lt_div_up(d.bv_h * d.p2, WARP_ITEMS * WARP_NB), lt_div_up(nslots, NSW));
+    const LtCamSlots cs = {f.slot_pos, f.chunk_cam, f.cams};
+    k_warp_planes<false, true><<<g, 256, 0, st>>>(f.und_cam, nullptr, h->planeR, h->planeB, nullptr, h->lab_yz, h->lab_cbrt, d,
+                                                  (unsigned)h->stream_pad, nslots, lt_und_cam_group_words(h), cs);
     LT_LAUNCH_CHECK();
     return 0;
 }
@@ -774,11 +1000,19 @@ __device__ __forceinline__ int lane_tap(const int2* __restrict__ rows, const LtD
 }
 
 // Lane overlay of four pixels of frame row y, columns 4q .. 4q + 3, held as three RGB words (12 bytes): only G changes.
+// CAMS: position s takes its overlay map and rows from its camera, cams[pos_cam[s]] (`map` unused).
+template <bool CAMS>
 __device__ __forceinline__ void overlay_words(uint32_t& w0, uint32_t& w1, uint32_t& w2, const int2* __restrict__ map,
                                               const int2* __restrict__ lane_rows, const int4* __restrict__ lane_bbox,
                                               const int* __restrict__ draw, const LtDims& d, int y, int q, int s,
-                                              const int* __restrict__ ids) {
-    if (draw[s] && y >= d.ov0 && y < d.ov1) {
+                                              const int* __restrict__ ids, const LtCamDev* __restrict__ cams,
+                                              const int* __restrict__ pos_cam) {
+    int ov0 = d.ov0, ov1 = d.ov1;
+    if (CAMS && draw[s]) {
+        const LtCamDev* cd = cams + __ldg(&pos_cam[s]);
+        map = cd->ov_map; ov0 = cd->ov0; ov1 = cd->ov1;
+    }
+    if (draw[s] && y >= ov0 && y < ov1) {
         // Q5 canvas coordinates of the four pixels; most of them cannot reach the polygon: one test against its
         // bounding box (taps of a pixel: columns sx, sx + 1, rows sy, sy + 1) skips the span look-ups
         const int4* mp = reinterpret_cast<const int4*>(map + (size_t)y * d.img_w + q * 4);
@@ -816,10 +1050,11 @@ __device__ __forceinline__ void overlay_words(uint32_t& w0, uint32_t& w1, uint32
     }
 }
 
+template <bool CAMS>
 __global__ void __launch_bounds__(256)
 k_overlay(const uint8_t* frames, uint8_t* out, const int2* __restrict__ map,
           const int2* __restrict__ lane_rows, const int4* __restrict__ lane_bbox, const int* __restrict__ draw, LtDims d, int row0,
-          const int* __restrict__ ids) {
+          const int* __restrict__ ids, const LtCamDev* __restrict__ cams, const int* __restrict__ pos_cam) {
     // one thread = 4 pixels = 12 bytes (three aligned 32-bit words); img_w % 4 == 0 is checked at create.
     // `out` may alias `frames` (in-place annotation): every thread reads and writes only its own 12 bytes.
     int q = blockIdx.x * blockDim.x + threadIdx.x;
@@ -829,17 +1064,18 @@ k_overlay(const uint8_t* frames, uint8_t* out, const int2* __restrict__ map,
     size_t base = (((size_t)s * d.img_h + y) * d.img_w + (size_t)q * 4) * 3;
     const uint32_t* src = reinterpret_cast<const uint32_t*>(frames + base);
     uint32_t w0 = src[0], w1 = src[1], w2 = src[2];
-    overlay_words(w0, w1, w2, map, lane_rows, lane_bbox, draw, d, y, q, s, ids);
+    overlay_words<CAMS>(w0, w1, w2, map, lane_rows, lane_bbox, draw, d, y, q, s, ids, cams, pos_cam);
     uint32_t* dst = reinterpret_cast<uint32_t*>(out + base);
     dst[0] = w0; dst[1] = w1; dst[2] = w2;
 }
 
 // k_overlay of NV12 frames: one thread converts 4 pixels (one luma word, one chroma word = two U,V pairs) to the three
 // RGB words k_overlay reads, blends them the same way and writes them to the RGB output (which cannot alias the input).
+template <bool CAMS>
 __global__ void __launch_bounds__(256)
 k_overlay_nv12(const uint8_t* __restrict__ frames, uint8_t* __restrict__ out, const int2* __restrict__ map,
                const int2* __restrict__ lane_rows, const int4* __restrict__ lane_bbox, const int* __restrict__ draw, LtDims d,
-               int row0, const int* __restrict__ ids) {
+               int row0, const int* __restrict__ ids, const LtCamDev* __restrict__ cams, const int* __restrict__ pos_cam) {
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
     const int y = row0 + blockIdx.y, s = blockIdx.z;
     if (q >= (d.img_w >> 2)) return;
@@ -848,7 +1084,7 @@ k_overlay_nv12(const uint8_t* __restrict__ frames, uint8_t* __restrict__ out, co
     const uint32_t uv = __ldg(reinterpret_cast<const uint32_t*>(f + (size_t)(d.img_h + (y >> 1)) * d.img_w) + q);
     uint32_t w0, w1, w2;
     nv12_to_rgb_words(luma, uv, w0, w1, w2);
-    overlay_words(w0, w1, w2, map, lane_rows, lane_bbox, draw, d, y, q, s, ids);
+    overlay_words<CAMS>(w0, w1, w2, map, lane_rows, lane_bbox, draw, d, y, q, s, ids, cams, pos_cam);
     uint32_t* dst = reinterpret_cast<uint32_t*>(out + (((size_t)s * d.img_h + y) * d.img_w + (size_t)q * 4) * 3);
     dst[0] = w0; dst[1] = w1; dst[2] = w2;
 }
@@ -874,13 +1110,13 @@ k_copy_rows(const uint4* __restrict__ src, uint4* __restrict__ dst, size_t frame
         if (i0 + (size_t)u * blockDim.x < total) fd[idx[u]] = v[u];
 }
 
-// k_overlay runs on the rows [ov0, ov1) that the lane overlay can reach; out of place, the other rows of the output
-// frame are a plain copy of the input.
+// k_overlay runs on the rows [ov0, ov1) that the lane overlay can reach (a camera batch: the union over its cameras);
+// out of place, the other rows of the output frame are a plain copy of the input.
 int lt_launch_overlay(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, const int* d_draw,
-                      const int* ids, cudaStream_t st) {
+                      const int* ids, cudaStream_t st, const LtFrontSet* cf) {
     const LtDims& d = h->d;
     const size_t row_bytes = (size_t)d.img_w * 3, frame_bytes = row_bytes * d.img_h;
-    int r0 = d.ov0, r1 = d.ov1;
+    int r0 = cf ? cf->cam_ov0 : d.ov0, r1 = cf ? cf->cam_ov1 : d.ov1;
     if (d_out != d_frames) {
         if (row_bytes % 16 || ((uintptr_t)d_frames | (uintptr_t)d_out) % 16) {
             r0 = 0; r1 = d.img_h;                       // generic path: k_overlay copies every row itself
@@ -895,7 +1131,12 @@ int lt_launch_overlay(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int
     }
     if (r1 > r0) {
         dim3 g(lt_div_up(d.img_w / 4, 256), r1 - r0, n);
-        k_overlay<<<g, 256, 0, st>>>(d_frames, d_out, h->ov_map, h->lane_rows, h->lane_bbox, d_draw, d, r0, ids);
+        if (cf)
+            k_overlay<true><<<g, 256, 0, st>>>(d_frames, d_out, nullptr, h->lane_rows, h->lane_bbox, d_draw, d, r0, ids, cf->cams,
+                                               cf->pos_cam);
+        else
+            k_overlay<false><<<g, 256, 0, st>>>(d_frames, d_out, h->ov_map, h->lane_rows, h->lane_bbox, d_draw, d, r0, ids,
+                                                nullptr, nullptr);
         LT_LAUNCH_CHECK();
     }
     return 0;
@@ -936,14 +1177,20 @@ int lt_launch_nv12_to_rgb(const uint8_t* d_nv12, uint8_t* d_rgb, int n, int w, i
 
 // The annotated RGB frames of NV12 input: k_overlay_nv12 on the rows the overlay can reach, the converter on the others.
 int lt_launch_overlay_nv12(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, const int* d_draw,
-                           const int* ids, cudaStream_t st) {
+                           const int* ids, cudaStream_t st, const LtFrontSet* cf) {
     const LtDims& d = h->d;
+    const int r0 = cf ? cf->cam_ov0 : d.ov0, r1 = cf ? cf->cam_ov1 : d.ov1;
     int rc;
-    if ((rc = lt_launch_nv12_to_rgb(d_frames, d_out, n, d.img_w, d.img_h, 0, d.ov0, st))) return rc;
-    if ((rc = lt_launch_nv12_to_rgb(d_frames, d_out, n, d.img_w, d.img_h, d.ov1, d.img_h, st))) return rc;
-    if (d.ov1 > d.ov0) {
-        dim3 g(lt_div_up(d.img_w / 4, 256), d.ov1 - d.ov0, n);
-        k_overlay_nv12<<<g, 256, 0, st>>>(d_frames, d_out, h->ov_map, h->lane_rows, h->lane_bbox, d_draw, d, d.ov0, ids);
+    if ((rc = lt_launch_nv12_to_rgb(d_frames, d_out, n, d.img_w, d.img_h, 0, r0, st))) return rc;
+    if ((rc = lt_launch_nv12_to_rgb(d_frames, d_out, n, d.img_w, d.img_h, r1, d.img_h, st))) return rc;
+    if (r1 > r0) {
+        dim3 g(lt_div_up(d.img_w / 4, 256), r1 - r0, n);
+        if (cf)
+            k_overlay_nv12<true><<<g, 256, 0, st>>>(d_frames, d_out, nullptr, h->lane_rows, h->lane_bbox, d_draw, d, r0, ids,
+                                                    cf->cams, cf->pos_cam);
+        else
+            k_overlay_nv12<false><<<g, 256, 0, st>>>(d_frames, d_out, h->ov_map, h->lane_rows, h->lane_bbox, d_draw, d, r0, ids,
+                                                     nullptr, nullptr);
         LT_LAUNCH_CHECK();
     }
     return 0;

@@ -750,11 +750,13 @@ __device__ void lane_rows_from_polylines(const int* xl, int nl, const int* xr, i
 // per-frame state update (lane_tracker.py:1142-1209)
 // ---------------------------------------------------------------------------
 
+// CAMS: position s takes mppv / mpph from its camera, cams[pos_cam[s]] (the handle's cfg otherwise).
+template <bool CAMS>
 __global__ void __launch_bounds__(SEARCH_THREADS)
 k_update_state(LtDims d, lt_config cfg, LtDevState* __restrict__ state, const LtAttemptOut* __restrict__ att1,
                const LtAttemptOut* __restrict__ att2, const int* __restrict__ retry, int* __restrict__ avg_x,
                int2* __restrict__ lane_rows, int4* __restrict__ lane_bbox, int* __restrict__ draw, lt_result* __restrict__ results,
-               const int* __restrict__ ids) {
+               const int* __restrict__ ids, const LtCamDev* __restrict__ cams, const int* __restrict__ pos_cam) {
     // s: batch position (attempt outputs, retry and draw flags, result record); sid: state slot of its stream
     const int s = blockIdx.x, sid = ids ? ids[s] : s, tid = threadIdx.x, W = d.bv_w, H = d.bv_h;
     extern __shared__ unsigned char smem_raw[];
@@ -825,9 +827,14 @@ k_update_state(LtDims d, lt_config cfg, LtDevState* __restrict__ state, const Lt
             // get_curve_radius (lane_tracker.py:530-549): the metric refit of the same pixels is the
             // analytic rescaling a' = a*mpph/mppv^2, b' = b*mpph/mppv of this frame's fit
             long long rad[2];
+            double mppv = cfg.mppv, mpph = cfg.mpph;
+            if (CAMS) {
+                const LtCamDev& cd = cams[pos_cam[s]];
+                mppv = cd.mppv; mpph = cd.mpph;
+            }
             for (int side = 0; side < 2; ++side) {
-                double am = a.fit[side][0] * cfg.mpph / (cfg.mppv * cfg.mppv), bm = a.fit[side][1] * cfg.mpph / cfg.mppv;
-                double g = 2.0 * am * (double)H * cfg.mppv + bm;
+                double am = a.fit[side][0] * mpph / (mppv * mppv), bm = a.fit[side][1] * mpph / mppv;
+                double g = 2.0 * am * (double)H * mppv + bm;
                 double r = pow(1.0 + g * g, 1.5) / fabs(2.0 * am);
                 rad[side] = (!(r == r) || r >= 9.2233720368547758e18) ? 0x7FFFFFFFFFFFFFFFLL : (long long)r;   // int(float)
             }
@@ -845,7 +852,7 @@ k_update_state(LtDims d, lt_config cfg, LtDevState* __restrict__ state, const Lt
             // get_eccentricity (lane_tracker.py:551-559)
             if (nkeep[0] > 0 && nkeep[1] > 0) {
                 int mid = W / 2, left = xl[nkeep[0] - 1], right = xr[nkeep[1] - 1];
-                st.eccentricity = mul64((double)((mid - left) - (right - mid)) / 2.0, cfg.mpph);
+                st.eccentricity = mul64((double)((mid - left) - (right - mid)) / 2.0, mpph);
             }
         }
         __syncthreads();
@@ -873,11 +880,17 @@ k_update_state(LtDims d, lt_config cfg, LtDevState* __restrict__ state, const Lt
 }
 
 int lt_launch_update_state(lt_handle* h, int n, const int* ids, lt_result* d_results, int attempts_allowed,
-                           cudaStream_t st) {
+                           cudaStream_t st, const LtFrontSet* cf) {
     size_t smem = (size_t)3 * h->d.bv_h * sizeof(int);
     const int* retry = attempts_allowed >= 2 ? h->draw_flags + h->S : nullptr;
-    k_update_state<<<n, SEARCH_THREADS, smem, st>>>(h->d, h->cfg, h->state, h->att, h->att + h->S, retry, h->avg_x,
-                                                    h->lane_rows, h->lane_bbox, h->draw_flags, d_results, ids);
+    if (cf)
+        k_update_state<true><<<n, SEARCH_THREADS, smem, st>>>(h->d, h->cfg, h->state, h->att, h->att + h->S, retry, h->avg_x,
+                                                              h->lane_rows, h->lane_bbox, h->draw_flags, d_results, ids,
+                                                              cf->cams, cf->pos_cam);
+    else
+        k_update_state<false><<<n, SEARCH_THREADS, smem, st>>>(h->d, h->cfg, h->state, h->att, h->att + h->S, retry, h->avg_x,
+                                                               h->lane_rows, h->lane_bbox, h->draw_flags, d_results, ids,
+                                                               nullptr, nullptr);
     LT_LAUNCH_CHECK();
     return 0;
 }

@@ -53,8 +53,11 @@ def shipped_calibration(scale=1.0):
 class RoadVideo:
     """Frame generator for one stream; ``frame(t)`` -> uint8 RGB [h, w, 3]."""
 
-    def __init__(self, seed=0, scale=1.0, separation=180.0):
-        cal = shipped_calibration(scale)
+    def __init__(self, seed=0, scale=1.0, separation=180.0, calibration=None):
+        """calibration: constructor arguments of ``LaneTracker`` (``shipped_calibration`` form) whose warp ``M`` renders
+        the road into the frame, for cameras mounted otherwise (None: ``shipped_calibration(scale)``).  The frames have
+        no lens distortion either way."""
+        cal = shipped_calibration(scale) if calibration is None else calibration
         self.seed = int(seed)
         self.scale = float(scale)
         self.separation = separation * scale

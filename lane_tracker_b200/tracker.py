@@ -85,6 +85,20 @@ def bilateral_adaptive_threshold(img, ksize=30, C=0, mode='floor', true_value=25
         return out.cpu().numpy()
 
 
+def _calibration(cam_matrix, dist_coeffs, warp_matrices, mpp_conversion):
+    """The calibration arguments of the constructor and of ``set_camera`` -> lt_camera (checked)."""
+    c = _lib.lt_camera()
+    c.cam_matrix[:] = [float(v) for v in np.asarray(cam_matrix, dtype=np.float64).reshape(9)]
+    d = np.asarray(dist_coeffs, dtype=np.float64).ravel()
+    if d.size > 5 and np.any(d[5:] != 0):
+        raise ValueError("only the 5-coefficient distortion model (k1,k2,p1,p2,k3) is supported")
+    c.dist_coeffs[:] = [float(v) for v in np.concatenate([d[:5], np.zeros(max(0, 5 - d.size))])]
+    c.M[:] = [float(v) for v in np.asarray(warp_matrices[0], dtype=np.float64).reshape(9)]
+    c.Minv[:] = [float(v) for v in np.asarray(warp_matrices[1], dtype=np.float64).reshape(9)]
+    c.mppv, c.mpph = float(mpp_conversion[0]), float(mpp_conversion[1])
+    return c
+
+
 def _ptr(t):
     return C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(0)
 
@@ -111,14 +125,9 @@ class BatchedLaneTracker:
         cfg = lt_config()
         cfg.img_w, cfg.img_h = self.img_size
         cfg.bv_w, cfg.bv_h = self.warped_size
-        cfg.cam_matrix[:] = [float(v) for v in np.asarray(cam_matrix, dtype=np.float64).reshape(9)]
-        d = np.asarray(dist_coeffs, dtype=np.float64).ravel()
-        if d.size > 5 and np.any(d[5:] != 0):
-            raise ValueError("only the 5-coefficient distortion model (k1,k2,p1,p2,k3) is supported")
-        cfg.dist_coeffs[:] = [float(v) for v in np.concatenate([d[:5], np.zeros(max(0, 5 - d.size))])]
-        cfg.M[:] = [float(v) for v in np.asarray(warp_matrices[0], dtype=np.float64).reshape(9)]
-        cfg.Minv[:] = [float(v) for v in np.asarray(warp_matrices[1], dtype=np.float64).reshape(9)]
-        cfg.mppv, cfg.mpph = float(mpp_conversion[0]), float(mpp_conversion[1])
+        cal = _calibration(cam_matrix, dist_coeffs, warp_matrices, mpp_conversion)
+        for name, _ in _lib.lt_camera._fields_:
+            setattr(cfg, name, getattr(cal, name))
         cfg.n_fail, cfg.n_reset, cfg.n_average = self.n_fail, self.n_reset, self.n_average
         cfg.print_frame_count = int(bool(print_frame_count))
         cfg.max_streams = self.n_streams
@@ -141,6 +150,35 @@ class BatchedLaneTracker:
         self.geometry = dict(roi_rows=(int(geo[0]), int(geo[1])), overlay_rows=(int(geo[2]), int(geo[3])),
                              plane_width=int(geo[4]), mask_words=int(geo[5]), pixel_capacity=int(geo[6]),
                              source_rows=(int(geo[7]), int(geo[8])))
+        self.camera_rows = {}                  # camera -> its rows (lt_debug_read 13), see ``set_camera``
+        self._read_camera_rows(0)
+        self.camera_epoch = 0                  # bumped by set_camera (GraphedProcess refuses to replay across it)
+
+    def _read_camera_rows(self, k):
+        v = np.zeros(6, dtype=np.int32)
+        check(self.lib.lt_debug_read(self._h, 13, int(k), v.ctypes.data_as(C.c_void_p), v.nbytes))
+        self.camera_rows[int(k)] = dict(roi_rows=(int(v[0]), int(v[1])), overlay_rows=(int(v[2]), int(v[3])),
+                                        source_rows=(int(v[4]), int(v[5])))
+
+    def rows_any_camera(self):
+        """(source rows, overlay rows) over camera 0 and every camera set: the frame rows the tracker may read, and
+        those the lane overlay may change, whichever cameras a batch uses (half-open; overlay (0, 0) if none)."""
+        src = [r["source_rows"] for r in self.camera_rows.values()]
+        ov = [r["overlay_rows"] for r in self.camera_rows.values() if r["overlay_rows"][1] > r["overlay_rows"][0]]
+        return ((min(a for a, _ in src), max(b for _, b in src)),
+                (min(a for a, _ in ov), max(b for _, b in ov)) if ov else (0, 0))
+
+    def set_camera(self, k, cam_matrix, dist_coeffs, warp_matrices, mpp_conversion):
+        """Set camera k (1 <= k < LT_MAX_CAMERAS) for the ``cameras=`` argument of the process calls: a calibration in
+        the constructor's forms (camera 0 is the constructor's and cannot change).  Image and bird's-eye sizes stay
+        the handle's.  Synchronises the device.  A stream whose camera was re-mounted keeps its tracking state: reset
+        it with ``reset(ids)``.  A ``GraphedProcess`` captured with cameras before this call can no longer replay."""
+        cal = _calibration(cam_matrix, dist_coeffs, warp_matrices, mpp_conversion)
+        with torch.cuda.device(self.device):
+            check(self.lib.lt_set_camera(self._h, int(k), C.byref(cal)))
+        self._read_camera_rows(k)
+        # a graph holds pointers to the camera tables and the camera undistort buffer, which this call may replace
+        self.camera_epoch += 1
 
     # -- lifetime -----------------------------------------------------------
     def close(self):
@@ -353,6 +391,29 @@ class BatchedLaneTracker:
                              % (int(a[bad[0]]), int(bad[0]), _lib.LT_MAX_PROFILES))
         return (C.c_int32 * n)(*[int(v) for v in a])
 
+    def _check_cameras(self, cameras, n):
+        """Camera indices of a batch of n frames -> ctypes int32 array (None: None).  Any int sequence, NumPy array or
+        CPU tensor of n indices in [0, LT_MAX_CAMERAS); frame i was filmed by camera cameras[i] (see ``set_camera``)."""
+        if cameras is None:
+            return None
+        if isinstance(cameras, torch.Tensor):
+            if cameras.is_cuda:
+                raise ValueError("cameras must be host data (a sequence, a NumPy array or a CPU tensor), not a CUDA tensor")
+            cameras = cameras.numpy()
+        a = np.asarray(cameras)
+        if a.ndim != 1 or (a.size and a.dtype.kind not in "iu"):
+            raise ValueError("cameras must be a 1-D sequence of integers")
+        if a.size != n:
+            raise ValueError("got %d camera indices for %d frames" % (a.size, n))
+        bad = np.flatnonzero((a < 0) | (a >= _lib.LT_MAX_CAMERAS))
+        if bad.size:
+            raise ValueError("camera %d at batch position %d outside [0, %d)"
+                             % (int(a[bad[0]]), int(bad[0]), _lib.LT_MAX_CAMERAS))
+        unset = [i for i, k in enumerate(a) if int(k) not in self.camera_rows]
+        if unset:
+            raise ValueError("camera %d at batch position %d is unset" % (int(a[unset[0]]), unset[0]))
+        return (C.c_int32 * n)(*[int(v) for v in a])
+
     @staticmethod
     def _no_params_with_profiles(profiles, params, kw):
         if profiles is not None and (params is not None or kw):
@@ -369,7 +430,8 @@ class BatchedLaneTracker:
         if out.data_ptr() % 4:
             raise ValueError("out must start at a 4-byte aligned address (the kernels access frames as 32-bit words)")
 
-    def process_async(self, frames, out=None, params=None, results_dev=None, ids=None, profiles=None, **kw):
+    def process_async(self, frames, out=None, params=None, results_dev=None, ids=None, profiles=None, cameras=None,
+                      **kw):
         """Enqueue one frame per stream on the current CUDA stream; returns the number of frames.
 
         frames: uint8 CUDA tensor [n, H, W, 3] (RGB) or [n, H * 3 / 2, W] (NV12: the luma plane, then interleaved
@@ -381,16 +443,25 @@ class BatchedLaneTracker:
         state.  out and the result records stay in batch order.
         profiles: None -- every frame uses ``params`` (or ``make_params(**kw)``); else n profile indices (any int
         sequence, NumPy array or CPU tensor; see ``set_profile``): frame i uses profile profiles[i], and ``params`` /
-        keyword options may not be given."""
-        return self._process_call(frames, out, None, params, results_dev, ids, kw, profiles)
+        keyword options may not be given.
+        cameras: None -- every frame comes from camera 0 (the constructor's calibration); else n camera indices (see
+        ``set_camera``): frame i was filmed by camera cameras[i].  A caller with one camera per stream passes
+        camera_of[ids]."""
+        return self._process_call(frames, out, None, params, results_dev, ids, kw, profiles, cameras)
 
-    def process_front_async(self, frames, buffer_set, params=None, profiles=None, **kw):
+    def process_front_async(self, frames, buffer_set, params=None, profiles=None, cameras=None, **kw):
         """First half of ``process_async`` (undistort, warp, first-attempt filter) into intermediate buffer set
         0 or 1, on the current CUDA stream.  Stateless.  See ``DevicePipeline``.  RGB or NV12 frames.  With
-        ``profiles``, the back half of this buffer set must be given the same profile indices."""
+        ``profiles`` or ``cameras``, the back half of this buffer set must be given the same indices."""
         n = self._input(frames)
         self._no_params_with_profiles(profiles, params, kw)
         h_prof = self._check_profiles(profiles, n)
+        h_cam = self._check_cameras(cameras, n)
+        if h_cam is not None:
+            p = None if h_prof is not None else (params if params is not None else make_params(**kw))
+            check(self.lib.lt_process_front_cameras(self._h, _ptr(frames), h_cam, n, C.byref(p) if p is not None else None,
+                                                    h_prof, int(buffer_set), _stream_ptr(self.device)))
+            return n
         if h_prof is not None:
             check(self.lib.lt_process_front_profiles(self._h, _ptr(frames), h_prof, n, int(buffer_set),
                                                      _stream_ptr(self.device)))
@@ -399,23 +470,35 @@ class BatchedLaneTracker:
         check(self.lib.lt_process_front(self._h, _ptr(frames), n, C.byref(p), int(buffer_set), _stream_ptr(self.device)))
         return n
 
-    def process_back_async(self, frames, out, buffer_set, params=None, results_dev=None, ids=None, profiles=None, **kw):
+    def process_back_async(self, frames, out, buffer_set, params=None, results_dev=None, ids=None, profiles=None,
+                           cameras=None, **kw):
         """Second half of ``process_async`` (searches, second attempt, state machine, overlay) from intermediate
         buffer set 0 or 1, on the current CUDA stream.  Advances the per-stream state of the streams in ``ids``
-        (None: streams 0..n-1), as ``process_async``.  RGB or NV12 frames, as given to the front half.  ``profiles``:
-        those the front half of this buffer set was given."""
-        return self._process_call(frames, out, buffer_set, params, results_dev, ids, kw, profiles)
+        (None: streams 0..n-1), as ``process_async``.  RGB or NV12 frames, as given to the front half.  ``profiles``,
+        ``cameras``: those the front half of this buffer set was given."""
+        return self._process_call(frames, out, buffer_set, params, results_dev, ids, kw, profiles, cameras)
 
-    def _process_call(self, frames, out, buffer_set, params, results_dev, ids, kw, profiles=None):
+    def _process_call(self, frames, out, buffer_set, params, results_dev, ids, kw, profiles=None, cameras=None):
         """Checks and C call of ``process_async`` (buffer_set None: both halves) or ``process_back_async``; -> n."""
         n = self._input(frames)
         self._check_out(out, frames)
         h_ids = self._check_ids(ids, n)
         self._no_params_with_profiles(profiles, params, kw)
         h_prof = self._check_profiles(profiles, n)
+        h_cam = self._check_cameras(cameras, n)
         res = self._results_dev if results_dev is None else results_dev
         if res.numel() < n * RESULT_DTYPE.itemsize or not res.is_cuda:
             raise ValueError("results buffer too small")
+        if h_cam is not None:
+            p = None if h_prof is not None else (params if params is not None else make_params(**kw))
+            pp = C.byref(p) if p is not None else None
+            if buffer_set is None:
+                check(self.lib.lt_process_cameras(self._h, _ptr(frames), _ptr(out), h_ids, h_cam, n, pp, h_prof,
+                                                  _ptr(res), _stream_ptr(self.device)))
+            else:
+                check(self.lib.lt_process_back_cameras(self._h, _ptr(frames), _ptr(out), h_ids, h_cam, n, pp, h_prof,
+                                                       int(buffer_set), _ptr(res), _stream_ptr(self.device)))
+            return n
         if h_prof is not None:
             if buffer_set is None:
                 check(self.lib.lt_process_profiles(self._h, _ptr(frames), _ptr(out), h_ids, h_prof, n, _ptr(res),
@@ -444,11 +527,11 @@ class BatchedLaneTracker:
         torch.cuda.current_stream(self.device).synchronize()
         return self._results_host[:nbytes].numpy().view(RESULT_DTYPE).copy()
 
-    def process(self, frames, out=None, params=None, ids=None, profiles=None, **kw):
+    def process(self, frames, out=None, params=None, ids=None, profiles=None, cameras=None, **kw):
         """``process_async`` followed by ``fetch_results``: the n result records, in batch order.  With ``ids``, frame
         i advances stream ids[i] and the other streams keep their state; with ``profiles``, frame i uses parameter
-        profile profiles[i] (``set_profile``)."""
-        n = self.process_async(frames, out, params, ids=ids, profiles=profiles, **kw)
+        profile profiles[i] (``set_profile``); with ``cameras``, frame i comes from camera cameras[i] (``set_camera``)."""
+        n = self.process_async(frames, out, params, ids=ids, profiles=profiles, cameras=cameras, **kw)
         return self.fetch_results(n)
 
     # -- stage methods (device tensors) ---------------------------------------
@@ -719,10 +802,12 @@ class GraphedProcess:
 
     With ``profiles`` (n profile indices, see ``BatchedLaneTracker.set_profile``) frame i uses profile profiles[i].
     The graph holds the profile indices and the profile table as they stood at capture time: a later ``set_profile``
-    does not reach it (capture a new ``GraphedProcess`` instead).
+    does not reach it (capture a new ``GraphedProcess`` instead).  With ``cameras`` (n camera indices, see
+    ``BatchedLaneTracker.set_camera``) frame i comes from camera cameras[i]; the graph then holds the camera tables and
+    buffers of capture time, and ``replay`` raises RuntimeError after a later ``set_camera``.
     """
 
-    def __init__(self, tracker, n=None, overlay=True, params=None, frame_format="rgb", profiles=None):
+    def __init__(self, tracker, n=None, overlay=True, params=None, frame_format="rgb", profiles=None, cameras=None):
         """frame_format 'nv12': ``self.frames`` is NV12 [n, H * 3 / 2, W]; ``self.out`` stays RGB."""
         if frame_format not in _FRAME_FORMATS:
             raise ValueError("frame_format must be 'rgb' or 'nv12'")
@@ -739,6 +824,9 @@ class GraphedProcess:
         self.params = params if params is not None or profiles is not None else make_params()
         self.profiles = None if profiles is None else np.array(profiles, dtype=np.int64)
         tracker._check_profiles(self.profiles, n)
+        self.cameras = None if cameras is None else np.array(cameras, dtype=np.int64)
+        tracker._check_cameras(self.cameras, n)
+        self.camera_epoch = tracker.camera_epoch
         # first-use initialisation (module load, shared-memory attributes) cannot happen inside a capture: run the
         # chain once for real on a side stream, with the tracking state saved and restored around it
         saved = [tracker.get_state(s) for s in range(n)]
@@ -746,18 +834,21 @@ class GraphedProcess:
         side.wait_stream(torch.cuda.current_stream(dev))
         with torch.cuda.stream(side):
             tracker.process_async(self.frames, self.out, params=self.params, results_dev=self.results_dev,
-                                  profiles=self.profiles)
+                                  profiles=self.profiles, cameras=self.cameras)
         side.synchronize()
         for s, (st, lx, rx) in enumerate(saved):
             tracker.set_state(s, st, lx, rx)
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph, stream=side):
             tracker.process_async(self.frames, self.out, params=self.params, results_dev=self.results_dev,
-                                  profiles=self.profiles)
+                                  profiles=self.profiles, cameras=self.cameras)
         torch.cuda.current_stream(dev).wait_stream(side)
 
     def replay(self):
         """Enqueue one frame per stream (read from ``self.frames``) on the current stream."""
+        if self.cameras is not None and self.t.camera_epoch != self.camera_epoch:
+            raise RuntimeError("set_camera ran after this graph was captured with cameras: the graph holds the camera "
+                               "tables and buffers it replaced; capture a new GraphedProcess")
         self.graph.replay()
 
     def fetch_results(self):
@@ -779,7 +870,8 @@ class DevicePipeline:
     ``submit(frames, out, ids=...)`` advances the listed streams only (see ``BatchedLaneTracker.process_async``);
     results stay in batch order.  ``frames`` may be RGB or NV12 (``out`` is RGB either way), batch by batch.
     ``submit(..., profiles=...)`` gives frame i parameter profile profiles[i] (``BatchedLaneTracker.set_profile``)
-    instead of the pipeline's ``params``.
+    instead of the pipeline's ``params``; ``submit(..., cameras=...)`` says that frame i comes from camera cameras[i]
+    (``BatchedLaneTracker.set_camera``).
     """
 
     def __init__(self, tracker, params=None):
@@ -794,11 +886,12 @@ class DevicePipeline:
         self.results_dev = [torch.zeros(tracker.n_streams * RESULT_DTYPE.itemsize, dtype=torch.uint8, device=dev)
                             for _ in range(2)]
 
-    def submit(self, frames, out=None, ids=None, profiles=None):
+    def submit(self, frames, out=None, ids=None, profiles=None, cameras=None):
         dev = self.t.device
         n = self.t._frame_format(frames)[0]
-        self.t._check_ids(ids, n)                      # refuse bad frames / ids / profiles before anything is enqueued
+        self.t._check_ids(ids, n)                      # refuse bad frames / ids / profiles / cameras before anything is enqueued
         self.t._check_profiles(profiles, n)
+        self.t._check_cameras(cameras, n)
         params = self.params if profiles is None else None
         k, bs = self._k, self._k & 1
         ready = torch.cuda.Event()
@@ -807,14 +900,14 @@ class DevicePipeline:
             self.s_front.wait_event(ready)
             if self._back_done[bs] is not None:
                 self.s_front.wait_event(self._back_done[bs])    # set `bs` is free again
-            self.t.process_front_async(frames, bs, params=params, profiles=profiles)
+            self.t.process_front_async(frames, bs, params=params, profiles=profiles, cameras=cameras)
             front_done = torch.cuda.Event()
             front_done.record(self.s_front)
         with torch.cuda.stream(self.s_back):
             self.s_back.wait_event(front_done)
             self.s_back.wait_event(ready)
             self.t.process_back_async(frames, out, bs, params=params, results_dev=self.results_dev[bs], ids=ids,
-                                      profiles=profiles)
+                                      profiles=profiles, cameras=cameras)
             done = torch.cuda.Event()
             done.record(self.s_back)
         self._back_done[bs] = done
@@ -860,7 +953,8 @@ class HostPipeline:
 
     ``submit(batch, ids=...)`` advances the listed streams only (see ``BatchedLaneTracker.process_async``); the
     frames and records of a finished batch are in batch order.  ``submit(batch, profiles=...)`` gives frame i
-    parameter profile profiles[i] (``BatchedLaneTracker.set_profile``) instead of the pipeline's ``params``.
+    parameter profile profiles[i] (``BatchedLaneTracker.set_profile``) instead of the pipeline's ``params``, and
+    ``submit(batch, cameras=...)`` says that frame i comes from camera cameras[i] (``BatchedLaneTracker.set_camera``).
     """
 
     def __init__(self, tracker, depth=3, overlay=True, params=None, inplace=False, frame_format="rgb"):
@@ -885,13 +979,6 @@ class HostPipeline:
             raise ValueError('inplace needs overlay=True')
         if self.inplace and self.nv12:
             raise ValueError("inplace annotation needs RGB frames: NV12 frames are annotated into separate RGB frames")
-        g = tracker.geometry
-        h_img = tracker.img_size[1]     # +-2 rows of slack: the fused remap variant samples the raw frame directly
-        self.rows_in = (max(0, min(g['source_rows'][0], g['overlay_rows'][0]) - 2),
-                        min(h_img, max(g['source_rows'][1], g['overlay_rows'][1]) + 2))
-        if self.nv12:       # the fused variant refuses NV12: the undistort reads exactly the source rows
-            self.rows_in = tuple(g['source_rows'])
-        self.rows_out = g['overlay_rows']
         self.rows_text = tracker.text_rows if tracker.text_enabled else (0, 0)   # putText rows: read and rewritten
         self.params = params if params is not None else make_params()
         dev = tracker.device
@@ -915,7 +1002,22 @@ class HostPipeline:
         self.tail = 0          # oldest slot in flight
         self.inflight = 0
 
-    def submit(self, host_frames, ids=None, profiles=None):
+    @property
+    def rows_in(self):
+        """Frame rows the partial host->device transfers move: over camera 0 and every camera set, so that any batch
+        is covered (set_camera may run between submissions)."""
+        src, ov = self.t.rows_any_camera()
+        if self.nv12:       # the fused variant refuses NV12: the undistort reads exactly the source rows
+            return src
+        h_img = self.t.img_size[1]     # +-2 rows of slack: the fused remap variant samples the raw frame directly
+        return max(0, min(src[0], ov[0]) - 2), min(h_img, max(src[1], ov[1]) + 2)
+
+    @property
+    def rows_out(self):
+        """Frame rows the lane overlay can change, over camera 0 and every camera set: what inplace mode copies back."""
+        return self.t.rows_any_camera()[1]
+
+    def submit(self, host_frames, ids=None, profiles=None, cameras=None):
         if self.inflight == self.depth:
             raise RuntimeError("pipeline full: collect a finished batch first")
         if not (host_frames.dtype == torch.uint8 and host_frames.is_pinned() and host_frames.is_contiguous()):
@@ -926,20 +1028,22 @@ class HostPipeline:
             raise ValueError("host_frames must be %s [n, %s] with 1 <= n <= %d, got %s"
                              % ("NV12" if self.nv12 else "RGB", ", ".join(map(str, sl["d_in"].shape[1:])),
                                 self.t.n_streams, list(host_frames.shape)))
-        self.t._check_ids(ids, n)                        # refuse bad ids / profiles before anything is enqueued
+        self.t._check_ids(ids, n)                        # refuse bad ids / profiles / cameras before anything is enqueued
         self.t._check_profiles(profiles, n)
+        self.t._check_cameras(cameras, n)
         params = self.params if profiles is None else None
+        rows_in, rows_out = self.rows_in, self.rows_out
         sl["n"] = n
         with torch.cuda.stream(self.s_in):
             self.s_in.wait_event(sl["e_run"])            # the kernels that last read this input buffer are done
             if self.inplace:
-                a, b = self.rows_in
+                a, b = rows_in
                 self.t.copy_rows(sl["d_in"], host_frames, a, b, True)
                 for ta, tb in _rows_minus(self.rows_text, (a, b)):      # text rows outside the rows already sent
                     self.t.copy_rows(sl["d_in"], host_frames, ta, tb, True)
                 sl["frames"] = host_frames
             elif self.nv12 and not self.overlay:
-                self.t.copy_rows(sl["d_in"], host_frames, self.rows_in[0], self.rows_in[1], True)
+                self.t.copy_rows(sl["d_in"], host_frames, rows_in[0], rows_in[1], True)
             else:
                 sl["d_in"][:n].copy_(host_frames, non_blocking=True)
             sl["e_in"].record(self.s_in)
@@ -949,7 +1053,7 @@ class HostPipeline:
             self.s_front.wait_event(sl["e_in"])
             if self._set_free[bs] is not None:
                 self.s_front.wait_event(self._set_free[bs])
-            self.t.process_front_async(sl["d_in"][:n], bs, params=params, profiles=profiles)
+            self.t.process_front_async(sl["d_in"][:n], bs, params=params, profiles=profiles, cameras=cameras)
             e_front = torch.cuda.Event()
             e_front.record(self.s_front)
         with torch.cuda.stream(self.s_run):
@@ -957,13 +1061,13 @@ class HostPipeline:
             self.s_run.wait_event(sl["e_out"])           # the previous D2H out of this output buffer is done
             d_out = sl["d_in"][:n] if self.inplace else (sl["d_out"][:n] if self.overlay else None)
             self.t.process_back_async(sl["d_in"][:n], d_out, bs, params=params, results_dev=sl["d_res"], ids=ids,
-                                      profiles=profiles)
+                                      profiles=profiles, cameras=cameras)
             sl["e_run"].record(self.s_run)
         self._set_free[bs] = sl["e_run"]
         with torch.cuda.stream(self.s_out):
             self.s_out.wait_event(sl["e_run"])
             if self.inplace:
-                a, b = self.rows_out
+                a, b = rows_out
                 if b > a:
                     self.t.copy_rows(host_frames, sl["d_in"][:n], a, b, False)
                 for ta, tb in _rows_minus(self.rows_text, (a, b)):      # text rows outside the rows already fetched
