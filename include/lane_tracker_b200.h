@@ -186,6 +186,28 @@ int lt_process_streams(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, co
 int lt_process_back_streams(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids, int32_t n,
                             const lt_params* params, int32_t set, lt_result* d_results, void* stream);
 
+/* Frame sequences: lt_process_streams in which ids may repeat.  The frames of one stream in the batch are consecutive
+ * frames of that stream, in batch-position order, so one batch can carry many frames of a single video.  The results
+ * equal, bit for bit, a series of lt_process_streams calls that feed each stream its frames one at a time.
+ *   h_ids: HOST int32 [n], 1 <= n <= max_streams, every id in [0, max_streams); repeats allowed.
+ * Addressing is that of lt_process_streams: frames, out frames, result records and masks by batch position, state by
+ * stream id.  After the call a stream's state, averaged polylines, cached lane polygon and captured pixel lists are
+ * those after its last frame in the batch; each out frame is drawn with the polygon and text of its own frame.
+ * The front half is lt_process_front, unchanged.  The back half runs in rounds: round r holds the positions that are
+ * the (r+1)-th frame of their stream in the batch, and the searches, second attempt and state update run round after
+ * round; the overlay and text then run once over the batch.  A batch without a repeated id enqueues exactly the
+ * launches of lt_process_streams.
+ * Refused before anything is enqueued, naming the position: n outside [1, max_streams], a null h_ids, an id out of
+ * range, and every other check of lt_process_streams except distinctness.  Nothing synchronises and the calls are
+ * capturable in a CUDA graph (the first sequence call with a repeated id allocates the handle's per-position snapshot
+ * buffers: make it before a capture).  Profiles and cameras are not available in these calls.
+ * lt_process_sequence(...) == lt_process_front(..., 0, stream) followed by lt_process_back_sequence(..., 0, ..., stream);
+ * lt_process_back_sequence is ordered like lt_process_back. */
+int lt_process_sequence(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids, int32_t n,
+                        const lt_params* params, lt_result* d_results, void* stream);
+int lt_process_back_sequence(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids, int32_t n,
+                             const lt_params* params, int32_t set, lt_result* d_results, void* stream);
+
 /* Parameter profiles: one batch whose frames use different lt_params and check_validity windows (cameras on different
  * roads or mounted differently; tracker_settings.md of the reference documents one set per demo video).
  * lt_set_profile stores profile `profile` (0 <= profile < LT_MAX_PROFILES) on the handle: `params`, checked like the

@@ -94,6 +94,8 @@ SIGNATURES = {
     "lt_process_back": (C.c_int, [P, P, P, i32, C.POINTER(lt_params), i32, P, P]),
     "lt_process_streams": (C.c_int, [P, P, P, C.POINTER(i32), i32, C.POINTER(lt_params), P, P]),
     "lt_process_back_streams": (C.c_int, [P, P, P, C.POINTER(i32), i32, C.POINTER(lt_params), i32, P, P]),
+    "lt_process_sequence": (C.c_int, [P, P, P, C.POINTER(i32), i32, C.POINTER(lt_params), P, P]),
+    "lt_process_back_sequence": (C.c_int, [P, P, P, C.POINTER(i32), i32, C.POINTER(lt_params), i32, P, P]),
     "lt_set_profile": (C.c_int, [P, i32, C.POINTER(lt_params), C.POINTER(lt_validity)]),
     "lt_process_profiles": (C.c_int, [P, P, P, C.POINTER(i32), C.POINTER(i32), i32, P, P]),
     "lt_process_front_profiles": (C.c_int, [P, P, C.POINTER(i32), i32, i32, P]),

@@ -167,7 +167,8 @@ extern "C" int lt_destroy(lt_handle* h) {
         for (void* p : cp) if (p) cudaFree(p);
     }
     void* ptrs[] = {h->und_map, h->bv_map, h->ov_map, h->bv_desc, h->und_desc, h->lab_yz, h->fused_desc, h->lab_gamma, h->lab_cbrt, h->lane_rows, h->lane_bbox, h->dl_bbox,
-                    h->avg_x, h->state, h->att, h->retry_list, h->retry_count, h->draw_flags, h->stream_ids, h->vis_scratch,
+                    h->avg_x, h->state, h->att, h->retry_list, h->retry_count, h->draw_flags, h->stream_ids, h->seq_pos,
+                    h->seq_rows, h->seq_bbox, h->seq_state, h->vis_scratch,
                     h->cap_pixels, h->cap_counts, h->cap_cents, h->cap_ncents, h->dl_rows, h->dl_flags, h->txt_state, h->txt_flags,
                     h->txt_tables, h->txt_char_start, h->txt_dy, h->txt_dx, h->txt_lut, h->txt_advance, h->txt_pair_overlap,
                     h->txt_bitmaps};
@@ -619,14 +620,42 @@ static int prepare_cameras(lt_handle* h, const int32_t* h_cams, int n, int set, 
 
 static bool allows_retry(int n_tries) { return n_tries >= 2 || n_tries == -1; }
 
+// The rounds of a sequence batch (lt_process_sequence): round r holds the positions that are the (r+1)-th occurrence
+// of their stream, in position order; pos[off[r] .. off[r+1]) are its positions.
+struct LtRounds {
+    std::vector<int> pos, off;
+};
+
+// Rounds of the ids h_ids[0..n) (in [0, S)); false when no id repeats (one round: the batch itself).
+static bool make_rounds(const int32_t* h_ids, int n, int S, LtRounds* r) {
+    std::vector<int> occ(n), seen(S, 0);
+    int R = 0;
+    for (int i = 0; i < n; ++i) {
+        occ[i] = seen[h_ids[i]]++;
+        R = occ[i] + 1 > R ? occ[i] + 1 : R;
+    }
+    if (R < 2) return false;
+    r->off.assign(R + 1, 0);
+    for (int i = 0; i < n; ++i) r->off[occ[i] + 1]++;
+    for (int k = 0; k < R; ++k) r->off[k + 1] += r->off[k];
+    std::vector<int> next(r->off.begin(), r->off.end() - 1);
+    r->pos.resize(n);
+    for (int i = 0; i < n; ++i) r->pos[next[occ[i]]++] = i;
+    return true;
+}
+
 // searches, second attempt of the streams that failed, state machine, overlay: advances the per-stream state.
 // h_ids (host, validated by check_ids) maps batch position i to state slot h_ids[i]; NULL: the identity.
 // fs: the buffer set whose profile snapshot the batch uses (NULL: p1 and the handle's windows for every position);
 // n_tries: of the batch (with profiles: 2 when some position may take a second attempt, else 1).
 // cf: the buffer set of a camera batch that is not on camera 0 alone (NULL otherwise).
+// rounds (NULL: every id distinct): a sequence batch, without profiles or cameras.  The searches, the second attempt
+// and the state update run round after round, each over its positions only, so that a frame sees the state its
+// stream's previous frame left; the update snapshots what the overlay and the text of each position read, and the
+// overlay and the text then run once over the batch from those snapshots.
 static int process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int n, int n_tries,
                         const LtAttemptParams& p1, lt_result* d_results, cudaStream_t st, bool own_begin,
-                        const int32_t* h_ids, const LtFrontSet* fs, const LtFrontSet* cf) {
+                        const int32_t* h_ids, const LtFrontSet* fs, const LtFrontSet* cf, const LtRounds* rounds = nullptr) {
     int rc;
     const LtAttemptParams p2 = second_attempt();
     const LtProfile* prof = fs ? fs->profiles : nullptr;
@@ -638,33 +667,50 @@ static int process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, i
         if ((rc = upload_stream_ids(h, h_ids, n, st))) return rc;
         ids = h->stream_ids;
     }
-    LtSearchArgs sa;
-    memset(&sa, 0, sizeof(sa));
-    sa.mask = h->mask; sa.mode = 0; sa.att = h->att; sa.do_fit = 1; sa.ids = ids;
+    // (h->seq_pos has one writer and its readers on this stream, as the stream ids: upload_stream_ids)
+    if (rounds && (rc = upload_ints(rounds->pos.data(), n, h->seq_pos, st))) return rc;
+    const int nr = rounds ? (int)rounds->off.size() - 1 : 1;
     const size_t S = h->S;
-    if (h->capture) {
-        sa.by_stream = 1; sa.pixels = h->cap_pixels; sa.pix_cap = h->pix_cap; sa.pix_counts = h->cap_counts;
-        sa.centroids = h->cap_cents; sa.ncentroids = h->cap_ncents;
-    }
-    if ((rc = lt_launch_search(h, n, p1, sa, nullptr, nullptr, st, prof, pos_prof, 1))) return rc;
-    lt_prof_mark(h, ST_SEARCH, st);
-    if (two) {
-        // second attempt only for the streams whose first attempt failed (lane_tracker.py:1071-1128).
-        // The reference re-runs undistort + warp here; their outputs are unchanged, so the planes are reused.
-        if ((rc = lt_launch_select_retry(h, n, n_tries, st, prof, pos_prof))) return rc;
-        lt_prof_mark(h, ST_RETRY_SELECT, st);
-        if ((rc = lt_launch_filter(h, n, p2, h->retry_list, h->retry_count, st))) return rc;
-        sa.att = h->att + h->S;
+    for (int r = 0; r < nr; ++r) {
+        const int* order = rounds ? h->seq_pos + rounds->off[r] : nullptr;
+        const int m = rounds ? rounds->off[r + 1] - rounds->off[r] : n;
+        LtSearchArgs sa;
+        memset(&sa, 0, sizeof(sa));
+        sa.mask = h->mask; sa.mode = 0; sa.att = h->att; sa.do_fit = 1; sa.ids = ids;
         if (h->capture) {
-            sa.pixels = h->cap_pixels + S * 2 * (size_t)h->pix_cap; sa.pix_counts = h->cap_counts + S * 2;
-            sa.centroids = h->cap_cents + S * 2 * LT_MAX_LEVELS; sa.ncentroids = h->cap_ncents + S * 2;
+            sa.by_stream = 1; sa.pixels = h->cap_pixels; sa.pix_cap = h->pix_cap; sa.pix_counts = h->cap_counts;
+            sa.centroids = h->cap_cents; sa.ncentroids = h->cap_ncents;
         }
-        if ((rc = lt_launch_search(h, n, p2, sa, h->retry_list, h->retry_count, st, prof, pos_prof, 0))) return rc;
+        if ((rc = lt_launch_search(h, m, p1, sa, order, nullptr, st, prof, pos_prof, 1))) return rc;
         lt_prof_mark(h, ST_SEARCH, st);
+        if (two) {
+            // second attempt only for the streams whose first attempt failed (lane_tracker.py:1071-1128).
+            // The reference re-runs undistort + warp here; their outputs are unchanged, so the planes are reused.
+            if ((rc = lt_launch_select_retry(h, m, n_tries, st, prof, pos_prof, order))) return rc;
+            lt_prof_mark(h, ST_RETRY_SELECT, st);
+            if ((rc = lt_launch_filter(h, m, p2, h->retry_list, h->retry_count, st))) return rc;
+            sa.att = h->att + h->S;
+            if (h->capture) {
+                sa.pixels = h->cap_pixels + S * 2 * (size_t)h->pix_cap; sa.pix_counts = h->cap_counts + S * 2;
+                sa.centroids = h->cap_cents + S * 2 * LT_MAX_LEVELS; sa.ncentroids = h->cap_ncents + S * 2;
+            }
+            if ((rc = lt_launch_search(h, m, p2, sa, h->retry_list, h->retry_count, st, prof, pos_prof, 0))) return rc;
+            lt_prof_mark(h, ST_SEARCH, st);
+        }
+        if ((rc = lt_launch_update_state(h, m, ids, d_results, two ? 2 : 1, st, cf, order))) return rc;
+        lt_prof_mark(h, ST_UPDATE, st);
     }
-    if ((rc = lt_launch_update_state(h, n, ids, d_results, two ? 2 : 1, st, cf))) return rc;
-    lt_prof_mark(h, ST_UPDATE, st);
     if (d_out) {
+        // a sequence batch draws every position from its snapshot: a view of the handle whose polygon rows, boxes and
+        // states are the snapshots, indexed by position (ids NULL), as lt_draw_lane and lt_draw_text draw
+        lt_handle view;
+        lt_handle* oh = h;
+        if (rounds) {
+            view = *h;
+            view.lane_rows = h->seq_rows; view.lane_bbox = h->seq_bbox; view.state = h->seq_state;
+            oh = &view;
+            ids = nullptr;
+        }
         // (copying the untouched rows on a side stream under the search kernels was measured: the copy saturates HBM
         // and slows the search by what it saves -- the plain in-order copy stays)
         // draw_lane writes its text into the frame BEFORE the blend (lane_tracker.py:653-662).  With the shipped
@@ -683,13 +729,13 @@ static int process_back(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, i
             } else if (d_out != d_frames) {
                 LT_CUDA(cudaMemcpyAsync(d_out, d_frames, (size_t)n * h->d.img_w * h->d.img_h * 3, cudaMemcpyDeviceToDevice, st));
             }
-            if ((rc = lt_launch_text(h, d_out, n, ids, st))) return rc;
-            if ((rc = lt_launch_overlay(h, d_out, d_out, n, h->draw_flags, ids, st, cf))) return rc;
+            if ((rc = lt_launch_text(oh, d_out, n, ids, st))) return rc;
+            if ((rc = lt_launch_overlay(oh, d_out, d_out, n, h->draw_flags, ids, st, cf))) return rc;
         } else {
-            if (nv12) rc = lt_launch_overlay_nv12(h, d_frames, d_out, n, h->draw_flags, ids, st, cf);
-            else rc = lt_launch_overlay(h, d_frames, d_out, n, h->draw_flags, ids, st, cf);
+            if (nv12) rc = lt_launch_overlay_nv12(oh, d_frames, d_out, n, h->draw_flags, ids, st, cf);
+            else rc = lt_launch_overlay(oh, d_frames, d_out, n, h->draw_flags, ids, st, cf);
             if (rc) return rc;
-            if ((rc = lt_launch_text(h, d_out, n, ids, st))) return rc;
+            if ((rc = lt_launch_text(oh, d_out, n, ids, st))) return rc;
         }
         lt_prof_mark(h, ST_OVERLAY, st);
     }
@@ -752,8 +798,9 @@ static int process_set(lt_handle* h, int set, int bandwidth) {
 }
 
 // Stream ids of lt_process_streams / lt_process_back_streams: 1 <= n <= S ids in [0, S), pairwise distinct (two
-// frames of one stream in a batch would race on its state).  Checked before anything is enqueued.
-static int check_ids(lt_handle* h, const int32_t* h_ids, int n) {
+// frames of one stream in a batch would race on its state) unless `repeats` (lt_process_sequence, whose back half
+// runs the frames of a stream in rounds).  Checked before anything is enqueued.
+static int check_ids(lt_handle* h, const int32_t* h_ids, int n, bool repeats = false) {
     int rc;
     if ((rc = check_n(h, n))) return rc;
     if (!h_ids) { lt_set_error("null stream id list"); return -1; }
@@ -761,7 +808,7 @@ static int check_ids(lt_handle* h, const int32_t* h_ids, int n) {
     for (int i = 0; i < n; ++i) {
         const int id = h_ids[i];
         if (id < 0 || id >= h->S) { lt_set_error("stream id %d at batch position %d outside [0, %d)", id, i, h->S); return -1; }
-        if (seen[id]) { lt_set_error("stream id %d appears twice in the batch (position %d)", id, i); return -1; }
+        if (seen[id] && !repeats) { lt_set_error("stream id %d appears twice in the batch (position %d)", id, i); return -1; }
         seen[id] = 1;
     }
     return 0;
@@ -809,7 +856,39 @@ static int check_cameras(lt_handle* h, const int32_t* h_cams, int n) {
 
 // What one process entry point does: the front half, the back half or both, with or without a stream id list, with
 // one lt_params or with a parameter profile per batch position, and with or without a camera per batch position.
-enum { PROC_FRONT = 1, PROC_BACK = 2, PROC_IDS = 4, PROC_PROFILES = 8, PROC_CAMERAS = 16 };
+// PROC_SEQ (with PROC_IDS): ids may repeat, the frames of a stream being its consecutive frames (lt_process_sequence).
+enum { PROC_FRONT = 1, PROC_BACK = 2, PROC_IDS = 4, PROC_PROFILES = 8, PROC_CAMERAS = 16, PROC_SEQ = 32 };
+
+// Grow the stage-timing event pool, keeping the events already recorded, so that `marks` more marks fit.
+static int prof_reserve(lt_handle* h, int marks) {
+    if (!h->prof_active || h->prof_n + marks <= h->prof_cap) return 0;
+    const int need = h->prof_n + marks, cap = need > 2 * h->prof_cap ? need : 2 * h->prof_cap;
+    cudaEvent_t* ev = new cudaEvent_t[cap];
+    int* stage = new int[cap];
+    for (int i = 0; i < h->prof_cap; ++i) { ev[i] = h->prof_ev[i]; stage[i] = h->prof_stage[i]; }
+    for (int i = h->prof_cap; i < cap; ++i)
+        if (cudaEventCreate(&ev[i]) != cudaSuccess) {
+            for (int k = h->prof_cap; k < i; ++k) cudaEventDestroy(ev[k]);
+            delete[] ev; delete[] stage;
+            lt_set_error("cannot create the stage-timing events");
+            return -2;
+        }
+    delete[] h->prof_ev; delete[] h->prof_stage;
+    h->prof_ev = ev; h->prof_stage = stage; h->prof_cap = cap;
+    return 0;
+}
+
+// Buffers of the sequence back half (LtRounds), allocated on first use like buffer set 1.
+static int alloc_sequence(lt_handle* h) {
+    if (h->seq_state) return 0;
+    LT_CUDA(cudaSetDevice(h->cfg.device));
+    const size_t S = h->S;
+    int rc = dev_alloc(&h->seq_pos, S);
+    if (!rc) rc = dev_alloc(&h->seq_rows, S * (size_t)h->d.bv_h);
+    if (!rc) rc = dev_alloc(&h->seq_bbox, S);
+    if (!rc) rc = dev_alloc(&h->seq_state, S);
+    return rc;
+}
 
 // The checks of the process entry points, in this order and all before anything is enqueued, then the halves.
 static int process_call(lt_handle* h, int what, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids, int n,
@@ -819,7 +898,7 @@ static int process_call(lt_handle* h, int what, const uint8_t* d_frames, uint8_t
     LtAttemptParams p1;
     const bool front = what & PROC_FRONT, back = what & PROC_BACK, profiles = what & PROC_PROFILES;
     const cudaStream_t st = (cudaStream_t)stream;
-    if ((what & PROC_IDS) && (rc = check_ids(h, h_ids, n))) return rc;
+    if ((what & PROC_IDS) && (rc = check_ids(h, h_ids, n, what & PROC_SEQ))) return rc;
     if (back && (rc = check_out(h, d_frames, d_out, n))) return rc;
     if ((rc = process_args(h, d_frames, n, profiles || params, set))) return rc;
     int bandwidth, n_tries;
@@ -881,6 +960,17 @@ static int process_call(lt_handle* h, int what, const uint8_t* d_frames, uint8_t
     }
     if ((rc = process_set(h, set, bandwidth))) return rc;
     if (back && !d_results) { lt_set_error("null argument"); return -1; }
+    // a sequence batch with a repeated id: its rounds, buffers and stage marks (a batch without one runs as
+    // lt_process_streams)
+    LtRounds rounds;
+    const bool seq = back && (what & PROC_SEQ) && make_rounds(h_ids, n, h->S, &rounds);
+    if (seq) {
+        if ((rc = alloc_sequence(h))) return rc;
+        // lt_profile_begin leaves room for the marks of its calls; a round adds up to six (search, retry selection,
+        // box, open5, search, update)
+        const int left = h->prof_max_calls - h->prof_calls;
+        if ((rc = prof_reserve(h, (32 + 2 * LT_MAX_PROFILES) * (left > 1 ? left : 1) + 6 * (int)rounds.off.size()))) return rc;
+    }
     LtFrontSet& fset = h->fs[set];
     if (front) {
         LtCamBatch cb = {nullptr, 0, 0};
@@ -900,7 +990,8 @@ static int process_call(lt_handle* h, int what, const uint8_t* d_frames, uint8_t
     if (!back) return 0;
     fset.cam_pending = 0;
     const LtFrontSet* cf = (cameras && !fset.cam_plain) ? &fset : nullptr;
-    return process_back(h, d_frames, d_out, n, n_tries, p1, d_results, st, !front, h_ids, profiles ? &fset : nullptr, cf);
+    return process_back(h, d_frames, d_out, n, n_tries, p1, d_results, st, !front, h_ids, profiles ? &fset : nullptr, cf,
+                        seq ? &rounds : nullptr);
 }
 
 extern "C" int lt_process(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, int32_t n, const lt_params* params,
@@ -926,6 +1017,18 @@ extern "C" int lt_process_streams(lt_handle* h, const uint8_t* d_frames, uint8_t
 extern "C" int lt_process_back_streams(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids,
                                        int32_t n, const lt_params* params, int32_t set, lt_result* d_results, void* stream) {
     return process_call(h, PROC_BACK | PROC_IDS, d_frames, d_out, h_ids, n, params, nullptr, set, d_results, stream);
+}
+
+extern "C" int lt_process_sequence(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids, int32_t n,
+                                   const lt_params* params, lt_result* d_results, void* stream) {
+    return process_call(h, PROC_FRONT | PROC_BACK | PROC_IDS | PROC_SEQ, d_frames, d_out, h_ids, n, params, nullptr, 0,
+                        d_results, stream);
+}
+
+extern "C" int lt_process_back_sequence(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids,
+                                        int32_t n, const lt_params* params, int32_t set, lt_result* d_results, void* stream) {
+    return process_call(h, PROC_BACK | PROC_IDS | PROC_SEQ, d_frames, d_out, h_ids, n, params, nullptr, set, d_results,
+                        stream);
 }
 
 extern "C" int lt_process_profiles(lt_handle* h, const uint8_t* d_frames, uint8_t* d_out, const int32_t* h_ids,
@@ -983,7 +1086,8 @@ void lt_prof_mark(lt_handle* h, int stage, cudaStream_t st) {
 extern "C" int lt_profile_begin(lt_handle* h, int32_t max_calls) {
     if (!h || max_calls < 1 || max_calls > 4096) { lt_set_error("bad argument"); return -1; }
     LT_CUDA(cudaSetDevice(h->cfg.device));
-    // a call marks at most about 20 boundaries, plus the threshold and noise stages once per filter group
+    // a call marks at most about 20 boundaries, plus the threshold and noise stages once per filter group (a sequence
+    // call with several rounds grows the pool before it enqueues: prof_reserve)
     int need = max_calls * (32 + 2 * LT_MAX_PROFILES);
     if (need > h->prof_cap) {
         cudaEvent_t* ev = new cudaEvent_t[need];

@@ -154,6 +154,12 @@ struct lt_handle {
     int* retry_list; int* retry_count;      // streams that need attempt 2
     int* draw_flags;             // [S]
     int* stream_ids;             // [S] state slot of each batch position of the last call with stream ids (lt_process_streams)
+    // sequence batches (lt_process_sequence), allocated on first use: the positions grouped by round, and per batch
+    // position what the overlay and the text of that frame read (k_update_state writes them, round by round)
+    int* seq_pos;                // [S]
+    int2* seq_rows;              // [S][bv_h]
+    int4* seq_bbox;              // [S]
+    LtDevState* seq_state;       // [S]
     int capture;                 // lt_set_capture
     uint32_t* cap_pixels;        // [2 attempts][S][2][pix_cap]
     int* cap_counts;             // [2][S][2]
@@ -275,11 +281,14 @@ struct LtSearchArgs {
 int lt_launch_search(lt_handle* h, int n, const LtAttemptParams& p, const LtSearchArgs& a, const int* list,
                      const int* count, cudaStream_t st, const LtProfile* prof = nullptr, const int* pos_prof = nullptr,
                      int prof_params = 0);
+// order (device, may be NULL; not with prof): the launch covers the batch positions order[0..n) instead of 0..n-1
 int lt_launch_select_retry(lt_handle* h, int n, int n_tries, cudaStream_t st, const LtProfile* prof = nullptr,
-                           const int* pos_prof = nullptr);
-// cf (may be NULL): the buffer set of a camera batch; position s then takes mppv / mpph from cf->cams[cf->pos_cam[s]]
+                           const int* pos_prof = nullptr, const int* order = nullptr);
+// cf (may be NULL): the buffer set of a camera batch; position s then takes mppv / mpph from cf->cams[cf->pos_cam[s]].
+// order (device, may be NULL; not with cf): CTA b updates batch position order[b] and also writes the position's
+// polygon rows, bounding box and state to h->seq_rows / seq_bbox / seq_state.
 int lt_launch_update_state(lt_handle* h, int n, const int* ids, lt_result* d_results, int attempts_allowed,
-                           cudaStream_t st, const LtFrontSet* cf = nullptr);
+                           cudaStream_t st, const LtFrontSet* cf = nullptr, const int* order = nullptr);
 int lt_launch_fit_pixels(lt_handle* h, const uint32_t* d_pixels, int cap, const int* d_counts, int n,
                          double* d_fits, cudaStream_t st);
 int lt_launch_validity(lt_handle* h, const double* d_fits, int n, int* d_valid, double* d_diffs, cudaStream_t st);

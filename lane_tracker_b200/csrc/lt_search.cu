@@ -619,14 +619,17 @@ int lt_launch_search(lt_handle* h, int n, const LtAttemptParams& p, const LtSear
 // attempt-2 selection (lane_tracker.py:1071)
 // ---------------------------------------------------------------------------
 
-// PROF: n_tries of position s is prof[pos_prof[s]].n_tries
-template <bool PROF>
+// PROF: n_tries of position s is prof[pos_prof[s]].n_tries.  ORDER: the batch positions are order[0..n) (one round
+// of a sequence batch) instead of 0..n-1.
+template <bool PROF, bool ORDER>
 __global__ void k_select_retry(const LtAttemptOut* __restrict__ att, int n, int n_tries, int* list, int* count,
-                               int* flags, const LtProfile* __restrict__ prof, const int* __restrict__ pos_prof) {
+                               int* flags, const LtProfile* __restrict__ prof, const int* __restrict__ pos_prof,
+                               const int* __restrict__ order) {
     // single CTA, ordered compaction so that the retry list is deterministic
     if (threadIdx.x == 0) {
         int c = 0;
-        for (int s = 0; s < n; ++s) {
+        for (int i = 0; i < n; ++i) {
+            const int s = ORDER ? order[i] : i;
             if (PROF) n_tries = prof[pos_prof[s]].n_tries;
             bool retry = ((!att[s].detected) | (!att[s].valid)) & ((n_tries >= 2) | (n_tries == -1));
             flags[s] = retry;
@@ -636,13 +639,17 @@ __global__ void k_select_retry(const LtAttemptOut* __restrict__ att, int n, int 
     }
 }
 
-int lt_launch_select_retry(lt_handle* h, int n, int n_tries, cudaStream_t st, const LtProfile* prof, const int* pos_prof) {
+int lt_launch_select_retry(lt_handle* h, int n, int n_tries, cudaStream_t st, const LtProfile* prof, const int* pos_prof,
+                           const int* order) {
     if (prof)
-        k_select_retry<true><<<1, 32, 0, st>>>(h->att, n, n_tries, h->retry_list, h->retry_count, h->draw_flags + h->S, prof,
-                                               pos_prof);
+        k_select_retry<true, false><<<1, 32, 0, st>>>(h->att, n, n_tries, h->retry_list, h->retry_count, h->draw_flags + h->S,
+                                                      prof, pos_prof, nullptr);
+    else if (order)
+        k_select_retry<false, true><<<1, 32, 0, st>>>(h->att, n, n_tries, h->retry_list, h->retry_count, h->draw_flags + h->S,
+                                                      nullptr, nullptr, order);
     else
-        k_select_retry<false><<<1, 32, 0, st>>>(h->att, n, n_tries, h->retry_list, h->retry_count, h->draw_flags + h->S,
-                                                nullptr, nullptr);
+        k_select_retry<false, false><<<1, 32, 0, st>>>(h->att, n, n_tries, h->retry_list, h->retry_count, h->draw_flags + h->S,
+                                                       nullptr, nullptr, nullptr);
     LT_LAUNCH_CHECK();
     return 0;
 }
@@ -750,15 +757,25 @@ __device__ void lane_rows_from_polylines(const int* xl, int nl, const int* xr, i
 // per-frame state update (lane_tracker.py:1142-1209)
 // ---------------------------------------------------------------------------
 
+// What the overlay and the text of one frame read, per batch position (LtSeqSnap): the update of a round of a sequence
+// batch copies them out of the stream's slot before a later frame of the stream overwrites it.
+struct LtSeqSnap {
+    int2* rows;                  // [S][bv_h] lane polygon rows: this frame's on a valid frame, the stream's cache otherwise
+    int4* bbox;                  // [S] their bounding box
+    LtDevState* state;           // [S] the stream's state after this frame (k_text formats from it)
+};
+
 // CAMS: position s takes mppv / mpph from its camera, cams[pos_cam[s]] (the handle's cfg otherwise).
-template <bool CAMS>
+// SEQ: CTA b updates batch position order[b] (one round of a sequence batch) and writes its snapshot to snap.
+template <bool CAMS, bool SEQ>
 __global__ void __launch_bounds__(SEARCH_THREADS)
 k_update_state(LtDims d, lt_config cfg, LtDevState* __restrict__ state, const LtAttemptOut* __restrict__ att1,
                const LtAttemptOut* __restrict__ att2, const int* __restrict__ retry, int* __restrict__ avg_x,
                int2* __restrict__ lane_rows, int4* __restrict__ lane_bbox, int* __restrict__ draw, lt_result* __restrict__ results,
-               const int* __restrict__ ids, const LtCamDev* __restrict__ cams, const int* __restrict__ pos_cam) {
+               const int* __restrict__ ids, const LtCamDev* __restrict__ cams, const int* __restrict__ pos_cam,
+               const int* __restrict__ order, LtSeqSnap snap) {
     // s: batch position (attempt outputs, retry and draw flags, result record); sid: state slot of its stream
-    const int s = blockIdx.x, sid = ids ? ids[s] : s, tid = threadIdx.x, W = d.bv_w, H = d.bv_h;
+    const int s = SEQ ? order[blockIdx.x] : blockIdx.x, sid = ids ? ids[s] : s, tid = threadIdx.x, W = d.bv_w, H = d.bv_h;
     extern __shared__ unsigned char smem_raw[];
     int* flags = reinterpret_cast<int*>(smem_raw);        // [H]
     int* stage = flags + H;                               // [2*H]
@@ -877,20 +894,35 @@ k_update_state(LtDims d, lt_config cfg, LtDevState* __restrict__ state, const Lt
         r.first_n_left = f1.n[0]; r.first_n_right = f1.n[1];
         for (int j = 0; j < 3; ++j) { r.first_left_fit[j] = f1.fit[0][j]; r.first_right_fit[j] = f1.fit[1][j]; }
     }
+    if (SEQ) {
+        static_assert(sizeof(LtDevState) % sizeof(int) == 0, "LtDevState is copied as words");
+        __syncthreads();                                  // the rows, box and state of this frame are complete
+        for (int y = tid; y < H; y += blockDim.x) snap.rows[(size_t)s * H + y] = lane_rows[(size_t)sid * H + y];
+        if (tid == 0) snap.bbox[s] = lane_bbox[sid];
+        const int* src = reinterpret_cast<const int*>(state + sid);
+        int* dst = reinterpret_cast<int*>(snap.state + s);
+        for (int i = tid; i < (int)(sizeof(LtDevState) / sizeof(int)); i += blockDim.x) dst[i] = src[i];
+    }
 }
 
 int lt_launch_update_state(lt_handle* h, int n, const int* ids, lt_result* d_results, int attempts_allowed,
-                           cudaStream_t st, const LtFrontSet* cf) {
+                           cudaStream_t st, const LtFrontSet* cf, const int* order) {
     size_t smem = (size_t)3 * h->d.bv_h * sizeof(int);
     const int* retry = attempts_allowed >= 2 ? h->draw_flags + h->S : nullptr;
+    const LtSeqSnap none = {nullptr, nullptr, nullptr};
     if (cf)
-        k_update_state<true><<<n, SEARCH_THREADS, smem, st>>>(h->d, h->cfg, h->state, h->att, h->att + h->S, retry, h->avg_x,
-                                                              h->lane_rows, h->lane_bbox, h->draw_flags, d_results, ids,
-                                                              cf->cams, cf->pos_cam);
+        k_update_state<true, false><<<n, SEARCH_THREADS, smem, st>>>(h->d, h->cfg, h->state, h->att, h->att + h->S, retry,
+                                                                     h->avg_x, h->lane_rows, h->lane_bbox, h->draw_flags,
+                                                                     d_results, ids, cf->cams, cf->pos_cam, nullptr, none);
+    else if (order)
+        k_update_state<false, true><<<n, SEARCH_THREADS, smem, st>>>(h->d, h->cfg, h->state, h->att, h->att + h->S, retry,
+                                                                     h->avg_x, h->lane_rows, h->lane_bbox, h->draw_flags,
+                                                                     d_results, ids, nullptr, nullptr, order,
+                                                                     {h->seq_rows, h->seq_bbox, h->seq_state});
     else
-        k_update_state<false><<<n, SEARCH_THREADS, smem, st>>>(h->d, h->cfg, h->state, h->att, h->att + h->S, retry, h->avg_x,
-                                                               h->lane_rows, h->lane_bbox, h->draw_flags, d_results, ids,
-                                                               nullptr, nullptr);
+        k_update_state<false, false><<<n, SEARCH_THREADS, smem, st>>>(h->d, h->cfg, h->state, h->att, h->att + h->S, retry,
+                                                                      h->avg_x, h->lane_rows, h->lane_bbox, h->draw_flags,
+                                                                      d_results, ids, nullptr, nullptr, nullptr, none);
     LT_LAUNCH_CHECK();
     return 0;
 }

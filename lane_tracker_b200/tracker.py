@@ -349,9 +349,10 @@ class BatchedLaneTracker:
             raise ValueError("frames must be RGB [n, %d, %d, 3] here, got NV12 frames" % (h, w))
         return n
 
-    def _check_ids(self, ids, n):
+    def _check_ids(self, ids, n, repeats=False):
         """Stream ids of a batch of n frames -> ctypes int32 array (None: None).  Any int sequence, NumPy array or CPU
-        tensor of n distinct ids in [0, n_streams); frame i belongs to stream ids[i]."""
+        tensor of n distinct ids in [0, n_streams); frame i belongs to stream ids[i].  repeats=True (a sequence batch):
+        ids may repeat."""
         if ids is None:
             return None
         if isinstance(ids, torch.Tensor):
@@ -367,7 +368,7 @@ class BatchedLaneTracker:
         if bad.size:
             raise ValueError("stream id %d outside [0, %d)" % (int(bad[0]), self.n_streams))
         u, counts = np.unique(a, return_counts=True)
-        if (counts > 1).any():
+        if not repeats and (counts > 1).any():
             raise ValueError("stream id %d appears more than once in the batch" % int(u[counts > 1][0]))
         return (C.c_int32 * n)(*[int(v) for v in a])
 
@@ -415,6 +416,15 @@ class BatchedLaneTracker:
         return (C.c_int32 * n)(*[int(v) for v in a])
 
     @staticmethod
+    def _check_sequence(sequence, ids, profiles, cameras):
+        if not sequence:
+            return
+        if ids is None:
+            raise ValueError("sequence=True needs ids: the stream of every frame")
+        if profiles is not None or cameras is not None:
+            raise ValueError("sequence=True takes neither profiles nor cameras")
+
+    @staticmethod
     def _no_params_with_profiles(profiles, params, kw):
         if profiles is not None and (params is not None or kw):
             raise ValueError("profiles= selects the parameters of every frame: pass it without params or keyword options")
@@ -431,7 +441,7 @@ class BatchedLaneTracker:
             raise ValueError("out must start at a 4-byte aligned address (the kernels access frames as 32-bit words)")
 
     def process_async(self, frames, out=None, params=None, results_dev=None, ids=None, profiles=None, cameras=None,
-                      **kw):
+                      sequence=False, **kw):
         """Enqueue one frame per stream on the current CUDA stream; returns the number of frames.
 
         frames: uint8 CUDA tensor [n, H, W, 3] (RGB) or [n, H * 3 / 2, W] (NV12: the luma plane, then interleaved
@@ -446,8 +456,14 @@ class BatchedLaneTracker:
         keyword options may not be given.
         cameras: None -- every frame comes from camera 0 (the constructor's calibration); else n camera indices (see
         ``set_camera``): frame i was filmed by camera cameras[i].  A caller with one camera per stream passes
-        camera_of[ids]."""
-        return self._process_call(frames, out, None, params, results_dev, ids, kw, profiles, cameras)
+        camera_of[ids].
+        sequence: True -- ids may repeat: the frames of one stream are consecutive frames of that stream, in batch
+        order, and the results equal feeding them one at a time (``ids`` required; no ``profiles`` or ``cameras``).
+        One video, 64 frames per call::
+
+            for chunk, out in chunks:          # [<= n_streams, H, W, 3] consecutive frames of stream 0
+                tracker.process_async(chunk, out, ids=[0] * len(chunk), sequence=True)"""
+        return self._process_call(frames, out, None, params, results_dev, ids, kw, profiles, cameras, sequence)
 
     def process_front_async(self, frames, buffer_set, params=None, profiles=None, cameras=None, **kw):
         """First half of ``process_async`` (undistort, warp, first-attempt filter) into intermediate buffer set
@@ -471,18 +487,21 @@ class BatchedLaneTracker:
         return n
 
     def process_back_async(self, frames, out, buffer_set, params=None, results_dev=None, ids=None, profiles=None,
-                           cameras=None, **kw):
+                           cameras=None, sequence=False, **kw):
         """Second half of ``process_async`` (searches, second attempt, state machine, overlay) from intermediate
         buffer set 0 or 1, on the current CUDA stream.  Advances the per-stream state of the streams in ``ids``
         (None: streams 0..n-1), as ``process_async``.  RGB or NV12 frames, as given to the front half.  ``profiles``,
-        ``cameras``: those the front half of this buffer set was given."""
-        return self._process_call(frames, out, buffer_set, params, results_dev, ids, kw, profiles, cameras)
+        ``cameras``: those the front half of this buffer set was given.  ``sequence``: as ``process_async`` (the
+        front half takes no ids)."""
+        return self._process_call(frames, out, buffer_set, params, results_dev, ids, kw, profiles, cameras, sequence)
 
-    def _process_call(self, frames, out, buffer_set, params, results_dev, ids, kw, profiles=None, cameras=None):
+    def _process_call(self, frames, out, buffer_set, params, results_dev, ids, kw, profiles=None, cameras=None,
+                      sequence=False):
         """Checks and C call of ``process_async`` (buffer_set None: both halves) or ``process_back_async``; -> n."""
         n = self._input(frames)
         self._check_out(out, frames)
-        h_ids = self._check_ids(ids, n)
+        self._check_sequence(sequence, ids, profiles, cameras)
+        h_ids = self._check_ids(ids, n, repeats=sequence)
         self._no_params_with_profiles(profiles, params, kw)
         h_prof = self._check_profiles(profiles, n)
         h_cam = self._check_cameras(cameras, n)
@@ -510,8 +529,12 @@ class BatchedLaneTracker:
         p = params if params is not None else make_params(**kw)
         if buffer_set is None:
             plain, streams, set_arg = self.lib.lt_process, self.lib.lt_process_streams, ()
+            if sequence:
+                streams = self.lib.lt_process_sequence
         else:
             plain, streams, set_arg = self.lib.lt_process_back, self.lib.lt_process_back_streams, (int(buffer_set),)
+            if sequence:
+                streams = self.lib.lt_process_back_sequence
         fn, ids_arg = (plain, ()) if h_ids is None else (streams, (h_ids,))
         check(fn(self._h, _ptr(frames), _ptr(out), *ids_arg, n, C.byref(p), *set_arg, _ptr(res),
                  _stream_ptr(self.device)))
@@ -527,11 +550,13 @@ class BatchedLaneTracker:
         torch.cuda.current_stream(self.device).synchronize()
         return self._results_host[:nbytes].numpy().view(RESULT_DTYPE).copy()
 
-    def process(self, frames, out=None, params=None, ids=None, profiles=None, cameras=None, **kw):
+    def process(self, frames, out=None, params=None, ids=None, profiles=None, cameras=None, sequence=False, **kw):
         """``process_async`` followed by ``fetch_results``: the n result records, in batch order.  With ``ids``, frame
         i advances stream ids[i] and the other streams keep their state; with ``profiles``, frame i uses parameter
-        profile profiles[i] (``set_profile``); with ``cameras``, frame i comes from camera cameras[i] (``set_camera``)."""
-        n = self.process_async(frames, out, params, ids=ids, profiles=profiles, cameras=cameras, **kw)
+        profile profiles[i] (``set_profile``); with ``cameras``, frame i comes from camera cameras[i] (``set_camera``);
+        with ``sequence=True``, ids may repeat and a stream's frames are its consecutive frames, in batch order."""
+        n = self.process_async(frames, out, params, ids=ids, profiles=profiles, cameras=cameras, sequence=sequence,
+                               **kw)
         return self.fetch_results(n)
 
     # -- stage methods (device tensors) ---------------------------------------
@@ -871,7 +896,11 @@ class DevicePipeline:
     results stay in batch order.  ``frames`` may be RGB or NV12 (``out`` is RGB either way), batch by batch.
     ``submit(..., profiles=...)`` gives frame i parameter profile profiles[i] (``BatchedLaneTracker.set_profile``)
     instead of the pipeline's ``params``; ``submit(..., cameras=...)`` says that frame i comes from camera cameras[i]
-    (``BatchedLaneTracker.set_camera``).
+    (``BatchedLaneTracker.set_camera``).  ``submit(frames, out, ids=..., sequence=True)`` lets ids repeat: the frames
+    of one stream are its consecutive frames, in batch order.  One video, 64 frames per batch::
+
+        for chunk, out in chunks:              # consecutive frames of one video, up to n_streams per chunk
+            pipe.submit(chunk, out, ids=[0] * len(chunk), sequence=True)
     """
 
     def __init__(self, tracker, params=None):
@@ -886,10 +915,11 @@ class DevicePipeline:
         self.results_dev = [torch.zeros(tracker.n_streams * RESULT_DTYPE.itemsize, dtype=torch.uint8, device=dev)
                             for _ in range(2)]
 
-    def submit(self, frames, out=None, ids=None, profiles=None, cameras=None):
+    def submit(self, frames, out=None, ids=None, profiles=None, cameras=None, sequence=False):
         dev = self.t.device
         n = self.t._frame_format(frames)[0]
-        self.t._check_ids(ids, n)                      # refuse bad frames / ids / profiles / cameras before anything is enqueued
+        self.t._check_sequence(sequence, ids, profiles, cameras)
+        self.t._check_ids(ids, n, repeats=sequence)    # refuse bad frames / ids / profiles / cameras before anything is enqueued
         self.t._check_profiles(profiles, n)
         self.t._check_cameras(cameras, n)
         params = self.params if profiles is None else None
@@ -907,7 +937,7 @@ class DevicePipeline:
             self.s_back.wait_event(front_done)
             self.s_back.wait_event(ready)
             self.t.process_back_async(frames, out, bs, params=params, results_dev=self.results_dev[bs], ids=ids,
-                                      profiles=profiles, cameras=cameras)
+                                      profiles=profiles, cameras=cameras, sequence=sequence)
             done = torch.cuda.Event()
             done.record(self.s_back)
         self._back_done[bs] = done
@@ -955,6 +985,8 @@ class HostPipeline:
     frames and records of a finished batch are in batch order.  ``submit(batch, profiles=...)`` gives frame i
     parameter profile profiles[i] (``BatchedLaneTracker.set_profile``) instead of the pipeline's ``params``, and
     ``submit(batch, cameras=...)`` says that frame i comes from camera cameras[i] (``BatchedLaneTracker.set_camera``).
+    ``submit(batch, ids=..., sequence=True)`` lets ids repeat: the frames of one stream are its consecutive frames, in
+    batch order (``pipe.submit(chunk, ids=[0] * len(chunk), sequence=True)`` for one video).
     """
 
     def __init__(self, tracker, depth=3, overlay=True, params=None, inplace=False, frame_format="rgb"):
@@ -1017,7 +1049,7 @@ class HostPipeline:
         """Frame rows the lane overlay can change, over camera 0 and every camera set: what inplace mode copies back."""
         return self.t.rows_any_camera()[1]
 
-    def submit(self, host_frames, ids=None, profiles=None, cameras=None):
+    def submit(self, host_frames, ids=None, profiles=None, cameras=None, sequence=False):
         if self.inflight == self.depth:
             raise RuntimeError("pipeline full: collect a finished batch first")
         if not (host_frames.dtype == torch.uint8 and host_frames.is_pinned() and host_frames.is_contiguous()):
@@ -1028,7 +1060,8 @@ class HostPipeline:
             raise ValueError("host_frames must be %s [n, %s] with 1 <= n <= %d, got %s"
                              % ("NV12" if self.nv12 else "RGB", ", ".join(map(str, sl["d_in"].shape[1:])),
                                 self.t.n_streams, list(host_frames.shape)))
-        self.t._check_ids(ids, n)                        # refuse bad ids / profiles / cameras before anything is enqueued
+        self.t._check_sequence(sequence, ids, profiles, cameras)
+        self.t._check_ids(ids, n, repeats=sequence)      # refuse bad ids / profiles / cameras before anything is enqueued
         self.t._check_profiles(profiles, n)
         self.t._check_cameras(cameras, n)
         params = self.params if profiles is None else None
@@ -1061,7 +1094,7 @@ class HostPipeline:
             self.s_run.wait_event(sl["e_out"])           # the previous D2H out of this output buffer is done
             d_out = sl["d_in"][:n] if self.inplace else (sl["d_out"][:n] if self.overlay else None)
             self.t.process_back_async(sl["d_in"][:n], d_out, bs, params=params, results_dev=sl["d_res"], ids=ids,
-                                      profiles=profiles, cameras=cameras)
+                                      profiles=profiles, cameras=cameras, sequence=sequence)
             sl["e_run"].record(self.s_run)
         self._set_free[bs] = sl["e_run"]
         with torch.cuda.stream(self.s_out):
