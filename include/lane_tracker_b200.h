@@ -121,7 +121,10 @@ typedef struct lt_validity {
  * Builds the fixed-point remap tables on the device.  Synchronous. */
 int lt_create(const lt_config* cfg, lt_handle** out);
 int lt_destroy(lt_handle* h);
-/* Re-zero the state of the listed streams (ids == NULL: all). Synchronous. */
+/* Re-zero the state of the listed streams (ids == NULL: all): one cudaMemcpy per id from host memory on the legacy
+ * default stream.  It is NOT ordered against work enqueued on other CUDA streams (non-blocking streams, such as the ones
+ * the pipelines run their back halves on, do not wait for it): use it only with no work of the handle in flight.  To
+ * start a new video on a stream while batches are in flight, use lt_reset_async on the stream of the back halves. */
 int lt_reset(lt_handle* h, const int32_t* ids, int32_t n);
 int lt_set_validity(lt_handle* h, const lt_validity* v);     /* NULL restores the shipped constants */
 int lt_get_validity(lt_handle* h, lt_validity* v);
@@ -263,7 +266,8 @@ int lt_set_camera(lt_handle* h, int32_t camera, const lt_camera* cam);
  *   h_cameras : HOST int32 [n], position i was filmed by camera h_cameras[i] (its undistort, warp, overlay and the
  *               metres per pixel of its curve radii and eccentricity).  Cameras belong to batch positions, like
  *               profiles: a caller that keeps one camera per stream passes camera_of[ids].  A stream may change camera
- *               between frames; its tracking state carries over (reset a re-mounted camera's stream with lt_reset).
+ *               between frames; its tracking state carries over (start a re-mounted camera's stream afresh with
+ *               lt_reset_async, enqueued before the back half of the batch that carries its first new frame).
  *               Copied when the call is enqueued: nothing synchronises and the calls are capturable in a CUDA graph.
  *   params / h_profiles: exactly one is non-NULL (lt_process_streams or lt_process_profiles semantics).
  *   h_ids     : as lt_process_streams; NULL means the identity 0..n-1.
@@ -472,6 +476,50 @@ int lt_get_state(lt_handle* h, int32_t stream_id, lt_state* h_state, int32_t* h_
                  int32_t* h_right_avg_x);   /* polylines: bv_h ints each, may be NULL. Synchronous. */
 int lt_set_state(lt_handle* h, int32_t stream_id, const lt_state* h_state, const int32_t* h_left_avg_x,
                  const int32_t* h_right_avg_x);
+
+/* ---- stream starts and state records (stream-ordered) ----------------------
+ * lt_reset_async: what lt_reset writes for the streams h_ids[0..n) (h_ids == NULL: every stream, n ignored), enqueued
+ *   on `stream`: the initial state of lt_create (last_detection = n_reset + 1, everything else zero).  The ids travel
+ *   as kernel arguments (one single-CTA launch per 1000 ids): h_ids may be reused when the call returns, nothing
+ *   synchronises, and the call is capturable in a CUDA graph.  Like lt_reset it writes the tracking state only: the
+ *   averaged polylines and the cached lane polygon of the old video stay in place but are not read again (nothing is
+ *   drawn on a failing frame before a valid one rebuilds them).
+ *   Usage: to start a new video on stream s in the batch you are about to enqueue, enqueue lt_reset_async({s}) on that
+ *   batch's back-half stream, after the previous back half and before this one (lane_tracker_b200 does this for
+ *   `starts=`).  Refused before anything is enqueued, naming the position: n outside [1, max_streams], an id out of
+ *   range, a repeated id.
+ *
+ * State records move streams between slots, handles and GPUs without stopping the device.  A record is
+ * lt_state_record_bytes(h) bytes (a multiple of 16: 18320 bytes at the shipped 1080x1100 bird's-eye view) and holds
+ * everything a later frame of the stream reads:
+ *   [0, 64)            header, int32 words: LT_RECORD_MAGIC, LT_ABI_VERSION, sizeof(lt_state), bv_w, bv_h, n_average,
+ *                      n_fail, n_reset, then zeros;
+ *   [64, A)            the tracking state (lt_state), zero-padded to 16 bytes: A = 64 + round_up(sizeof(lt_state), 16);
+ *   [A, A + 8 bv_h)    the averaged polylines, int32 [2][bv_h] (left, right; vertex i of side k on row
+ *                      bv_h - n_k_avg + i);
+ *   [R = A + 8 bv_h, R + 8 bv_h)   the cached lane polygon rows, int32 [bv_h][2] (first, last column; empty: first > last);
+ *   [B = round_up(R + 8 bv_h, 16), B + 16)   their bounding box, int32 [4] (min first, max last, first row, last row);
+ *   zeros to the end.
+ * Captured pixel lists (lt_set_capture) and per-batch outputs (result records, draw flags) are not state: they are not
+ * carried.
+ * lt_export_states gathers the records of streams h_ids[i] into d_dst + i * record_bytes; lt_import_states scatters the
+ *   records d_src + i * record_bytes into slots h_ids[i].  Both on `stream`, ordered like the back halves they sit
+ *   between; nothing synchronises and both are capturable.  h_ids: HOST int32 [n], 1 <= n <= max_streams, distinct ids
+ *   in [0, max_streams) (refused before anything is enqueued, naming the position).  d_dst / d_src: device memory of
+ *   the handle's GPU, 16-byte aligned.
+ * lt_import_states checks every record on the device before it writes any of it: the header against the handle's
+ *   (LT_RECORD_BAD_HEADER), and every field a kernel later uses as an index or a loop bound (LT_RECORD_BAD_STATE):
+ *   ring_len and radii_len in [0, n_average], n_left_avg and n_right_avg in [0, bv_h], every non-empty polygon row and
+ *   a non-empty bounding box inside the bird's-eye view.  A refused record is not applied: the slot keeps its bytes.
+ *   d_status (device int32 [n], may be NULL) receives LT_RECORD_OK or the code of each record. */
+#define LT_RECORD_MAGIC 0x5253544CU    /* "LTSR" */
+#define LT_RECORD_OK 0
+#define LT_RECORD_BAD_HEADER 1
+#define LT_RECORD_BAD_STATE 2
+int lt_reset_async(lt_handle* h, const int32_t* h_ids, int32_t n, void* stream);
+int64_t lt_state_record_bytes(lt_handle* h);
+int lt_export_states(lt_handle* h, const int32_t* h_ids, int32_t n, void* d_dst, void* stream);
+int lt_import_states(lt_handle* h, const int32_t* h_ids, int32_t n, const void* d_src, int32_t* d_status, void* stream);
 
 /* Debug/test access to internal buffers of the last lt_process / stage call.  stream_id is a batch position for
  * items 3-8 (buffers of the last batch) and a stream id for item 9 (per-stream cache); the two coincide for lt_process.

@@ -17,6 +17,8 @@ LT_MAX_CAMERAS = 64
 LT_MAX_LEVELS = 128
 LT_ABI_VERSION = 4
 LT_NSTAGES = 16
+# lt_import_states status codes
+LT_RECORD_OK, LT_RECORD_BAD_HEADER, LT_RECORD_BAD_STATE = 0, 1, 2
 
 i32, f64 = C.c_int32, C.c_double
 
@@ -136,6 +138,10 @@ SIGNATURES = {
     "lt_get_state": (C.c_int, [P, i32, C.POINTER(lt_state), P, P]),
     "lt_set_state": (C.c_int, [P, i32, C.POINTER(lt_state), P, P]),
     "lt_debug_read": (C.c_int64, [P, i32, i32, P, C.c_int64]),
+    "lt_reset_async": (C.c_int, [P, C.POINTER(i32), i32, P]),
+    "lt_state_record_bytes": (C.c_int64, [P]),
+    "lt_export_states": (C.c_int, [P, C.POINTER(i32), i32, P, P]),
+    "lt_import_states": (C.c_int, [P, C.POINTER(i32), i32, P, P, P]),
 }
 
 _lib = None

@@ -167,7 +167,7 @@ extern "C" int lt_destroy(lt_handle* h) {
         for (void* p : cp) if (p) cudaFree(p);
     }
     void* ptrs[] = {h->und_map, h->bv_map, h->ov_map, h->bv_desc, h->und_desc, h->lab_yz, h->fused_desc, h->lab_gamma, h->lab_cbrt, h->lane_rows, h->lane_bbox, h->dl_bbox,
-                    h->avg_x, h->state, h->att, h->retry_list, h->retry_count, h->draw_flags, h->stream_ids, h->seq_pos,
+                    h->avg_x, h->state, h->init, h->att, h->retry_list, h->retry_count, h->draw_flags, h->stream_ids, h->seq_pos,
                     h->seq_rows, h->seq_bbox, h->seq_state, h->vis_scratch,
                     h->cap_pixels, h->cap_counts, h->cap_cents, h->cap_ncents, h->dl_rows, h->dl_flags, h->txt_state, h->txt_flags,
                     h->txt_tables, h->txt_char_start, h->txt_dy, h->txt_dx, h->txt_lut, h->txt_advance, h->txt_pair_overlap,
@@ -349,7 +349,7 @@ extern "C" int lt_create(const lt_config* cfg, lt_handle** out) {
     if (!rc) rc = alloc_front_set(h, 0);
     if (!rc) select_set(h, 0);
     A(lane_rows, S * (size_t)d.bv_h); A(lane_bbox, S); A(avg_x, S * 2 * (size_t)d.bv_h);
-    A(state, S); A(att, 2 * S); A(retry_list, S); A(retry_count, 1); A(draw_flags, 2 * S); A(stream_ids, S);
+    A(state, S); A(init, 1); A(att, 2 * S); A(retry_list, S); A(retry_count, 1); A(draw_flags, 2 * S); A(stream_ids, S);
 #undef A
     if (rc) { lt_destroy(h); return rc; }
     if (cudaStreamCreateWithFlags(&h->side, cudaStreamNonBlocking) != cudaSuccess ||
@@ -363,6 +363,13 @@ extern "C" int lt_create(const lt_config* cfg, lt_handle** out) {
     cudaMemset(h->draw_flags, 0, 2 * S * sizeof(int));
     cudaMemset(h->retry_count, 0, sizeof(int));
     cudaMemset(h->att, 0, 2 * S * sizeof(LtAttemptOut));
+    {
+        LtDevState z;
+        init_state(h, &z.s);
+        if (cudaMemcpy(h->init, &z, sizeof(z), cudaMemcpyHostToDevice) != cudaSuccess) {
+            lt_set_error("cannot write the initial state"); lt_destroy(h); return -2;
+        }
+    }
     *out = h;
     rc = lt_reset(h, nullptr, 0);
     if (rc) { lt_destroy(h); *out = nullptr; return rc; }
@@ -1698,6 +1705,197 @@ extern "C" int lt_set_state(lt_handle* h, int32_t id, const lt_state* hs, const 
         if (rc) return rc;
     }
     return 0;
+}
+
+// ---------------------------------------------------------------------------
+// stream starts (lt_reset_async) and state records (lt_export_states / lt_import_states)
+// ---------------------------------------------------------------------------
+
+// lt_reset_async: the initial state h->init copied into the slots of a chunk of ids, one word per thread and step.
+__global__ void __launch_bounds__(256) k_reset_states(const __grid_constant__ LtIdsChunk c, const LtDevState* __restrict__ init,
+                                                      LtDevState* __restrict__ state) {
+    constexpr int W = sizeof(LtDevState) / sizeof(int);
+    static_assert(sizeof(LtDevState) % sizeof(int) == 0, "LtDevState is copied as words");
+    const int* src = reinterpret_cast<const int*>(init);
+    for (int i = threadIdx.x; i < c.count * W; i += blockDim.x)
+        reinterpret_cast<int*>(state + c.ids[i / W])[i % W] = __ldg(&src[i % W]);
+}
+
+// Byte offsets of the parts of one state record (include/lane_tracker_b200.h), from the bird's-eye height.
+struct LtRecordLayout {
+    int state, avg, rows, bbox, bytes;
+};
+static constexpr int LT_RECORD_HEADER_BYTES = 64;
+__host__ __device__ static inline int lt_align16(int v) { return (v + 15) & ~15; }
+__host__ __device__ static inline LtRecordLayout lt_record_layout(int H) {
+    LtRecordLayout r;
+    r.state = LT_RECORD_HEADER_BYTES;
+    r.avg = r.state + lt_align16((int)sizeof(LtDevState));
+    r.rows = r.avg + 2 * H * (int)sizeof(int);
+    r.bbox = lt_align16(r.rows + H * (int)sizeof(int2));
+    r.bytes = r.bbox + (int)sizeof(int4);
+    return r;
+}
+
+struct LtRecordHeader {          // the 64-byte header, int32 words
+    uint32_t magic;
+    int abi, state_bytes, bv_w, bv_h, n_average, n_fail, n_reset;
+    int zero[8];
+};
+static_assert(sizeof(LtRecordHeader) == LT_RECORD_HEADER_BYTES, "record header is 64 bytes");
+
+// What the record kernels read and write of a handle: its header and its per-stream arrays.
+struct LtRecordDev {
+    LtRecordHeader hdr;
+    LtDevState* state; int* avg_x; int2* rows; int4* bbox;
+};
+
+// The ids of a record launch.  Kept at 512 so that they and LtRecordDev fit the classic 4 KB of kernel arguments.
+#define LT_RECORD_CHUNK 512
+struct LtRecordIds {
+    int offset, count;
+    int ids[LT_RECORD_CHUNK];
+};
+
+__device__ static inline void zero_bytes(uint8_t* p, int a, int b) {
+    for (int i = a + (int)threadIdx.x; i < b; i += blockDim.x) p[i] = 0;
+}
+
+// One CTA per record: record offset + blockIdx.x of dst <- stream ids[blockIdx.x] (16-byte aligned records).
+__global__ void __launch_bounds__(256) k_export_states(const __grid_constant__ LtRecordIds c, const __grid_constant__ LtRecordDev r,
+                                                       uint8_t* __restrict__ dst) {
+    const int H = r.hdr.bv_h, sid = c.ids[blockIdx.x], tid = threadIdx.x;
+    const LtRecordLayout L = lt_record_layout(H);
+    uint8_t* rec = dst + (size_t)(c.offset + blockIdx.x) * L.bytes;
+    if (tid < LT_RECORD_HEADER_BYTES / 4)
+        reinterpret_cast<int*>(rec)[tid] = reinterpret_cast<const int*>(&r.hdr)[tid];
+    const int* st = reinterpret_cast<const int*>(r.state + sid);
+    for (int i = tid; i < (int)(sizeof(LtDevState) / 4); i += blockDim.x) reinterpret_cast<int*>(rec + L.state)[i] = st[i];
+    zero_bytes(rec, L.state + (int)sizeof(LtDevState), L.avg);
+    const int* ax = r.avg_x + (size_t)sid * 2 * H;
+    for (int i = tid; i < 2 * H; i += blockDim.x) reinterpret_cast<int*>(rec + L.avg)[i] = ax[i];
+    const int2* rows = r.rows + (size_t)sid * H;
+    for (int i = tid; i < H; i += blockDim.x) reinterpret_cast<int2*>(rec + L.rows)[i] = rows[i];
+    zero_bytes(rec, L.rows + H * (int)sizeof(int2), L.bbox);
+    if (tid == 0) *reinterpret_cast<int4*>(rec + L.bbox) = r.bbox[sid];
+}
+
+// One CTA per record: checks record offset + blockIdx.x of src, and applies it to slot ids[blockIdx.x] only if it
+// passes (status: LT_RECORD_OK / LT_RECORD_BAD_HEADER / LT_RECORD_BAD_STATE).
+__global__ void __launch_bounds__(256) k_import_states(const __grid_constant__ LtRecordIds c, const __grid_constant__ LtRecordDev r,
+                                                       const uint8_t* __restrict__ src, int* __restrict__ status) {
+    const int H = r.hdr.bv_h, W = r.hdr.bv_w, sid = c.ids[blockIdx.x], tid = threadIdx.x;
+    const LtRecordLayout L = lt_record_layout(H);
+    const int i = c.offset + blockIdx.x;
+    const uint8_t* rec = src + (size_t)i * L.bytes;
+    __shared__ int code;
+    if (tid == 0) {
+        const LtRecordHeader& g = *reinterpret_cast<const LtRecordHeader*>(rec);
+        int k = LT_RECORD_OK;
+        if (g.magic != r.hdr.magic || g.abi != r.hdr.abi || g.state_bytes != r.hdr.state_bytes || g.bv_w != W ||
+            g.bv_h != H || g.n_average != r.hdr.n_average || g.n_fail != r.hdr.n_fail || g.n_reset != r.hdr.n_reset) {
+            k = LT_RECORD_BAD_HEADER;
+        } else {
+            const lt_state& s = reinterpret_cast<const LtDevState*>(rec + L.state)->s;
+            const int nav = r.hdr.n_average;
+            const int4 b = *reinterpret_cast<const int4*>(rec + L.bbox);
+            if (s.ring_len < 0 || s.ring_len > nav || s.radii_len < 0 || s.radii_len > nav || s.n_left_avg < 0 ||
+                s.n_left_avg > H || s.n_right_avg < 0 || s.n_right_avg > H ||
+                (b.x <= b.y && (b.x < 0 || b.y >= W || b.z < 0 || b.z > b.w || b.w >= H)))
+                k = LT_RECORD_BAD_STATE;
+        }
+        code = k;
+    }
+    __syncthreads();
+    int bad_row = 0;
+    if (code == LT_RECORD_OK) {
+        const int2* rows = reinterpret_cast<const int2*>(rec + L.rows);
+        for (int y = tid; y < H; y += blockDim.x) {
+            const int2 q = rows[y];
+            bad_row |= q.x <= q.y && (q.x < 0 || q.y >= W);
+        }
+    }
+    bad_row = __syncthreads_or(bad_row);
+    const int k = code != LT_RECORD_OK ? code : (bad_row ? LT_RECORD_BAD_STATE : LT_RECORD_OK);
+    if (tid == 0 && status) status[i] = k;
+    if (k != LT_RECORD_OK) return;
+    const int* st = reinterpret_cast<const int*>(rec + L.state);
+    for (int j = tid; j < (int)(sizeof(LtDevState) / 4); j += blockDim.x) reinterpret_cast<int*>(r.state + sid)[j] = st[j];
+    const int* ax = reinterpret_cast<const int*>(rec + L.avg);
+    for (int j = tid; j < 2 * H; j += blockDim.x) r.avg_x[(size_t)sid * 2 * H + j] = ax[j];
+    const int2* rows = reinterpret_cast<const int2*>(rec + L.rows);
+    for (int j = tid; j < H; j += blockDim.x) r.rows[(size_t)sid * H + j] = rows[j];
+    if (tid == 0) r.bbox[sid] = *reinterpret_cast<const int4*>(rec + L.bbox);
+}
+
+extern "C" int lt_reset_async(lt_handle* h, const int32_t* h_ids, int32_t n, void* stream) {
+    int rc;
+    if (!h) { lt_set_error("null handle"); return -1; }
+    std::vector<int32_t> all;
+    if (!h_ids) {
+        all.resize(h->S);
+        for (int i = 0; i < h->S; ++i) all[i] = i;
+        h_ids = all.data();
+        n = h->S;
+    } else if ((rc = check_ids(h, h_ids, n))) {
+        return rc;
+    }
+    const cudaStream_t st = (cudaStream_t)stream;
+    LtIdsChunk c;
+    for (int off = 0; off < n; off += LT_IDS_CHUNK) {
+        c.offset = off;
+        c.count = n - off < LT_IDS_CHUNK ? n - off : LT_IDS_CHUNK;
+        memcpy(c.ids, h_ids + off, (size_t)c.count * sizeof(int32_t));
+        k_reset_states<<<1, 256, 0, st>>>(c, h->init, h->state);
+        LT_LAUNCH_CHECK();
+    }
+    return 0;
+}
+
+extern "C" int64_t lt_state_record_bytes(lt_handle* h) {
+    if (!h) { lt_set_error("null handle"); return -1; }
+    return lt_record_layout(h->d.bv_h).bytes;
+}
+
+static LtRecordDev record_dev(const lt_handle* h) {
+    LtRecordDev r;
+    memset(&r, 0, sizeof(r));
+    r.hdr.magic = LT_RECORD_MAGIC; r.hdr.abi = LT_ABI_VERSION; r.hdr.state_bytes = (int)sizeof(lt_state);
+    r.hdr.bv_w = h->d.bv_w; r.hdr.bv_h = h->d.bv_h;
+    r.hdr.n_average = h->cfg.n_average; r.hdr.n_fail = h->cfg.n_fail; r.hdr.n_reset = h->cfg.n_reset;
+    r.state = h->state; r.avg_x = h->avg_x; r.rows = h->lane_rows; r.bbox = h->lane_bbox;
+    return r;
+}
+
+// export (d_status unused) or import of the records of streams h_ids[0..n), all checks before anything is enqueued
+static int move_states(lt_handle* h, bool to_handle, const int32_t* h_ids, int n, const void* d_rec, int32_t* d_status,
+                       void* stream) {
+    int rc;
+    if ((rc = check_ids(h, h_ids, n))) return rc;
+    if (!d_rec) { lt_set_error("null record buffer"); return -1; }
+    if ((uintptr_t)d_rec & 15) { lt_set_error("the record buffer must be 16-byte aligned (got address %p)", d_rec); return -1; }
+    if ((uintptr_t)d_status & 3) { lt_set_error("d_status must be 4-byte aligned (got address %p)", (void*)d_status); return -1; }
+    const cudaStream_t st = (cudaStream_t)stream;
+    const LtRecordDev r = record_dev(h);
+    LtRecordIds c;
+    for (int off = 0; off < n; off += LT_RECORD_CHUNK) {
+        c.offset = off;
+        c.count = n - off < LT_RECORD_CHUNK ? n - off : LT_RECORD_CHUNK;
+        memcpy(c.ids, h_ids + off, (size_t)c.count * sizeof(int32_t));
+        if (to_handle) k_import_states<<<c.count, 256, 0, st>>>(c, r, (const uint8_t*)d_rec, d_status);
+        else k_export_states<<<c.count, 256, 0, st>>>(c, r, (uint8_t*)d_rec);
+        LT_LAUNCH_CHECK();
+    }
+    return 0;
+}
+
+extern "C" int lt_export_states(lt_handle* h, const int32_t* h_ids, int32_t n, void* d_dst, void* stream) {
+    return move_states(h, false, h_ids, n, d_dst, nullptr, stream);
+}
+
+extern "C" int lt_import_states(lt_handle* h, const int32_t* h_ids, int32_t n, const void* d_src, int32_t* d_status,
+                                void* stream) {
+    return move_states(h, true, h_ids, n, d_src, d_status, stream);
 }
 
 extern "C" int64_t lt_debug_read(lt_handle* h, int32_t what, int32_t id, void* dst, int64_t cap) {

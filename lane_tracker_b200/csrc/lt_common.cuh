@@ -150,6 +150,7 @@ struct lt_handle {
     int4* lane_bbox;             // [S] bounding box of the polygon rows: (min lo, max hi, first row, last row); empty: (W, -1, H, -1)
     int* avg_x;                  // [S][2][bv_h]   averaged polylines (state)
     LtDevState* state;           // [S]
+    LtDevState* init;            // [1] the initial state (init_state), written at lt_create: what lt_reset_async copies
     LtAttemptOut* att;           // [S]
     int* retry_list; int* retry_count;      // streams that need attempt 2
     int* draw_flags;             // [S]

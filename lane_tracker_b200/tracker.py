@@ -171,8 +171,9 @@ class BatchedLaneTracker:
     def set_camera(self, k, cam_matrix, dist_coeffs, warp_matrices, mpp_conversion):
         """Set camera k (1 <= k < LT_MAX_CAMERAS) for the ``cameras=`` argument of the process calls: a calibration in
         the constructor's forms (camera 0 is the constructor's and cannot change).  Image and bird's-eye sizes stay
-        the handle's.  Synchronises the device.  A stream whose camera was re-mounted keeps its tracking state: reset
-        it with ``reset(ids)``.  A ``GraphedProcess`` captured with cameras before this call can no longer replay."""
+        the handle's.  Synchronises the device.  A stream whose camera was re-mounted keeps its tracking state: flag
+        its first frame from the new mounting in ``starts=`` to start it afresh.  A ``GraphedProcess`` captured with
+        cameras before this call can no longer replay."""
         cal = _calibration(cam_matrix, dist_coeffs, warp_matrices, mpp_conversion)
         with torch.cuda.device(self.device):
             check(self.lib.lt_set_camera(self._h, int(k), C.byref(cal)))
@@ -193,11 +194,73 @@ class BatchedLaneTracker:
             pass
 
     def reset(self, ids=None):
+        """Re-zero the state of the streams ``ids`` (None: all) synchronously, outside every CUDA stream: only with no
+        work of this tracker in flight.  ``reset_async`` and ``starts=`` are ordered with the batches."""
         if ids is None:
             check(self.lib.lt_reset(self._h, None, 0))
         else:
             arr = (C.c_int32 * len(ids))(*[int(i) for i in ids])
             check(self.lib.lt_reset(self._h, arr, len(ids)))
+
+    def reset_async(self, ids=None):
+        """Enqueue on the current CUDA stream what ``reset(ids)`` writes (None: every stream): the next frame of each
+        stream is processed as by a freshly reset stream.  Capturable in a CUDA graph."""
+        arr = None if ids is None else self._check_ids(ids, len(ids))
+        with torch.cuda.device(self.device):
+            check(self.lib.lt_reset_async(self._h, arr, 0 if ids is None else len(ids), _stream_ptr(self.device)))
+
+    @property
+    def record_bytes(self):
+        """Size of one stream's state record (``export_states`` / ``import_states``)."""
+        return int(check(self.lib.lt_state_record_bytes(self._h)))
+
+    def export_states(self, ids, out=None):
+        """The state records of streams ``ids`` (distinct) -> CUDA uint8 tensor [n, record_bytes] (``out`` if given),
+        gathered on the current CUDA stream: tracking state, averaged polylines and cached lane polygon, everything a
+        later frame of the stream reads (layout: include/lane_tracker_b200.h).  Capturable in a CUDA graph."""
+        h_ids = self._check_ids(ids, len(ids))
+        n, rb = len(ids), self.record_bytes
+        if out is None:
+            out = torch.empty((n, rb), dtype=torch.uint8, device=self.device)
+        self._check_records(out, n, "out")
+        with torch.cuda.device(self.device):
+            check(self.lib.lt_export_states(self._h, h_ids, n, _ptr(out), _stream_ptr(self.device)))
+        return out
+
+    def import_states(self, ids, records, check=True):
+        """Write the state records ``records`` [n, record_bytes] (from ``export_states`` of this or another tracker of
+        the same bird's-eye size, n_average, n_fail and n_reset, moved to this tracker's device) into slots ``ids``, on
+        the current CUDA stream.  Each record is checked on the device first; a refused one is not applied and its
+        slot keeps its state.  -> int32 CUDA tensor [n] of status codes (LT_RECORD_OK, LT_RECORD_BAD_HEADER,
+        LT_RECORD_BAD_STATE).  check=True synchronises the current stream and raises ValueError naming the first
+        refused position."""
+        do_check = check
+        h_ids = self._check_ids(ids, len(ids))
+        n = len(ids)
+        self._check_records(records, n, "records")
+        status = torch.empty(n, dtype=torch.int32, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.lt_import_states(self._h, h_ids, n, _ptr(records), _ptr(status),
+                                                 _stream_ptr(self.device)))
+        if do_check:
+            got = status.cpu().numpy()        # synchronises the current stream
+            bad = np.flatnonzero(got != _lib.LT_RECORD_OK)
+            if bad.size:
+                i = int(bad[0])
+                why = {_lib.LT_RECORD_BAD_HEADER: "its header does not match this tracker (magic, ABI version, state "
+                                                  "size, bird's-eye size, n_average, n_fail or n_reset)",
+                       _lib.LT_RECORD_BAD_STATE: "its state is inconsistent (ring_len, radii_len, polyline lengths, "
+                                                 "polygon rows or box out of range)"}.get(int(got[i]), "code %d" % got[i])
+                raise ValueError("state record at position %d (stream %d) refused: %s" % (i, int(ids[i]), why))
+        return status
+
+    def _check_records(self, t, n, name):
+        rb = self.record_bytes
+        if not (isinstance(t, torch.Tensor) and t.dtype == torch.uint8 and t.device == self.device and
+                t.is_contiguous() and tuple(t.shape) == (n, rb)):
+            raise ValueError("%s must be a contiguous uint8 tensor [%d, %d] on %s" % (name, n, rb, self.device))
+        if t.data_ptr() % 16:
+            raise ValueError("%s must start at a 16-byte aligned address" % name)
 
     def set_validity(self, **kw):
         """Override the acceptance windows of check_validity (lane_tracker.py:588-593, 617); no arguments restores
@@ -425,6 +488,38 @@ class BatchedLaneTracker:
             raise ValueError("sequence=True takes neither profiles nor cameras")
 
     @staticmethod
+    def _check_starts(starts, ids, n, sequence):
+        """``starts`` of a batch of n frames -> the stream ids to start (None: no starts).  One bool per batch position:
+        position i starts a new video on its stream (ids[i], or i without ids).  In a sequence batch a start may only
+        be at a stream's first position in the batch."""
+        if starts is None:
+            return None
+        if isinstance(starts, torch.Tensor):
+            if starts.is_cuda:
+                raise ValueError("starts must be host data (a sequence, a NumPy array or a CPU tensor), not a CUDA tensor")
+            starts = starts.numpy()
+        if isinstance(starts, np.ndarray) and starts.ndim != 1:
+            raise ValueError("starts must be a 1-D sequence of bools")
+        a = list(starts)
+        if len(a) != n:
+            raise ValueError("got %d starts for %d frames" % (len(a), n))
+        for i, v in enumerate(a):
+            if not isinstance(v, (bool, np.bool_)):
+                raise ValueError("starts[%d] is %r: starts must be bools" % (i, v))
+        sids = [int(ids[i]) if ids is not None else i for i in range(n)]
+        if sequence:
+            first = {}
+            for i, s in enumerate(sids):
+                first.setdefault(s, i)
+            for i, v in enumerate(a):
+                if v and first[sids[i]] != i:
+                    raise ValueError("starts[%d]: stream %d starts a new video after its frame at position %d of this "
+                                     "sequence batch; a start must be a stream's first position: split the batch there"
+                                     % (i, sids[i], first[sids[i]]))
+        flagged = [s for s, v in zip(sids, a) if v]
+        return flagged or None
+
+    @staticmethod
     def _no_params_with_profiles(profiles, params, kw):
         if profiles is not None and (params is not None or kw):
             raise ValueError("profiles= selects the parameters of every frame: pass it without params or keyword options")
@@ -441,7 +536,7 @@ class BatchedLaneTracker:
             raise ValueError("out must start at a 4-byte aligned address (the kernels access frames as 32-bit words)")
 
     def process_async(self, frames, out=None, params=None, results_dev=None, ids=None, profiles=None, cameras=None,
-                      sequence=False, **kw):
+                      sequence=False, starts=None, **kw):
         """Enqueue one frame per stream on the current CUDA stream; returns the number of frames.
 
         frames: uint8 CUDA tensor [n, H, W, 3] (RGB) or [n, H * 3 / 2, W] (NV12: the luma plane, then interleaved
@@ -462,8 +557,16 @@ class BatchedLaneTracker:
         One video, 64 frames per call::
 
             for chunk, out in chunks:          # [<= n_streams, H, W, 3] consecutive frames of stream 0
-                tracker.process_async(chunk, out, ids=[0] * len(chunk), sequence=True)"""
-        return self._process_call(frames, out, None, params, results_dev, ids, kw, profiles, cameras, sequence)
+                tracker.process_async(chunk, out, ids=[0] * len(chunk), sequence=True)
+
+        starts: None, or one bool per frame: frame i is the first frame of a new video on its stream (ids[i], or i
+        without ids) and is processed as by a freshly reset stream (``reset_async`` of the flagged streams, enqueued
+        right before the back half).  In a sequence batch only a stream's first position may start.  Refused before
+        anything is enqueued: a wrong length or an entry that is not a bool.  The reset is enqueued after every check
+        made here and before the library call; a batch the library itself then refuses (LaneTrackerError: an unset
+        profile, parameters out of range, a back half whose profiles or cameras differ from its front half's) has
+        already reset its flagged streams, which start their new videos with the next frames they are given."""
+        return self._process_call(frames, out, None, params, results_dev, ids, kw, profiles, cameras, sequence, starts)
 
     def process_front_async(self, frames, buffer_set, params=None, profiles=None, cameras=None, **kw):
         """First half of ``process_async`` (undistort, warp, first-attempt filter) into intermediate buffer set
@@ -487,16 +590,17 @@ class BatchedLaneTracker:
         return n
 
     def process_back_async(self, frames, out, buffer_set, params=None, results_dev=None, ids=None, profiles=None,
-                           cameras=None, sequence=False, **kw):
+                           cameras=None, sequence=False, starts=None, **kw):
         """Second half of ``process_async`` (searches, second attempt, state machine, overlay) from intermediate
         buffer set 0 or 1, on the current CUDA stream.  Advances the per-stream state of the streams in ``ids``
         (None: streams 0..n-1), as ``process_async``.  RGB or NV12 frames, as given to the front half.  ``profiles``,
-        ``cameras``: those the front half of this buffer set was given.  ``sequence``: as ``process_async`` (the
-        front half takes no ids)."""
-        return self._process_call(frames, out, buffer_set, params, results_dev, ids, kw, profiles, cameras, sequence)
+        ``cameras``: those the front half of this buffer set was given.  ``sequence``, ``starts``: as
+        ``process_async`` (the front half takes no ids; a start only touches the state the back half reads)."""
+        return self._process_call(frames, out, buffer_set, params, results_dev, ids, kw, profiles, cameras, sequence,
+                                  starts)
 
     def _process_call(self, frames, out, buffer_set, params, results_dev, ids, kw, profiles=None, cameras=None,
-                      sequence=False):
+                      sequence=False, starts=None):
         """Checks and C call of ``process_async`` (buffer_set None: both halves) or ``process_back_async``; -> n."""
         n = self._input(frames)
         self._check_out(out, frames)
@@ -505,9 +609,13 @@ class BatchedLaneTracker:
         self._no_params_with_profiles(profiles, params, kw)
         h_prof = self._check_profiles(profiles, n)
         h_cam = self._check_cameras(cameras, n)
+        started = self._check_starts(starts, ids, n, sequence)
         res = self._results_dev if results_dev is None else results_dev
         if res.numel() < n * RESULT_DTYPE.itemsize or not res.is_cuda:
             raise ValueError("results buffer too small")
+        if started is not None:
+            # the new videos begin right before the back half that reads their first frames, on its stream
+            self.reset_async(started)
         if h_cam is not None:
             p = None if h_prof is not None else (params if params is not None else make_params(**kw))
             pp = C.byref(p) if p is not None else None
@@ -550,13 +658,15 @@ class BatchedLaneTracker:
         torch.cuda.current_stream(self.device).synchronize()
         return self._results_host[:nbytes].numpy().view(RESULT_DTYPE).copy()
 
-    def process(self, frames, out=None, params=None, ids=None, profiles=None, cameras=None, sequence=False, **kw):
+    def process(self, frames, out=None, params=None, ids=None, profiles=None, cameras=None, sequence=False, starts=None,
+                **kw):
         """``process_async`` followed by ``fetch_results``: the n result records, in batch order.  With ``ids``, frame
         i advances stream ids[i] and the other streams keep their state; with ``profiles``, frame i uses parameter
         profile profiles[i] (``set_profile``); with ``cameras``, frame i comes from camera cameras[i] (``set_camera``);
-        with ``sequence=True``, ids may repeat and a stream's frames are its consecutive frames, in batch order."""
+        with ``sequence=True``, ids may repeat and a stream's frames are its consecutive frames, in batch order; with
+        ``starts``, the flagged frames begin new videos on their streams."""
         n = self.process_async(frames, out, params, ids=ids, profiles=profiles, cameras=cameras, sequence=sequence,
-                               **kw)
+                               starts=starts, **kw)
         return self.fetch_results(n)
 
     # -- stage methods (device tensors) ---------------------------------------
@@ -853,16 +963,15 @@ class GraphedProcess:
         tracker._check_cameras(self.cameras, n)
         self.camera_epoch = tracker.camera_epoch
         # first-use initialisation (module load, shared-memory attributes) cannot happen inside a capture: run the
-        # chain once for real on a side stream, with the tracking state saved and restored around it
-        saved = [tracker.get_state(s) for s in range(n)]
+        # chain once for real on a side stream, with the state records of its streams exported before and imported
+        # after it on that stream
         side = torch.cuda.Stream(dev)
         side.wait_stream(torch.cuda.current_stream(dev))
         with torch.cuda.stream(side):
+            saved = tracker.export_states(range(n))
             tracker.process_async(self.frames, self.out, params=self.params, results_dev=self.results_dev,
                                   profiles=self.profiles, cameras=self.cameras)
-        side.synchronize()
-        for s, (st, lx, rx) in enumerate(saved):
-            tracker.set_state(s, st, lx, rx)
+            tracker.import_states(range(n), saved, check=False)
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph, stream=side):
             tracker.process_async(self.frames, self.out, params=self.params, results_dev=self.results_dev,
@@ -901,6 +1010,11 @@ class DevicePipeline:
 
         for chunk, out in chunks:              # consecutive frames of one video, up to n_streams per chunk
             pipe.submit(chunk, out, ids=[0] * len(chunk), sequence=True)
+
+    ``submit(..., starts=...)`` flags the frames that begin a new video on their stream (see
+    ``BatchedLaneTracker.process_async``): the start is enqueued on the back stream, after every back half submitted
+    before and before this batch's, so the pipeline need not be drained.  ``export_states`` / ``import_states`` move
+    state records on the back stream in the same order.
     """
 
     def __init__(self, tracker, params=None):
@@ -915,13 +1029,14 @@ class DevicePipeline:
         self.results_dev = [torch.zeros(tracker.n_streams * RESULT_DTYPE.itemsize, dtype=torch.uint8, device=dev)
                             for _ in range(2)]
 
-    def submit(self, frames, out=None, ids=None, profiles=None, cameras=None, sequence=False):
+    def submit(self, frames, out=None, ids=None, profiles=None, cameras=None, sequence=False, starts=None):
         dev = self.t.device
         n = self.t._frame_format(frames)[0]
         self.t._check_sequence(sequence, ids, profiles, cameras)
         self.t._check_ids(ids, n, repeats=sequence)    # refuse bad frames / ids / profiles / cameras before anything is enqueued
         self.t._check_profiles(profiles, n)
         self.t._check_cameras(cameras, n)
+        self.t._check_starts(starts, ids, n, sequence)
         params = self.params if profiles is None else None
         k, bs = self._k, self._k & 1
         ready = torch.cuda.Event()
@@ -937,13 +1052,25 @@ class DevicePipeline:
             self.s_back.wait_event(front_done)
             self.s_back.wait_event(ready)
             self.t.process_back_async(frames, out, bs, params=params, results_dev=self.results_dev[bs], ids=ids,
-                                      profiles=profiles, cameras=cameras, sequence=sequence)
+                                      profiles=profiles, cameras=cameras, sequence=sequence, starts=starts)
             done = torch.cuda.Event()
             done.record(self.s_back)
         self._back_done[bs] = done
         self._last = done
         self._k = k + 1
         return done
+
+    def export_states(self, ids):
+        """State records of streams ``ids`` as they stand after every batch submitted so far (and before any submitted
+        later), gathered on the back stream -> (uint8 CUDA tensor [n, record_bytes], torch.cuda.Event after which it
+        is complete)."""
+        return _on_stream(self.t, self.s_back, lambda: self.t.export_states(ids))
+
+    def import_states(self, ids, records):
+        """Write state records into slots ``ids`` on the back stream, after every batch submitted so far and before any
+        submitted later.  ``records`` are read after the work enqueued so far on the current stream.  -> (int32 CUDA
+        status tensor [n], see ``BatchedLaneTracker.import_states``; torch.cuda.Event after which it is complete)."""
+        return _on_stream(self.t, self.s_back, lambda: self.t.import_states(ids, records, check=False), records)
 
     def last_results_dev(self):
         """Device buffer holding the lt_result records of the most recently submitted batch."""
@@ -957,6 +1084,22 @@ class DevicePipeline:
         """Results of the most recently submitted batch as a structured array (synchronises)."""
         self.join()
         return self.t.fetch_results(n, self.last_results_dev())
+
+
+def _on_stream(tracker, stream, fn, reads=None):
+    """Run ``fn`` (a state-record call of ``tracker``) on a pipeline's back stream, after the work enqueued so far on
+    the current stream (``reads``, a tensor it reads, is kept alive for that stream) -> (fn's tensor, its event)."""
+    dev = tracker.device
+    ready = torch.cuda.Event()
+    ready.record(torch.cuda.current_stream(dev))
+    with torch.cuda.stream(stream):
+        stream.wait_event(ready)
+        if reads is not None:
+            reads.record_stream(stream)
+        t = fn()
+        done = torch.cuda.Event()
+        done.record(stream)
+    return t, done
 
 
 def _rows_minus(rows, covered):
@@ -986,7 +1129,9 @@ class HostPipeline:
     parameter profile profiles[i] (``BatchedLaneTracker.set_profile``) instead of the pipeline's ``params``, and
     ``submit(batch, cameras=...)`` says that frame i comes from camera cameras[i] (``BatchedLaneTracker.set_camera``).
     ``submit(batch, ids=..., sequence=True)`` lets ids repeat: the frames of one stream are its consecutive frames, in
-    batch order (``pipe.submit(chunk, ids=[0] * len(chunk), sequence=True)`` for one video).
+    batch order (``pipe.submit(chunk, ids=[0] * len(chunk), sequence=True)`` for one video).  ``submit(batch,
+    starts=...)`` flags the frames that begin a new video on their stream, and ``export_states`` / ``import_states``
+    move state records, all in submission order on the stream of the back halves (see ``DevicePipeline``).
     """
 
     def __init__(self, tracker, depth=3, overlay=True, params=None, inplace=False, frame_format="rgb"):
@@ -1049,7 +1194,7 @@ class HostPipeline:
         """Frame rows the lane overlay can change, over camera 0 and every camera set: what inplace mode copies back."""
         return self.t.rows_any_camera()[1]
 
-    def submit(self, host_frames, ids=None, profiles=None, cameras=None, sequence=False):
+    def submit(self, host_frames, ids=None, profiles=None, cameras=None, sequence=False, starts=None):
         if self.inflight == self.depth:
             raise RuntimeError("pipeline full: collect a finished batch first")
         if not (host_frames.dtype == torch.uint8 and host_frames.is_pinned() and host_frames.is_contiguous()):
@@ -1064,6 +1209,7 @@ class HostPipeline:
         self.t._check_ids(ids, n, repeats=sequence)      # refuse bad ids / profiles / cameras before anything is enqueued
         self.t._check_profiles(profiles, n)
         self.t._check_cameras(cameras, n)
+        self.t._check_starts(starts, ids, n, sequence)
         params = self.params if profiles is None else None
         rows_in, rows_out = self.rows_in, self.rows_out
         sl["n"] = n
@@ -1094,7 +1240,7 @@ class HostPipeline:
             self.s_run.wait_event(sl["e_out"])           # the previous D2H out of this output buffer is done
             d_out = sl["d_in"][:n] if self.inplace else (sl["d_out"][:n] if self.overlay else None)
             self.t.process_back_async(sl["d_in"][:n], d_out, bs, params=params, results_dev=sl["d_res"], ids=ids,
-                                      profiles=profiles, cameras=cameras, sequence=sequence)
+                                      profiles=profiles, cameras=cameras, sequence=sequence, starts=starts)
             sl["e_run"].record(self.s_run)
         self._set_free[bs] = sl["e_run"]
         with torch.cuda.stream(self.s_out):
@@ -1112,6 +1258,14 @@ class HostPipeline:
         sl["busy"] = True
         self.head = (self.head + 1) % self.depth
         self.inflight += 1
+
+    def export_states(self, ids):
+        """As ``DevicePipeline.export_states``, on the stream of the back halves."""
+        return _on_stream(self.t, self.s_run, lambda: self.t.export_states(ids))
+
+    def import_states(self, ids, records):
+        """As ``DevicePipeline.import_states``, on the stream of the back halves."""
+        return _on_stream(self.t, self.s_run, lambda: self.t.import_states(ids, records, check=False), records)
 
     def _collect(self, block):
         sl = self.slots[self.tail]
