@@ -37,7 +37,7 @@ typedef struct lt_handle lt_handle;
  * calibration read by utils.load_camera_calib / load_warp_params (utils.py:13-55). */
 typedef struct lt_config {
     int32_t img_w, img_h;         /* img_size    (width, height) */
-    int32_t bv_w, bv_h;           /* warped_size (width, height); bv_w must be even */
+    int32_t bv_w, bv_h;           /* warped_size (width, height); bv_w must be even (see lt_create) */
     double  cam_matrix[9];        /* row-major 3x3 */
     double  dist_coeffs[5];       /* k1 k2 p1 p2 k3 */
     double  M[9];                 /* warp_matrices[0] */
@@ -118,7 +118,11 @@ typedef struct lt_validity {
 /* ---- lifetime ------------------------------------------------------------ */
 
 /* LaneTracker.__init__ (lane_tracker.py:101-176) for `max_streams` streams.
- * Builds the fixed-point remap tables on the device.  Synchronous. */
+ * Builds the fixed-point remap tables on the device.  Synchronous.
+ * Accepted geometry: img_w in [64, 32767] and a multiple of 4, img_h in [16, 32767], bv_w even and in [66, 32767],
+ * bv_h in [16, 65535].  A bv_w at which a threshold kernel could not launch with some parameter set the process calls
+ * accept (shared memory beyond the device's per-block opt-in limit) is refused as well: on a B200 (227 KB) the widest
+ * accepted bird's-eye view is 3614 columns. */
 int lt_create(const lt_config* cfg, lt_handle** out);
 int lt_destroy(lt_handle* h);
 /* Re-zero the state of the listed streams (ids == NULL: all): one cudaMemcpy per id from host memory on the legacy

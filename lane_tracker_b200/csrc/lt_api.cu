@@ -66,7 +66,9 @@ static LtAttemptParams second_attempt() {
     return attempt_from(p);
 }
 
-static int check_params(const lt_handle* h, const LtAttemptParams& a) {
+// The filter options alone: lt_filter_lane_points takes no search options, so a view narrower or shorter than the
+// default search windows must not refuse it.
+static int check_filter_params(const LtAttemptParams& a) {
     if (a.filter_type != 0 && a.filter_type != 1) {
         lt_set_error("Unexpected filter mode. Expected modes are 'bilateral' or 'neighborhood'.");
         return -1;
@@ -79,6 +81,12 @@ static int check_params(const lt_handle* h, const LtAttemptParams& a) {
         lt_set_error("'neighborhood' block sizes must be odd and >= 3 (cv2.adaptiveThreshold)");
         return -1;
     }
+    return 0;
+}
+
+static int check_params(const lt_handle* h, const LtAttemptParams& a) {
+    int rc;
+    if ((rc = check_filter_params(a))) return rc;
     if (a.window_width < 1 || a.window_width > 64 || a.window_height < 1 || a.window_height > h->d.bv_h) {
         lt_set_error("window_width must lie in [1, 64] and window_height in [1, warped height]");
         return -1;
@@ -300,10 +308,12 @@ static int build_camera(lt_handle* h, LtCamera& c) {
 
 extern "C" int lt_create(const lt_config* cfg, lt_handle** out) {
     if (!cfg || !out) { lt_set_error("null argument"); return -1; }
-    if (cfg->img_w < 64 || cfg->img_h < 16 || cfg->bv_w < 64 || cfg->bv_h < 16 || (cfg->img_w & 3) || cfg->bv_h > 65535 ||
-        cfg->bv_w > 32767 || cfg->img_w > 32767 || cfg->img_h > 32767) {
-        lt_set_error("unsupported geometry: img %dx%d (width must be a multiple of 4), warped %dx%d", cfg->img_w,
-                     cfg->img_h, cfg->bv_w, cfg->bv_h);
+    // bv_w >= 66: pair planes at least 2 * LT_HALO_X wide, so that every packed column feeds at most one of the two
+    // seam halos the erosion epilogue of the morphology writes
+    if (cfg->img_w < 64 || cfg->img_h < 16 || cfg->bv_w < 66 || cfg->bv_h < 16 || (cfg->img_w & 3) || (cfg->bv_w & 1) ||
+        cfg->bv_h > 65535 || cfg->bv_w > 32767 || cfg->img_w > 32767 || cfg->img_h > 32767) {
+        lt_set_error("unsupported geometry: img %dx%d (width must be a multiple of 4), warped %dx%d (width must be even and "
+                     "at least 66)", cfg->img_w, cfg->img_h, cfg->bv_w, cfg->bv_h);
         return -1;
     }
     if (cfg->max_streams < 1 || cfg->n_average < 1 || cfg->n_average > LT_MAX_AVERAGE) {
@@ -311,6 +321,18 @@ extern "C" int lt_create(const lt_config* cfg, lt_handle** out) {
         return -1;
     }
     LT_CUDA(cudaSetDevice(cfg->device));
+    {
+        // a view so wide that a threshold kernel could not launch would fail in the middle of a batch: refuse it here
+        int optin = 0;
+        LT_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, cfg->device));
+        if (lt_filter_smem_bytes(cfg->bv_w) > (size_t)optin) {
+            int widest = 66;
+            while (lt_filter_smem_bytes(widest + 2) <= (size_t)optin) widest += 2;
+            lt_set_error("unsupported geometry: img %dx%d (width must be a multiple of 4), warped %dx%d (width must be "
+                         "even and at most %d on this device)", cfg->img_w, cfg->img_h, cfg->bv_w, cfg->bv_h, widest);
+            return -1;
+        }
+    }
     lt_handle* h = new lt_handle();
     memset(h, 0, sizeof(*h));
     h->cfg = *cfg;
@@ -1361,7 +1383,7 @@ extern "C" int lt_filter_lane_points(lt_handle* h, const uint8_t* d_bv_rgb, uint
     LtAttemptParams p = attempt_from(dp);
     p.filter_type = filter_type; p.ksize_r = ksize_r; p.C_r = C_r; p.ksize_b = ksize_b; p.C_b = C_b;
     p.mask_noise = mask_noise; p.ksize_noise = ksize_noise; p.C_noise = C_noise; p.noise_thresh = noise_thresh;
-    if ((rc = check_params(h, p))) return rc;
+    if ((rc = check_filter_params(p))) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     if (d_bv_rgb) {   // NULL: reuse the planes left by the last lt_remap / lt_process
         if ((rc = lt_launch_planes_from_bv(h, d_bv_rgb, n, st))) return rc;

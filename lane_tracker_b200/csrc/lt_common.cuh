@@ -261,6 +261,9 @@ struct LtFilterGroup {
 // first and their lists are consecutive in one device array, so that g[0].list covers all their positions (the
 // morphology runs once over them).  count != NULL (device count of a retry list) only with ng == 1.
 int lt_launch_filter_groups(lt_handle* h, int n, const LtFilterGroup* g, int ng, const int* count, cudaStream_t st);
+// Largest dynamic shared memory a threshold launch takes at warped width bv_w, over every kernel size the parameter
+// checks accept (lt_create refuses widths at which this exceeds the device's opt-in limit).
+size_t lt_filter_smem_bytes(int bv_w);
 int lt_launch_morph_pair(lt_handle* h, bool tophat, int n, const int* list, const int* count, cudaStream_t st);
 int lt_launch_mask_to_u8(lt_handle* h, const uint32_t* bits, uint8_t* d_mask, int n, cudaStream_t st);
 int lt_launch_u8_to_mask(lt_handle* h, const uint8_t* d_mask, uint32_t* bits, int n, cudaStream_t st);

@@ -748,6 +748,29 @@ static int crossh_pitch(const LtDims& d, int k) {                  // in half-wo
 }
 constexpr size_t CROSSH_SMEM_MAX = 200 * 1024;
 
+static int box_pitch(const LtDims& d, int half) {                  // in half-words: 2 * odd, like crossh_pitch
+    int pitch = d.p2 + 2 * ((half + 2) & ~1) + 4;
+    while (((pitch >> 1) & 1) == 0 || (pitch & 1)) ++pitch;
+    return pitch;
+}
+
+// The row kernels are the only threshold kernels whose shared memory grows with the width: the packed one while its
+// tile fits CROSSH_SMEM_MAX (k <= 127), the prefix-sum one (k > 127 or unpacked lanes, at any width) and the box one
+// (block 255).  The column kernels, the morphology and the opening stage fixed-width strips, independent of
+// bv_w.
+size_t lt_filter_smem_bytes(int bv_w) {
+    LtDims d;
+    memset(&d, 0, sizeof(d));
+    d.bv_w = bv_w;
+    d.p2 = 32 * ((bv_w + 63) / 64);
+    const size_t packed = (size_t)CROSSH_ROWS * crossh_pitch(d, 127) * sizeof(unsigned short);
+    const size_t wide = (size_t)ROWK_WARPS * 2 * ((bv_w + 32) & ~31) * sizeof(uint32_t);
+    const size_t box = (size_t)CROSSH_ROWS * box_pitch(d, 255 / 2) * sizeof(unsigned short);
+    size_t m = wide > box ? wide : box;
+    if (packed <= CROSSH_SMEM_MAX && packed > m) m = packed;
+    return m;
+}
+
 // horizontal half of one plane, or of two planes in one launch (plane1 != nullptr; both must take the packed kernel)
 static int launch_cross_h(lt_handle* h, const uint32_t* plane, uint32_t* bits, int k, int C, int accumulate, int n,
                           const int* list, const int* count, cudaStream_t st, const uint32_t* plane1 = nullptr, int k1 = 0,
@@ -843,12 +866,7 @@ static int launch_box_pair(lt_handle* h, int block_r, int c_r, int block_b, int 
     // the top-hat planes, unused by this filter type, hold the row sums
     const LtDims& d = h->d;
     const int half_r = block_r / 2, half_b = block_b / 2;
-    auto box_pitch = [&](int half) {                  // in half-words: 2 * odd, like crossh_pitch
-        int pitch = d.p2 + 2 * ((half + 2) & ~1) + 4;
-        while (((pitch >> 1) & 1) == 0 || (pitch & 1)) ++pitch;
-        return pitch;
-    };
-    const int pitch_r = box_pitch(half_r), pitch_b = box_pitch(half_b);
+    const int pitch_r = box_pitch(d, half_r), pitch_b = box_pitch(d, half_b);
     size_t smem = (size_t)CROSSH_ROWS * (pitch_r > pitch_b ? pitch_r : pitch_b) * sizeof(unsigned short);
     { int rc = lt_ensure_smem((const void*)k_box_h, smem); if (rc) return rc; }
     const int zs = count ? (n < 8 ? n : 8) : n;     // retry-list launches: few slots, each CTA loops over the list
